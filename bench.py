@@ -2,6 +2,7 @@
 """Benchmark of the TT-LSTM / TT-GRU recurrence path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs 1,2,3,4,5] [--headline 3]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): TT-LSTM cell-steps/sec = batch x T / seconds of one forward(+backward) pass over the whole
 stack.  One "step" = one such pass over one batch of synthetic input of the config's shape.
@@ -71,8 +72,13 @@ CONFIGS = {
     7: dict(name="cfg3-dense GE2E speaker encoder 3xLSTM (dense baseline)", cell="lstm", I=40, H=256, L=3, d=0, r=0, B=640, T=160,
             mode="fwd+bwd", grad="hT", inp="uniform", seed=11, dense=True),
 }
-# per-config caps on (warmup, steps): cfg5 moves ~100 GB per step
-STEP_CAP = {5: (3, 3), 4: (3, 5)}
+# per-config (warmup, steps) when --warmup / --steps are not given (3 / 10 otherwise): cfg5 moves ~100 GB per step.
+# Given on the command line, --warmup / --steps apply to every config.
+STEP_DEFAULT = {5: (3, 3), 4: (3, 5)}
+# --dump-outputs: an output array with more elements than this is written as a fixed, seeded sample of this many elements;
+# all the arrays of one run together stay under DUMP_BYTES
+DUMP_ELEMS = 1 << 18
+DUMP_BYTES = 64 << 20
 # CPU sample (batch, T) per config for the in-line cpu_baseline: about 5-15 s of CPU work each
 CPU_SAMPLE = {1: (64, 784), 2: (64, 784), 3: (96, 160), 4: (32, 160), 5: (8, 200), 6: (96, 160), 7: (96, 160), 8: (96, 160), 9: (96, 160)}
 KINDS = ["k_ttlinear_fwd", "k_rnn_fwd", "k_rnn_bwd", "k_ttlinear_bwd", "gemm_ih_fwd", "gemm_dx", "gemm_dw"]
@@ -303,6 +309,7 @@ class GpuBench(object):
         self.lib = _lib.load()
         self.flush_buf = torch.empty(256 << 20, dtype=torch.uint8, device=self.dev)
         self.windows = []                              # host-time windows of the timed regions (clock sampling)
+        self.dumped_bytes = 0
         self.peak = self.measure_ffma_peak()
 
     def barrier(self):
@@ -324,8 +331,28 @@ class GpuBench(object):
             peak = max(peak, flops.value / (e0.elapsed_time(e1) * 1e-3) / 1e12)
         return peak
 
-    def run(self, cid, cfg, B_rank, steps, warmup, scaling, with_e2e=True):
-        """One config at per-rank batch B_rank.  Returns the record (rank 0) or None."""
+    def dump(self, out_dir, prefix, arrays):
+        """Write each tensor as out_dir/<prefix><name>.npy (float32; float64 stays float64).  A tensor of more than
+        DUMP_ELEMS elements is written as the flat elements at DUMP_ELEMS indices drawn from a generator seeded with 0,
+        in ascending order: the same positions in every run, so two builds compare element for element."""
+        os.makedirs(out_dir, exist_ok=True)
+        for name, t in sorted(arrays.items()):
+            t = t.detach()
+            if t.numel() > DUMP_ELEMS:
+                idx = torch.randint(t.numel(), (DUMP_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+                a = t[torch.unravel_index(idx.to(t.device), t.shape)].cpu().numpy()
+            else:
+                a = t.cpu().numpy()
+            if a.dtype != np.float64:
+                a = a.astype(np.float32)
+            self.dumped_bytes += a.nbytes
+            if self.dumped_bytes > DUMP_BYTES:
+                raise SystemExit("--dump-outputs: more than %d bytes of outputs" % DUMP_BYTES)
+            np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+    def run(self, cid, cfg, B_rank, steps, warmup, scaling, with_e2e=True, dump_dir=None):
+        """One config at per-rank batch B_rank.  Returns the record (rank 0) or None.  With `dump_dir`, rank 0 writes
+        what the last timed step computed there (see dump())."""
         from tensorized_rnn_b200.dist import allreduce_gradients
         lib, dev, dist = self.lib, self.dev, self.dist
         torch.manual_seed(cfg["seed"])
@@ -342,7 +369,8 @@ class GpuBench(object):
             cls = self.tr.TTLSTM if cfg["cell"] == "lstm" else self.tr.TTGRU
             with redirect_stdout(io.StringIO()):
                 model = cls(cfg["I"], cfg["H"], cfg["L"], torch.device("cpu"), n_cores=cfg["d"], tt_rank=cfg["r"]).to(dev)
-        params = [p for p in (enc if ge2e else model).parameters()]
+        named = list((enc if ge2e else model).named_parameters())
+        params = [p for _, p in named]
         B, T, H = B_rank, cfg["T"], cfg["H"]
         if ge2e and B % ge2e[1] != 0:
             raise SystemExit("the GE2E step needs a per-rank batch that is a multiple of the utterances per speaker")
@@ -353,10 +381,22 @@ class GpuBench(object):
         train = cfg["mode"] != "fwd"
         dense_dout = torch.rand(B, T, H, device=dev) if cfg["grad"] == "dense" else None
 
-        def one_pass(x):
+        def results(res):
+            """What the recurrent stack returns to its caller: outputs and final state(s)."""
+            if cfg["cell"] == "lstm":
+                return {"out": res[0], "h_T": res[1][0], "c_T": res[1][1]}
+            return {"out": res[0], "h_T": res[1]}
+
+        def grads():
+            return {"grad." + n: p.grad for n, p in named if p.grad is not None}
+
+        def one_pass(x, keep=None):
+            """One step; with a dict `keep`, also hands it what the step computed."""
             if not train:
                 with torch.no_grad():
                     res = model(x)
+                if keep is not None:
+                    keep.update(results(res))
                 return res[1][0] if cfg["cell"] == "lstm" else res[1]
             for p in params:
                 p.grad = None
@@ -366,8 +406,12 @@ class GpuBench(object):
                 loss.backward()
                 if dist is not None:
                     allreduce_gradients(params)
+                if keep is not None:
+                    keep.update(embeds=embeds, loss=loss, **grads())
                 return loss
             res = model(x)
+            if keep is not None:
+                keep.update(results(res))
             out = res[0]
             hT = res[1][0] if cfg["cell"] == "lstm" else res[1]
             if dense_dout is not None:
@@ -379,6 +423,8 @@ class GpuBench(object):
                 result = loss
             if dist is not None:
                 allreduce_gradients(params)             # one flat NCCL all-reduce of every TT-core / bias gradient
+            if keep is not None:
+                keep.update(grads())
             return result
 
         for _ in range(warmup):
@@ -388,22 +434,26 @@ class GpuBench(object):
         lib.ttrnn_launch_count(1)
         lib.ttrnn_tc_launch_count(1)
 
-        def timed(n):
+        def timed(n, keep=None):
             ev = []
             self.barrier()
             w0 = time.perf_counter()
-            for _ in range(n):
+            for i in range(n):
                 self.flush_buf.fill_(1)
                 e0, e1 = torch.cuda.Event(True), torch.cuda.Event(True)
                 e0.record()
-                one_pass(x_dev)
+                one_pass(x_dev, keep if i == n - 1 else None)
                 e1.record()
                 ev.append((e0, e1))
             self.barrier()
             self.windows.append((w0, time.perf_counter()))
             return sum(a.elapsed_time(b) for a, b in ev)
 
-        total_ms = timed(steps)
+        last = {}
+        total_ms = timed(steps, last)
+        if dump_dir and self.rank == 0:
+            self.dump(dump_dir, "cfg%d_" % cid, last)
+        last.clear()
         launches = int(lib.ttrnn_launch_count(0))
         tc_launches = int(lib.ttrnn_tc_launch_count(0))
         # ---- per-kernel times: a second pass with the library's event pairs around every launch.  While that timing is
@@ -585,8 +635,8 @@ class GpuBench(object):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps of every config (default: 10; 5 for cfg4, 3 for cfg5)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed warm-up steps of every config (default: 3)")
     ap.add_argument("--headline", type=int, default=3, choices=sorted(CONFIGS))
     ap.add_argument("--config", type=int, default=0, help="shorthand: headline = this config and run only it")
     ap.add_argument("--configs", default="1,2,3,4,5,6,7,8,9", help="configs measured into all_configs")
@@ -595,7 +645,19 @@ def main():
     ap.add_argument("--seq-len", type=int, default=0, help="override T of the headline config (profiling only)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the weak-scaling measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of every config computed (outputs, final states, parameter "
+                         "gradients) as DIR/cfg<id>_<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup is not None and args.warmup < 0:
+        ap.error("--warmup must not be negative")
+
+    def steps_for(cid):
+        dw, ds = STEP_DEFAULT.get(cid, (3, 10))
+        return (dw if args.warmup is None else args.warmup), (ds if args.steps is None else args.steps)
+
     if args.config:
         args.headline, args.configs = args.config, str(args.config)
     ids = [int(v) for v in args.configs.split(",") if v.strip()]
@@ -620,18 +682,19 @@ def main():
         # batch of the bounded sample: a pilot pass at batch 32 sizes it so that (warmup + steps) passes take ~150 s;
         # T stays at the config value (the reference's cost is per-step dispatch and its O(T^2) backward)
         T = head["T"]
+        warmup, steps = steps_for(args.headline)
         _, pilot = run_cpu_oracle(head, 32, T, 1, 0)
-        budget = 150.0 / (args.steps + args.warmup)
+        budget = 150.0 / (steps + warmup)
         Bs = int(max(16, min(head["B"], 32 * budget / pilot)))
         Bs = max(16, (Bs // 16) * 16) if Bs < head["B"] else head["B"]
-        val, sec = run_cpu_oracle(head, Bs, T, args.steps, args.warmup)
+        val, sec = run_cpu_oracle(head, Bs, T, steps, warmup)
         sample = "batch %d of the config's %d sequences x T %d per step (pilot pass at batch 32 took %.1f s); oracle port of " \
                  "the reference PyTorch path, %d threads" % (Bs, head["B"], T, pilot, torch.get_num_threads())
         cj = config_json(head, Bs, 1, "none")
         cj["parallelism"] = "host CPU, %d threads" % torch.get_num_threads()
         cj["sample_of_global_batch"] = head["B"]
         line = {"impl": "reference", "metric": metric, "value": val, "unit": "cell-steps/s", "n_gpus": args.gpus,
-                "steps": args.steps, "warmup": args.warmup, "ms_per_step": sec * 1e3, "higher_is_better": True,
+                "steps": steps, "warmup": warmup, "ms_per_step": sec * 1e3, "higher_is_better": True,
                 "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": cj,
                 "sample": sample,
                 "cpu_baseline": {"value": val, "unit": "cell-steps/s", "cores": torch.get_num_threads(), "kind": "port",
@@ -657,10 +720,6 @@ def main():
     def split(B):
         return (B + world - 1) // world
 
-    def steps_for(cid):
-        cw, cs = STEP_CAP.get(cid, (args.warmup, args.steps))
-        return min(args.warmup, cw), min(args.steps, cs)
-
     records = []
     head_rec = None
     order = [args.headline] + [i for i in ids if i != args.headline]
@@ -671,7 +730,7 @@ def main():
     for cid in order:
         cfg = cfgs[cid]
         w, s = steps_for(cid)
-        rec = gb.run(cid, cfg, split(cfg["B"]), s, w, "strong")
+        rec = gb.run(cid, cfg, split(cfg["B"]), s, w, "strong", dump_dir=args.dump_outputs)
         weak = None
         if world > 1 and not args.no_weak:
             weak = gb.run(cid, cfg, cfg["B"], min(s, 5), min(w, 3), "weak", with_e2e=False)

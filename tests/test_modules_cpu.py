@@ -161,40 +161,85 @@ def test_every_registered_static_kernel_fits_shared_memory():
     assert {r[0] for r in rows} == {"rnn_fwd", "rnn_bwd", "ttl_fwd", "ttl_bwd"}
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tensorized_rnn"), reason="needs the reference checkout (build container only)")
-def test_patch_reference_switches_the_callers_over():
-    """compat.patch_reference(): the reference's MNIST_Classifier then builds the B200 modules, with the
-    reference's own state_dict layout (keys and shapes identical to an unpatched build)."""
-    import io
+# A stand-in for the reference's import layout: the module names compat.patch_reference() rewrites, and a caller that,
+# like the reference's experiments/digit_classification/mnist_classifier.py, imports the classes by name at import time
+# and picks them at construction time.  The stand-in classes only need to be distinct from the B200 ones.
+_STANDIN_REFERENCE = {
+    "tensorized_rnn/__init__.py": "",
+    "tensorized_rnn/rnn_utils.py": "class ActivGradLogger(object):\n    pass\n",
+    "tensorized_rnn/tt_lstm.py": "import torch\n\nclass TTLSTMCell(torch.nn.Module):\n    pass\n\n"
+                                 "class TTLSTM(torch.nn.Module):\n    def __init__(self, *args, **kwargs):\n"
+                                 "        super().__init__()\n",
+    "tensorized_rnn/gru.py": "import torch\nfrom tensorized_rnn.rnn_utils import ActivGradLogger\n\n"
+                             "class GRUCell(torch.nn.Module):\n    pass\n\nclass GRU(torch.nn.Module):\n    pass\n\n"
+                             "class TTGRUCell(torch.nn.Module):\n    pass\n\n"
+                             "class TTGRU(torch.nn.Module):\n    def __init__(self, *args, **kwargs):\n"
+                             "        super().__init__()\n",
+    "tensorized_rnn/lstm.py": "import torch\nfrom tensorized_rnn.rnn_utils import ActivGradLogger\n\n"
+                              "class LSTMCell(torch.nn.Module):\n    pass\n\nclass LSTM(torch.nn.Module):\n    pass\n",
+    "tensorized_rnn/tt_linearset.py": "import torch\n\nclass TTLinearSet(torch.nn.Module):\n    pass\n",
+    "t3nsor/__init__.py": "from t3nsor.layers import TTLinear\n",
+    "t3nsor/layers.py": "import torch\n\nclass TTLinear(torch.nn.Module):\n    def __init__(self, *args, **kwargs):\n"
+                        "        super().__init__()\n",
+    "mnist_classifier.py": "import torch\nfrom tensorized_rnn.tt_lstm import TTLSTM\nfrom tensorized_rnn.gru import TTGRU\n"
+                           "from t3nsor.layers import TTLinear\n\n"
+                           "class MNIST_Classifier(torch.nn.Module):\n"
+                           "    def __init__(self, in_size, emb_size, hidden, n_layers, device, tt, gru, n_cores, tt_rank):\n"
+                           "        super().__init__()\n"
+                           "        cls = TTGRU if gru else TTLSTM\n"
+                           "        self.rnn = cls(in_size, hidden, n_layers, device, n_cores=n_cores, tt_rank=tt_rank)\n"
+                           "        self.linear = TTLinear(in_features=hidden, out_features=emb_size, bias=True,\n"
+                           "                               auto_shapes=True, d=n_cores, tt_rank=tt_rank)\n",
+}
+
+
+def test_patch_reference_switches_the_callers_over(tmp_path):
+    """compat.patch_reference(): a caller of the reference's modules then builds the B200 modules, with the
+    reference's own state_dict layout and, from the same seed, the reference's own parameters (the stored
+    parameters of the reference TTLSTM of the golden case lstm_d2r2_L2_small); unpatch_reference() restores the
+    reference's classes."""
     import sys
-    from contextlib import redirect_stdout
     import tensorized_rnn_b200.compat as compat
-    sys.path.insert(0, "/root/reference")
-    sys.path.insert(0, "/root/reference/experiments/digit_classification")
+    for rel, text in _STANDIN_REFERENCE.items():
+        path = tmp_path / rel
+        path.parent.mkdir(parents=True, exist_ok=True)
+        path.write_text(text)
+    case = next(c for c in golden_index() if c["name"] == "lstm_d2r2_L2_small")
+    g = load_golden(case["name"])
+    args = (case["input_size"], 10, case["hidden_size"], case["num_layers"], torch.device("cpu"))
+    kw = dict(tt=True, gru=False, n_cores=case["n_cores"], tt_rank=case["tt_rank"])
+    standin = ("tensorized_rnn", "t3nsor", "mnist_classifier")
+    sys.path.insert(0, str(tmp_path))
     try:
         import mnist_classifier as mc
+        import tensorized_rnn.tt_lstm as ref_tt
+        ref_cls = ref_tt.TTLSTM
+        ref = mc.MNIST_Classifier(*args, **kw)
         with redirect_stdout(io.StringIO()):
-            torch.manual_seed(0)
-            ref = mc.MNIST_Classifier(28, 10, 64, 1, torch.device("cpu"), tt=True, gru=False, n_cores=2, tt_rank=2)
             n = compat.patch_reference()
             assert n >= 4
-            torch.manual_seed(0)
-            ours = mc.MNIST_Classifier(28, 10, 64, 1, torch.device("cpu"), tt=True, gru=False, n_cores=2, tt_rank=2)
+            torch.manual_seed(case["seed"])
+            ours = mc.MNIST_Classifier(*args, **kw)
         assert isinstance(ours.rnn, tr.TTLSTM) and not isinstance(ref.rnn, tr.TTLSTM)
-        assert isinstance(ours.linear, tr.TTLinear)
-        sd_ref, sd = ref.state_dict(), ours.state_dict()
-        assert list(sd.keys()) == list(sd_ref.keys())
-        for k in sd:
-            assert tuple(sd[k].shape) == tuple(sd_ref[k].shape), k
-            assert torch.equal(sd[k], sd_ref[k].contiguous()), k      # same RNG stream -> identical parameters
-        ours.load_state_dict(sd_ref)
+        assert isinstance(ours.linear, tr.TTLinear) and not isinstance(ref.linear, tr.TTLinear)
+        sd = ours.state_dict()
+        ref_rnn = {"rnn." + k: v for k, v in state_dict_from_golden(g).items()}
+        # state_dict layout of the reference's TTLinear (d = 2, with bias), from its stored fixture
+        ref_linear = ["linear." + k for k in state_dict_from_golden(load_golden("ttlinear_0"))]
+        assert case["n_cores"] == 2
+        assert list(sd.keys()) == list(ref_rnn.keys()) + ref_linear
+        for k, v in ref_rnn.items():
+            assert tuple(sd[k].shape) == tuple(v.shape), k
+            assert torch.equal(sd[k], v), k                                  # same RNG stream -> identical parameters
+        ours.rnn.load_state_dict(state_dict_from_golden(g))                  # reference checkpoints load
+        compat.unpatch_reference()
+        assert ref_tt.TTLSTM is ref_cls and mc.TTLSTM is ref_cls
     finally:
         compat.unpatch_reference()
-        for p in ("/root/reference/experiments/digit_classification", "/root/reference"):
-            if p in sys.path:
-                sys.path.remove(p)
-    import tensorized_rnn.tt_lstm as ref_tt
-    assert ref_tt.TTLSTM is not tr.TTLSTM
+        sys.path.remove(str(tmp_path))
+        for name in list(sys.modules):
+            if name.split(".")[0] in standin:
+                del sys.modules[name]
 
 
 def test_ih_route_selection_is_host_logic():
