@@ -303,6 +303,10 @@ int ttrnn_static_kernel_table(char *buf, int32_t cap);
  *                   backward scratch buffers.  0 = everything on the caller's stream
  *   "save_bytes"    budget for keeping chain activations of two-core chains for backward instead of
  *                   recomputing them (default 0 = recompute)
+ *   "merge_cores"   d3 r8 LSTM chains: run static kernels with TT cores 0 and 1 contracted into one core while staging
+ *                   (same parameters and gradients, one chain stage fewer).  1 (default) = the dX-only BPTT kernels only:
+ *                   forward results stay bit-identical to 0, gradients differ by rounding; 2 = the forward kernels as well
+ *                   (faster, but h_t is rounded differently); 0 = the three-core chain.  Stamped into the workspace plan.
  * returns 0 if the key is known. */
 int ttrnn_set_option(const char *key, int64_t value);
 

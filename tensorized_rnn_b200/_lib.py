@@ -118,7 +118,7 @@ def load() -> C.CDLL:
                      ("row_plan", "TTRNN_ROW_PLAN"), ("gemm_wide", "TTRNN_GEMM_WIDE"), ("split_kept", "TTRNN_SPLIT_KEPT"),
                      ("dense_hh_dw", "TTRNN_DENSE_HH_DW"), ("tc_gemm", "TTRNN_TC_GEMM"),
                      ("rank_pad", "TTRNN_RANK_PAD"), ("bwd_overlap", "TTRNN_BWD_OVERLAP"),
-                     ("row_groups", "TTRNN_ROW_GROUPS")):
+                     ("row_groups", "TTRNN_ROW_GROUPS"), ("merge_cores", "TTRNN_MERGE_CORES")):
         if os.environ.get(env):
             lib.ttrnn_set_option(key.encode(), int(os.environ[env]))
     _lib = lib

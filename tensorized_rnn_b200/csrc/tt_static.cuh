@@ -9,6 +9,7 @@
 //   gates aligned with the first output mode (i_0 % G == 0), final-stage tiles <= one per thread.
 #pragma once
 #include <cuda_runtime.h>
+#include <type_traits>
 #include "tt_plan.h"
 
 namespace tts {
@@ -154,6 +155,53 @@ template <class S, int k> struct COff { static constexpr int v = COff<S, k - 1>:
 template <class S> struct COff<S, 0> { static constexpr int v = 0; };
 template <class S> constexpr int core_floats() { return COff<S, S::D - 1>::v + St<S, S::D - 1>::CORE; }
 
+// ---- contracted chain: cores 0 and 1 of a three-core shape merged into one core ------------------
+//   W01[i0*I1 + i1][j0*J1 + j1][a2] = sum_a1 G0[i0][j0][a1] G1[a1][i1][j1][a2]
+// Adjacent modes merge in row-major order, so h_t keeps its [J0*J1][J2] layout in the first stage and the gate
+// stays the high part of the first output mode: the two-core chain over (W01, G2) computes the same W_hh h with
+// one stage, one block barrier and one shared-memory round trip fewer per step (d3 r8: 589 824 instead of
+// 655 360 FLOPs per row-step).  The kernels read the original three-core blob and contract while staging;
+// parameter and gradient blobs keep the three-core layout.
+template <class S3>
+struct Merge01 {
+    static_assert(S3::D == 3 && S3::RK[0] == 1 && S3::RK[3] == 1, "Merge01 contracts cores 0 and 1 of a three-core chain");
+    using Src = S3;
+    static constexpr int D = 2, G = S3::G;
+    static constexpr int J[7] = {S3::J[0] * S3::J[1], S3::J[2]};
+    static constexpr int I[7] = {S3::I[0] * S3::I[1], S3::I[2]};
+    static constexpr int RK[7] = {1, S3::RK[2], 1};
+};
+// shape whose blob the kernels of S read (S itself, or the three-core source of a Merge01)
+template <class S, class = void> struct SrcOf { using type = S; static constexpr bool merged = false; };
+template <class S> struct SrcOf<S, std::void_t<typename S::Src>> { using type = typename S::Src; static constexpr bool merged = true; };
+template <class S> constexpr int blob_floats() { return core_floats<typename SrcOf<S>::type>(); }
+
+// element e (blob order r,i,j,r') of core k of S; a contracted core is summed over a1 in a fixed order, so every CTA
+// and both directions stage bit-identical weights
+template <class S, int k>
+TTS_DEV float core_elem(const float *__restrict__ cores, int e) {
+    if constexpr (SrcOf<S>::merged) {
+        using S3 = typename SrcOf<S>::type;
+        if constexpr (k == 0) {
+            using T = St<S, 0>;
+            constexpr int J1 = S3::J[1], I1 = S3::I[1], R1 = S3::RK[1], R2 = S3::RK[2];
+            const int ap = e % T::rn;
+            const int t = e / T::rn;
+            const int j = t % T::J, i = t / T::J;              // r_0 = 1
+            const float *g0 = cores + COff<S3, 0>::v + ((i / I1) * S3::J[0] + j / J1) * R1;
+            const float *g1 = cores + COff<S3, 1>::v + ((i % I1) * J1 + j % J1) * R2 + ap;
+            float s = 0.f;
+#pragma unroll
+            for (int a1 = 0; a1 < R1; ++a1) s = fmaf(__ldg(g0 + a1), __ldg(g1 + a1 * (I1 * J1 * R2)), s);
+            return s;
+        } else {
+            return __ldg(cores + COff<S3, k + 1>::v + e);
+        }
+    } else {
+        return __ldg(cores + COff<S, k>::v + e);
+    }
+}
+
 // ---- stage the cores: blob (r,i,j,r') -> shared W layouts --------------------------------------
 template <class S, int k>
 TTS_DEV void stage_weights_k(const float *__restrict__ cores, float *__restrict__ wsm, int tid) {
@@ -175,7 +223,7 @@ TTS_DEV void stage_weights_k(const float *__restrict__ cores, float *__restrict_
         int col;
         if (k == 0 && T::PACK) col = gate_col<S>(i % I0p, i / I0p);   // gate index = i / I0p (gates are the high part of i_0)
         else col = i * T::r + a;
-        wsm[WOff<S, k>::v + (j * T::rn + ap) * T::NS + col] = __ldg(cores + COff<S, k>::v + e);
+        wsm[WOff<S, k>::v + (j * T::rn + ap) * T::NS + col] = core_elem<S, k>(cores, e);
     }
     if constexpr (k + 1 < S::D) stage_weights_k<S, k + 1>(cores, wsm, tid);
 }
@@ -697,7 +745,7 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_fwd_s(const __grid_constant_
             if (t + 1 < a.steps) fetch_in(t + 1);
             // ---- stages d-1 .. 1
             const float *X0 = fwd_chain_pp<S, R, TU, S::D - 1>(hs, P, Q, wsm, tid);
-            if (a.x0_save) {
+            if (!SrcOf<S>::merged && a.x0_save) {
                 // X_0 tile -> HBM (coalesced float4), overlapped with the final stage which only reads it
                 using T0s = St<S, 0>;
                 constexpr int X0F = T0s::Mrow * T0s::K;
@@ -804,7 +852,7 @@ TTS_DEV void stage_weights_t(const float *__restrict__ cores, float *__restrict_
         const int i = t % T::I;
         const int a = t / T::I;
         const int row = (k == 0 && T::PACK) ? gate_col<S>(i % I0p, i / I0p) : i * T::r + a;
-        wt[WTOff<S, k>::v + row * TT_::KST + j * T::rn + ap] = __ldg(cores + COff<S, k>::v + e);
+        wt[WTOff<S, k>::v + row * TT_::KST + j * T::rn + ap] = core_elem<S, k>(cores, e);
     }
     if constexpr (k + 1 < S::D) stage_weights_t<S, k + 1>(cores, wt, tid);
 }
@@ -1246,6 +1294,7 @@ template <class S, int CELL, int R, int MODE, class TB, bool DWI = true, int SV 
 __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant__ RnnBwdSArgs a) {
     constexpr bool SAVED = (SV == 1), SAVEU = (SV != 0);
     static_assert(!SAVED || (S::D == 2 && DWI), "saved-activation backward is implemented for two-core chains");
+    static_assert(!SrcOf<S>::merged || (!DWI && SV == 2), "contracted chains run the dX-only kernel with kept gates");
     // DWI = false with kept gates: nothing of the forward chain is needed (gates come from the forward pass, the
     // core gradients from the dense accumulation outside): the kernel runs the gate gradients and the dX chain only
     constexpr bool RECOMPUTE = !SAVED && (DWI || !SAVEU);
@@ -1584,16 +1633,16 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
     }
     // ---- flush gradients of this CTA into its slot
     if (!a.partial) return;
-    float *slot = a.partial + (long long)blockIdx.x * (core_floats<S>() + 3 * GH);
+    float *slot = a.partial + (long long)blockIdx.x * (blob_floats<S>() + 3 * GH);
     if constexpr (DWI) flush_all<S, R, TB, 0>(dw, xs, slot, tid);
 #pragma unroll
     for (int n = 0; n < NE; ++n)
 #pragma unroll
         for (int g = 0; g < G; ++g) {
             const int col = g * H + hid[n];
-            slot[core_floats<S>() + col] += g_bhh[n][g];
-            slot[core_floats<S>() + GH + col] += g_weff[n][g];
-            slot[core_floats<S>() + 2 * GH + col] += g_bih[n][g];
+            slot[blob_floats<S>() + col] += g_bhh[n][g];
+            slot[blob_floats<S>() + GH + col] += g_weff[n][g];
+            slot[blob_floats<S>() + 2 * GH + col] += g_bih[n][g];
         }
 }
 

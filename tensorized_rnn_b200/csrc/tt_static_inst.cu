@@ -58,14 +58,24 @@ template <class S> constexpr long long x0_floats() {
 }
 #define TTS_FWD(S, CELL, R, MODE, ...)                                                                     \
     {#S, CELL, MODE, R, x0_floats<S>(), tts::FwdSmem<S, R, __VA_ARGS__>::BYTES, &match_shape<S>,            \
-     &launch_fwd<S, CELL, R, MODE, __VA_ARGS__>, &prepare_fwd<S, CELL, R, MODE, __VA_ARGS__>}
+     &launch_fwd<S, CELL, R, MODE, __VA_ARGS__>, &prepare_fwd<S, CELL, R, MODE, __VA_ARGS__>, 0}
+// contracted chain (tts::Merge01) of the three-core shape S3: registered under S3, reads S3's blob, keeps no X_0
+#define TTS_FWD_M01(S3, CELL, R, MODE, ...)                                                                \
+    {#S3 "(m01)", CELL, MODE, R, 0, tts::FwdSmem<tts::Merge01<S3>, R, __VA_ARGS__>::BYTES, &match_shape<S3>, \
+     &launch_fwd<tts::Merge01<S3>, CELL, R, MODE, __VA_ARGS__>, &prepare_fwd<tts::Merge01<S3>, CELL, R, MODE, __VA_ARGS__>, 1}
 
 // Tune<FTMr, FTI, FSK, TM1, TN1, TM2, TN2, TM3, TN3>: final-stage tile (rows, first-mode slices, k-split)
 // and (rows, columns) of the thread tile of stages 1..3
 using tts::Tune;
 #define TTS_FWD2(S, CELL, R, MODE, ...)                                                                    \
     {#S "(2 CTAs/SM)", CELL, MODE, R, x0_floats<S>(), tts::FwdSmem<S, R, __VA_ARGS__>::BYTES, &match_shape<S>, \
-     &launch_fwd<S, CELL, R, MODE, __VA_ARGS__, 2>, &prepare_fwd<S, CELL, R, MODE, __VA_ARGS__, 2>}
+     &launch_fwd<S, CELL, R, MODE, __VA_ARGS__, 2>, &prepare_fwd<S, CELL, R, MODE, __VA_ARGS__, 2>, 0}
+// d3 r8 chain with cores 0 and 1 contracted (J = [32, 8], I = [64, 16], RK = [1, 8, 1]): the final stage contracts
+// K = 256; two first-mode slices per thread with k split in halves (FTI = FSK = 2): per k-step R + 8 LDS.128 feed 16 R
+// FFMA2.  Four slices / four k-splits measured within 0.1 % of it on cfg3 (B200) and need three times the exchange
+// space of the reduce-scatter, so the smaller tile stays.
+using TU_m01_R2 = Tune<1, 2, 2, 2, 8>;
+using TU_m01_R5 = Tune<1, 2, 2, 1, 8>;
 const TtsRnnFwdEntry kFwd[] = {
     TTS_FWD(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_RANK1, Tune<1, 2, 2, 1, 8>),
     TTS_FWD(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, Tune<1, 2, 2, 1, 8>),
@@ -87,6 +97,11 @@ const TtsRnnFwdEntry kFwd[] = {
     TTS_FWD(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 3, tts::MODE_XG, Tune<1, 1, 1, 1, 8, 1, 8>),
     TTS_FWD(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 4, tts::MODE_XG, Tune<1, 1, 1, 1, 8, 1, 8>),
     TTS_FWD(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 5, tts::MODE_XG, Tune<1, 1, 1, 1, 8, 1, 8>),
+    TTS_FWD_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, TU_m01_R2),
+    TTS_FWD_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_XG, TU_m01_R2),
+    TTS_FWD_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 3, tts::MODE_XG, TU_m01_R5),
+    TTS_FWD_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 4, tts::MODE_XG, TU_m01_R5),
+    TTS_FWD_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 5, tts::MODE_XG, TU_m01_R5),
     TTS_FWD(HH_H768_d2r4_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_XG, Tune<1, 3, 1, 1, 8>),
     TTS_FWD(HH_H768_d2r4_lstm, TTRNN_CELL_LSTM, 4, tts::MODE_XG, Tune<1, 3, 1, 1, 8>),
     TTS_FWD(HH_H256_d4r16_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, Tune<4, 1, 4, 8, 8, 8, 8, 4, 8>),
@@ -107,29 +122,36 @@ int prepare_bwd(int *occ) {
     return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, k, tts::NTHR, tts::BwdSmem<S, R, TB, DWI, SV>::BYTES);
 }
 template <class S>
-constexpr long long slot_floats() { return tts::core_floats<S>() + 3LL * S::G * tts::n_in<S>(); }
+constexpr long long slot_floats() { return tts::blob_floats<S>() + 3LL * S::G * tts::n_in<S>(); }
 
 #define TTS_BWD(S, CELL, R, MODE, ...)                                                                      \
     {#S, CELL, MODE, R, 0, 0, tts::BwdSmem<S, R, __VA_ARGS__, true>::BYTES, slot_floats<S>(), &match_shape<S>, \
-     &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, true>, &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true>}
+     &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, true>, &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true>, 0}
 #define TTS_BWD_SAVED(S, CELL, R, MODE, ...)                                                                \
     {#S "(saved)", CELL, MODE, R, 0, 1, tts::BwdSmem<S, R, __VA_ARGS__, true, 1>::BYTES, slot_floats<S>(),   \
      &match_shape<S>, &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 1>,                                   \
-     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 1>}
+     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 1>, 0}
 #define TTS_BWD_SAVEU(S, CELL, R, MODE, ...)                                                                \
     {#S "(kept u)", CELL, MODE, R, 0, 2, tts::BwdSmem<S, R, __VA_ARGS__, true, 2>::BYTES, slot_floats<S>(),  \
      &match_shape<S>, &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 2>,                                   \
-     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 2>}
+     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 2>, 0}
 #define TTS_BWD_SPLIT(S, CELL, R, MODE, ...)                                                                \
     {#S "(split)", CELL, MODE, R, 1, 0, tts::BwdSmem<S, R, __VA_ARGS__, false>::BYTES, slot_floats<S>(),     \
      &match_shape<S>, &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, false>,                                     \
-     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, false>}
+     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, false>, 0}
 
 // kept gates + split: gate gradients and the dX chain only (no recompute, no in-kernel core gradients)
 #define TTS_BWD_SPLIT_SAVEU(S, CELL, R, MODE, ...)                                                          \
     {#S "(split, kept u)", CELL, MODE, R, 1, 2, tts::BwdSmem<S, R, __VA_ARGS__, false, 2>::BYTES, slot_floats<S>(), \
      &match_shape<S>, &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, false, 2>,                                  \
-     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, false, 2>}
+     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, false, 2>, 0}
+
+// contracted d3 r8 chain (tts::Merge01), dX-only with kept gates: registered under S3; the gradient slot keeps the
+// layout of S3's blob (only the bias gradients are written: the hh core gradients come from the dense accumulation)
+#define TTS_BWD_SPLIT_SAVEU_M01(S3, CELL, R, MODE, ...)                                                     \
+    {#S3 "(m01, split, kept u)", CELL, MODE, R, 1, 2, tts::BwdSmem<tts::Merge01<S3>, R, __VA_ARGS__, false, 2>::BYTES, \
+     slot_floats<S3>(), &match_shape<S3>, &launch_bwd<tts::Merge01<S3>, CELL, R, MODE, __VA_ARGS__, false, 2>,    \
+     &prepare_bwd<tts::Merge01<S3>, CELL, R, MODE, __VA_ARGS__, false, 2>, 1}
 
 // the same with the register budget of two co-resident CTAs per SM (one-row variants: 80 KB of shared memory each).
 // Measured dead end (round 2, cfg3 shape, 196 / 296 rows): two co-resident one-row CTAs take 2.61 ms per layer-pass
@@ -137,7 +159,7 @@ constexpr long long slot_floats() { return tts::core_floats<S>() + 3LL * S::G * 
 #define TTS_BWD_SPLIT_SAVEU2(S, CELL, R, MODE, ...)                                                         \
     {#S "(split, kept u, 2 CTAs/SM)", CELL, MODE, R, 1, 2, tts::BwdSmem<S, R, __VA_ARGS__, false, 2>::BYTES, slot_floats<S>(), \
      &match_shape<S>, &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, false, 2, 2>,                               \
-     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, false, 2, 2>}
+     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, false, 2, 2>, 0}
 
 // TuneB<forward Tune, BTM0..3 (rows per thread of bwd-data stage k), BSP (split of the last bwd-data
 // stage), WTK0..3 (kappa rows of the register tile of bwd-weight stage k)>
@@ -155,6 +177,9 @@ using TB_d3_split_R3 = TuneB<Tune<1, 1, 1, 1, 8, 1, 8>, 2, 2, 1, 1, 8, 4, 8, 4, 
 // H = 768 d2 r4: dX-only kernel with kept gates (the fused variant's core-gradient tiles do not divide 256 threads)
 using TB_h768_split = TuneB<Tune<1, 3, 1, 1, 8>, 1, 1, 1, 1, 2, 8, 8, 8, 8>;
 using TB_d4r16_split = TuneB<Tune<4, 1, 4, 8, 8, 8, 8, 4, 8>, 8, 8, 4, 1, 4, 4, 4, 4, 4>;
+// contracted d3 r8 chain, dX only: bwd-data stage 0 (K = 256, 64 gate rows) two rows per thread, stage 1 as stage 2 of
+// the three-core chain (split 8 ways); the forward tile only sets the ownership of hidden units (one per thread)
+using TB_m01_split = TuneB<Tune<1, 1, 1, 1, 8>, 2, 1, 1, 1, 8, 4, 8, 4, 4>;
 const TtsRnnBwdEntry kBwd[] = {
     TTS_BWD(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_RANK1, TB_d2),
     TTS_BWD(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 4, tts::MODE_RANK1, TB_d2),
@@ -204,6 +229,11 @@ const TtsRnnBwdEntry kBwd[] = {
     TTS_BWD_SPLIT_SAVEU(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, TB_d3_split_R2),
     TTS_BWD_SPLIT_SAVEU(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_XG, TB_d3_split_R2),
     TTS_BWD_SPLIT_SAVEU(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 3, tts::MODE_XG, TB_d3_split_R3),
+    // four rows fit once the contracted chain drops the second X_k slot (209 KB; 246 KB for the three-core chain)
+    TTS_BWD_SPLIT_SAVEU_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, TB_m01_split),
+    TTS_BWD_SPLIT_SAVEU_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_XG, TB_m01_split),
+    TTS_BWD_SPLIT_SAVEU_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 3, tts::MODE_XG, TB_m01_split),
+    TTS_BWD_SPLIT_SAVEU_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 4, tts::MODE_XG, TB_m01_split),
 };
 
 
@@ -294,6 +324,16 @@ const TtsTtlBwdEntry *tts_find_ttl_bwd(const ttrnn_tt_shape *s, long long rows, 
 // kept gates (saved == 2): a "split" variant (gate gradients + dX chain only; core gradients by the dense
 // accumulation outside) does a third of the work per row of the fused variant and is preferred when the caller
 // can run the dense accumulation (split_kept_ok)
+// merge != 0: the contracted-chain variants (merged = 1) replace the three-core ones wherever one of them passes `ok`;
+// otherwise only the three-core variants compete.  Returns the `merged` value the candidates must have.
+template <class E, size_t N, class F>
+static int merged_wanted(const E (&tab)[N], int merge, F ok) {
+    if (merge)
+        for (const auto &e : tab)
+            if (e.merged && ok(e)) return 1;
+    return 0;
+}
+
 static bool use_split_kept(const ttrnn_tt_shape *hh, int cell, int mode, int saved, int split_kept_ok) {
     if (saved != 2 || !split_kept_ok) return false;
     for (const auto &e : kBwd)
@@ -302,18 +342,20 @@ static bool use_split_kept(const ttrnn_tt_shape *hh, int cell, int mode, int sav
 }
 
 const TtsRnnBwdEntry *tts_find_rnn_bwd(const ttrnn_tt_shape *hh, int cell, int mode, long long B, int sms, int prefer_R,
-                                       int saved, int split_kept_ok) {
+                                       int saved, int split_kept_ok, int merge) {
     const TtsRnnBwdEntry *best = nullptr;
     const bool only_split = use_split_kept(hh, cell, mode, saved, split_kept_ok);
+    auto ok = [&](const TtsRnnBwdEntry &e) {
+        return e.cell == cell && e.mode == mode && e.saved == saved && e.match(hh) && e.smem <= kMaxSmem &&
+               (saved != 2 || (e.split != 0) == only_split);
+    };
+    const int mw = merged_wanted(kBwd, merge, ok);
     if (prefer_R > 0)
         for (const auto &e : kBwd)
-            if (e.cell == cell && e.mode == mode && e.saved == saved && e.match(hh) && e.smem <= kMaxSmem &&
-                e.R == prefer_R && (saved != 2 || (e.split != 0) == only_split))
-                return &e;
+            if (ok(e) && e.merged == mw && e.R == prefer_R) return &e;
     long long best_cost = 0;
     for (const auto &e : kBwd) {
-        if (e.cell != cell || e.mode != mode || e.saved != saved || !e.match(hh) || e.smem > kMaxSmem) continue;
-        if (saved == 2 && (e.split != 0) != only_split) continue;
+        if (!ok(e) || e.merged != mw) continue;
         const long long tiles = (B + e.R - 1) / e.R;
         const long long waves = (tiles + sms - 1) / sms;
         const long long cost = waves * (2 * e.R + 3);
@@ -326,19 +368,21 @@ const TtsRnnBwdEntry *tts_find_rnn_bwd(const ttrnn_tt_shape *hh, int cell, int m
 }
 
 int tts_plan_rnn_bwd(const ttrnn_tt_shape *hh, int cell, int mode, long long B, int sms, int prefer_R, int saved,
-                     int split_kept_ok, const TtsRnnBwdEntry *entry[2], long long row0[2], long long rows[2]) {
+                     int split_kept_ok, int merge, const TtsRnnBwdEntry *entry[2], long long row0[2], long long rows[2]) {
     entry[0] = entry[1] = nullptr;
     row0[0] = row0[1] = rows[0] = rows[1] = 0;
     if (prefer_R > 0) {
-        entry[0] = tts_find_rnn_bwd(hh, cell, mode, B, sms, prefer_R, saved, split_kept_ok);
+        entry[0] = tts_find_rnn_bwd(hh, cell, mode, B, sms, prefer_R, saved, split_kept_ok, merge);
         rows[0] = B;
         return entry[0] ? 1 : 0;
     }
     const bool only_split = use_split_kept(hh, cell, mode, saved, split_kept_ok);
-    auto ok = [&](const TtsRnnBwdEntry &e) {
+    auto ok0 = [&](const TtsRnnBwdEntry &e) {
         return e.cell == cell && e.mode == mode && e.saved == saved && e.match(hh) && e.smem <= kMaxSmem &&
                (saved != 2 || (e.split != 0) == only_split);
     };
+    const int mw = merged_wanted(kBwd, merge, ok0);
+    auto ok = [&](const TtsRnnBwdEntry &e) { return ok0(e) && e.merged == mw; };
     // cost of a wave of R rows per CTA ~ (1 + R): one unit of per-step overhead (barriers, gate phase) per row of work
     auto wave_cost = [&](const TtsRnnBwdEntry &e, long long nrows) {
         const long long tiles = (nrows + e.R - 1) / e.R;
@@ -371,14 +415,17 @@ int tts_plan_rnn_bwd(const ttrnn_tt_shape *hh, int cell, int mode, long long B, 
     return n;
 }
 
-const TtsRnnFwdEntry *tts_find_rnn_fwd(const ttrnn_tt_shape *hh, int cell, int mode, long long B, int sms, int prefer_R) {
+const TtsRnnFwdEntry *tts_find_rnn_fwd(const ttrnn_tt_shape *hh, int cell, int mode, long long B, int sms, int prefer_R,
+                                       int merge) {
     const TtsRnnFwdEntry *best = nullptr;
+    auto ok = [&](const TtsRnnFwdEntry &e) { return e.cell == cell && e.mode == mode && e.match(hh) && e.smem <= kMaxSmem; };
+    const int mw = merged_wanted(kFwd, merge, ok);
     if (prefer_R > 0)
         for (const auto &e : kFwd)
-            if (e.cell == cell && e.mode == mode && e.match(hh) && e.smem <= kMaxSmem && e.R == prefer_R) return &e;
+            if (ok(e) && e.merged == mw && e.R == prefer_R) return &e;
     long long best_cost = 0;
     for (const auto &e : kFwd) {
-        if (e.cell != cell || e.mode != mode || !e.match(hh) || e.smem > kMaxSmem) continue;
+        if (!ok(e) || e.merged != mw) continue;
         const long long tiles = (B + e.R - 1) / e.R;
         const long long waves = (tiles + sms - 1) / sms;
         // time of a wave of R rows per CTA ~ (1.5 + R): a latency floor per step (barriers, shared-memory round trips) plus

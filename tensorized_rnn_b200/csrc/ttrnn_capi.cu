@@ -62,6 +62,13 @@ std::atomic<long long> g_opt_bwd_overlap{1};
 // runs beside the head group of layer l + 1 (forward) / l - 1 (backward).  0 = one group (every launch on the caller's stream),
 // 1 = planned, >= 4 = force group 0 to that many rows whatever the plan says (tests)
 std::atomic<long long> g_opt_row_groups{1};
+// d3 r8 TT-LSTM chains: run static kernels with cores 0 and 1 contracted (tts::Merge01: one stage and 10 % of the
+// multiply-adds fewer per step).  1 (default) = the dX-only BPTT kernels only: the forward keeps the three-core chain, so
+// outputs, states and everything computed from them stay bit-identical to merge_cores = 0 and only the BPTT sums are
+// reordered; 2 = the forward kernels as well (another ~3 % on cfg3, but h_t is rounded differently, which a GE2E loss
+// backward amplifies: cfg9 parameter gradients move by ~1e-5 relative); 0 = the three-core chain everywhere.  The fused BPTT
+// kernels, the runtime-shape kernels and the gradient-logging path always run the three-core chain.
+std::atomic<long long> g_opt_merge_cores{1};
 
 // Snapshot of every option that decides a buffer layout or a kernel route.  ttrnn_rnn_workspace_bytes() takes it from the
 // process-wide options and stamps it into ttrnn_rnn_workspace.plan; forward and backward run from THAT copy, so a
@@ -69,14 +76,16 @@ std::atomic<long long> g_opt_row_groups{1};
 // the scratch buffers are interpreted.  Helpers read the calling thread's current snapshot `t_opt`.
 struct Opts {
     long long rows, chunk, chunk_bytes, stat, srows_fwd, srows_bwd, save_bytes, save_u_bytes, row_plan, dense_ih, gemm_wide,
-        dense_hh, split_kept, dense_ratio, tc_gemm, rank_pad, bwd_overlap, row_groups;
+        dense_hh, split_kept, dense_ratio, tc_gemm, rank_pad, bwd_overlap, row_groups, merge_cores;
 };
 constexpr int kOptFields = sizeof(Opts) / sizeof(long long);
-constexpr long long kPlanMagic = 0x7474726E6E706C34LL;          // "ttrnnpl4"
+constexpr long long kPlanMagic = 0x7474726E6E706C35LL;          // "ttrnnpl5"
 // plan words: [0] magic, [1 .. kOptFields] options, then the row-group split (group count, rows of group 0)
 constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2;
 static_assert(kOptFields + 3 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
 thread_local Opts t_opt;
+inline int merge_fwd() { return t_opt.merge_cores >= 2 ? 1 : 0; }    // contracted forward variants (merge_cores = 2)
+inline int merge_bwd() { return t_opt.merge_cores >= 1 ? 1 : 0; }    // contracted dX-only BPTT variants (merge_cores >= 1)
 
 Opts snapshot_options() {
     Opts o;
@@ -86,6 +95,7 @@ Opts snapshot_options() {
     o.dense_ih = g_opt_dense_ih.load(); o.gemm_wide = g_opt_gemm_wide.load(); o.dense_hh = g_opt_dense_hh.load();
     o.split_kept = g_opt_split_kept.load(); o.dense_ratio = g_opt_dense_ratio.load(); o.tc_gemm = g_opt_tc_gemm.load();
     o.rank_pad = g_opt_rank_pad.load(); o.bwd_overlap = g_opt_bwd_overlap.load(); o.row_groups = g_opt_row_groups.load();
+    o.merge_cores = g_opt_merge_cores.load();
     return o;
 }
 void plan_store(const Opts &o, int64_t *plan) {
@@ -386,7 +396,7 @@ int make_eff_desc(const ttrnn_rnn_desc *d, const DevInfo *dv, EffDesc *e) {
     if (!any) return 0;
     for (int l = 0; l < d->num_layers; ++l) {
         const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        if (!tts_find_rnn_fwd(&p.hh[l], d->cell, mode, d->batch, dv->sms, 0)) return 0;     // padding would not reach a static kernel
+        if (!tts_find_rnn_fwd(&p.hh[l], d->cell, mode, d->batch, dv->sms, 0, merge_fwd())) return 0;     // padding would not reach a static kernel
     }
     RnnPlan pad;
     if (build_rnn_plan(&p, &pad)) return 0;
@@ -510,15 +520,15 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
         int mode1[TTRNN_MAX_LAYERS] = {}, mode2[TTRNN_MAX_LAYERS] = {};
         for (int l = 0; l < L; ++l) {
             const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-            const TtsRnnFwdEntry *se = tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd);
+            const TtsRnnFwdEntry *se = tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd, merge_fwd());
             if (!se) continue;
-            if (se->x0_floats > 0 && tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 1)) {
+            if (se->x0_floats > 0 && tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 1, 0, merge_bwd())) {
                 mode1[l] = 1;
                 lo->x0f[l] = se->x0_floats;
                 extra1 += r4(B * T * se->x0_floats) + r4(B * T * 4 * H);
             }
             const int oks = split_kept_ok(rp.layer[l].hh, mode, tc, T) ? 1 : 0;
-            if (tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 2, oks)) {
+            if (tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 2, oks, merge_bwd())) {
                 mode2[l] = 1;
                 extra2 += r4(B * T * 4 * H);
             }
@@ -583,8 +593,8 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
             const bool okd = dense_hh_dw_ok(rp.layer[l].hh);
             const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
             const int oks = split_kept_ok(rp.layer[l].hh, mode, tc, T) ? 1 : 0;
-            const TtsRnnBwdEntry *be = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 0);
-            const TtsRnnBwdEntry *b2 = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 2, oks);
+            const TtsRnnBwdEntry *be = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd());
+            const TtsRnnBwdEntry *b2 = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 2, oks, merge_bwd());
             if (okd && ((be && be->split) || (b2 && b2->split)) && dense_bwd_floats(rp.layer[l].hh) > dhh)
                 dhh = dense_bwd_floats(rp.layer[l].hh);
         }
@@ -946,16 +956,16 @@ bool group_launches(const ttrnn_rnn_desc *d, const RnnPlan &rp, const RnnLayout 
     };
     for (int l = 0; l < d->num_layers; ++l) {
         const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        const TtsRnnFwdEntry *se = tts_find_rnn_fwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_fwd);
+        const TtsRnnFwdEntry *se = tts_find_rnn_fwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_fwd, merge_fwd());
         if (!se) return false;
         push(fq, Bg, se->R);
     }
     for (int l = d->num_layers - 1; l >= 0; --l) {
         const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        const TtsRnnBwdEntry *be = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_bwd);
+        const TtsRnnBwdEntry *be = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd());
         if (lo.save_mode[l] != 0)
             if (const TtsRnnBwdEntry *bs = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_bwd, lo.save_mode[l],
-                                                            split_kept_ok(rp.layer[l].hh, mode, lo.Tc, d->seq_len)))
+                                                            split_kept_ok(rp.layer[l].hh, mode, lo.Tc, d->seq_len), merge_bwd()))
                 be = bs;
         if (!be) return false;
         const TtsRnnBwdEntry *pe[2] = {be, nullptr};
@@ -963,7 +973,7 @@ bool group_launches(const ttrnn_rnn_desc *d, const RnnPlan &rp, const RnnLayout 
         int np = 1;
         if ((!be->split || be->saved == 2) && t_opt.row_plan) {
             const int q = tts_plan_rnn_bwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_bwd, be->saved,
-                                           be->split && be->saved == 2, pe, pr0, pr);
+                                           be->split && be->saved == 2, merge_bwd(), pe, pr0, pr);
             if (q >= 1) np = q; else { pe[0] = be; pr[0] = Bg; }
         }
         for (int q = 0; q < np; ++q) push(bq, pr[q], pe[q]->R);
@@ -1138,6 +1148,7 @@ int ttrnn_set_option(const char *key, int64_t value) {
     if (!strcmp(key, "rank_pad")) { g_opt_rank_pad.store(value); return 0; }
     if (!strcmp(key, "bwd_overlap")) { g_opt_bwd_overlap.store(value); return 0; }
     if (!strcmp(key, "row_groups")) { g_opt_row_groups.store(value); return 0; }
+    if (!strcmp(key, "merge_cores")) { g_opt_merge_cores.store(value); return 0; }
     if (!strcmp(key, "tc_red_ts")) { ttc::tc_red_variant() = value ? 1 : 0; return 0; }   // A/B switch, not part of a plan
     if (!strcmp(key, "tc_rows_ts")) { ttc::tc_rows_variant() = value ? 1 : 0; return 0; } // A/B switch, not part of a plan
     return 1;
@@ -1242,14 +1253,14 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
         const char *route = rank1 ? "rank_one" : (dense ? "dense" : "tt_chain");
         const bool tc_f = dense && tc_rows_use(B * (long long)lo.Tc, lp.ih.n_in, GH, false);
         const bool tc_r = dense && t_opt.tc_gemm && ttc::tc_red_ok(B * (long long)lo.Tc, lp.ih.n_in, GH);
-        const TtsRnnFwdEntry *se = t_opt.stat ? tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd) : nullptr;
+        const TtsRnnFwdEntry *se = t_opt.stat ? tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd, merge_fwd()) : nullptr;
         put("layer=%d ih_route=%s ih_fwd_tc=%d ih_dw_tc=%d fwd_kernel=%s fwd_rows=%d save_mode=%d", l, route, (int)tc_f, (int)tc_r,
             se ? tok(se->name).c_str() : "runtime", se ? se->R : 0, lo.save_mode[l]);
         if (training) {
-            const TtsRnnBwdEntry *be = t_opt.stat ? tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd) : nullptr;
+            const TtsRnnBwdEntry *be = t_opt.stat ? tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd()) : nullptr;
             if (t_opt.stat && lo.save_mode[l] != 0)
                 if (const TtsRnnBwdEntry *bs = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, lo.save_mode[l],
-                                                                split_kept_ok(lp.hh, mode, lo.Tc, d->seq_len)))
+                                                                split_kept_ok(lp.hh, mode, lo.Tc, d->seq_len), merge_bwd()))
                     be = bs;
             if (!be) {
                 put(" bwd_kernel=runtime bwd_rows=0");
@@ -1259,7 +1270,7 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
                 int np = 1;
                 if ((!be->split || be->saved == 2) && t_opt.row_plan) {
                     const int q = tts_plan_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, be->saved,
-                                                   be->split && be->saved == 2, pe, pr0, pr);
+                                                   be->split && be->saved == 2, merge_bwd(), pe, pr0, pr);
                     if (q >= 1) np = q; else { pe[0] = be; pr[0] = B; }
                 }
                 put(" bwd_kernel=%s bwd_rows=%d bwd_phase_rows=%lld", tok(pe[0]->name).c_str(), pe[0]->R, pr[0]);
@@ -1402,7 +1413,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
 
         // ---- statically specialised kernel for this hh shape, if one is registered -------------------
         const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        const TtsRnnFwdEntry *se = t_opt.stat ? tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd) : nullptr;
+        const TtsRnnFwdEntry *se = t_opt.stat ? tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd, merge_fwd()) : nullptr;
         if (se) {
             int occ = 0;
             int rc = se->prepare(&occ);
@@ -1665,11 +1676,11 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
         // per-step gradient logging is emitted by the runtime-shape BPTT kernel (it recomputes from hs / cs, which every
         // training forward keeps, so it can follow a forward that ran on the static kernels)
         const bool logging = t_log.dh != nullptr;
-        const TtsRnnBwdEntry *be = (t_opt.stat && !logging) ? tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd) : nullptr;
+        const TtsRnnBwdEntry *be = (t_opt.stat && !logging) ? tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd()) : nullptr;
         if (t_opt.stat && !logging && lo.save_mode[l] != 0 && sv) {
             // forward kept (X_0 and) the hh pre-activations of this layer: use the kernel that consumes them
             if (const TtsRnnBwdEntry *bs = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd,
-                                                            lo.save_mode[l], split_kept_ok(lp.hh, mode, lo.Tc, T)))
+                                                            lo.save_mode[l], split_kept_ok(lp.hh, mode, lo.Tc, T), merge_bwd()))
                 be = bs;
         }
         // split variants behind a projected input take the hh bias gradient from the ih side (LSTM only); the rank-one
@@ -1690,7 +1701,7 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
                 const TtsRnnBwdEntry *pe[2];
                 long long pr0[2], pr[2];
                 const int np = tts_plan_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, be->saved,
-                                                be->split && be->saved == 2, pe, pr0, pr);
+                                                be->split && be->saved == 2, merge_bwd(), pe, pr0, pr);
                 if (np >= 1) {
                     nph = np;
                     for (int q = 0; q < np; ++q) { ph_e[q] = pe[q]; ph_row0[q] = pr0[q]; ph_rows[q] = pr[q]; }
