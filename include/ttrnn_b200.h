@@ -253,7 +253,7 @@ int ttrnn_rnn_ih_route(const ttrnn_rnn_desc *desc, int32_t layer, int64_t *chain
 
 /* Execution plan of `desc` under the current options, as text: first line "chunk_steps=.. sms=.. tc_gemm=.. rank_padded=.. bwd_overlap=..", then one
  * line per layer of key=value pairs (ih_route, ih_fwd_tc / ih_dw_tc = tensor-core GEMMs used, fwd_kernel, fwd_rows =
- * batch rows per CTA, save_mode, and with training != 0: bwd_kernel, bwd_rows, bwd_phase_rows, optional second phase,
+ * batch rows per CTA, save_mode = 2 with kept gate activations else 0, and with training != 0: bwd_kernel, bwd_rows, bwd_phase_rows, optional second phase,
  * hh_dw, hh_dw_tc).  Needs a CUDA device (the plan depends on its SM count).  Returns characters written, < 0 on error. */
 int ttrnn_rnn_describe(const ttrnn_rnn_desc *desc, int32_t training, char *buf, int32_t cap);
 /* Row-group split of `desc` under the current options (round 2, "row_groups"): multi-layer stacks whose batch does not
@@ -301,8 +301,6 @@ int ttrnn_static_kernel_table(char *buf, int32_t cap);
  *                   layer l - 1, planned for the SMs that kernel leaves idle; the second stream is forked from and joined back
  *                   into the caller's stream inside ttrnn_rnn_backward (capturable).  Costs a second set of the per-layer
  *                   backward scratch buffers.  0 = everything on the caller's stream
- *   "save_bytes"    budget for keeping chain activations of two-core chains for backward instead of
- *                   recomputing them (default 0 = recompute)
  *   "merge_cores"   d3 r8 LSTM chains: run static kernels with TT cores 0 and 1 contracted into one core while staging
  *                   (same parameters and gradients, one chain stage fewer).  1 (default) = the dX-only BPTT kernels only:
  *                   forward results stay bit-identical to 0, gradients differ by rounding; 2 = the forward kernels as well

@@ -114,7 +114,7 @@ def load() -> C.CDLL:
                      ("chunk_bytes", "TTRNN_CHUNK_BYTES"), ("static_rows_fwd", "TTRNN_STATIC_ROWS_FWD"),
                      ("static_rows_bwd", "TTRNN_STATIC_ROWS_BWD"), ("static_kernels", "TTRNN_STATIC_KERNELS"),
                      ("dense_ih", "TTRNN_DENSE_IH"), ("dense_ih_ratio", "TTRNN_DENSE_IH_RATIO"),
-                     ("save_bytes", "TTRNN_SAVE_BYTES"), ("save_u_bytes", "TTRNN_SAVE_U_BYTES"),
+                     ("save_u_bytes", "TTRNN_SAVE_U_BYTES"),
                      ("row_plan", "TTRNN_ROW_PLAN"), ("gemm_wide", "TTRNN_GEMM_WIDE"), ("split_kept", "TTRNN_SPLIT_KEPT"),
                      ("dense_hh_dw", "TTRNN_DENSE_HH_DW"), ("tc_gemm", "TTRNN_TC_GEMM"),
                      ("rank_pad", "TTRNN_RANK_PAD"), ("bwd_overlap", "TTRNN_BWD_OVERLAP"),

@@ -614,10 +614,8 @@ struct RnnFwdSArgs {
     long long out_bstride;
     float *c_save;
     float *h_out, *c_out;
-    // optional (training, two-core chains): keep X_0 (output of stage 1) and the hh pre-activations of every
-    // step so that backward does not recompute the chain.  Row b, step t at  base + b*bstride + t*per_step.
-    float *x0_save;          // per step: Mrow_0 * K_0 floats (unpadded rows)
-    long long x0_bstride;
+    // optional (training): keep the gate activations of every step so that backward skips the final stage of the
+    // chain recompute.  Row b, step t at  base + b*bstride + t*per_step.
     float *u_save;           // per step: H x 4 floats [h][gate]: the gate activations (LSTM i,f,g,o; GRU r,z,n and u_n)
     long long u_bstride;
 };
@@ -745,17 +743,6 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_fwd_s(const __grid_constant_
             if (t + 1 < a.steps) fetch_in(t + 1);
             // ---- stages d-1 .. 1
             const float *X0 = fwd_chain_pp<S, R, TU, S::D - 1>(hs, P, Q, wsm, tid);
-            if (!SrcOf<S>::merged && a.x0_save) {
-                // X_0 tile -> HBM (coalesced float4), overlapped with the final stage which only reads it
-                using T0s = St<S, 0>;
-                constexpr int X0F = T0s::Mrow * T0s::K;
-                for (int e = tid * 4; e < R * X0F; e += NTHR * 4) {
-                    const int b = e / X0F, rem = e % X0F;
-                    if (row0 + b < a.B)
-                        *reinterpret_cast<float4 *>(a.x0_save + (row0 + b) * a.x0_bstride + (long long)t * X0F + rem) =
-                            ld4(X0 + b * T0s::BS + T0s::roff(rem / T0s::K) + (rem % T0s::K));
-                }
-            }
             // ---- stage 0 (split over K) + reduce-scatter + gate math + state update
             float pre[R][NE][4];
             {
@@ -1184,7 +1171,7 @@ struct BwdSmem {
     using TU = typename TB::F;
     using FM = FinMap<S, R, TU::FTMr, TU::FTI, TU::FSK>;
     // forward-layout cores are only staged by the kernels that recompute (part of) the chain
-    static constexpr int W = (SV == 1 || (!DWI && SV != 0)) ? 0 : w_floats<S>();
+    static constexpr int W = (!DWI && SV != 0) ? 0 : w_floats<S>();
     static constexpr int WT = wt_floats<S>();
     static constexpr int stage_bs(int k) { return slot_floats_of<S>(k); }
     static constexpr int HS0 = cr4(R * stage_bs(S::D - 1));
@@ -1224,10 +1211,8 @@ struct RnnBwdSArgs {
     const float *dh_in, *dc_in;
     float *dh_out, *dc_out;
     float *partial;          // [gridDim.x][core_floats + 3*G*H]: cores, db_hh, d_weff, db_ih  (+= at the end)
-    const float *x0_save;    // SAVED kernels: X_0 tiles / hh pre-activations written by the forward kernel
-    long long x0_bstride;    //   (whole sequence, not offset by t0; row stride in floats)
-    const float *u_save;
-    long long u_bstride;
+    const float *u_save;     // kept-gates kernels: gate activations written by the forward kernel
+    long long u_bstride;     //   (whole sequence, not offset by t0; row stride in floats)
 };
 
 // LASTSYNC = false: no barrier after stage 1 (the caller's next phase does not read X_0 and ends with a barrier)
@@ -1286,18 +1271,18 @@ TTS_DEV void flush_all(DwRegs<S, R, TB> &dw, float *stg, float *slot, int tid) {
     if constexpr (k + 1 < S::D) flush_all<S, R, TB, k + 1>(dw, stg, slot, tid);
 }
 
-// SV = 0: recompute the whole chain;  SV = 1: forward kept X_0 and the hh pre-activations (two-core chains);
-// SV = 2: forward kept only the hh pre-activations u (G*H floats per row and step): stages d-1..1 are
+// SV = 0: recompute the whole chain;
+// SV = 2: forward kept the hh pre-activations u (G*H floats per row and step): stages d-1..1 are
 //         recomputed (their X_k feed the core gradients) but the final stage, its reduce-scatter and two
 //         barriers are skipped -- for two-core chains that is 60 % of the recomputed multiply-adds
 template <class S, int CELL, int R, int MODE, class TB, bool DWI = true, int SV = 0, int MINB = 1>
 __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant__ RnnBwdSArgs a) {
-    constexpr bool SAVED = (SV == 1), SAVEU = (SV != 0);
-    static_assert(!SAVED || (S::D == 2 && DWI), "saved-activation backward is implemented for two-core chains");
+    static_assert(SV == 0 || SV == 2, "save mode");
+    constexpr bool SAVEU = (SV != 0);
     static_assert(!SrcOf<S>::merged || (!DWI && SV == 2), "contracted chains run the dX-only kernel with kept gates");
     // DWI = false with kept gates: nothing of the forward chain is needed (gates come from the forward pass, the
     // core gradients from the dense accumulation outside): the kernel runs the gate gradients and the dX chain only
-    constexpr bool RECOMPUTE = !SAVED && (DWI || !SAVEU);
+    constexpr bool RECOMPUTE = DWI || !SAVEU;
     constexpr bool NEED_H = DWI || !SAVEU || (CELL != TTRNN_CELL_LSTM);
     extern __shared__ __align__(16) float smem[];
     using SM = BwdSmem<S, R, TB, DWI, SV>;
@@ -1411,17 +1396,6 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
                 else st4(dho_s + e, make_float4(0.f, 0.f, 0.f, 0.f));
             }
         };
-        auto fetch_x0 = [&](int tgl) {                    // saved X_0 tile of global step tgl -> its slot
-            using T0s = St<S, 0>;
-            constexpr int X0F = T0s::Mrow * T0s::K;
-            float *dst = xs + SM::template XOff<0>::v;
-            for (int e = tid * 4; e < R * X0F; e += NTHR * 4) {
-                const int b = e / X0F, rem = e % X0F;
-                float *d4 = dst + b * T0s::BS + T0s::roff(rem / T0s::K) + (rem % T0s::K);
-                if (row0 + b < a.B) cp_async16(d4, a.x0_save + (row0 + b) * a.x0_bstride + (long long)tgl * X0F + rem);
-                else st4(d4, make_float4(0.f, 0.f, 0.f, 0.f));
-            }
-        };
         auto fetch_regs = [&](int tl) {                   // operands of local step tl (recompute kernels)
             const int tgl = a.t0 + tl;
 #pragma unroll
@@ -1482,15 +1456,13 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
         } else {
             fetch_regs(a.steps - 1);
         }
-        if (SAVED) fetch_x0(a.t0 + a.steps - 1);
         cp_async_wait_all();
         __syncthreads();
         for (int t = a.steps - 1; t >= 0; --t) {
             const int tg = a.t0 + t;
             float *hcur = smem + ((t & 1) ? HOFF1 : HOFF0);
             // the last barrier of the previous step's backward chain already ordered everything this step reads (dh chain,
-            // cp.async tiles); only the kept-X_0 kernels issue more cp.async after it
-            if constexpr (SAVED) __syncthreads();
+            // cp.async tiles)
             // operands of this step
             float xin[R][NE][4], x1[R], cprev[R][NE], hprev[R][NE], dho[R][NE], pre[R][NE][4];
 #pragma unroll
@@ -1610,7 +1582,6 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
                         g_bhh[n][g] += d_hh[g];
                     }
                 }
-            if (SAVED) cp_async_wait_all();               // X_0 tile of this step (and h_{t-2}) have landed
             __syncthreads();
             if constexpr (SAVEU) {
                 if (t > 0) fetch_dho(tg - 1);             // the tile of this step has been consumed by every thread
@@ -1618,7 +1589,6 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
             // ---- backward chain: core gradients (register tiles) and dh_{t-1}
             bwd_chain<S, R, TB, 0, true, DWI>(xs, hcur, dy0, dhc, wt, xch, dw, tid);
             cp_async_wait_all();
-            if (SAVED && t > 0) fetch_x0(tg - 1);         // the X_0 slot is free again: refill for the next step
         }
         __syncthreads();
 #pragma unroll

@@ -13,7 +13,6 @@ struct TtlBwdSArgs;
 struct TtsRnnFwdEntry {
     const char *name;
     int cell, mode, R;
-    long long x0_floats;                                                      // > 0: the kernel can keep X_0 (floats per row-step)
     size_t smem;
     bool (*match)(const ttrnn_tt_shape *hh);
     int (*launch)(const tts::RnnFwdSArgs *args, int grid, cudaStream_t st);   // 0 = ok, else cudaError_t
@@ -30,7 +29,7 @@ struct TtsRnnBwdEntry {
     const char *name;
     int cell, mode, R;
     int split;                                                               // 1: core gradients come from a batched kernel
-    int saved;                                                               // 1: consumes X_0 + hh pre-activations kept by forward, 2: pre-activations only
+    int saved;                                                               // 2: consumes the gate activations kept by the forward, 0: recomputes
     size_t smem;
     long long slot_floats;                                                   // floats per gradient slot
     bool (*match)(const ttrnn_tt_shape *hh);

@@ -53,22 +53,19 @@ int prepare_fwd(int *occ) {
     return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, k, tts::NTHR, tts::FwdSmem<S, R, TU>::BYTES);
 }
 
-template <class S> constexpr long long x0_floats() {
-    return S::D == 2 ? (long long)tts::St<S, 0>::Mrow * tts::St<S, 0>::K : 0;
-}
 #define TTS_FWD(S, CELL, R, MODE, ...)                                                                     \
-    {#S, CELL, MODE, R, x0_floats<S>(), tts::FwdSmem<S, R, __VA_ARGS__>::BYTES, &match_shape<S>,            \
+    {#S, CELL, MODE, R, tts::FwdSmem<S, R, __VA_ARGS__>::BYTES, &match_shape<S>,                            \
      &launch_fwd<S, CELL, R, MODE, __VA_ARGS__>, &prepare_fwd<S, CELL, R, MODE, __VA_ARGS__>, 0}
-// contracted chain (tts::Merge01) of the three-core shape S3: registered under S3, reads S3's blob, keeps no X_0
+// contracted chain (tts::Merge01) of the three-core shape S3: registered under S3, reads S3's blob
 #define TTS_FWD_M01(S3, CELL, R, MODE, ...)                                                                \
-    {#S3 "(m01)", CELL, MODE, R, 0, tts::FwdSmem<tts::Merge01<S3>, R, __VA_ARGS__>::BYTES, &match_shape<S3>, \
+    {#S3 "(m01)", CELL, MODE, R, tts::FwdSmem<tts::Merge01<S3>, R, __VA_ARGS__>::BYTES, &match_shape<S3>,    \
      &launch_fwd<tts::Merge01<S3>, CELL, R, MODE, __VA_ARGS__>, &prepare_fwd<tts::Merge01<S3>, CELL, R, MODE, __VA_ARGS__>, 1}
 
 // Tune<FTMr, FTI, FSK, TM1, TN1, TM2, TN2, TM3, TN3>: final-stage tile (rows, first-mode slices, k-split)
 // and (rows, columns) of the thread tile of stages 1..3
 using tts::Tune;
 #define TTS_FWD2(S, CELL, R, MODE, ...)                                                                    \
-    {#S "(2 CTAs/SM)", CELL, MODE, R, x0_floats<S>(), tts::FwdSmem<S, R, __VA_ARGS__>::BYTES, &match_shape<S>, \
+    {#S "(2 CTAs/SM)", CELL, MODE, R, tts::FwdSmem<S, R, __VA_ARGS__>::BYTES, &match_shape<S>,                \
      &launch_fwd<S, CELL, R, MODE, __VA_ARGS__, 2>, &prepare_fwd<S, CELL, R, MODE, __VA_ARGS__, 2>, 0}
 // d3 r8 chain with cores 0 and 1 contracted (J = [32, 8], I = [64, 16], RK = [1, 8, 1]): the final stage contracts
 // K = 256; two first-mode slices per thread with k split in halves (FTI = FSK = 2): per k-step R + 8 LDS.128 feed 16 R
@@ -127,10 +124,6 @@ constexpr long long slot_floats() { return tts::blob_floats<S>() + 3LL * S::G * 
 #define TTS_BWD(S, CELL, R, MODE, ...)                                                                      \
     {#S, CELL, MODE, R, 0, 0, tts::BwdSmem<S, R, __VA_ARGS__, true>::BYTES, slot_floats<S>(), &match_shape<S>, \
      &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, true>, &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true>, 0}
-#define TTS_BWD_SAVED(S, CELL, R, MODE, ...)                                                                \
-    {#S "(saved)", CELL, MODE, R, 0, 1, tts::BwdSmem<S, R, __VA_ARGS__, true, 1>::BYTES, slot_floats<S>(),   \
-     &match_shape<S>, &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 1>,                                   \
-     &prepare_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 1>, 0}
 #define TTS_BWD_SAVEU(S, CELL, R, MODE, ...)                                                                \
     {#S "(kept u)", CELL, MODE, R, 0, 2, tts::BwdSmem<S, R, __VA_ARGS__, true, 2>::BYTES, slot_floats<S>(),  \
      &match_shape<S>, &launch_bwd<S, CELL, R, MODE, __VA_ARGS__, true, 2>,                                   \
@@ -189,10 +182,6 @@ const TtsRnnBwdEntry kBwd[] = {
     TTS_BWD(HH_H256_d2r4_gru, TTRNN_CELL_GRU, 7, tts::MODE_RANK1, TB_d2),
     TTS_BWD(HH_H256_d2r4_gru, TTRNN_CELL_GRU, 4, tts::MODE_XG, TB_d2),
     TTS_BWD(HH_H256_d2r4_gru, TTRNN_CELL_GRU, 7, tts::MODE_XG, TB_d2),
-    TTS_BWD_SAVED(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_RANK1, TB_d2),
-    TTS_BWD_SAVED(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 4, tts::MODE_RANK1, TB_d2),
-    TTS_BWD_SAVED(HH_H256_d2r4_gru, TTRNN_CELL_GRU, 4, tts::MODE_RANK1, TB_d2),
-    TTS_BWD_SAVED(HH_H256_d2r4_gru, TTRNN_CELL_GRU, 7, tts::MODE_RANK1, TB_d2),
     TTS_BWD_SAVEU(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_RANK1, TB_d2),
     TTS_BWD_SAVEU(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, TB_d2),
     TTS_BWD_SAVEU(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_RANK1, TB_d2),

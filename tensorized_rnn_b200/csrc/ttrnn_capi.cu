@@ -28,9 +28,6 @@ std::atomic<long long> g_opt_chunk{0};
 std::atomic<long long> g_opt_chunk_bytes{4LL << 30};
 std::atomic<long long> g_opt_static{1};
 std::atomic<long long> g_opt_srows_fwd{0}, g_opt_srows_bwd{0};
-// budget for kept chain activations (0 = always recompute).  Off by default: measured on cfg2 it trades
-// +0.9 ms forward (X_0 stores) for -1.2 ms backward and costs 9 GB, a 1.6 % net gain.
-std::atomic<long long> g_opt_save_bytes{0};
 // budget for keeping only the hh pre-activations u (G*H floats per row and step) so that backward skips the
 // final stage of the chain recompute (measured on cfg2: see profiles/)
 std::atomic<long long> g_opt_save_u_bytes{16LL << 30};
@@ -75,11 +72,11 @@ std::atomic<long long> g_opt_merge_cores{1};
 // ttrnn_set_option() between a forward and its backward (another model, another thread) cannot change how `saved` and
 // the scratch buffers are interpreted.  Helpers read the calling thread's current snapshot `t_opt`.
 struct Opts {
-    long long rows, chunk, chunk_bytes, stat, srows_fwd, srows_bwd, save_bytes, save_u_bytes, row_plan, dense_ih, gemm_wide,
+    long long rows, chunk, chunk_bytes, stat, srows_fwd, srows_bwd, save_u_bytes, row_plan, dense_ih, gemm_wide,
         dense_hh, split_kept, dense_ratio, tc_gemm, rank_pad, bwd_overlap, row_groups, merge_cores;
 };
 constexpr int kOptFields = sizeof(Opts) / sizeof(long long);
-constexpr long long kPlanMagic = 0x7474726E6E706C35LL;          // "ttrnnpl5"
+constexpr long long kPlanMagic = 0x7474726E6E706C36LL;          // "ttrnnpl6"
 // plan words: [0] magic, [1 .. kOptFields] options, then the row-group split (group count, rows of group 0)
 constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2;
 static_assert(kOptFields + 3 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
@@ -91,7 +88,7 @@ Opts snapshot_options() {
     Opts o;
     o.rows = g_opt_rows.load(); o.chunk = g_opt_chunk.load(); o.chunk_bytes = g_opt_chunk_bytes.load();
     o.stat = g_opt_static.load(); o.srows_fwd = g_opt_srows_fwd.load(); o.srows_bwd = g_opt_srows_bwd.load();
-    o.save_bytes = g_opt_save_bytes.load(); o.save_u_bytes = g_opt_save_u_bytes.load(); o.row_plan = g_opt_row_plan.load();
+    o.save_u_bytes = g_opt_save_u_bytes.load(); o.row_plan = g_opt_row_plan.load();
     o.dense_ih = g_opt_dense_ih.load(); o.gemm_wide = g_opt_gemm_wide.load(); o.dense_hh = g_opt_dense_hh.load();
     o.split_kept = g_opt_split_kept.load(); o.dense_ratio = g_opt_dense_ratio.load(); o.tc_gemm = g_opt_tc_gemm.load();
     o.rank_pad = g_opt_rank_pad.load(); o.bwd_overlap = g_opt_bwd_overlap.load(); o.row_groups = g_opt_row_groups.load();
@@ -336,6 +333,21 @@ int build_rnn_plan(const ttrnn_rnn_desc *d, RnnPlan *rp) {
     return 0;
 }
 
+// ---- kernel routes of a recurrent layer -------------------------------------------------------------------------
+// Every caller that needs to know which recurrent kernel a layer runs (workspace layout, row-group planner, describe,
+// the launch paths) asks these functions, so that the plan they report and model is the one that launches.
+
+// input mode of layer l: a single input feature (I = 1) is folded into the recurrent kernel as a rank-one term
+inline int layer_mode(const ttrnn_rnn_desc *d, int l) {
+    return (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
+}
+
+// statically specialised forward kernel of layer l at B rows on `sms` SMs, or nullptr (runtime-shape kernel)
+const TtsRnnFwdEntry *fwd_route(const ttrnn_rnn_desc *d, int l, long long B, int sms) {
+    if (!t_opt.stat) return nullptr;
+    return tts_find_rnn_fwd(&d->hh[l], d->cell, layer_mode(d, l), B, sms, (int)t_opt.srows_fwd, merge_fwd());
+}
+
 // ---- rank padding -----------------------------------------------------------------------------------------------
 // The statically specialised kernels need inner TT ranks that are multiples of 4 (tt_static.cuh).  A chain whose ranks
 // are not (the reference's own GE2E default is n_cores = 2, rank = 2: encoder/params_model.py:15-16) is mathematically
@@ -394,10 +406,8 @@ int make_eff_desc(const ttrnn_rnn_desc *d, const DevInfo *dv, EffDesc *e) {
             }
         }
     if (!any) return 0;
-    for (int l = 0; l < d->num_layers; ++l) {
-        const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        if (!tts_find_rnn_fwd(&p.hh[l], d->cell, mode, d->batch, dv->sms, 0, merge_fwd())) return 0;     // padding would not reach a static kernel
-    }
+    for (int l = 0; l < d->num_layers; ++l)
+        if (!fwd_route(&p, l, d->batch, dv->sms)) return 0;     // padding would not reach a static kernel
     RnnPlan pad;
     if (build_rnn_plan(&p, &pad)) return 0;
     const int GH = real.G * d->hidden_size;
@@ -456,10 +466,59 @@ bool dense_hh_dw_ok(const ChainPlan &hh) {
     return t_opt.dense_hh && hh.n_out % ttg::BN == 0 && hh.n_in % 4 == 0 && hh.n_in <= 2048;
 }
 
-// kept gates: may the dX-only ("split") BPTT variants be used for this layer?  They need the dense accumulation of the hh
-// core gradients; with a rank-one input the delta buffer must also hold the whole sequence (single-chunk plans)
-bool split_kept_ok(const ChainPlan &hh, int mode, long long Tc, long long T) {
-    return dense_hh_dw_ok(hh) && t_opt.split_kept && (mode != tts::MODE_RANK1 || Tc >= T);
+// Static BPTT route of layer l at B rows on `sms` SMs.  `mode` is an argument because a rank-one layer 0 whose input
+// gradient is requested runs the MODE_XG kernels.  `kept`: the forward kept this layer's gate activations (the kept-gates
+// kernels are then preferred where registered); Tc: timesteps per chunk of the layout.
+struct BwdRoute {
+    int nph = 0;                                       // phases of the row plan; 0 = runtime-shape kernel
+    const TtsRnnBwdEntry *e[2] = {nullptr, nullptr};   // kernel of each phase
+    long long row0[2] = {0, 0}, rows[2] = {0, 0};      // first row and row count of each phase
+    bool kept = false;       // the kernels consume the kept gate activations
+    bool split = false;      // dX-only kernels: the hh core gradients are computed outside the recurrent kernel ...
+    bool dense_hh = false;   // ... by the dense accumulation dW_hh^T = H_prev^T delta (else a second chain pass)
+    bool split_r1 = false;   // split behind a rank-one input: bias / W_ih-column gradients stay in the kernel's slots
+};
+
+int bwd_route(const ttrnn_rnn_desc *d, const RnnPlan &rp, int l, int mode, long long B, int sms, bool kept, long long Tc,
+              BwdRoute *r) {
+    *r = BwdRoute();
+    if (!t_opt.stat) return 0;
+    const ttrnn_tt_shape *hh = &d->hh[l];
+    const int srows = (int)t_opt.srows_bwd;
+    const TtsRnnBwdEntry *be = tts_find_rnn_bwd(hh, d->cell, mode, B, sms, srows, 0, 0, merge_bwd());
+    if (kept) {
+        // the dX-only ("split") variants need the dense accumulation of the hh core gradients; with a rank-one input the
+        // delta buffer must also hold the whole sequence (single-chunk plans)
+        const bool split_ok = dense_hh_dw_ok(rp.layer[l].hh) && t_opt.split_kept && (mode != tts::MODE_RANK1 || Tc >= d->seq_len);
+        if (const TtsRnnBwdEntry *bs = tts_find_rnn_bwd(hh, d->cell, mode, B, sms, srows, 2, split_ok, merge_bwd())) be = bs;
+    }
+    if (!be) return 0;
+    r->nph = 1;
+    r->e[0] = be;
+    r->rows[0] = B;
+    // row plan: one phase, or two when a tail variant beats a mostly idle last wave
+    if ((!be->split || be->saved == 2) && t_opt.row_plan) {
+        const TtsRnnBwdEntry *pe[2];
+        long long pr0[2], pr[2];
+        const int np = tts_plan_rnn_bwd(hh, d->cell, mode, B, sms, srows, be->saved, be->split && be->saved == 2, merge_bwd(),
+                                        pe, pr0, pr);
+        if (np >= 1) {
+            r->nph = np;
+            for (int q = 0; q < np; ++q) { r->e[q] = pe[q]; r->row0[q] = pr0[q]; r->rows[q] = pr[q]; }
+        }
+    }
+    r->kept = r->e[0]->saved == 2;
+    r->split = r->e[0]->split != 0;
+    r->dense_hh = r->split && dense_hh_dw_ok(rp.layer[l].hh);
+    r->split_r1 = r->split && mode == tts::MODE_RANK1;
+    // split variants behind a projected input take the hh bias gradient from the ih side (LSTM only); the rank-one
+    // variants keep every bias / W_ih-column gradient in the kernel's own slot and work for both cells
+    if (r->split && d->cell != TTRNN_CELL_LSTM && !r->split_r1)
+        return fail("internal: split BPTT variants with a projected input compute the hh bias gradient from the ih side "
+                    "(LSTM only); %s is registered for a GRU", r->e[0]->name);
+    if (r->split_r1 && !r->dense_hh)
+        return fail("internal: rank-one split BPTT variant %s selected without the dense hh core-gradient route", r->e[0]->name);
+    return 0;
 }
 
 struct DenseIh {
@@ -488,9 +547,9 @@ struct RnnLayout {
     // backward overlap: the per-layer buffers (everything from b_xg on) exist twice, set (l & 1) at + set * set_stride
     int overlap = 0;
     long long set_stride = 0;
-    // kept chain activations (two-core static chains, within the save_bytes budget): per layer offsets into `saved`
-    int save_mode[TTRNN_MAX_LAYERS] = {};
-    long long sv_x0[TTRNN_MAX_LAYERS] = {}, sv_u[TTRNN_MAX_LAYERS] = {}, x0f[TTRNN_MAX_LAYERS] = {};
+    // kept gate activations (static kernels, within the save_u_bytes budget): per layer flag and offset into `saved`
+    bool kept[TTRNN_MAX_LAYERS] = {};
+    long long sv_u[TTRNN_MAX_LAYERS] = {};
 };
 
 int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, RnnLayout *lo) {
@@ -511,35 +570,27 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
     lo->sv_hs = 0;
     lo->sv_cs = r4((L - 1) * lo->BTH);
     lo->sv_total = lo->sv_cs + (lstm ? r4(L * lo->BTH) : 0);
-    // kept activations of the static recurrent kernels, per layer:
-    //   mode 1 (two-core chains, "save_bytes" budget, off by default): X_0 tiles + gate activations
-    //   mode 2 ("save_u_bytes" budget, default 16 GiB): gate activations only (4*H floats per row and step: LSTM
-    //           i,f,g,o; GRU r,z,n,u_n) -- backward skips the final stage of the recompute and all gate math
-    if (t_opt.stat) {
-        long long extra1 = 0, extra2 = 0;
-        int mode1[TTRNN_MAX_LAYERS] = {}, mode2[TTRNN_MAX_LAYERS] = {};
+    // kept gate activations of the static recurrent kernels ("save_u_bytes" budget, default 16 GiB): 4*H floats per row
+    // and step (LSTM i,f,g,o; GRU r,z,n,u_n) -- backward skips the final stage of the recompute and all gate math.  Every
+    // layer whose forward and kept-gates backward are static keeps them, or none does.  The dense accumulation of the hh
+    // core gradients is sized for a split backward with or without kept gates.
+    bool can_keep[TTRNN_MAX_LAYERS] = {};
+    long long kept_floats = 0, dhh = 0;
+    if (t_opt.stat)
         for (int l = 0; l < L; ++l) {
-            const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-            const TtsRnnFwdEntry *se = tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd, merge_fwd());
-            if (!se) continue;
-            if (se->x0_floats > 0 && tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 1, 0, merge_bwd())) {
-                mode1[l] = 1;
-                lo->x0f[l] = se->x0_floats;
-                extra1 += r4(B * T * se->x0_floats) + r4(B * T * 4 * H);
-            }
-            const int oks = split_kept_ok(rp.layer[l].hh, mode, tc, T) ? 1 : 0;
-            if (tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 2, oks, merge_bwd())) {
-                mode2[l] = 1;
-                extra2 += r4(B * T * 4 * H);
-            }
+            BwdRoute recompute, keep;
+            if (bwd_route(d, rp, l, layer_mode(d, l), B, dv.sms, false, tc, &recompute) ||
+                bwd_route(d, rp, l, layer_mode(d, l), B, dv.sms, true, tc, &keep))
+                return 1;
+            can_keep[l] = keep.kept && fwd_route(d, l, B, dv.sms);
+            if (can_keep[l]) kept_floats += r4(B * T * 4 * H);
+            if ((recompute.dense_hh || keep.dense_hh) && dense_bwd_floats(rp.layer[l].hh) > dhh)
+                dhh = dense_bwd_floats(rp.layer[l].hh);
         }
-        const bool use1 = extra1 > 0 && extra1 * 4 <= t_opt.save_bytes;
-        const bool use2 = !use1 && extra2 > 0 && extra2 * 4 <= t_opt.save_u_bytes;
-        for (int l = 0; l < L; ++l) {
-            lo->save_mode[l] = (use1 && mode1[l]) ? 1 : ((use2 && mode2[l]) ? 2 : 0);
-            if (lo->save_mode[l] == 1) { lo->sv_x0[l] = lo->sv_total; lo->sv_total += r4(B * T * lo->x0f[l]); }
-            if (lo->save_mode[l] != 0) { lo->sv_u[l] = lo->sv_total; lo->sv_total += r4(B * T * 4 * H); }
-        }
+    const bool keep_all = kept_floats > 0 && kept_floats * 4 <= t_opt.save_u_bytes;
+    for (int l = 0; l < L; ++l) {
+        lo->kept[l] = keep_all && can_keep[l];
+        if (lo->kept[l]) { lo->sv_u[l] = lo->sv_total; lo->sv_total += r4(B * T * 4 * H); }
     }
     // forward scratch
     long long o = 0;
@@ -587,18 +638,7 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
     lo->b_spill = o; o += r4(spill) * lo->nslots;
     lo->b_aux = o; o += 2 * r4(GH) + 4;                   // rank-one input mode: W_ih column, its gradient, a 1.0f
     lo->b_dense = o; o += dbw;
-    long long dhh = 0;                                    // split backward: dense accumulation of the hh core gradients
-    if (t_opt.stat)
-        for (int l = 0; l < L; ++l) {
-            const bool okd = dense_hh_dw_ok(rp.layer[l].hh);
-            const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-            const int oks = split_kept_ok(rp.layer[l].hh, mode, tc, T) ? 1 : 0;
-            const TtsRnnBwdEntry *be = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd());
-            const TtsRnnBwdEntry *b2 = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 2, oks, merge_bwd());
-            if (okd && ((be && be->split) || (b2 && b2->split)) && dense_bwd_floats(rp.layer[l].hh) > dhh)
-                dhh = dense_bwd_floats(rp.layer[l].hh);
-        }
-    lo->b_dense_hh = o; o += dhh;
+    lo->b_dense_hh = o; o += dhh;                         // split backward: dense accumulation of the hh core gradients
     lo->overlap = (t_opt.bwd_overlap && t_opt.stat && L > 1 && tc == T) ? 1 : 0;
     if (lo->overlap) {
         lo->set_stride = r4(o - set_base);
@@ -606,6 +646,23 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
     }
     lo->b_total = o;
     return 0;
+}
+
+// Everything a call derives from its descriptor: the effective (possibly rank-padded) descriptor, its parameter plan and
+// its workspace layout on the device `dv`.
+struct CallPlan {
+    DevInfo dv;
+    EffDesc eff;
+    RnnPlan rp;         // of eff.d
+    RnnLayout lo;
+    const ttrnn_rnn_desc *d() const { return &eff.d; }
+};
+
+int plan_call(const ttrnn_rnn_desc *d_in, const DevInfo &dv, CallPlan *cp) {
+    cp->dv = dv;
+    if (build_rnn_plan(d_in, &cp->rp) || make_eff_desc(d_in, &dv, &cp->eff)) return 1;
+    if (cp->eff.padded && build_rnn_plan(&cp->eff.d, &cp->rp)) return 1;
+    return build_layout(&cp->eff.d, cp->rp, dv, &cp->lo);
 }
 
 // ---- launch helpers ------------------------------------------------------------------------
@@ -945,38 +1002,26 @@ double sim_makespan(const std::vector<SimLaunch> *q, int nq, int sms) {
 
 // launches of the recurrent kernels of one group of `Bg` rows: forward layers 0..L-1 into fq, backward L-1..0 into bq.
 // Cost of a wave of R rows per CTA ~ (0.4 + R) (measured on the d3r8 chain: forward 2.67 / 4.43 / 6.59 / 10.5 us per step
-// at R = 1 / 2 / 3 / 5, backward 2.96 / 4.86 / 7.0 at R = 1 / 2 / 3).  false: a layer has no static kernel.
-bool group_launches(const ttrnn_rnn_desc *d, const RnnPlan &rp, const RnnLayout &lo, long long Bg, int sms,
-                    std::vector<SimLaunch> *fq, std::vector<SimLaunch> *bq) {
+// at R = 1 / 2 / 3 / 5, backward 2.96 / 4.86 / 7.0 at R = 1 / 2 / 3).  The routes are those of a call on `Bg` rows with
+// the kept gates and chunking of the layout `cp.lo`.  false: a layer has no static kernel.
+bool group_launches(const CallPlan &cp, long long Bg, std::vector<SimLaunch> *fq, std::vector<SimLaunch> *bq) {
     constexpr double kFloor = 0.4;
+    const ttrnn_rnn_desc *d = cp.d();
+    const int sms = cp.dv.sms;
     auto push = [&](std::vector<SimLaunch> *q, long long rows, int R) {
         const long long tiles = (rows + R - 1) / R;
         const long long waves = (tiles + sms - 1) / sms;
         q->push_back({(int)(tiles < sms ? tiles : sms), (double)waves * (kFloor + R)});
     };
     for (int l = 0; l < d->num_layers; ++l) {
-        const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        const TtsRnnFwdEntry *se = tts_find_rnn_fwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_fwd, merge_fwd());
+        const TtsRnnFwdEntry *se = fwd_route(d, l, Bg, sms);
         if (!se) return false;
         push(fq, Bg, se->R);
     }
     for (int l = d->num_layers - 1; l >= 0; --l) {
-        const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        const TtsRnnBwdEntry *be = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd());
-        if (lo.save_mode[l] != 0)
-            if (const TtsRnnBwdEntry *bs = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_bwd, lo.save_mode[l],
-                                                            split_kept_ok(rp.layer[l].hh, mode, lo.Tc, d->seq_len), merge_bwd()))
-                be = bs;
-        if (!be) return false;
-        const TtsRnnBwdEntry *pe[2] = {be, nullptr};
-        long long pr0[2] = {0, 0}, pr[2] = {Bg, 0};
-        int np = 1;
-        if ((!be->split || be->saved == 2) && t_opt.row_plan) {
-            const int q = tts_plan_rnn_bwd(&d->hh[l], d->cell, mode, Bg, sms, (int)t_opt.srows_bwd, be->saved,
-                                           be->split && be->saved == 2, merge_bwd(), pe, pr0, pr);
-            if (q >= 1) np = q; else { pe[0] = be; pr[0] = Bg; }
-        }
-        for (int q = 0; q < np; ++q) push(bq, pr[q], pe[q]->R);
+        BwdRoute br;
+        if (bwd_route(d, cp.rp, l, layer_mode(d, l), Bg, sms, cp.lo.kept[l], cp.lo.Tc, &br) || !br.nph) return false;
+        for (int q = 0; q < br.nph; ++q) push(bq, br.rows[q], br.e[q]->R);
     }
     return true;
 }
@@ -1023,24 +1068,18 @@ int plan_row_groups(const ttrnn_rnn_desc *d_in, GroupPlan *gp, const DevInfo *de
         e.used = true; e.d = *d_in; e.o = t_opt; e.sms = dv.sms; e.gp = *gp;
         return 0;
     };
-    RnnPlan rp;
-    if (build_rnn_plan(d_in, &rp)) return 1;
-    EffDesc eff;
-    if (make_eff_desc(d_in, &dv, &eff)) return 1;
-    const ttrnn_rnn_desc *d = &eff.d;
-    if (eff.padded && build_rnn_plan(d, &rp)) return 1;
-    RnnLayout lo;
-    if (build_layout(d, rp, dv, &lo)) return 1;
-    const long long B = d->batch;
-    if (lo.Tc != d->seq_len || B < 8 || B > 16LL * dv.sms) return remember();
+    CallPlan cp;
+    if (plan_call(d_in, dv, &cp)) return 1;
+    const long long B = d_in->batch;
+    if (cp.lo.Tc != d_in->seq_len || B < 8 || B > 16LL * dv.sms) return remember();
     std::vector<SimLaunch> f1, b1;
-    if (!group_launches(d, rp, lo, B, dv.sms, &f1, &b1)) return remember();
+    if (!group_launches(cp, B, &f1, &b1)) return remember();
     const double fwd1 = sim_makespan(&f1, 1, dv.sms), bwd1 = sim_makespan(&b1, 1, dv.sms);
     double best = fwd1 + bwd1;
     const long long step = B <= 1024 ? 4 : 16;
     for (long long r0 = step; r0 < B; r0 += step) {
         std::vector<SimLaunch> fq[kMaxGroups], bq[kMaxGroups];
-        if (!group_launches(d, rp, lo, r0, dv.sms, &fq[0], &bq[0]) || !group_launches(d, rp, lo, B - r0, dv.sms, &fq[1], &bq[1]))
+        if (!group_launches(cp, r0, &fq[0], &bq[0]) || !group_launches(cp, B - r0, &fq[1], &bq[1]))
             continue;
         const double f2 = sim_makespan(fq, 2, dv.sms), b2 = sim_makespan(bq, 2, dv.sms);
         // ties go to the later candidate: the larger group 0 (issued first, on the caller's stream) is the critical path
@@ -1134,7 +1173,6 @@ int ttrnn_set_option(const char *key, int64_t value) {
     if (!strcmp(key, "chunk_steps")) { g_opt_chunk.store(value); return 0; }
     if (!strcmp(key, "chunk_bytes")) { g_opt_chunk_bytes.store(value > 0 ? value : (4LL << 30)); return 0; }
     if (!strcmp(key, "static_kernels")) { g_opt_static.store(value); return 0; }
-    if (!strcmp(key, "save_bytes")) { g_opt_save_bytes.store(value); return 0; }
     if (!strcmp(key, "save_u_bytes")) { g_opt_save_u_bytes.store(value); return 0; }
     if (!strcmp(key, "static_rows_fwd")) { g_opt_srows_fwd.store(value); return 0; }
     if (!strcmp(key, "static_rows_bwd")) { g_opt_srows_bwd.store(value); return 0; }
@@ -1200,8 +1238,10 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
     t_opt = snapshot_options();
     // with two row groups the layer lines describe group 0 (the full waves); the header names the split and the
     // rows per CTA the remainder group runs at
+    DevInfo dv;
+    if (get_dev(&dv)) return -1;
     GroupPlan gp;
-    if (plan_row_groups(d_full, &gp)) return -1;
+    if (plan_row_groups(d_full, &gp, &dv)) return -1;
     ttrnn_rnn_desc d_g0;
     const ttrnn_rnn_desc *d_in = d_full;
     if (gp.n == 2) {
@@ -1209,16 +1249,11 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
         d_g0.batch = gp.rows[0];
         d_in = &d_g0;
     }
-    RnnPlan rp;
-    if (build_rnn_plan(d_in, &rp)) return -1;
-    DevInfo dv;
-    if (get_dev(&dv)) return -1;
-    EffDesc eff;
-    if (make_eff_desc(d_in, &dv, &eff)) return -1;
-    const ttrnn_rnn_desc *d = &eff.d;
-    if (eff.padded && build_rnn_plan(d, &rp)) return -1;
-    RnnLayout lo;
-    if (build_layout(d, rp, dv, &lo)) return -1;
+    CallPlan cp;
+    if (plan_call(d_in, dv, &cp)) return -1;
+    const ttrnn_rnn_desc *d = cp.d();
+    const RnnPlan &rp = cp.rp;
+    const RnnLayout &lo = cp.lo;
     const long long B = d->batch;
     const int GH = rp.G * d->hidden_size;
     int n = 0;
@@ -1236,48 +1271,38 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
             if (c == ' ') c = '_';
         return t;
     };
-    put("chunk_steps=%d sms=%d tc_gemm=%lld rank_padded=%d bwd_overlap=%d row_groups=%d", lo.Tc, dv.sms, t_opt.tc_gemm, (int)eff.padded,
-        lo.overlap, gp.n);
+    put("chunk_steps=%d sms=%d tc_gemm=%lld rank_padded=%d bwd_overlap=%d row_groups=%d", lo.Tc, dv.sms, t_opt.tc_gemm,
+        (int)cp.eff.padded, lo.overlap, gp.n);
     if (gp.n == 2) {
         std::vector<SimLaunch> fq, bq;
         put(" group_rows0=%lld group_rows1=%lld", gp.rows[0], gp.rows[1]);
-        if (group_launches(d, rp, lo, gp.rows[1], dv.sms, &fq, &bq) && !fq.empty() && !bq.empty())
+        if (group_launches(cp, gp.rows[1], &fq, &bq) && !fq.empty() && !bq.empty())
             put(" group1_fwd_ctas=%d group1_bwd_ctas=%d", fq.back().ctas, bq.front().ctas);
     }
     put("\n");
     for (int l = 0; l < d->num_layers; ++l) {
         const LayerPlan &lp = rp.layer[l];
-        const bool rank1 = (l == 0 && d->input_size == 1);
-        const int mode = rank1 ? tts::MODE_RANK1 : tts::MODE_XG;
+        const int mode = layer_mode(d, l);
+        const bool rank1 = mode == tts::MODE_RANK1;
         const bool dense = !rank1 && dense_ih_ok(lp.ih, &d->ih[l]);
         const char *route = rank1 ? "rank_one" : (dense ? "dense" : "tt_chain");
         const bool tc_f = dense && tc_rows_use(B * (long long)lo.Tc, lp.ih.n_in, GH, false);
         const bool tc_r = dense && t_opt.tc_gemm && ttc::tc_red_ok(B * (long long)lo.Tc, lp.ih.n_in, GH);
-        const TtsRnnFwdEntry *se = t_opt.stat ? tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd, merge_fwd()) : nullptr;
+        const TtsRnnFwdEntry *se = fwd_route(d, l, B, dv.sms);
+        // save_mode 2 = kept gate activations, 0 = recompute
         put("layer=%d ih_route=%s ih_fwd_tc=%d ih_dw_tc=%d fwd_kernel=%s fwd_rows=%d save_mode=%d", l, route, (int)tc_f, (int)tc_r,
-            se ? tok(se->name).c_str() : "runtime", se ? se->R : 0, lo.save_mode[l]);
+            se ? tok(se->name).c_str() : "runtime", se ? se->R : 0, lo.kept[l] ? 2 : 0);
         if (training) {
-            const TtsRnnBwdEntry *be = t_opt.stat ? tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd()) : nullptr;
-            if (t_opt.stat && lo.save_mode[l] != 0)
-                if (const TtsRnnBwdEntry *bs = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, lo.save_mode[l],
-                                                                split_kept_ok(lp.hh, mode, lo.Tc, d->seq_len), merge_bwd()))
-                    be = bs;
-            if (!be) {
+            BwdRoute br;
+            if (bwd_route(d, rp, l, mode, B, dv.sms, lo.kept[l], lo.Tc, &br)) return -1;
+            if (!br.nph) {
                 put(" bwd_kernel=runtime bwd_rows=0");
             } else {
-                const TtsRnnBwdEntry *pe[2] = {be, nullptr};
-                long long pr0[2] = {0, 0}, pr[2] = {B, 0};
-                int np = 1;
-                if ((!be->split || be->saved == 2) && t_opt.row_plan) {
-                    const int q = tts_plan_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, be->saved,
-                                                   be->split && be->saved == 2, merge_bwd(), pe, pr0, pr);
-                    if (q >= 1) np = q; else { pe[0] = be; pr[0] = B; }
-                }
-                put(" bwd_kernel=%s bwd_rows=%d bwd_phase_rows=%lld", tok(pe[0]->name).c_str(), pe[0]->R, pr[0]);
-                if (np == 2) put(" bwd_kernel2=%s bwd_rows2=%d bwd_phase_rows2=%lld", tok(pe[1]->name).c_str(), pe[1]->R, pr[1]);
-                const bool hh_dense = be->split && dense_hh_dw_ok(lp.hh);
-                put(" hh_dw=%s hh_dw_tc=%d", be->split ? (hh_dense ? "dense" : "tt_chain") : "fused",
-                    (int)(hh_dense && t_opt.tc_gemm && ttc::tc_red_ok(B * (long long)lo.Tc, d->hidden_size, GH)));
+                put(" bwd_kernel=%s bwd_rows=%d bwd_phase_rows=%lld", tok(br.e[0]->name).c_str(), br.e[0]->R, br.rows[0]);
+                if (br.nph == 2)
+                    put(" bwd_kernel2=%s bwd_rows2=%d bwd_phase_rows2=%lld", tok(br.e[1]->name).c_str(), br.e[1]->R, br.rows[1]);
+                put(" hh_dw=%s hh_dw_tc=%d", br.split ? (br.dense_hh ? "dense" : "tt_chain") : "fused",
+                    (int)(br.dense_hh && t_opt.tc_gemm && ttc::tc_red_ok(B * (long long)lo.Tc, d->hidden_size, GH)));
             }
         }
         put("\n");
@@ -1293,18 +1318,12 @@ int64_t ttrnn_rnn_param_count(const ttrnn_rnn_desc *desc) {
 
 // byte sizes of ONE row group (the whole batch when the plan has a single group), under the calling thread's options
 static int workspace_one(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *ws) {
-    RnnPlan rp;
-    if (build_rnn_plan(desc, &rp)) return 1;
     DevInfo dv;
-    if (get_dev(&dv)) return 1;
-    EffDesc eff;
-    if (make_eff_desc(desc, &dv, &eff)) return 1;
-    if (eff.padded && build_rnn_plan(&eff.d, &rp)) return 1;
-    RnnLayout lo;
-    if (build_layout(&eff.d, rp, dv, &lo)) return 1;
-    ws->saved_bytes = lo.sv_total * 4;
-    ws->fwd_scratch_bytes = (lo.f_total + eff.pad_floats) * 4;             // + the rank-padded parameter blob
-    ws->bwd_scratch_bytes = (lo.b_total + 2 * eff.pad_floats) * 4;         // + padded parameters and padded gradients
+    CallPlan cp;
+    if (get_dev(&dv) || plan_call(desc, dv, &cp)) return 1;
+    ws->saved_bytes = cp.lo.sv_total * 4;
+    ws->fwd_scratch_bytes = (cp.lo.f_total + cp.eff.pad_floats) * 4;       // + the rank-padded parameter blob
+    ws->bwd_scratch_bytes = (cp.lo.b_total + 2 * cp.eff.pad_floats) * 4;   // + padded parameters and padded gradients
     return 0;
 }
 
@@ -1345,17 +1364,14 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
 static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
                        const float *c0, const float *params_in, float *out, float *hT, float *cT, void *saved, void *scratch,
                        void *stream) {
-    RnnPlan rp;
-    if (build_rnn_plan(d_in, &rp)) return 1;
     if (!x || !params_in || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     DevInfo dv;
-    if (get_dev(&dv)) return 1;
-    EffDesc eff;
-    if (make_eff_desc(d_in, &dv, &eff)) return 1;
-    const ttrnn_rnn_desc *d = &eff.d;
-    if (eff.padded && build_rnn_plan(d, &rp)) return 1;
-    RnnLayout lo;
-    if (build_layout(d, rp, dv, &lo)) return 1;
+    CallPlan cp;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp)) return 1;
+    const ttrnn_rnn_desc *d = cp.d();
+    const RnnPlan &rp = cp.rp;
+    const RnnLayout &lo = cp.lo;
+    const EffDesc &eff = cp.eff;
     if ((lo.f_total + eff.pad_floats) * 4 != ws->fwd_scratch_bytes || lo.sv_total * 4 != ws->saved_bytes)
         return fail("ttrnn_rnn_forward: workspace struct does not belong to this descriptor (scratch %lld vs %lld bytes)",
                     (long long)(lo.f_total + eff.pad_floats) * 4, (long long)ws->fwd_scratch_bytes);
@@ -1394,7 +1410,8 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
 
         // ---- batched ih projection of one time chunk: xg[b, t, :] = W_ih x[b, t0+t, :] + b_ih (+ b_hh for LSTM),
         // through the TT chain or, when that is the cheaper contraction order, through dense W_ih^T
-        const bool dense = dense_ih_ok(lp.ih, &d->ih[l]) && !(l == 0 && d->input_size == 1);
+        const int mode = layer_mode(d, l);
+        const bool dense = mode == tts::MODE_XG && dense_ih_ok(lp.ih, &d->ih[l]);
         DenseIh D;
         if (dense) {
             dense_carve(sc + lo.f_dense, lp.ih, false, &D);
@@ -1412,8 +1429,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
         };
 
         // ---- statically specialised kernel for this hh shape, if one is registered -------------------
-        const int mode = (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
-        const TtsRnnFwdEntry *se = t_opt.stat ? tts_find_rnn_fwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_fwd, merge_fwd()) : nullptr;
+        const TtsRnnFwdEntry *se = fwd_route(d, l, B, dv.sms);
         if (se) {
             int occ = 0;
             int rc = se->prepare(&occ);
@@ -1454,10 +1470,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                 sa.c_in = first ? c0 : st_c;
                 sa.out = lout + (long long)t0 * H; sa.out_bstride = (long long)T * H;
                 sa.c_save = csave ? csave + (long long)t0 * H : nullptr;
-                if (sv && lo.save_mode[l] == 1 && se->x0_floats == lo.x0f[l]) {
-                    sa.x0_save = sv + lo.sv_x0[l] + (long long)t0 * lo.x0f[l]; sa.x0_bstride = (long long)T * lo.x0f[l];
-                }
-                if (sv && lo.save_mode[l] != 0) {
+                if (sv && lo.kept[l]) {
                     sa.u_save = sv + lo.sv_u[l] + (long long)t0 * 4 * H;       sa.u_bstride = (long long)T * 4 * H;
                 }
                 sa.h_out = (last && l == L - 1 && hT) ? hT : st_h;
@@ -1537,38 +1550,32 @@ static SideCtx *side_ctx() {
 }
 
 // body of ttrnn_rnn_backward on the effective (possibly rank-padded) descriptor
-static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const RnnLayout &lo, const DevInfo &dv, const float *x,
-                             const float *h0, const float *c0, const float *params, const float *out, const void *saved,
-                             const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0,
-                             float *d_c0, void *scratch, cudaStream_t st);
+static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0, const float *c0, const float *params,
+                             const float *out, const void *saved, const float *d_out, const float *d_hT, const float *d_cT,
+                             float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, cudaStream_t st);
 
 static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
                         const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
                         const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
                         void *scratch, void *stream) {
-    RnnPlan rp;
-    if (build_rnn_plan(d_in, &rp)) return 1;
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     DevInfo dv;
-    if (get_dev(&dv)) return 1;
-    EffDesc eff;
-    if (make_eff_desc(d_in, &dv, &eff)) return 1;
-    const ttrnn_rnn_desc *d = &eff.d;
-    if (eff.padded && build_rnn_plan(d, &rp)) return 1;
-    RnnLayout lo;
-    if (build_layout(d, rp, dv, &lo)) return 1;
+    CallPlan cp;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp)) return 1;
+    const RnnLayout &lo = cp.lo;
+    const EffDesc &eff = cp.eff;
     if ((lo.b_total + 2 * eff.pad_floats) * 4 != ws->bwd_scratch_bytes || lo.sv_total * 4 != ws->saved_bytes)
         return fail("ttrnn_rnn_backward: workspace struct does not belong to this descriptor (scratch %lld vs %lld bytes)",
                     (long long)(lo.b_total + 2 * eff.pad_floats) * 4, (long long)ws->bwd_scratch_bytes);
     cudaStream_t st = (cudaStream_t)stream;
     if (!eff.padded)
-        return rnn_backward_impl(d, rp, lo, dv, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch, st);
+        return rnn_backward_impl(cp, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch, st);
     float *pp = (float *)scratch + lo.b_total, *dpp = pp + eff.pad_floats;
     CU_CHECK(cudaMemsetAsync(pp, 0, (size_t)eff.pad_floats * 4, st));
     k_pad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, params, pp);
     ++g_launches;
     CU_CHECK(cudaGetLastError());
-    if (rnn_backward_impl(d, rp, lo, dv, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st)) return 1;
+    if (rnn_backward_impl(cp, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st)) return 1;
     // the gradient wrt a real core is the matching block of the padded core's gradient
     k_unpad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, dpp, d_params);
     ++g_launches;
@@ -1576,10 +1583,13 @@ static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
     return 0;
 }
 
-static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const RnnLayout &lo, const DevInfo &dv, const float *x,
-                             const float *h0, const float *c0, const float *params, const float *out, const void *saved,
-                             const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0,
-                             float *d_c0, void *scratch, cudaStream_t st) {
+static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0, const float *c0, const float *params,
+                             const float *out, const void *saved, const float *d_out, const float *d_hT, const float *d_cT,
+                             float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, cudaStream_t st) {
+    const ttrnn_rnn_desc *d = cp.d();
+    const RnnPlan &rp = cp.rp;
+    const RnnLayout &lo = cp.lo;
+    const DevInfo &dv = cp.dv;
     const long long B = d->batch;
     const int T = d->seq_len, H = d->hidden_size, L = d->num_layers, G = rp.G;
     const int GH = G * H;
@@ -1624,7 +1634,8 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
         const float *b_hh = d->has_bias ? params + lp.off_hh_bias : nullptr;
 
         // ---- ih projection (recompute) and its backward per time chunk: TT chain or dense route ---------
-        const int mode = (l == 0 && d->input_size == 1 && !d_x) ? tts::MODE_RANK1 : tts::MODE_XG;
+        // a rank-one layer 0 whose input gradient is wanted runs the projected-input kernels (delta_ih feeds dX)
+        const int mode = d_x ? tts::MODE_XG : layer_mode(d, l);
         const bool dense = mode == tts::MODE_XG && dense_ih_bwd_ok(lp.ih, dlin != nullptr, &d->ih[l]);
         DenseIh D;
         if (dense) {
@@ -1674,48 +1685,22 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
 
         // ---- statically specialised BPTT kernel for this hh shape, if one is registered ---------------
         // per-step gradient logging is emitted by the runtime-shape BPTT kernel (it recomputes from hs / cs, which every
-        // training forward keeps, so it can follow a forward that ran on the static kernels)
+        // training forward keeps, so it can follow a forward that ran on the static kernels).  Where the forward kept the
+        // gate activations of this layer, the route prefers the kernels that consume them.
         const bool logging = t_log.dh != nullptr;
-        const TtsRnnBwdEntry *be = (t_opt.stat && !logging) ? tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, 0, 0, merge_bwd()) : nullptr;
-        if (t_opt.stat && !logging && lo.save_mode[l] != 0 && sv) {
-            // forward kept (X_0 and) the hh pre-activations of this layer: use the kernel that consumes them
-            if (const TtsRnnBwdEntry *bs = tts_find_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd,
-                                                            lo.save_mode[l], split_kept_ok(lp.hh, mode, lo.Tc, T), merge_bwd()))
-                be = bs;
-        }
-        // split variants behind a projected input take the hh bias gradient from the ih side (LSTM only); the rank-one
-        // variants keep every bias / W_ih-column gradient in the kernel's own slot and work for both cells
-        const bool split_r1 = be && be->split && mode == tts::MODE_RANK1;
-        if (be && be->split && !lstm && !split_r1)
-            return fail("internal: split BPTT variants with a projected input compute the hh bias gradient from the ih side "
-                        "(LSTM only); %s is registered for a GRU", be->name);
-        if (split_r1 && !dense_hh_dw_ok(lp.hh))
-            return fail("internal: rank-one split BPTT variant %s selected without the dense hh core-gradient route", be->name);
-        if (be) {
-            // row plan: one phase, or two when a tail variant beats a mostly idle last wave
-            const TtsRnnBwdEntry *ph_e[2] = {be, nullptr};
-            long long ph_row0[2] = {0, 0}, ph_rows[2] = {B, 0};
+        BwdRoute br;
+        if (!logging && bwd_route(d, rp, l, mode, B, dv.sms, lo.kept[l] && sv, lo.Tc, &br)) return 1;
+        if (br.nph) {
+            const bool split = br.split, split_r1 = br.split_r1, dense_hh = br.dense_hh;
             int ph_grid[2] = {0, 0};
-            int nph = 1;
-            if ((!be->split || be->saved == 2) && t_opt.row_plan) {
-                const TtsRnnBwdEntry *pe[2];
-                long long pr0[2], pr[2];
-                const int np = tts_plan_rnn_bwd(&d->hh[l], d->cell, mode, B, dv.sms, (int)t_opt.srows_bwd, be->saved,
-                                                be->split && be->saved == 2, merge_bwd(), pe, pr0, pr);
-                if (np >= 1) {
-                    nph = np;
-                    for (int q = 0; q < np; ++q) { ph_e[q] = pe[q]; ph_row0[q] = pr0[q]; ph_rows[q] = pr[q]; }
-                    be = ph_e[0];
-                }
-            }
             int rc = 0;
             int sgrid = 0;
-            for (int q = 0; q < nph; ++q) {
+            for (int q = 0; q < br.nph; ++q) {
                 int occ = 0;
-                rc = ph_e[q]->prepare(&occ);
-                if (rc || occ < 1) return fail("static kernel %s cannot be configured (cuda error %d)", ph_e[q]->name, rc);
+                rc = br.e[q]->prepare(&occ);
+                if (rc || occ < 1) return fail("static kernel %s cannot be configured (cuda error %d)", br.e[q]->name, rc);
                 long long g = (long long)occ * dv.sms;
-                const long long tiles = (ph_rows[q] + ph_e[q]->R - 1) / ph_e[q]->R;
+                const long long tiles = (br.rows[q] + br.e[q]->R - 1) / br.e[q]->R;
                 if (g > tiles) g = tiles;
                 if (g > lo.nslots) g = lo.nslots;
                 ph_grid[q] = (int)g;
@@ -1724,10 +1709,10 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
             // launch every phase of the plan on its rows (row-indexed pointers are offset; gradient slots are shared
             // and accumulated: the phases run back to back on the stream)
             auto launch_plan = [&](const tts::RnnBwdSArgs &base) -> int {
-                for (int q = 0; q < nph; ++q) {
+                for (int q = 0; q < br.nph; ++q) {
                     tts::RnnBwdSArgs a2 = base;
-                    const long long r0 = ph_row0[q];
-                    a2.B = ph_rows[q];
+                    const long long r0 = br.row0[q];
+                    a2.B = br.rows[q];
                     if (a2.xg) a2.xg += r0 * a2.xg_bstride;
                     if (a2.x1) a2.x1 += r0 * a2.x1_bstride;
                     if (a2.hs) a2.hs += r0 * (long long)T * H;
@@ -1739,38 +1724,35 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
                     if (a2.dc_in) a2.dc_in += r0 * H;
                     if (a2.dh_out) a2.dh_out += r0 * H;
                     if (a2.dc_out) a2.dc_out += r0 * H;
-                    if (a2.x0_save) a2.x0_save += r0 * a2.x0_bstride;
                     if (a2.u_save) a2.u_save += r0 * a2.u_bstride;
                     int e;
                     {
-                        KernelTimer tm(TTRNN_K_RNN_BWD, st, ph_e[q]->R, ph_grid[q], ph_rows[q], a2.steps);
-                        e = ph_e[q]->launch(&a2, ph_grid[q], st);
+                        KernelTimer tm(TTRNN_K_RNN_BWD, st, br.e[q]->R, ph_grid[q], br.rows[q], a2.steps);
+                        e = br.e[q]->launch(&a2, ph_grid[q], st);
                     }
                     ++g_launches;
-                    if (e) return fail("static kernel %s launch failed: %s", ph_e[q]->name, cudaGetErrorString((cudaError_t)e));
+                    if (e) return fail("static kernel %s launch failed: %s", br.e[q]->name, cudaGetErrorString((cudaError_t)e));
                 }
                 return 0;
             };
-            const long long slot = be->slot_floats;
+            const long long slot = br.e[0]->slot_floats;
             if (slot > lo.part_stride) return fail("internal: gradient slot too small");
             const long long ih_slot = lp.ih.core_floats + GH;
             const long long hhw_slot = lp.hh.core_floats + GH;       // slot layout of the batched hh-dW kernel (split mode)
             int hh_used = 0;
-            CU_CHECK(cudaMemsetAsync(part_hh, 0, (size_t)((be->split && !split_r1) ? hhw_slot * lo.nslots : slot * sgrid) * 4, st));
+            CU_CHECK(cudaMemsetAsync(part_hh, 0, (size_t)((split && !split_r1) ? hhw_slot * lo.nslots : slot * sgrid) * 4, st));
             CU_CHECK(cudaMemsetAsync(part_ih, 0, (size_t)ih_slot * lo.nslots * 4, st));
             tts::RnnBwdSArgs sa;
             memset(&sa, 0, sizeof sa);
             sa.B = B; sa.T = T;
             sa.cores = params + lp.off_hh_cores;
             sa.hs = lout; sa.cs = lcs; sa.h0 = h0; sa.c0 = c0; sa.dhs = dhs;
-            sa.partial = (be->split && !split_r1) ? nullptr : part_hh;
-            if (be->saved == 1) { sa.x0_save = sv + lo.sv_x0[l]; sa.x0_bstride = (long long)T * lo.x0f[l]; }
-            if (be->saved != 0) { sa.u_save = sv + lo.sv_u[l];   sa.u_bstride = (long long)T * 4 * H; }
+            sa.partial = (split && !split_r1) ? nullptr : part_hh;
+            if (br.kept) { sa.u_save = sv + lo.sv_u[l]; sa.u_bstride = (long long)T * 4 * H; }
             float *aux = ss + lo.b_aux;
             float *aux_g = aux + r4(GH);
             float *one = aux_g + r4(GH);
             int ih_used = 0;
-            const bool dense_hh = be->split && dense_hh_dw_ok(lp.hh);
             DenseIh DH;
             int hh_dense_calls = 0;
             if (dense_hh) {
@@ -1812,17 +1794,16 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
                     const bool last = (t0 + tc == T);
                     // the kept-gates kernels take the gate activations from the forward pass and only WRITE delta_ih
                     // into xg: recomputing the ih projection of the chunk would be wasted work
-                    if (be->saved == 0 && project(t0, tc)) return 1;
+                    if (!br.kept && project(t0, tc)) return 1;
                     sa.t0 = t0; sa.steps = tc;
                     sa.xg = xg; sa.xg_bstride = (long long)tc * GH;
                     sa.dh_in = last ? (l == L - 1 ? d_hT : nullptr) : sdh;
                     sa.dc_in = last ? (l == L - 1 ? d_cT : nullptr) : sdc;
                     sa.dh_out = sdh; sa.dc_out = sdc;
                     if (launch_plan(sa)) return 1;
-                    // bwd_overlap = 1: fork only when this layer's BPTT grid leaves >= 24 SMs idle; 2: always (the deferred
-                    // GEMMs then fill whatever the recurrent kernels of BOTH row groups leave idle)
+                    // bwd_overlap: fork only when this layer's BPTT grid leaves >= 24 SMs idle
                     const int idle_sms = dv.sms - sgrid;
-                    if (side && l > 0 && nchunks == 1 && dense && dlin && (idle_sms >= 24 || t_opt.bwd_overlap >= 2)) {
+                    if (side && l > 0 && nchunks == 1 && dense && dlin && idle_sms >= 24) {
                         // overlap: dX (the next layer's input) first, then everything that only produces parameter gradients
                         // moves to the side stream, planned for the SMs the next BPTT kernel leaves idle
                         if (project_dx(t0, tc)) return 1;
@@ -1831,9 +1812,9 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
                         CU_CHECK(cudaStreamWaitEvent(side->s, side->fork, 0));
                         ws = side->s;
                         join.used = true;
-                        dvw.sms = idle_sms >= 24 ? idle_sms : 48;
+                        dvw.sms = idle_sms;
                     }
-                    if (be->split) {
+                    if (split) {
                         // hh core gradients over rows (h_{t-1}, delta_t) of this chunk: dense accumulation of
                         // dW_hh^T = H_prev^T delta (projected onto the cores after the last chunk), or a batched
                         // TT-matvec backward (second chain pass) when the dense order is disabled / does not fit
@@ -1890,7 +1871,7 @@ static int rnn_backward_impl(const ttrnn_rnn_desc *d, const RnnPlan &rp, const R
                                         lo.nslots, ss + lo.b_spill, 0, ws, &ih_used))
                     return 1;
                 if (reduce_partials(part_ih, ih_used, ih_slot, 0, lp.ih.core_floats, d_params + lp.off_ih_cores, ws)) return 1;
-            } else if (be->split) {
+            } else if (split) {
                 if (reduce_partials(part_hh, hh_used, hhw_slot, 0, (int)cf, d_params + lp.off_hh_cores, ws)) return 1;
             } else if (reduce_partials(part_hh, sgrid, slot, 0, (int)cf, d_params + lp.off_hh_cores, ws)) {
                 return 1;
@@ -2147,18 +2128,12 @@ int ttrnn_rnn_saved_layout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace
     if (!ws || !plan_load(ws->plan, &t_opt)) return fail("ttrnn_rnn_saved_layout: `ws` must come from ttrnn_rnn_workspace_bytes()");
     if (ws->plan[kPlanGroups] > 1) return fail("ttrnn_rnn_saved_layout needs a whole-batch plan (TTRNN_WS_WHOLE_BATCH)");
     if (!hs_off || !cs_off) return fail("hs_off and cs_off must be non-null");
-    RnnPlan rp;
-    if (build_rnn_plan(d_in, &rp)) return 1;
-    if (layer < 0 || layer >= d_in->num_layers) return fail("layer %d out of range", layer);
     DevInfo dv;
-    if (get_dev(&dv)) return 1;
-    EffDesc eff;
-    if (make_eff_desc(d_in, &dv, &eff)) return 1;
-    if (eff.padded && build_rnn_plan(&eff.d, &rp)) return 1;
-    RnnLayout lo;
-    if (build_layout(&eff.d, rp, dv, &lo)) return 1;
-    *hs_off = (layer == d_in->num_layers - 1) ? -1 : lo.sv_hs + (long long)layer * lo.BTH;
-    *cs_off = (d_in->cell == TTRNN_CELL_LSTM) ? lo.sv_cs + (long long)layer * lo.BTH : -1;
+    CallPlan cp;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp)) return 1;
+    if (layer < 0 || layer >= d_in->num_layers) return fail("layer %d out of range", layer);
+    *hs_off = (layer == d_in->num_layers - 1) ? -1 : cp.lo.sv_hs + (long long)layer * cp.lo.BTH;
+    *cs_off = (d_in->cell == TTRNN_CELL_LSTM) ? cp.lo.sv_cs + (long long)layer * cp.lo.BTH : -1;
     return 0;
 }
 

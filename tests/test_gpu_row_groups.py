@@ -156,3 +156,79 @@ def test_options_changed_between_forward_and_backward_do_not_move_the_split():
         torch.cuda.synchronize()
     assert rel_err(h, h_ref) <= FWD_TOL
     assert_grads([p.grad for p in m.flat_parameters()], g_ref)
+
+
+def recorded_recurrent_launches(m, x):
+    """(kind, rows per CTA, CTAs, rows) of every recurrent-kernel launch of one forward + backward step, in issue order
+    (kernel timing runs the row groups back to back on one stream)."""
+    lib = _lib.load()
+    kms, kcnt = (ctypes.c_double * 7)(), (ctypes.c_int64 * 7)()
+    lib.ttrnn_kernel_times(kms, kcnt)
+    lib.ttrnn_kernel_timing(1)
+    try:
+        m(x)[0].sum().backward()
+        torch.cuda.synchronize()
+    finally:
+        lib.ttrnn_kernel_timing(0)
+    lib.ttrnn_kernel_times(kms, kcnt)
+    n = lib.ttrnn_kernel_launch_records(None, 0)
+    buf = (ctypes.c_double * (6 * max(n, 1)))()
+    lib.ttrnn_kernel_launch_records(buf, n)
+    recs = [tuple(int(buf[6 * i + j]) for j in range(4)) for i in range(n)]
+    return [r for r in recs if r[0] in (1, 2)]
+
+
+def described_launches(plan, rows):
+    """(kind, rows per CTA, rows) of the forward and backward recurrent launches that a describe_plan() result of a call
+    on `rows` rows names."""
+    fwd = [(1, lay["fwd_rows"], rows) for lay in plan[1:]]
+    bwd = []
+    for lay in reversed(plan[1:]):
+        bwd.append((2, lay["bwd_rows"], lay["bwd_phase_rows"]))
+        if "bwd_rows2" in lay:
+            bwd.append((2, lay["bwd_rows2"], lay["bwd_phase_rows2"]))
+    return fwd, bwd
+
+
+DESCRIBED = [
+    # name, cell, I, H, L, d, r, B, T, options
+    ("cfg3_shape_640_rows", "lstm", 40, 256, 3, 3, 8, 640, 6, {}),
+    ("cfg3_shape_640_rows_one_group", "lstm", 40, 256, 3, 3, 8, 640, 6, {"row_groups": 0}),
+    ("cfg1_shape_256_rows", "lstm", 1, 256, 1, 2, 4, 256, 12, {}),
+]
+
+
+@pytest.mark.parametrize("case", DESCRIBED, ids=[c[0] for c in DESCRIBED])
+def test_describe_matches_the_recorded_launches(case):
+    """describe_plan() is what the tests and the benchmark read the kernel routes from: the recurrent launches of one
+    training step must be the ones it names, per row group (rows per CTA, rows per launch, two-phase backward row plans,
+    the CTAs of group 1), in issue order."""
+    name, cell, I, H, L, d, r, B, T, extra = case
+    _, m = make_pair(cell, I, H, L, d, r)
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    x = torch.rand(B, T, I, generator=torch.Generator().manual_seed(5)).to(DEV)
+    with options(**extra):
+        plan = _lib.describe_plan(m.spec().desc(B, T), training=True)
+        head = plan[0]
+        groups = [head["group_rows0"], head["group_rows1"]] if head["row_groups"] == 2 else [B]
+        plans = [plan]
+        if len(groups) == 2:
+            with options(row_groups=0):                    # group 1 runs the single-group routes of its own rows
+                plans.append(_lib.describe_plan(m.spec().desc(groups[1], T), training=True))
+        recs = recorded_recurrent_launches(m, x)
+    if name == "cfg3_shape_640_rows" and sms == 148:
+        assert groups == [444, 196], head
+    if name == "cfg1_shape_256_rows":
+        assert plan[1]["ih_route"] == "rank_one" and "split" in plan[1]["bwd_kernel"], plan[1]
+    fwd, bwd = [], []
+    for rows, p in zip(groups, plans):
+        f, b = described_launches(p, rows)
+        fwd += f
+        bwd += b
+    assert [rc[:2] + rc[3:] for rc in recs] == fwd + bwd, (plans, recs)
+    for kind, R, ctas, rows in recs:
+        tiles = -(-rows // R)
+        assert ctas == tiles if tiles <= sms else sms <= ctas <= tiles, (kind, R, ctas, rows)
+    if len(groups) == 2:
+        g1_fwd, g1_bwd = recs[2 * L - 1], recs[2 * L + len(described_launches(plans[0], groups[0])[1])]
+        assert (g1_fwd[2], g1_bwd[2]) == (head["group1_fwd_ctas"], head["group1_bwd_ctas"]), (head, recs)

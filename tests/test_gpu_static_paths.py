@@ -111,9 +111,8 @@ def test_static_kernels_match_oracle(case):
 
 
 def test_saved_activation_backward_matches_recompute():
-    """Three backward variants of the static BPTT kernel must agree: full recompute (both budgets 0), kept
-    hh pre-activations only (`save_u_bytes`, the default: backward skips the final stage of the recompute) and
-    kept X_0 + pre-activations (`save_bytes`, two-core chains)."""
+    """Two backward variants of the static BPTT kernel must agree: full recompute (`save_u_bytes` 0) and kept
+    gate activations (`save_u_bytes`, the default: backward skips the final stage of the recompute)."""
     dev = torch.device("cuda:0")
     lib = _lib.load()
     cases = [("gru", tr.TTGRU, 1, 256, 1, 2, 4), ("lstm", tr.TTLSTM, 1, 256, 1, 2, 4), ("lstm", tr.TTLSTM, 40, 256, 2, 3, 8)]
@@ -122,8 +121,7 @@ def test_saved_activation_backward_matches_recompute():
         m = quiet(cls, I, H, L, torch.device("cpu"), n_cores=d, tt_rank=r).to(dev)
         x = torch.rand(19, 23, I, device=dev)
         res = []
-        for save_all, save_u in ((0, 0), (0, 1 << 30), (1 << 30, 0)):
-            lib.ttrnn_set_option(b"save_bytes", save_all)
+        for save_u in (0, 1 << 30):
             lib.ttrnn_set_option(b"save_u_bytes", save_u)
             try:
                 for p in m.parameters():
@@ -134,7 +132,6 @@ def test_saved_activation_backward_matches_recompute():
                 (out.sum() + 3 * h.sum()).backward()
                 res.append((out.detach().clone(), [p.grad.clone() for p in m.parameters()]))
             finally:
-                lib.ttrnn_set_option(b"save_bytes", 0)
                 lib.ttrnn_set_option(b"save_u_bytes", 16 << 30)
         for other in res[1:]:
             assert torch.equal(res[0][0], other[0])

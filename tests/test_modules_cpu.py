@@ -274,6 +274,7 @@ def test_ih_route_selection_is_host_logic():
     finally:
         lib.ttrnn_set_option(b"dense_ih", 1)
     assert lib.ttrnn_set_option(b"no_such_option", 1) != 0
+    assert lib.ttrnn_set_option(b"save_bytes", 1) != 0
 
 
 def test_header_is_valid_c_and_matches_the_binding():
