@@ -32,7 +32,9 @@ extern "C" {
 #define TTRNN_ABI_VERSION 4   /* 2: + cell step, ih route query, static kernel table; 3: execution plan carried by
                                  ttrnn_rnn_workspace, GEMM probe, GE2E head, dense cells; 4: row groups in the plan
                                  (ttrnn_rnn_row_groups, ttrnn_rnn_workspace_bytes_ex), per-step logging entry points,
-                                 per-launch timing records -- additive: every ABI 3 signature is unchanged */
+                                 per-launch timing records -- additive: every ABI 3 signature is unchanged.  Still 4 with
+                                 per-layer states: one more flag value (TTRNN_WS_LAYER_STATES) and two new symbols
+                                 (ttrnn_dense_rnn_forward_ex / _backward_ex); no existing signature or default changes */
 #define TTRNN_MAX_CORES   6
 #define TTRNN_MAX_LAYERS  8
 
@@ -94,13 +96,20 @@ const char *ttrnn_last_error(void);            /* thread-local, never NULL */
 int64_t ttrnn_rnn_param_count(const ttrnn_rnn_desc *desc);
 
 int ttrnn_rnn_workspace_bytes(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *ws);
-/* The same with flags.  TTRNN_WS_WHOLE_BATCH: plan one row group, so that every layer's h_t / c_t sequence is one
- * (B,T,H) block of `saved` (required by ttrnn_rnn_saved_layout / ttrnn_rnn_backward_logged). */
+/* The same with flags (they combine).  TTRNN_WS_WHOLE_BATCH: plan one row group, so that every layer's h_t / c_t
+ * sequence is one (B,T,H) block of `saved` (required by ttrnn_rnn_saved_layout / ttrnn_rnn_backward_logged).
+ * TTRNN_WS_LAYER_STATES: the forward / backward calls that run from this plan take PER-LAYER states, the contract of
+ * torch.nn.LSTM: h0, c0, hT, cT, d_hT, d_cT, d_h0 and d_c0 are (L, B, H), layer l's block starting at l * B * H.  Each
+ * may be NULL (an input state NULL = zeros).  Layer l starts from its own (h0, c0), returns its own (h_T, c_T), the
+ * upstream d_hT / d_cT of layer l enters that layer's BPTT at its last step, and d_h0 / d_c0 receive each layer's own
+ * gradient (not summed).  With it a stack can run one sequence in pieces: the final states of one call are the initial
+ * states of the next.  The flag changes no kernel route, buffer size or result of the shared-state contract. */
 #define TTRNN_WS_WHOLE_BATCH 1
+#define TTRNN_WS_LAYER_STATES 2
 int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrnn_rnn_workspace *ws);
 
 /* Forward over the whole stack.  h0 / c0 may be NULL (zeros); one (h0, c0) seeds
- * every layer (lstm.py:120-121).  c0 / cT / d_c* are ignored for GRU.
+ * every layer (lstm.py:120-121) unless the plan carries TTRNN_WS_LAYER_STATES (see above).  c0 / cT / d_c* are ignored for GRU.
  * `ws` = the struct ttrnn_rnn_workspace_bytes() filled for this desc (sizes + execution plan).
  * `saved` NULL = inference (nothing kept for backward).  Returns outputs of the
  * last layer for every t, and (h_T, c_T) of the last layer (lstm.py:135). */
@@ -113,7 +122,7 @@ int ttrnn_rnn_forward(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
  * (SURVEY.md section 8a-10).  d_out (B,T,H), d_hT, d_cT: upstream gradients (any may be
  * NULL = zero).  d_params is OVERWRITTEN with the gradient blob.  d_x (B,T,I) may
  * be NULL.  d_h0 / d_c0 (B,H) may be NULL; they receive the SUM over layers
- * because every layer shares the same initial state. */
+ * because every layer shares the same initial state (per layer under TTRNN_WS_LAYER_STATES). */
 int ttrnn_rnn_backward(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
                        const float *x, const float *h0, const float *c0,
                        const float *params, const float *out, const void *saved,
@@ -195,6 +204,16 @@ int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *desc, const float *x, const
                              const float *d_out, const float *d_hT, const float *d_cT,
                              float *d_params, float *d_x, float *d_h0, float *d_c0,
                              void *scratch, void *stream);
+/* The same with flags: TTRNN_WS_LAYER_STATES makes every state buffer (L, B, H), as for ttrnn_rnn_forward.  Pass the same
+ * flags to a forward and its backward.  (Under that flag d_h0 / d_c0 of a layer are written where its h0 / c0 is given.) */
+int ttrnn_dense_rnn_forward_ex(const ttrnn_dense_desc *desc, const float *x, const float *h0, const float *c0,
+                               const float *params, float *out, float *hT, float *cT,
+                               void *saved, void *scratch, void *stream, int32_t flags);
+int ttrnn_dense_rnn_backward_ex(const ttrnn_dense_desc *desc, const float *x, const float *h0, const float *c0,
+                                const float *params, const float *out, void *saved,
+                                const float *d_out, const float *d_hT, const float *d_cT,
+                                float *d_params, float *d_x, float *d_h0, float *d_c0,
+                                void *scratch, void *stream, int32_t flags);
 
 /* GE2E head on the device (SURVEY.md 8f-4): the part of the speaker-encoder training step the reference runs on the CPU
  * after every RNN pass (experiments/speaker_verification/encoder/main.py:279-280 moves the embeddings to `loss_device`).

@@ -15,6 +15,7 @@ MAX_CORES = 6
 MAX_LAYERS = 8
 PLAN_WORDS = 24
 WS_WHOLE_BATCH = 1
+WS_LAYER_STATES = 2      # per-layer (L, B, H) initial / final states and their gradients
 CELL_LSTM, CELL_GRU = 0, 1
 
 _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc", "libttrnn_b200.so")
@@ -71,6 +72,8 @@ SYMBOLS = {
     "ttrnn_dense_rnn_workspace_bytes": (C.c_int, [C.POINTER(DenseDesc), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "ttrnn_dense_rnn_forward": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 10),
     "ttrnn_dense_rnn_backward": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 15),
+    "ttrnn_dense_rnn_forward_ex": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 10 + [C.c_int32]),
+    "ttrnn_dense_rnn_backward_ex": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 15 + [C.c_int32]),
     "ttrnn_embed_forward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 4),
     "ttrnn_embed_backward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 6),
     "ttrnn_ge2e_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),

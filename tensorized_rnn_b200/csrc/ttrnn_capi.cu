@@ -77,9 +77,10 @@ struct Opts {
 };
 constexpr int kOptFields = sizeof(Opts) / sizeof(long long);
 constexpr long long kPlanMagic = 0x7474726E6E706C36LL;          // "ttrnnpl6"
-// plan words: [0] magic, [1 .. kOptFields] options, then the row-group split (group count, rows of group 0)
-constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2;
-static_assert(kOptFields + 3 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
+// plan words: [0] magic, [1 .. kOptFields] options, then the row-group split (group count, rows of group 0), then 1 when
+// the state buffers are per layer (TTRNN_WS_LAYER_STATES)
+constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2, kPlanLayerStates = kOptFields + 3;
+static_assert(kOptFields + 4 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
 thread_local Opts t_opt;
 inline int merge_fwd() { return t_opt.merge_cores >= 2 ? 1 : 0; }    // contracted forward variants (merge_cores = 2)
 inline int merge_bwd() { return t_opt.merge_cores >= 1 ? 1 : 0; }    // contracted dX-only BPTT variants (merge_cores >= 1)
@@ -174,6 +175,20 @@ int get_dev(DevInfo *d) {
     d->ok = true;
     return 0;
 }
+
+// Where layer l's initial state, final state and their gradients live.  stride 0 is the reference's contract
+// (lstm.py:120-121,135): one (B, H) block seeds every layer, only the last layer's final state comes back and takes an
+// upstream gradient, and d_h0 / d_c0 receive the sum over layers.  stride > 0 (TTRNN_WS_LAYER_STATES): every state buffer
+// is (L, B, H) and layer l's block starts l * stride floats in.  The stride is the FULL batch's B * H, also inside a row
+// group, whose pointers the entry points have already moved to the group's first row.
+struct StateMap {
+    long long stride = 0;
+    template <class P> P init(P p, int l) const { return (p && stride) ? p + l * stride : p; }               // h0, c0, d_h0, d_c0
+    template <class P> P fin(P p, int l, int L) const {                                                       // hT, cT, d_hT, d_cT
+        if (stride) return p ? p + l * stride : p;
+        return l == L - 1 ? p : nullptr;
+    }
+};
 
 inline int gates_of(int cell) { return cell == TTRNN_CELL_LSTM ? 4 : 3; }
 inline long long r4(long long v) { return (v + 3) & ~3LL; }
@@ -1357,13 +1372,14 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
     plan_store(t_opt, ws->plan);
     ws->plan[kPlanGroups] = gp.n;
     ws->plan[kPlanRows0] = gp.rows[0];
+    ws->plan[kPlanLayerStates] = (flags & TTRNN_WS_LAYER_STATES) ? 1 : 0;
     return 0;
 }
 
 // forward of ONE row group on stream `stream`; `ws` carries the byte sizes of this group, t_opt is already loaded
-static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
-                       const float *c0, const float *params_in, float *out, float *hT, float *cT, void *saved, void *scratch,
-                       void *stream) {
+static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
+                       const float *h0, const float *c0, const float *params_in, float *out, float *hT, float *cT, void *saved,
+                       void *scratch, void *stream) {
     if (!x || !params_in || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     DevInfo dv;
     CallPlan cp;
@@ -1407,6 +1423,9 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
         float *csave = (sv && lstm) ? sv + lo.sv_cs + (long long)l * lo.BTH : nullptr;
         const float *b_ih = d->has_bias ? params + lp.off_ih_bias : nullptr;
         const float *b_hh = d->has_bias ? params + lp.off_hh_bias : nullptr;
+        // this layer's initial state, read by its first chunk, and where its last chunk leaves the final state
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
+        float *hTl = sm.fin(hT, l, L), *cTl = sm.fin(cT, l, L);
 
         // ---- batched ih projection of one time chunk: xg[b, t, :] = W_ih x[b, t0+t, :] + b_ih (+ b_hh for LSTM),
         // through the TT chain or, when that is the cheaper contraction order, through dense W_ih^T
@@ -1466,15 +1485,15 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                 }
                 const bool first = (t0 == 0), last = (t0 + tc == T);
                 sa.steps = tc;
-                sa.h_in = first ? h0 : st_h;
-                sa.c_in = first ? c0 : st_c;
+                sa.h_in = first ? h0l : st_h;
+                sa.c_in = first ? c0l : st_c;
                 sa.out = lout + (long long)t0 * H; sa.out_bstride = (long long)T * H;
                 sa.c_save = csave ? csave + (long long)t0 * H : nullptr;
                 if (sv && lo.kept[l]) {
                     sa.u_save = sv + lo.sv_u[l] + (long long)t0 * 4 * H;       sa.u_bstride = (long long)T * 4 * H;
                 }
-                sa.h_out = (last && l == L - 1 && hT) ? hT : st_h;
-                sa.c_out = (last && l == L - 1 && cT) ? cT : st_c;
+                sa.h_out = (last && hTl) ? hTl : st_h;
+                sa.c_out = (last && cTl) ? cTl : st_c;
                 {
                     KernelTimer tm(TTRNN_K_RNN_FWD, st, se->R, (int)g, B, tc);
                     rc = se->launch(&sa, (int)g, st);
@@ -1510,12 +1529,12 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
             const bool first = (t0 == 0), last = (t0 + tc == T);
             a.steps = tc;
             a.xg = xg; a.xg_bstride = (long long)tc * GH;
-            a.h_in = first ? h0 : st_h;
-            a.c_in = first ? c0 : st_c;
+            a.h_in = first ? h0l : st_h;
+            a.c_in = first ? c0l : st_c;
             a.out = lout + (long long)t0 * H; a.out_bstride = (long long)T * H;
             a.c_save = csave ? csave + (long long)t0 * H : nullptr;
-            a.h_out = (last && l == L - 1 && hT) ? hT : st_h;
-            a.c_out = (last && l == L - 1 && cT) ? cT : st_c;
+            a.h_out = (last && hTl) ? hTl : st_h;
+            a.c_out = (last && cTl) ? cTl : st_c;
             {
                 KernelTimer tm(TTRNN_K_RNN_FWD, st, R, grid, B, tc);
                 k_rnn_fwd<<<grid, TT_NTHREADS, smem, st>>>(a);
@@ -1550,14 +1569,15 @@ static SideCtx *side_ctx() {
 }
 
 // body of ttrnn_rnn_backward on the effective (possibly rank-padded) descriptor
-static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0, const float *c0, const float *params,
-                             const float *out, const void *saved, const float *d_out, const float *d_hT, const float *d_cT,
-                             float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, cudaStream_t st);
+static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float *x, const float *h0, const float *c0,
+                             const float *params, const float *out, const void *saved, const float *d_out, const float *d_hT,
+                             const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch,
+                             cudaStream_t st);
 
-static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
-                        const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
-                        const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
-                        void *scratch, void *stream) {
+static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
+                        const float *h0, const float *c0, const float *params, const float *out, const void *saved,
+                        const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0,
+                        float *d_c0, void *scratch, void *stream) {
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     DevInfo dv;
     CallPlan cp;
@@ -1569,13 +1589,14 @@ static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
                     (long long)(lo.b_total + 2 * eff.pad_floats) * 4, (long long)ws->bwd_scratch_bytes);
     cudaStream_t st = (cudaStream_t)stream;
     if (!eff.padded)
-        return rnn_backward_impl(cp, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch, st);
+        return rnn_backward_impl(cp, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
+                                 st);
     float *pp = (float *)scratch + lo.b_total, *dpp = pp + eff.pad_floats;
     CU_CHECK(cudaMemsetAsync(pp, 0, (size_t)eff.pad_floats * 4, st));
     k_pad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, params, pp);
     ++g_launches;
     CU_CHECK(cudaGetLastError());
-    if (rnn_backward_impl(cp, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st)) return 1;
+    if (rnn_backward_impl(cp, sm, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st)) return 1;
     // the gradient wrt a real core is the matching block of the padded core's gradient
     k_unpad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, dpp, d_params);
     ++g_launches;
@@ -1583,9 +1604,10 @@ static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
     return 0;
 }
 
-static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0, const float *c0, const float *params,
-                             const float *out, const void *saved, const float *d_out, const float *d_hT, const float *d_cT,
-                             float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, cudaStream_t st) {
+static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float *x, const float *h0, const float *c0,
+                             const float *params, const float *out, const void *saved, const float *d_out, const float *d_hT,
+                             const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch,
+                             cudaStream_t st) {
     const ttrnn_rnn_desc *d = cp.d();
     const RnnPlan &rp = cp.rp;
     const RnnLayout &lo = cp.lo;
@@ -1632,6 +1654,9 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
         float *dlin = (l == 0) ? d_x : sc + lo.b_dhs + (l & 1) * r4(lo.BTH);
         const float *b_ih = d->has_bias ? params + lp.off_ih_bias : nullptr;
         const float *b_hh = d->has_bias ? params + lp.off_hh_bias : nullptr;
+        // this layer's initial state and the upstream gradient of its final state (enters its last step)
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
+        const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L);
 
         // ---- ih projection (recompute) and its backward per time chunk: TT chain or dense route ---------
         // a rank-one layer 0 whose input gradient is wanted runs the projected-input kernels (delta_ih feeds dX)
@@ -1746,7 +1771,7 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
             memset(&sa, 0, sizeof sa);
             sa.B = B; sa.T = T;
             sa.cores = params + lp.off_hh_cores;
-            sa.hs = lout; sa.cs = lcs; sa.h0 = h0; sa.c0 = c0; sa.dhs = dhs;
+            sa.hs = lout; sa.cs = lcs; sa.h0 = h0l; sa.c0 = c0l; sa.dhs = dhs;
             sa.partial = (split && !split_r1) ? nullptr : part_hh;
             if (br.kept) { sa.u_save = sv + lo.sv_u[l]; sa.u_bstride = (long long)T * 4 * H; }
             float *aux = ss + lo.b_aux;
@@ -1770,8 +1795,8 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
                 sa.x1 = lin; sa.x1_bstride = T;
                 sa.t0 = 0; sa.steps = T;
                 if (split_r1) { sa.xg = xg; sa.xg_bstride = (long long)T * GH; }      // delta_hh of every step
-                sa.dh_in = (l == L - 1) ? d_hT : nullptr;
-                sa.dc_in = (l == L - 1) ? d_cT : nullptr;
+                sa.dh_in = dhTl;
+                sa.dc_in = dcTl;
                 sa.dh_out = sdh; sa.dc_out = sdc;
                 if (launch_plan(sa)) return 1;
                 if (split_r1) {
@@ -1783,7 +1808,7 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
                         return 0;
                     };
                     if (T > 1 && hh_dw1(lout, (long long)T * H, xg + GH, B * (T - 1), T - 1)) return 1;
-                    if (h0 && hh_dw1(h0, H, xg, B, 1)) return 1;
+                    if (h0l && hh_dw1(h0l, H, xg, B, 1)) return 1;
                 }
             } else {
                 sa.bias_hh = lstm ? nullptr : b_hh;
@@ -1797,8 +1822,8 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
                     if (!br.kept && project(t0, tc)) return 1;
                     sa.t0 = t0; sa.steps = tc;
                     sa.xg = xg; sa.xg_bstride = (long long)tc * GH;
-                    sa.dh_in = last ? (l == L - 1 ? d_hT : nullptr) : sdh;
-                    sa.dc_in = last ? (l == L - 1 ? d_cT : nullptr) : sdc;
+                    sa.dh_in = last ? dhTl : sdh;
+                    sa.dc_in = last ? dcTl : sdc;
                     sa.dh_out = sdh; sa.dc_out = sdc;
                     if (launch_plan(sa)) return 1;
                     // bwd_overlap: fork only when this layer's BPTT grid leaves >= 24 SMs idle
@@ -1834,7 +1859,7 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
                             if (hh_dw(lout + (long long)(t0 - 1) * H, (long long)T * H, xg, B * tc, tc)) return 1;
                         } else {
                             if (tc > 1 && hh_dw(lout, (long long)T * H, xg + GH, B * (tc - 1), tc - 1)) return 1;
-                            if (h0 && hh_dw(h0, H, xg, B, 1)) return 1;
+                            if (h0l && hh_dw(h0l, H, xg, B, 1)) return 1;
                         }
                     }
                     if (project_bwd(t0, tc, &ih_used)) return 1;
@@ -1908,8 +1933,8 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
                 CU_CHECK(cudaEventRecord(side->done[set], ws));
                 set_busy[set] = true;
             }
-            if (d_h0 && axpy1(sdh, d_h0, lo.BH, l != L - 1, st)) return 1;
-            if (lstm && d_c0 && axpy1(sdc, d_c0, lo.BH, l != L - 1, st)) return 1;
+            if (d_h0 && axpy1(sdh, sm.init(d_h0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
+            if (lstm && d_c0 && axpy1(sdc, sm.init(d_c0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
             continue;
         }
 
@@ -1925,7 +1950,7 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
         a.cell = d->cell; a.H = H; a.G = G; a.B = B; a.T = T;
         a.cores = params + lp.off_hh_cores;
         a.bias_hh = lstm ? nullptr : b_hh;
-        a.hs = lout; a.cs = lcs; a.h0 = h0; a.c0 = c0; a.dhs = dhs;
+        a.hs = lout; a.cs = lcs; a.h0 = h0l; a.c0 = c0l; a.dhs = dhs;
         if (logging) {
             a.dh_log = t_log.dh + (long long)l * t_log.layer_stride;
             a.dc_log = (lstm && t_log.dc) ? t_log.dc + (long long)l * t_log.layer_stride : nullptr;
@@ -1951,8 +1976,8 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
             // (2) reverse-time recurrence: xg <- delta_ih, hh core grads, dh/dc carried across chunks
             a.t0 = t0; a.steps = tc;
             a.xg = xg; a.xg_bstride = (long long)tc * GH;
-            a.dh_in = last ? (l == L - 1 ? d_hT : nullptr) : sdh;
-            a.dc_in = last ? (l == L - 1 ? d_cT : nullptr) : sdc;
+            a.dh_in = last ? dhTl : sdh;
+            a.dc_in = last ? dcTl : sdc;
             a.dh_out = sdh; a.dc_out = sdc;
             {
                 KernelTimer tm(TTRNN_K_RNN_BWD, st, R, grid, B, tc);
@@ -1979,11 +2004,19 @@ static int rnn_backward_impl(const CallPlan &cp, const float *x, const float *h0
                 if (reduce_partials(part_hh, grid, hh_slot, lp.hh.core_floats, GH, d_params + lp.off_hh_bias, st)) return 1;
             }
         }
-        // (5) gradient wrt the shared initial state: sum over layers
-        if (d_h0 && axpy1(sdh, d_h0, lo.BH, l != L - 1, st)) return 1;
-        if (lstm && d_c0 && axpy1(sdc, d_c0, lo.BH, l != L - 1, st)) return 1;
+        // (5) gradient wrt the initial state: this layer's own block, or the sum over layers when the state is shared
+        if (d_h0 && axpy1(sdh, sm.init(d_h0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
+        if (lstm && d_c0 && axpy1(sdc, sm.init(d_c0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
     }
     return 0;
+}
+
+// per-layer state buffers (TTRNN_WS_LAYER_STATES in the plan) are strided by the full batch's B * H, so that a row group
+// reaches layer l's rows from a pointer moved to its first row
+static StateMap state_map(const ttrnn_rnn_desc *d_full, const ttrnn_rnn_workspace *ws) {
+    StateMap sm;
+    if (ws->plan[kPlanLayerStates]) sm.stride = (long long)d_full->batch * d_full->hidden_size;
+    return sm;
 }
 
 // ---- public entry points: one call of the single-group path per row group ---------------------------------------
@@ -2031,7 +2064,9 @@ int ttrnn_rnn_forward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws,
                       void *stream) {
     if (!ws || !plan_load(ws->plan, &t_opt))
         return fail("ttrnn_rnn_forward: `ws` must be the struct filled by ttrnn_rnn_workspace_bytes() for this descriptor");
-    if (ws->plan[kPlanGroups] <= 1) return forward_one(d_in, ws, x, h0, c0, params, out, hT, cT, saved, scratch, stream);
+    if (!d_in) return fail("null descriptor");
+    const StateMap sm = state_map(d_in, ws);
+    if (ws->plan[kPlanGroups] <= 1) return forward_one(d_in, ws, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream);
     if (!x || !params || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_forward")) return 1;
@@ -2048,7 +2083,7 @@ int ttrnn_rnn_forward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws,
     for (int g = 0; g < gs.n && !rc; ++g) {
         const long long r0 = gs.row0[g];
         t_group = g;
-        rc = forward_one(&gs.d[g], &gs.w[g], x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
+        rc = forward_one(&gs.d[g], &gs.w[g], sm, x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
                          out + r0 * T * H, hT ? hT + r0 * H : nullptr, cT ? cT + r0 * H : nullptr,
                          saved ? (char *)saved + gs.sv_off[g] : nullptr, (char *)scratch + gs.f_off[g],
                          (g == 0 || serial) ? (void *)st : (void *)gc->s);
@@ -2067,8 +2102,11 @@ int ttrnn_rnn_backward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                        void *scratch, void *stream) {
     if (!ws || !plan_load(ws->plan, &t_opt))
         return fail("ttrnn_rnn_backward: `ws` must be the struct the matching forward ran with");
+    if (!d_in) return fail("null descriptor");
+    const StateMap sm = state_map(d_in, ws);
     if (ws->plan[kPlanGroups] <= 1)
-        return backward_one(d_in, ws, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch, stream);
+        return backward_one(d_in, ws, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
+                            stream);
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_backward")) return 1;
@@ -2087,7 +2125,7 @@ int ttrnn_rnn_backward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
         const long long r0 = gs.row0[g];
         float *dp = g == 0 ? d_params : (float *)((char *)scratch + gs.dp_off[g]);
         t_group = g;
-        rc = backward_one(&gs.d[g], &gs.w[g], x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
+        rc = backward_one(&gs.d[g], &gs.w[g], sm, x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
                           out + r0 * T * H, saved ? (const char *)saved + gs.sv_off[g] : nullptr,
                           d_out ? d_out + r0 * T * H : nullptr, d_hT ? d_hT + r0 * H : nullptr, d_cT ? d_cT + r0 * H : nullptr, dp,
                           d_x ? d_x + r0 * T * I : nullptr, d_h0 ? d_h0 + r0 * H : nullptr, d_c0 ? d_c0 + r0 * H : nullptr,
@@ -2352,8 +2390,8 @@ int ttrnn_dense_rnn_workspace_bytes(const ttrnn_dense_desc *desc, int64_t *saved
     return 0;
 }
 
-int ttrnn_dense_rnn_forward(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
-                            float *out, float *hT, float *cT, void *saved, void *scratch, void *stream) {
+static int dense_forward(const ttrnn_dense_desc *d, const StateMap &sm, const float *x, const float *h0, const float *c0,
+                         const float *params, float *out, float *hT, float *cT, void *saved, void *scratch, void *stream) {
     t_opt = snapshot_options();
     DensePlan dp;
     if (build_dense_plan(d, &dp)) return 1;
@@ -2391,8 +2429,9 @@ int ttrnn_dense_rnn_forward(const ttrnn_dense_desc *d, const float *x, const flo
         } else if (dense_linear(dv, B * (long long)T, T, lin, (long long)T * o.nin, o.nin, w_ih_hi, w_ih_lo, wt_ih, GH,
                          o.has_bih ? params + o.b_ih : nullptr, ab, (long long)T * GH, false, st))
             return 1;
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
         for (int t = 0; t < T; ++t) {
-            const float *hp = t == 0 ? h0 : lout + (long long)(t - 1) * H;
+            const float *hp = t == 0 ? h0l : lout + (long long)(t - 1) * H;
             const long long ldhp = t == 0 ? H : (long long)T * H;
             // u_t = h_{t-1} W_hh^T + b_hh  (h_{-1} = 0: u_0 = b_hh)
             if (hp) {
@@ -2410,7 +2449,7 @@ int ttrnn_dense_rnn_forward(const ttrnn_dense_desc *d, const float *x, const flo
             a.a = ab + (long long)t * GH; a.lda = (long long)T * GH;
             a.u = ub + (long long)t * GH; a.ldu = (long long)T * GH;
             a.h_prev = hp; a.ldhp = ldhp;
-            a.c_prev = t == 0 ? c0 : cs + (long long)(t - 1) * H; a.ldcp = t == 0 ? H : (long long)T * H;
+            a.c_prev = t == 0 ? c0l : cs + (long long)(t - 1) * H; a.ldcp = t == 0 ? H : (long long)T * H;
             a.h = lout + (long long)t * H; a.ldh = (long long)T * H;
             a.c = lstm ? cs + (long long)t * H : nullptr; a.ldc = (long long)T * H;
             {
@@ -2421,19 +2460,18 @@ int ttrnn_dense_rnn_forward(const ttrnn_dense_desc *d, const float *x, const flo
             ++g_launches;
         }
         CU_CHECK(cudaGetLastError());
-        if (l == L - 1) {
-            if (hT) CU_CHECK(cudaMemcpy2DAsync(hT, (size_t)H * 4, lout + (long long)(T - 1) * H, (size_t)T * H * 4, (size_t)H * 4, B,
-                                               cudaMemcpyDeviceToDevice, st));
-            if (lstm && cT) CU_CHECK(cudaMemcpy2DAsync(cT, (size_t)H * 4, cs + (long long)(T - 1) * H, (size_t)T * H * 4, (size_t)H * 4,
-                                                       B, cudaMemcpyDeviceToDevice, st));
-        }
+        float *hTl = sm.fin(hT, l, L), *cTl = sm.fin(cT, l, L);
+        if (hTl) CU_CHECK(cudaMemcpy2DAsync(hTl, (size_t)H * 4, lout + (long long)(T - 1) * H, (size_t)T * H * 4, (size_t)H * 4, B,
+                                            cudaMemcpyDeviceToDevice, st));
+        if (lstm && cTl) CU_CHECK(cudaMemcpy2DAsync(cTl, (size_t)H * 4, cs + (long long)(T - 1) * H, (size_t)T * H * 4, (size_t)H * 4,
+                                                    B, cudaMemcpyDeviceToDevice, st));
     }
     return 0;
 }
 
-int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
-                             const float *out, void *saved, const float *d_out, const float *d_hT, const float *d_cT,
-                             float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream) {
+static int dense_backward(const ttrnn_dense_desc *d, const StateMap &sm, const float *x, const float *h0, const float *c0,
+                          const float *params, const float *out, void *saved, const float *d_out, const float *d_hT,
+                          const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream) {
     t_opt = snapshot_options();
     DensePlan dp;
     if (build_dense_plan(d, &dp)) return 1;
@@ -2470,20 +2508,22 @@ int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const fl
         // dh_{t-1} += du_t W_hh : rows GEMM with Bt = W_hh^T (H x GH)
         if (transpose_to(W_hh, wT, GH, H, st)) return 1;                         // wT = W_hh^T (H x GH)
         if (split_tf32(wT, wT_hi, wT_lo, r4(nhh), st)) return 1;
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
+        const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L);
         for (int t = T - 1; t >= 0; --t) {
             ttd::DenseStepArgs a;
             memset(&a, 0, sizeof a);
             a.B = B; a.H = H;
             a.a = ab + (long long)t * GH; a.lda = (long long)T * GH;
             a.u = ub + (long long)t * GH; a.ldu = (long long)T * GH;
-            a.h_prev = t == 0 ? h0 : lout + (long long)(t - 1) * H; a.ldhp = t == 0 ? H : (long long)T * H;
-            a.c_prev = t == 0 ? c0 : (lstm ? cs + (long long)(t - 1) * H : nullptr); a.ldcp = t == 0 ? H : (long long)T * H;
+            a.h_prev = t == 0 ? h0l : lout + (long long)(t - 1) * H; a.ldhp = t == 0 ? H : (long long)T * H;
+            a.c_prev = t == 0 ? c0l : (lstm ? cs + (long long)(t - 1) * H : nullptr); a.ldcp = t == 0 ? H : (long long)T * H;
             a.dout = dhs ? dhs + (long long)t * H : nullptr; a.lddo = (long long)T * H;
             a.first = t == T - 1;
             a.dh_gemm = a.first ? nullptr : dh_gemm;
             a.dh_direct = (a.first || lstm) ? nullptr : dhd[(t + 1) & 1];
-            a.dh_T = (a.first && l == L - 1) ? d_hT : nullptr;
-            a.dc_T = (a.first && l == L - 1) ? d_cT : nullptr;
+            a.dh_T = a.first ? dhTl : nullptr;
+            a.dc_T = a.first ? dcTl : nullptr;
             a.da = ab + (long long)t * GH; a.ldda = (long long)T * GH;
             a.du = ub + (long long)t * GH; a.lddu = (long long)T * GH;
             a.dh_direct_out = dhd[t & 1];
@@ -2494,7 +2534,7 @@ int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const fl
                 else ttd::k_dense_cell_bwd<false><<<(unsigned)blocks, 256, 0, st>>>(a);
             }
             ++g_launches;
-            if (t > 0 || (d_h0 && h0)) {
+            if (t > 0 || (d_h0 && h0l)) {
                 // dh_gemm = du_t W_hh
                 if (dense_linear(dv, B, 1, ub + (long long)t * GH, (long long)T * GH, GH, wT_hi, wT_lo, W_hh, H, nullptr,
                                  dh_gemm, H, true, st))
@@ -2502,13 +2542,13 @@ int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const fl
             }
         }
         CU_CHECK(cudaGetLastError());
-        // gradient wrt the shared initial state: sum over layers
-        if (d_h0 && h0) {
+        // gradient wrt the initial state: this layer's own block, or the sum over layers when the state is shared
+        if (d_h0 && h0l) {
             ttd::k_add2<<<(unsigned)blocks, 256, 0, st>>>(dh_gemm, lstm ? nullptr : dhd[0], sc + lo.s_dh + 4 * r4(lo.BH), lo.BH);
             ++g_launches;
-            if (axpy1(sc + lo.s_dh + 4 * r4(lo.BH), d_h0, lo.BH, l != L - 1, st)) return 1;
+            if (axpy1(sc + lo.s_dh + 4 * r4(lo.BH), sm.init(d_h0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
         }
-        if (lstm && d_c0 && c0 && axpy1(dcc, d_c0, lo.BH, l != L - 1, st)) return 1;
+        if (lstm && d_c0 && c0l && axpy1(dcc, sm.init(d_c0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
         // dW_hh^T (H x GH) = sum_t h_{t-1}^T du_t ; db_hh = column sums of du (all T steps)
         {
             bool acc = false;
@@ -2517,8 +2557,8 @@ int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const fl
                     return 1;
                 acc = true;
             }
-            if (h0) {
-                if (dense_dw(dv, B, 1, h0, H, H, ub, (long long)T * GH, GH, D, acc, false, st)) return 1;
+            if (h0l) {
+                if (dense_dw(dv, B, 1, h0l, H, H, ub, (long long)T * GH, GH, D, acc, false, st)) return 1;
                 acc = true;
             }
             if (acc) {
@@ -2563,6 +2603,36 @@ int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const fl
 }
 
 // ---- GE2E head (SURVEY.md 8f-4) ------------------------------------------------------------------------------------
+int ttrnn_dense_rnn_forward(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
+                            float *out, float *hT, float *cT, void *saved, void *scratch, void *stream) {
+    return dense_forward(d, StateMap(), x, h0, c0, params, out, hT, cT, saved, scratch, stream);
+}
+int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
+                             const float *out, void *saved, const float *d_out, const float *d_hT, const float *d_cT,
+                             float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream) {
+    return dense_backward(d, StateMap(), x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
+                          stream);
+}
+static int dense_state_map(const ttrnn_dense_desc *d, int32_t flags, StateMap *sm) {
+    if (!d) return fail("null descriptor");
+    if (flags & ~TTRNN_WS_LAYER_STATES) return fail("dense cells: unknown flags 0x%x (only TTRNN_WS_LAYER_STATES applies)", flags);
+    if (flags & TTRNN_WS_LAYER_STATES) sm->stride = d->batch * (long long)d->hidden_size;
+    return 0;
+}
+int ttrnn_dense_rnn_forward_ex(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
+                               float *out, float *hT, float *cT, void *saved, void *scratch, void *stream, int32_t flags) {
+    StateMap sm;
+    if (dense_state_map(d, flags, &sm)) return 1;
+    return dense_forward(d, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream);
+}
+int ttrnn_dense_rnn_backward_ex(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
+                                const float *out, void *saved, const float *d_out, const float *d_hT, const float *d_cT,
+                                float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream, int32_t flags) {
+    StateMap sm;
+    if (dense_state_map(d, flags, &sm)) return 1;
+    return dense_backward(d, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch, stream);
+}
+
 int ttrnn_embed_forward(int64_t rows, int32_t E, const float *x, float *y, float *inv_norm, void *stream) {
     if (rows < 1 || E < 1) return fail("ttrnn_embed_forward: rows and E must be >= 1");
     if (!x || !y || !inv_norm) return fail("ttrnn_embed_forward: null operand");

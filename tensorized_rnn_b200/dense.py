@@ -21,8 +21,10 @@ from .functional import _bytes_to_floats, _dense16, _ptr, _require_cuda_f32
 
 
 class _DenseRnnFunction(torch.autograd.Function):
+    """`layer_states`: h0 / c0 and the returned final states are (L, B, H), one block per layer (TTRNN_WS_LAYER_STATES)."""
+
     @staticmethod
-    def forward(ctx, cell: str, hidden_size: int, num_layers: int, has_bias: bool, x, h0, c0, *params):
+    def forward(ctx, cell: str, hidden_size: int, num_layers: int, has_bias: bool, layer_states: bool, x, h0, c0, *params):
         lib = _lib.load()
         _require_cuda_f32("input", x)
         for i, p in enumerate(params):
@@ -31,11 +33,13 @@ class _DenseRnnFunction(torch.autograd.Function):
             raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
         B, T, I = x.shape
         H = hidden_size
+        state_shape = (num_layers, B, H) if layer_states else (B, H)
+        flags = _lib.WS_LAYER_STATES if layer_states else 0
         for name, s in (("h0", h0), ("c0", c0)):
             if s is not None:
                 _require_cuda_f32(name, s)
-                if tuple(s.shape) != (B, H):
-                    raise ValueError("%s must have shape (%d, %d), got %s" % (name, B, H, tuple(s.shape)))
+                if tuple(s.shape) != state_shape:
+                    raise ValueError("%s must have shape %s, got %s" % (name, state_shape, tuple(s.shape)))
         x, h0c, c0c = _dense16(x), _dense16(h0), _dense16(c0)
         desc = _lib.DenseDesc(_lib.CELL_LSTM if cell == "lstm" else _lib.CELL_GRU, num_layers, I, H, int(has_bias), T, B)
         with torch.cuda.device(x.device):
@@ -48,14 +52,15 @@ class _DenseRnnFunction(torch.autograd.Function):
             sb, wb = C.c_int64(0), C.c_int64(0)
             _lib.check(lib.ttrnn_dense_rnn_workspace_bytes(C.byref(desc), C.byref(sb), C.byref(wb)), "ttrnn_dense_rnn_workspace_bytes")
             out = torch.empty((B, T, H), device=x.device, dtype=torch.float32)
-            hT = torch.empty((B, H), device=x.device, dtype=torch.float32)
-            cT = torch.empty((B, H), device=x.device, dtype=torch.float32) if cell == "lstm" else None
+            hT = torch.empty(state_shape, device=x.device, dtype=torch.float32)
+            cT = torch.empty(state_shape, device=x.device, dtype=torch.float32) if cell == "lstm" else None
             saved = torch.empty(_bytes_to_floats(sb.value), device=x.device, dtype=torch.float32)
             scratch = torch.empty(_bytes_to_floats(wb.value), device=x.device, dtype=torch.float32)
             stream = torch.cuda.current_stream(x.device).cuda_stream
-            _lib.check(lib.ttrnn_dense_rnn_forward(C.byref(desc), _ptr(x), _ptr(h0c), _ptr(c0c), _ptr(blob), _ptr(out), _ptr(hT),
-                                                   _ptr(cT), _ptr(saved), _ptr(scratch), stream), "ttrnn_dense_rnn_forward")
+            _lib.check(lib.ttrnn_dense_rnn_forward_ex(C.byref(desc), _ptr(x), _ptr(h0c), _ptr(c0c), _ptr(blob), _ptr(out), _ptr(hT),
+                                                      _ptr(cT), _ptr(saved), _ptr(scratch), stream, flags), "ttrnn_dense_rnn_forward")
         ctx.desc, ctx.cell = desc, cell
+        ctx.flags, ctx.state_shape = flags, state_shape
         ctx.shapes = [tuple(p.shape) for p in params]
         ctx.scratch_floats = _bytes_to_floats(wb.value)
         ctx.has_h0, ctx.has_c0 = h0 is not None, c0 is not None
@@ -77,23 +82,25 @@ class _DenseRnnFunction(torch.autograd.Function):
         B, H = x.shape[0], out.shape[2]
         with torch.cuda.device(x.device):
             d_blob = torch.empty_like(blob)
-            d_x = torch.empty_like(x) if ctx.needs_input_grad[4] else None
-            d_h0 = torch.empty((B, H), device=x.device, dtype=torch.float32) if (ctx.has_h0 and ctx.needs_input_grad[5]) else None
-            d_c0 = torch.empty((B, H), device=x.device, dtype=torch.float32) \
-                if (lstm and ctx.has_c0 and ctx.needs_input_grad[6]) else None
+            d_x = torch.empty_like(x) if ctx.needs_input_grad[5] else None
+            d_h0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
+                if (ctx.has_h0 and ctx.needs_input_grad[6]) else None
+            d_c0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
+                if (lstm and ctx.has_c0 and ctx.needs_input_grad[7]) else None
             scratch = torch.empty(ctx.scratch_floats, device=x.device, dtype=torch.float32)
             stream = torch.cuda.current_stream(x.device).cuda_stream
-            _lib.check(lib.ttrnn_dense_rnn_backward(C.byref(ctx.desc), _ptr(x), _ptr(h0), _ptr(c0), _ptr(blob), _ptr(out), _ptr(saved),
-                                                    _ptr(d_out), _ptr(d_hT), _ptr(d_cT), _ptr(d_blob), _ptr(d_x), _ptr(d_h0),
-                                                    _ptr(d_c0), _ptr(scratch), stream), "ttrnn_dense_rnn_backward")
+            _lib.check(lib.ttrnn_dense_rnn_backward_ex(C.byref(ctx.desc), _ptr(x), _ptr(h0), _ptr(c0), _ptr(blob), _ptr(out),
+                                                       _ptr(saved), _ptr(d_out), _ptr(d_hT), _ptr(d_cT), _ptr(d_blob), _ptr(d_x),
+                                                       _ptr(d_h0), _ptr(d_c0), _ptr(scratch), stream, ctx.flags),
+                       "ttrnn_dense_rnn_backward")
         d_params, off = [], 0
         for i, shp in enumerate(ctx.shapes):
             n = 1
             for v in shp:
                 n *= v
-            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[7 + i] else None)
+            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[8 + i] else None)
             off += n
-        return (None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
+        return (None, None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
 
 
 class _DenseCell(nn.Module):
@@ -160,11 +167,11 @@ class _DenseRnnBase(nn.Module):
     def flat_parameters(self):
         return [p for c in self._all_layers for p in c.flat_parameters()]
 
-    def _run(self, input, h0, c0):
+    def _run(self, input, h0, c0, layer_states=False):
         if input.shape[1] == 0:
             raise NameError("name 'x' is not defined")       # the reference fails the same way on T = 0 (lstm.py:135)
-        return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.num_layers, bool(self.bias), input, h0, c0,
-                                       *self.flat_parameters())
+        return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.num_layers, bool(self.bias), layer_states, input,
+                                       h0, c0, *self.flat_parameters())
 
 
 class LSTM(_DenseRnnBase):
@@ -180,6 +187,13 @@ class LSTM(_DenseRnnBase):
         out, h, c = self._run(input, h0, c0)
         return out, (h, c)
 
+    def forward_states(self, input, states=None):
+        """Per-layer states, as torch.nn.LSTM takes them: `states` = (h, c), each (num_layers, batch, hidden), or None
+        (zeros).  Returns (outputs, (h_n, c_n)) with every layer's final state, so a sequence can be run in pieces."""
+        h0, c0 = states if states is not None else (None, None)
+        out, h, c = self._run(input, h0, c0, layer_states=True)
+        return out, (h, c)
+
 
 class GRU(_DenseRnnBase):
     """Dense GRU stack, drop-in for reference tensorized_rnn.gru.GRU (gru.py:52-136)."""
@@ -191,3 +205,8 @@ class GRU(_DenseRnnBase):
     def forward(self, input, init_states=None):
         out, h = self._run(input, init_states, None)
         return out, h
+
+    def forward_states(self, input, states=None):
+        """Per-layer states: `states` (num_layers, batch, hidden) or None (zeros) -> (outputs, h_n (num_layers, batch,
+        hidden))."""
+        return self._run(input, states, None, layer_states=True)

@@ -90,10 +90,12 @@ def _step_stats(lib, v: torch.Tensor, stream) -> torch.Tensor:
 class _RnnFunction(torch.autograd.Function):
     """`step_log` (None or an object with .activations(layer, var, stats) / .gradients(layer, var, stats)): fused
     log_grads.  The training forward reports the per-step statistics of every layer's h_t / c_t sequence, the
-    backward those of the total gradients reaching them, (2, T) tensors each (reference rnn_utils.py:127-172)."""
+    backward those of the total gradients reaching them, (2, T) tensors each (reference rnn_utils.py:127-172).
+    `layer_states`: h0 / c0 and the returned final states are (L, B, H), one block per layer (TTRNN_WS_LAYER_STATES);
+    else (B, H), shared by every layer on the way in and the last layer's on the way out."""
 
     @staticmethod
-    def forward(ctx, spec: RnnSpec, grad_enabled: bool, step_log, x, h0, c0, *params):
+    def forward(ctx, spec: RnnSpec, grad_enabled: bool, step_log, layer_states: bool, x, h0, c0, *params):
         lib = _lib.load()
         _require_cuda_f32("input", x)
         for i, p in enumerate(params):
@@ -104,11 +106,12 @@ class _RnnFunction(torch.autograd.Function):
         H = spec.hidden_size
         if I != spec.input_size:
             raise ValueError("input has %d features, the module was built for %d" % (I, spec.input_size))
+        state_shape = (spec.num_layers, B, H) if layer_states else (B, H)
         for name, s in (("h0", h0), ("c0", c0)):
             if s is not None:
                 _require_cuda_f32(name, s)
-                if tuple(s.shape) != (B, H):
-                    raise ValueError("%s must have shape (%d, %d), got %s" % (name, B, H, tuple(s.shape)))
+                if tuple(s.shape) != state_shape:
+                    raise ValueError("%s must have shape %s, got %s" % (name, state_shape, tuple(s.shape)))
         x = _dense16(x)
         h0c = _dense16(h0)
         c0c = _dense16(c0)
@@ -121,16 +124,16 @@ class _RnnFunction(torch.autograd.Function):
             if want != blob.numel():
                 raise RuntimeError("parameter blob has %d floats, descriptor expects %d" % (blob.numel(), want))
             ws = _lib.RnnWorkspace()
-            _lib.check(lib.ttrnn_rnn_workspace_bytes_ex(C.byref(desc), _lib.WS_WHOLE_BATCH if step_log is not None else 0,
-                                                        C.byref(ws)), "ttrnn_rnn_workspace_bytes")
+            flags = (_lib.WS_WHOLE_BATCH if step_log is not None else 0) | (_lib.WS_LAYER_STATES if layer_states else 0)
+            _lib.check(lib.ttrnn_rnn_workspace_bytes_ex(C.byref(desc), flags, C.byref(ws)), "ttrnn_rnn_workspace_bytes")
             # grad mode is always off inside Function.forward and needs_input_grad stays True for nn.Parameters under
             # torch.no_grad(): the caller captures torch.is_grad_enabled() before .apply (ADVICE r1)
-            training = bool(grad_enabled) and any(ctx.needs_input_grad[3:])
+            training = bool(grad_enabled) and any(ctx.needs_input_grad[4:])
             if step_log is not None and not training:
                 raise RuntimeError("fused per-step logging needs a training forward (it reads the kept h_t / c_t sequences)")
             out = torch.empty((B, T, H), device=x.device, dtype=torch.float32)
-            hT = torch.empty((B, H), device=x.device, dtype=torch.float32)
-            cT = torch.empty((B, H), device=x.device, dtype=torch.float32) if spec.cell == "lstm" else None
+            hT = torch.empty(state_shape, device=x.device, dtype=torch.float32)
+            cT = torch.empty(state_shape, device=x.device, dtype=torch.float32) if spec.cell == "lstm" else None
             saved = torch.empty(_bytes_to_floats(ws.saved_bytes), device=x.device, dtype=torch.float32) \
                 if training else None
             scratch = torch.empty(_bytes_to_floats(ws.fwd_scratch_bytes), device=x.device, dtype=torch.float32)
@@ -154,6 +157,7 @@ class _RnnFunction(torch.autograd.Function):
             ctx.ws = ws                    # sizes + execution plan: backward runs from the same plan as this forward
             ctx.bwd_floats = _bytes_to_floats(ws.bwd_scratch_bytes)
             ctx.has_h0, ctx.has_c0 = h0 is not None, c0 is not None
+            ctx.state_shape = state_shape
             ctx.set_materialize_grads(False)
             ctx.save_for_backward(x, h0c, c0c, blob, out, saved)
         if spec.cell == "lstm":
@@ -176,11 +180,11 @@ class _RnnFunction(torch.autograd.Function):
         d_cT = _dense16(d_cT)
         with torch.cuda.device(x.device):
             d_blob = torch.empty_like(blob)
-            d_x = torch.empty_like(x) if ctx.needs_input_grad[3] else None
-            d_h0 = torch.empty((B, H), device=x.device, dtype=torch.float32) \
-                if (ctx.has_h0 and ctx.needs_input_grad[4]) else None
-            d_c0 = torch.empty((B, H), device=x.device, dtype=torch.float32) \
-                if (spec.cell == "lstm" and ctx.has_c0 and ctx.needs_input_grad[5]) else None
+            d_x = torch.empty_like(x) if ctx.needs_input_grad[4] else None
+            d_h0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
+                if (ctx.has_h0 and ctx.needs_input_grad[5]) else None
+            d_c0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
+                if (spec.cell == "lstm" and ctx.has_c0 and ctx.needs_input_grad[6]) else None
             scratch = torch.empty(ctx.bwd_floats, device=x.device, dtype=torch.float32)
             stream = torch.cuda.current_stream(x.device).cuda_stream
             args = (C.byref(desc), C.byref(ctx.ws), _ptr(x), _ptr(h0), _ptr(c0), _ptr(blob), _ptr(out),
@@ -203,17 +207,19 @@ class _RnnFunction(torch.autograd.Function):
             n = 1
             for v in shp:
                 n *= v
-            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[6 + i] else None)
+            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[7 + i] else None)
             off += n
-        return (None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
+        return (None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
 
 
 def rnn_sequence(spec: RnnSpec, x: torch.Tensor, h0: Optional[torch.Tensor], c0: Optional[torch.Tensor],
-                 params: Sequence[torch.Tensor], step_log=None):
-    """Run the whole stack over the whole sequence.  Returns (out, hT[, cT]).  `step_log`: see _RnnFunction."""
+                 params: Sequence[torch.Tensor], step_log=None, layer_states: bool = False):
+    """Run the whole stack over the whole sequence.  Returns (out, hT[, cT]).  `step_log`: see _RnnFunction.
+    `layer_states=True`: h0 / c0 and the returned hT / cT are (num_layers, batch, hidden), one state per layer, so that
+    the final states of one call can seed the next call over the rest of the sequence."""
     if x.dim() != 3:
         raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
-    return _RnnFunction.apply(spec, torch.is_grad_enabled(), step_log, x, h0, c0, *params)
+    return _RnnFunction.apply(spec, torch.is_grad_enabled(), step_log, bool(layer_states), x, h0, c0, *params)
 
 
 class _TTLinearFunction(torch.autograd.Function):

@@ -254,6 +254,19 @@ class _TTRNNBase(nn.Module):
             # the reference falls off its time loop with unbound locals (lstm.py:135 / gru.py:136)
             raise NameError("zero-length sequence: the reference raises NameError here and so does this module")
 
+    def _layer_states_in(self, input, states):
+        """Per-layer initial states of the cell-step loop: a list of num_layers (batch, hidden) tensors per state
+        variable; None = zeros."""
+        shape = (self.num_layers, input.size(0), self.hidden_size)
+        out = []
+        for s in states:
+            if s is None:
+                s = torch.zeros(shape, device=input.device)
+            elif tuple(s.shape) != shape:
+                raise ValueError("per-layer states must have shape %s, got %s" % (shape, tuple(s.shape)))
+            out.append(list(s.unbind(0)))
+        return out
+
 
 class TTLSTM(_TTRNNBase):
     """Drop-in for reference tensorized_rnn.tt_lstm.TTLSTM (tt_lstm.py:43-62)."""
@@ -276,17 +289,34 @@ class TTLSTM(_TTRNNBase):
         out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink)
         return out, (h, c)
 
-    def _forward_cell_steps(self, input, init_states):
-        """The reference's own loop (lstm.py:116-135): step-major, layer-minor, one shared initial state.
+    def forward_states(self, input, states=None):
+        """Per-layer states, the contract of torch.nn.LSTM: `states` = (h, c), each (num_layers, batch, hidden), or None
+        (zeros).  Returns (outputs (batch, seq_len, hidden), (h_n, c_n)) with every layer's final state, each
+        (num_layers, batch, hidden): feeding them to the next call continues the sequence exactly where this one
+        stopped (streaming inference, truncated BPTT)."""
+        self._check_input(input)
+        sink = self._fused_step_log()
+        if self.cell_step_mode and sink is None:
+            return self._forward_cell_steps(input, states, layer_states=True)
+        h0, c0 = (None, None) if states is None else states
+        out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink, layer_states=True)
+        return out, (h, c)
+
+    def _forward_cell_steps(self, input, init_states, layer_states=False):
+        """The reference's own loop (lstm.py:116-135): step-major, layer-minor, one shared initial state
+        (`layer_states`: one per layer, and every layer's final state is returned).
         Outputs are stacked at the end instead of written in place, which spares autograd the
         reference's T CopySlices nodes; values are identical."""
         batch_size, seq_len, _ = input.size()
-        if init_states is None:
-            h = torch.zeros(batch_size, self.hidden_size, device=input.device)
-            c = torch.zeros(batch_size, self.hidden_size, device=input.device)
+        if layer_states:
+            internal_state = list(zip(*self._layer_states_in(input, init_states if init_states is not None else (None, None))))
         else:
-            h, c = init_states
-        internal_state = [(h, c)] * self.num_layers
+            if init_states is None:
+                h = torch.zeros(batch_size, self.hidden_size, device=input.device)
+                c = torch.zeros(batch_size, self.hidden_size, device=input.device)
+            else:
+                h, c = init_states
+            internal_state = [(h, c)] * self.num_layers
         outputs = []
         for step in range(seq_len):
             x = input[:, step, :]
@@ -295,6 +325,8 @@ class TTLSTM(_TTRNNBase):
                 x, new_c = cell(x, h, c)
                 internal_state[i] = (x, new_c)
             outputs.append(x)
+        if layer_states:
+            return torch.stack(outputs, dim=1), tuple(torch.stack(s) for s in zip(*internal_state))
         return torch.stack(outputs, dim=1), (x, new_c)
 
 
@@ -315,11 +347,23 @@ class TTGRU(_TTRNNBase):
         out, h = rnn_sequence(self.spec(), input, init_states, None, self.flat_parameters(), step_log=sink)
         return out, h
 
-    def _forward_cell_steps(self, input, init_states):
-        """The reference's own loop (gru.py:119-136)."""
+    def forward_states(self, input, states=None):
+        """Per-layer states, the contract of torch.nn.GRU: `states` (num_layers, batch, hidden) or None (zeros).
+        Returns (outputs (batch, seq_len, hidden), h_n (num_layers, batch, hidden)) with every layer's final state."""
+        self._check_input(input)
+        sink = self._fused_step_log()
+        if self.cell_step_mode and sink is None:
+            return self._forward_cell_steps(input, states, layer_states=True)
+        return rnn_sequence(self.spec(), input, states, None, self.flat_parameters(), step_log=sink, layer_states=True)
+
+    def _forward_cell_steps(self, input, init_states, layer_states=False):
+        """The reference's own loop (gru.py:119-136); `layer_states` as for TTLSTM."""
         batch_size, seq_len, _ = input.size()
-        h = torch.zeros(batch_size, self.hidden_size, device=input.device) if init_states is None else init_states
-        internal_state = [h] * self.num_layers
+        if layer_states:
+            internal_state, = self._layer_states_in(input, (init_states,))
+        else:
+            h = torch.zeros(batch_size, self.hidden_size, device=input.device) if init_states is None else init_states
+            internal_state = [h] * self.num_layers
         outputs = []
         for step in range(seq_len):
             x = input[:, step, :]
@@ -327,4 +371,6 @@ class TTGRU(_TTRNNBase):
                 x = cell(x, internal_state[i])
                 internal_state[i] = x
             outputs.append(x)
+        if layer_states:
+            return torch.stack(outputs, dim=1), torch.stack(internal_state)
         return torch.stack(outputs, dim=1), x
