@@ -34,7 +34,9 @@ extern "C" {
                                  (ttrnn_rnn_row_groups, ttrnn_rnn_workspace_bytes_ex), per-step logging entry points,
                                  per-launch timing records -- additive: every ABI 3 signature is unchanged.  Still 4 with
                                  per-layer states: one more flag value (TTRNN_WS_LAYER_STATES) and two new symbols
-                                 (ttrnn_dense_rnn_forward_ex / _backward_ex); no existing signature or default changes */
+                                 (ttrnn_dense_rnn_forward_ex / _backward_ex); no existing signature or default changes.
+                                 Still 4 with bidirectional stacks: two new symbols (ttrnn_time_reverse_add,
+                                 ttrnn_bidir_join), nothing existing changes */
 #define TTRNN_MAX_CORES   6
 #define TTRNN_MAX_LAYERS  8
 
@@ -147,6 +149,28 @@ int ttrnn_rnn_backward_logged(const ttrnn_rnn_desc *desc, const ttrnn_rnn_worksp
                               float *d_params, float *d_x, float *d_h0, float *d_c0,
                               void *scratch, void *stream, float *dh_log, float *dc_log);
 int ttrnn_step_norms(const float *v, int64_t B, int32_t T, int32_t H, float *out, void *stream);
+
+/* Bidirectional stacks (the contract of torch.nn.LSTM(bidirectional=True)).  The library has no whole-stack
+ * bidirectional call: the reverse direction of a layer is the ordinary one-layer ttrnn_rnn_forward / _backward (or
+ * ttrnn_dense_rnn_*) run on the layer input reversed in time, whose outputs then come back reversed in time.  These two
+ * memory-bound calls move the (B, T, .) blocks between the directions.  Every output element takes at most one FP32 add.
+ *
+ * ttrnn_time_reverse_add: y[b,t,:] = a[b,t,:] + r[b,T-1-t,:] over (B, T, F); a or r may be NULL (= zero).  With a NULL
+ * it reverses a layer-0 input for the reverse direction; with both it forms the layer-0 input gradient
+ * d_x = d_x_forward + reverse(d_x_reverse).  y must not alias a or r.
+ *
+ * ttrnn_bidir_join, H = hidden size, out_f / out_r = the forward / reverse direction's outputs (B, T, H), the latter in
+ * reversed time:
+ *   backward == 0: p = out_f, q = out_r (both required); writes the next layer's input u = y (B, T, 2H),
+ *                  y[b,t] = [out_f[b,t] | out_r[b,T-1-t]], and, unless v is NULL (the last layer), v = y_rev (B, T, 2H),
+ *                  y_rev[b,s] = y[b,T-1-s], the input of the next layer's reverse direction;
+ *   backward != 0: p = dy, q = dy_rev (the gradients of y and y_rev; either may be NULL = zero); writes
+ *                  u = d_out_f[b,t] = dy[b,t,:H] + dy_rev[b,T-1-t,:H] and v = d_out_r[b,s] = dy[b,T-1-s,H:] + dy_rev[b,s,H:],
+ *                  (B, T, H) each.
+ * Outputs must not alias inputs. */
+int ttrnn_time_reverse_add(int64_t B, int32_t T, int32_t F, const float *a, const float *r, float *y, void *stream);
+int ttrnn_bidir_join(int64_t B, int32_t T, int32_t H, int32_t backward, const float *p, const float *q, float *u,
+                     float *v, void *stream);
 
 /* Stand-alone TT linear map y = x W^T + bias over `rows` rows:
  * replaces TTLinear.forward (t3nsor/layers.py:121-127) -> tt_dense_matmul

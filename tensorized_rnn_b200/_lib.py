@@ -60,6 +60,8 @@ SYMBOLS = {
                                          C.POINTER(C.c_int64)]),
     "ttrnn_rnn_backward_logged": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 17),
     "ttrnn_step_norms": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P]),
+    "ttrnn_time_reverse_add": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P]),
+    "ttrnn_bidir_join": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "ttrnn_rnn_forward": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 10),
     "ttrnn_rnn_backward": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 15),
     "ttrnn_ttlinear_param_count": (C.c_int64, [C.POINTER(TTShape)]),

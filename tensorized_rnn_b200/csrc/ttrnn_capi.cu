@@ -15,6 +15,7 @@
 #include "tt_tc.cuh"
 #include "tt_ge2e.cuh"
 #include "tt_dense.cuh"
+#include "tt_bidir.cuh"
 #include "tt_static.cuh"
 #include "tt_static_api.h"
 
@@ -2178,6 +2179,53 @@ int ttrnn_rnn_saved_layout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace
 int ttrnn_step_norms(const float *v, int64_t B, int32_t T, int32_t H, float *out, void *stream) {
     if (!v || !out || B < 1 || T < 1 || H < 1) return fail("ttrnn_step_norms: bad arguments");
     k_step_norms<<<(unsigned)T, 256, 0, (cudaStream_t)stream>>>(v, B, T, H, out);
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+// ---- bidirectional stacks: time-reversed moves around the one-layer calls (tt_bidir.cuh) ---------------------------
+static bool aligned16(const void *p) { return ((uintptr_t)p & 15) == 0; }
+
+int ttrnn_time_reverse_add(int64_t B, int32_t T, int32_t F, const float *a, const float *r, float *y, void *stream) {
+    if (B < 1 || T < 1 || F < 1) return fail("ttrnn_time_reverse_add: B, T and F must be >= 1 (got %lld, %d, %d)",
+                                             (long long)B, T, F);
+    if (!y) return fail("ttrnn_time_reverse_add: y is NULL");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (F % 4 == 0 && aligned16(a) && aligned16(r) && aligned16(y)) {
+        const long long n = B * (long long)T * (F / 4);
+        bidir::k_reverse_add<4><<<bidir::grid_for(n, dv.sms), bidir::NT, 0, st>>>(a, r, y, n, T, F / 4);
+    } else {
+        const long long n = B * (long long)T * F;
+        bidir::k_reverse_add<1><<<bidir::grid_for(n, dv.sms), bidir::NT, 0, st>>>(a, r, y, n, T, F);
+    }
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int ttrnn_bidir_join(int64_t B, int32_t T, int32_t H, int32_t backward, const float *p, const float *q, float *u,
+                     float *v, void *stream) {
+    if (B < 1 || T < 1 || H < 1) return fail("ttrnn_bidir_join: B, T and H must be >= 1 (got %lld, %d, %d)",
+                                             (long long)B, T, H);
+    if (!u || (backward && !v)) return fail("ttrnn_bidir_join: missing output");
+    if (!backward && (!p || !q)) return fail("ttrnn_bidir_join: the forward needs both directions' outputs");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool vec = H % 4 == 0 && aligned16(p) && aligned16(q) && aligned16(u) && aligned16(v);
+    const int V = vec ? 4 : 1;
+    const long long n = B * (long long)T * (H / V) * (backward ? 1 : 2);
+    const unsigned grid = bidir::grid_for(n, dv.sms);
+    if (backward) {
+        if (vec) bidir::k_join_bwd<4><<<grid, bidir::NT, 0, st>>>(p, q, u, v, n, T, H / 4);
+        else bidir::k_join_bwd<1><<<grid, bidir::NT, 0, st>>>(p, q, u, v, n, T, H);
+    } else {
+        if (vec) bidir::k_join_fwd<4><<<grid, bidir::NT, 0, st>>>(p, q, u, v, n, T, H / 4);
+        else bidir::k_join_fwd<1><<<grid, bidir::NT, 0, st>>>(p, q, u, v, n, T, H);
+    }
     ++g_launches;
     CU_CHECK(cudaGetLastError());
     return 0;

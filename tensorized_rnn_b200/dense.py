@@ -7,6 +7,8 @@ convention (the dense LSTM cell gives its input map NO bias, lstm.py:17-18; the 
 gru.py:19-23), `init_hidden`, `param_count`, and the forward contract of lstm.py:101-135 / gru.py:104-136.  These are the
 modules `pmnist_test.py` builds without `--tt` and `SpeakerEncoder` builds with `compression=None`: with them the
 paper's dense-vs-TT comparison runs on the same device path (C ABI `ttrnn_dense_rnn_*`, csrc/tt_dense.cuh).
+`bidirectional=True` adds `cell{i}_reverse` per layer and runs the stack as one-layer calls per (layer, direction), as the TT
+modules do (functional.bidirectional_stack, DESIGN.md §4.17).
 """
 from __future__ import annotations
 
@@ -17,7 +19,8 @@ import torch
 from torch import nn
 
 from . import _lib
-from .functional import _bytes_to_floats, _dense16, _ptr, _require_cuda_f32
+from .functional import _bytes_to_floats, _dense16, _ptr, _require_cuda_f32, bidirectional_stack, \
+    shared_bidirectional_state
 
 
 class _DenseRnnFunction(torch.autograd.Function):
@@ -148,18 +151,22 @@ class _DenseRnnBase(nn.Module):
     cell_kind = ""
     cell_cls = None
 
-    def __init__(self, input_size, hidden_size, num_layers, device, bias=True, log_grads=False):
+    def __init__(self, input_size, hidden_size, num_layers, device, bias=True, log_grads=False, bidirectional=False):
         super().__init__()
         self.input_size, self.hidden_size, self.num_layers = input_size, hidden_size, num_layers
         self.bias, self.device, self.log_grads = bias, device, log_grads
+        self.bidirectional = bool(bidirectional)
         if log_grads:
             raise NotImplementedError("log_grads=True is implemented for the TT modules (TTLSTM / TTGRU); the dense baselines "
                                       "run as one fused sequence call and expose no per-step hooks")
+        # bidirectional: cell{i}_reverse after cell{i}, and the layers above the first take both directions' outputs
         self._all_layers = []
         for i in range(num_layers):
-            cell = self.cell_cls(input_size if i == 0 else hidden_size, hidden_size, bias, device)
-            setattr(self, "cell{}".format(i), cell)
-            self._all_layers.append(cell)
+            in_size = input_size if i == 0 else (2 * hidden_size if self.bidirectional else hidden_size)
+            for name in ("cell{}", "cell{}_reverse") if self.bidirectional else ("cell{}",):
+                cell = self.cell_cls(in_size, hidden_size, bias, device)
+                setattr(self, name.format(i), cell)
+                self._all_layers.append(cell)
 
     def param_count(self):
         return int(sum(p.numel() for c in self._all_layers for p in c.parameters()))
@@ -170,8 +177,27 @@ class _DenseRnnBase(nn.Module):
     def _run(self, input, h0, c0, layer_states=False):
         if input.shape[1] == 0:
             raise NameError("name 'x' is not defined")       # the reference fails the same way on T = 0 (lstm.py:135)
+        if self.bidirectional:
+            return self._run_bidirectional(input, h0, c0, layer_states)
         return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.num_layers, bool(self.bias), layer_states, input,
                                        h0, c0, *self.flat_parameters())
+
+    def _run_bidirectional(self, input, h0, c0, layer_states):
+        """Every (layer, direction) is a one-layer sequence call (functional.bidirectional_stack).  layer_states: h0 / c0
+        are (2L, B, H) and so are the returned final states; else one (B, H) state seeds every layer and both directions
+        and the last layer's two directions' final states come back as (2, B, H)."""
+        def run(layer, direction, x, h, c=None):
+            cell = self._all_layers[2 * layer + direction]
+            return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, 1, bool(self.bias), False, x, h, c,
+                                           *cell.flat_parameters())
+
+        states = [h0, c0] if self.cell_kind == "lstm" else [h0]
+        if not layer_states:
+            states = [shared_bidirectional_state(s, self.num_layers, input.size(0), self.hidden_size) for s in states]
+        out, fin = bidirectional_stack(input, states, self.num_layers, self.hidden_size, run)
+        if not layer_states:
+            fin = [f[-2:] for f in fin]
+        return (out, *fin)
 
 
 class LSTM(_DenseRnnBase):

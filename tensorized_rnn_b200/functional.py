@@ -222,6 +222,151 @@ def rnn_sequence(spec: RnnSpec, x: torch.Tensor, h0: Optional[torch.Tensor], c0:
     return _RnnFunction.apply(spec, torch.is_grad_enabled(), step_log, bool(layer_states), x, h0, c0, *params)
 
 
+# ---- bidirectional stacks (DESIGN.md §4.17) --------------------------------------------------------------------------
+class _BidirInputFunction(torch.autograd.Function):
+    """Layer-0 input of a bidirectional stack: x for the forward direction, x reversed in time for the reverse one
+    (ttrnn_time_reverse_add with a = NULL).  The backward forms d_x = d_x_forward + reverse(d_x_reverse) in the same
+    kernel, so the two directions' input gradients are summed by the library, not by autograd."""
+
+    @staticmethod
+    def forward(ctx, x):
+        lib = _lib.load()
+        _require_cuda_f32("input", x)
+        B, T, F = x.shape
+        x = _dense16(x)
+        with torch.cuda.device(x.device):
+            x_rev = torch.empty_like(x)
+            _lib.check(lib.ttrnn_time_reverse_add(B, T, F, None, _ptr(x), _ptr(x_rev),
+                                                  torch.cuda.current_stream(x.device).cuda_stream),
+                       "ttrnn_time_reverse_add")
+        ctx.set_materialize_grads(False)
+        return x, x_rev
+
+    @staticmethod
+    def backward(ctx, d_x_f, d_x_r):
+        if d_x_f is None and d_x_r is None:
+            return None
+        lib = _lib.load()
+        d_x_f, d_x_r = _dense16(d_x_f), _dense16(d_x_r)
+        like = d_x_f if d_x_f is not None else d_x_r
+        B, T, F = like.shape
+        with torch.cuda.device(like.device):
+            d_x = torch.empty_like(like)
+            _lib.check(lib.ttrnn_time_reverse_add(B, T, F, _ptr(d_x_f), _ptr(d_x_r), _ptr(d_x),
+                                                  torch.cuda.current_stream(like.device).cuda_stream),
+                       "ttrnn_time_reverse_add")
+        return d_x
+
+
+class _BidirJoinFunction(torch.autograd.Function):
+    """Joins the two directions of one layer (ttrnn_bidir_join): y[b,t] = [out_f[b,t] | out_r[b,T-1-t]], the next
+    layer's (or the module's) output, and unless `last`, y reversed in time, the next layer's reverse-direction input."""
+
+    @staticmethod
+    def forward(ctx, last: bool, out_f, out_r):
+        lib = _lib.load()
+        out_f, out_r = _dense16(out_f), _dense16(out_r)
+        B, T, H = out_f.shape
+        with torch.cuda.device(out_f.device):
+            y = torch.empty((B, T, 2 * H), device=out_f.device, dtype=torch.float32)
+            y_rev = None if last else torch.empty_like(y)
+            _lib.check(lib.ttrnn_bidir_join(B, T, H, 0, _ptr(out_f), _ptr(out_r), _ptr(y), _ptr(y_rev),
+                                            torch.cuda.current_stream(out_f.device).cuda_stream), "ttrnn_bidir_join")
+        ctx.set_materialize_grads(False)
+        return y if last else (y, y_rev)
+
+    @staticmethod
+    def backward(ctx, dy, dy_rev=None):
+        if dy is None and dy_rev is None:
+            return None, None, None
+        lib = _lib.load()
+        dy, dy_rev = _dense16(dy), _dense16(dy_rev)
+        like = dy if dy is not None else dy_rev
+        B, T, H2 = like.shape
+        with torch.cuda.device(like.device):
+            d_f = torch.empty((B, T, H2 // 2), device=like.device, dtype=torch.float32)
+            d_r = torch.empty_like(d_f)
+            _lib.check(lib.ttrnn_bidir_join(B, T, H2 // 2, 1, _ptr(dy), _ptr(dy_rev), _ptr(d_f), _ptr(d_r),
+                                            torch.cuda.current_stream(like.device).cuda_stream), "ttrnn_bidir_join")
+        return None, d_f, d_r
+
+
+_side_streams = {}
+
+
+def _side_stream(device: torch.device) -> torch.cuda.Stream:
+    """The stream the reverse directions run on: one per device, created on first use."""
+    idx = device.index if device.index is not None else torch.cuda.current_device()
+    s = _side_streams.get(idx)
+    if s is None:
+        s = _side_streams[idx] = torch.cuda.Stream(device=idx)
+    return s
+
+
+def shared_bidirectional_state(state: Optional[torch.Tensor], num_layers: int, batch: int, hidden_size: int):
+    """forward()'s one (B, H) initial state, which seeds every layer and both directions, as (2L, B, H) views of it."""
+    if state is None:
+        return None
+    if tuple(state.shape) != (batch, hidden_size):
+        raise ValueError("init_states must have shape %s, got %s" % ((batch, hidden_size), tuple(state.shape)))
+    return state.unsqueeze(0).expand(2 * num_layers, batch, hidden_size)
+
+
+def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]], num_layers: int, hidden_size: int,
+                        run):
+    """A bidirectional stack composed of one-layer calls, the contract of torch.nn.LSTM / GRU(bidirectional=True).
+
+    `run(layer, direction, x, *states)` runs direction 0 (forward) or 1 (reverse) of one layer over x (B, T, F) from its
+    (B, H) initial states (None = zeros) with the existing one-layer call and returns (out (B, T, H), *final states).
+    `states`: one entry per state variable (h, and c for an LSTM), each (2L, B, H) with direction d of layer l at
+    2l + d, or None (zeros).  Returns (out (B, T, 2H), [final states, each (2L, B, H) in the same order]).
+
+    The reverse direction of a layer sees its input reversed in time and returns its outputs reversed in time; the join
+    kernel writes the next layer's input and, for its reverse direction, the same tensor reversed.  The reverse
+    direction is issued on a side stream forked from the caller's current stream and joined back into it with events,
+    so that the two directions of a layer run concurrently.  Autograd runs each backward on the stream of its forward,
+    so the two directions' backward passes overlap as well, and it synchronises (and records) the gradients it hands
+    from one stream to the other; the forward's own cross-stream tensors are recorded here."""
+    if x.dim() != 3:
+        raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
+    _require_cuda_f32("input", x)
+    B = x.shape[0]
+    shape = (2 * num_layers, B, hidden_size)
+    for s in states:
+        if s is not None:
+            _require_cuda_f32("state", s)
+            if tuple(s.shape) != shape:
+                raise ValueError("bidirectional states must have shape %s (2 * num_layers, batch, hidden), got %s"
+                                 % (shape, tuple(s.shape)))
+    dev = x.device
+    with torch.cuda.device(dev):
+        main = torch.cuda.current_stream(dev)
+        side = _side_stream(dev)
+        inp_f, inp_r = _BidirInputFunction.apply(x)
+        finals = []
+        for l in range(num_layers):
+            st_f = [None if s is None else s[2 * l] for s in states]
+            st_r = [None if s is None else s[2 * l + 1] for s in states]
+            side.wait_stream(main)                      # fork: the reverse input and states are ready
+            for t in [inp_r] + st_r:
+                if t is not None:
+                    t.record_stream(side)
+            with torch.cuda.stream(side):
+                res_r = run(l, 1, inp_r, *st_r)
+            res_f = run(l, 0, inp_f, *st_f)
+            main.wait_stream(side)                      # join
+            for t in res_r:
+                t.record_stream(main)
+            last = l == num_layers - 1
+            if last:
+                out = _BidirJoinFunction.apply(True, res_f[0], res_r[0])
+            else:
+                inp_f, inp_r = _BidirJoinFunction.apply(False, res_f[0], res_r[0])
+            finals.append((res_f[1:], res_r[1:]))
+    fin = [torch.stack([f[k] for pair in finals for f in pair]) for k in range(len(finals[0][0]))]
+    return out, fin
+
+
 class _TTLinearFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, shape: _lib.TTShape, n_in: int, n_out: int, x, bias, *cores):

@@ -21,6 +21,10 @@ Two execution modes, chosen per module:
   step, and one reduction per (layer, variable) turns them into the four logged statistics
   (`ttrnn_rnn_backward_logged`, `ttrnn_step_norms`) that are appended to the same loggers.
   `new_core='first'/'last'` (rnn_utils.py:29-34) only changes the TT shapes and runs in either mode.
+
+`bidirectional=True` (no reference counterpart; the contract of torch.nn.LSTM(bidirectional=True)) adds a reverse cell
+per layer, `cell{i}_reverse`, and runs every (layer, direction) as a one-layer sequence call, the two directions of a
+layer on two streams (functional.bidirectional_stack, DESIGN.md §4.17).  It needs the fused mode.
 """
 from __future__ import annotations
 
@@ -29,7 +33,7 @@ from typing import List, Optional
 import torch
 from torch import nn
 
-from .functional import RnnSpec, rnn_sequence
+from .functional import RnnSpec, bidirectional_stack, rnn_sequence, shared_bidirectional_state
 from .functional import cell_step
 from .layers import TTLinear, TTLinearSet
 from .rnn_utils import ActivGradLogger
@@ -162,8 +166,11 @@ class _TTRNNBase(nn.Module):
     cell_kind = ""
 
     def __init__(self, input_size, hidden_size, num_layers, device, n_cores, tt_rank, bias=True,
-                 is_naive=False, log_grads=False, new_core=None):
+                 is_naive=False, log_grads=False, new_core=None, bidirectional=False):
         assert new_core in [None, 'first', 'last']
+        if bidirectional and (is_naive or log_grads):
+            raise NotImplementedError("bidirectional=True runs on the sequence kernels only; is_naive=True and "
+                                      "log_grads=True need the cell-step mode, which has no bidirectional form")
         super().__init__()
         self.n_cores = n_cores
         self.tt_rank = tt_rank
@@ -175,11 +182,17 @@ class _TTRNNBase(nn.Module):
         self.bias = bias
         self.device = device
         self.log_grads = log_grads
+        self.bidirectional = bool(bidirectional)
         self._all_layers = []
         for i in range(self.num_layers):
             cell = self._create_first_layer_cell() if i == 0 else self._create_other_layer_cell()
             setattr(self, 'cell{}'.format(i), cell)
             self._all_layers.append(cell)
+            if self.bidirectional:
+                # the reverse direction's cell of layer i, created right after the forward one (RNG order)
+                cell = self._make_cell(cell.input_size)
+                setattr(self, 'cell{}_reverse'.format(i), cell)
+                self._all_layers.append(cell)
         self._spec: Optional[RnnSpec] = None
         # log_grads: keep training forwards on the sequence kernels (see the module docstring); False = the reference's
         # per-step hooks in cell-step mode
@@ -225,7 +238,7 @@ class _TTRNNBase(nn.Module):
         return self._make_cell(self.input_size)
 
     def _create_other_layer_cell(self):
-        return self._make_cell(self.hidden_size)
+        return self._make_cell(2 * self.hidden_size if self.bidirectional else self.hidden_size)
 
     def param_count(self):
         total = 0
@@ -235,6 +248,9 @@ class _TTRNNBase(nn.Module):
         return total
 
     def spec(self) -> RnnSpec:
+        if self.bidirectional:
+            raise NotImplementedError("a bidirectional stack runs one-layer calls per (layer, direction); their "
+                                      "descriptors are cell{l}[_reverse]._single_step_spec()")
         if self._spec is None:
             self._spec = RnnSpec(self.cell_kind, self.input_size, self.hidden_size, bool(self.bias),
                                  [c.input_weights.tt_modes() for c in self._all_layers],
@@ -242,6 +258,8 @@ class _TTRNNBase(nn.Module):
         return self._spec
 
     def flat_parameters(self) -> List[torch.Tensor]:
+        """Every cell's parameters in C-ABI blob order, cells in creation order (bidirectional: cell0, cell0_reverse,
+        cell1, ...)."""
         out: List[torch.Tensor] = []
         for cell in self._all_layers:
             out += cell.flat_parameters()
@@ -253,6 +271,18 @@ class _TTRNNBase(nn.Module):
         if input.size(1) == 0:
             # the reference falls off its time loop with unbound locals (lstm.py:135 / gru.py:136)
             raise NameError("zero-length sequence: the reference raises NameError here and so does this module")
+
+    def _run_bidirectional(self, input, states):
+        """Bidirectional stack (functional.bidirectional_stack): every (layer, direction) is a one-layer sequence call.
+        `states`: per state variable (2L, B, H) or None."""
+        def run(layer, direction, x, h0, c0=None):
+            cell = self._all_layers[2 * layer + direction]
+            return rnn_sequence(cell._single_step_spec(), x, h0, c0, cell.flat_parameters())
+
+        return bidirectional_stack(input, states, self.num_layers, self.hidden_size, run)
+
+    def _shared_to_bidirectional(self, input, state):
+        return shared_bidirectional_state(state, self.num_layers, input.size(0), self.hidden_size)
 
     def _layer_states_in(self, input, states):
         """Per-layer initial states of the cell-step loop: a list of num_layers (batch, hidden) tensors per state
@@ -280,8 +310,15 @@ class TTLSTM(_TTRNNBase):
 
     def forward(self, input, init_states=None):
         """input (batch, seq_len, input_size) -> outputs (batch, seq_len, hidden), (h_T, c_T) of the last layer.
-        `init_states` = (h0, c0), each (batch, hidden), shared by every layer; None = zeros."""
+        `init_states` = (h0, c0), each (batch, hidden), shared by every layer; None = zeros.
+        bidirectional: outputs (batch, seq_len, 2 * hidden); (h0, c0) seed every layer and both directions; h_T, c_T
+        are (2, batch, hidden): the last layer's forward direction after the last step, then its reverse direction
+        after the first step."""
         self._check_input(input)
+        if self.bidirectional:
+            h0, c0 = (None, None) if init_states is None else init_states
+            out, (h, c) = self._run_bidirectional(input, [self._shared_to_bidirectional(input, s) for s in (h0, c0)])
+            return out, (h[-2:], c[-2:])
         sink = self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, init_states)
@@ -293,8 +330,13 @@ class TTLSTM(_TTRNNBase):
         """Per-layer states, the contract of torch.nn.LSTM: `states` = (h, c), each (num_layers, batch, hidden), or None
         (zeros).  Returns (outputs (batch, seq_len, hidden), (h_n, c_n)) with every layer's final state, each
         (num_layers, batch, hidden): feeding them to the next call continues the sequence exactly where this one
-        stopped (streaming inference, truncated BPTT)."""
+        stopped (streaming inference, truncated BPTT).
+        bidirectional: the states are (2 * num_layers, batch, hidden), direction d of layer l at 2l + d, in and out, as
+        torch.nn.LSTM(bidirectional=True) takes them; outputs are (batch, seq_len, 2 * hidden)."""
         self._check_input(input)
+        if self.bidirectional:
+            out, (h, c) = self._run_bidirectional(input, [None, None] if states is None else list(states))
+            return out, (h, c)
         sink = self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, states, layer_states=True)
@@ -339,8 +381,12 @@ class TTGRU(_TTRNNBase):
         return torch.zeros(batch_size, self.hidden_size).to(self.device)
 
     def forward(self, input, init_states=None):
-        """input (batch, seq_len, input_size) -> outputs (batch, seq_len, hidden), h_T of the last layer."""
+        """input (batch, seq_len, input_size) -> outputs (batch, seq_len, hidden), h_T of the last layer.
+        bidirectional: as for TTLSTM (outputs (batch, seq_len, 2 * hidden), h_T (2, batch, hidden))."""
         self._check_input(input)
+        if self.bidirectional:
+            out, (h,) = self._run_bidirectional(input, [self._shared_to_bidirectional(input, init_states)])
+            return out, h[-2:]
         sink = self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, init_states)
@@ -349,8 +395,12 @@ class TTGRU(_TTRNNBase):
 
     def forward_states(self, input, states=None):
         """Per-layer states, the contract of torch.nn.GRU: `states` (num_layers, batch, hidden) or None (zeros).
-        Returns (outputs (batch, seq_len, hidden), h_n (num_layers, batch, hidden)) with every layer's final state."""
+        Returns (outputs (batch, seq_len, hidden), h_n (num_layers, batch, hidden)) with every layer's final state.
+        bidirectional: states (2 * num_layers, batch, hidden), outputs (batch, seq_len, 2 * hidden), as torch.nn.GRU."""
         self._check_input(input)
+        if self.bidirectional:
+            out, (h,) = self._run_bidirectional(input, [states])
+            return out, h
         sink = self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, states, layer_states=True)
