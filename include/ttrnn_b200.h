@@ -36,7 +36,9 @@ extern "C" {
                                  per-layer states: one more flag value (TTRNN_WS_LAYER_STATES) and two new symbols
                                  (ttrnn_dense_rnn_forward_ex / _backward_ex); no existing signature or default changes.
                                  Still 4 with bidirectional stacks: two new symbols (ttrnn_time_reverse_add,
-                                 ttrnn_bidir_join), nothing existing changes */
+                                 ttrnn_bidir_join), nothing existing changes.  Still 4 with inter-layer dropout: one more
+                                 flag value (TTRNN_WS_DROPOUT), one struct and three new symbols (ttrnn_rnn_forward_dropout,
+                                 ttrnn_rnn_backward_dropout, ttrnn_dropout_apply) */
 #define TTRNN_MAX_CORES   6
 #define TTRNN_MAX_LAYERS  8
 
@@ -108,6 +110,11 @@ int ttrnn_rnn_workspace_bytes(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *w
  * states of the next.  The flag changes no kernel route, buffer size or result of the shared-state contract. */
 #define TTRNN_WS_WHOLE_BATCH 1
 #define TTRNN_WS_LAYER_STATES 2
+/* TTRNN_WS_DROPOUT: the plan is for ttrnn_rnn_forward_dropout / ttrnn_rnn_backward_dropout (below).  `saved` grows by
+ * (L-1) * B * T * H floats, the masked inputs of layers 1 .. L-1, and the forward scratch by one (B, T, H) block; every
+ * other size, offset and route is the one of the plan without the flag.  ttrnn_rnn_forward / ttrnn_rnn_backward /
+ * ttrnn_rnn_backward_logged reject a plan that carries it. */
+#define TTRNN_WS_DROPOUT 4
 int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrnn_rnn_workspace *ws);
 
 /* Forward over the whole stack.  h0 / c0 may be NULL (zeros); one (h0, c0) seeds
@@ -149,6 +156,43 @@ int ttrnn_rnn_backward_logged(const ttrnn_rnn_desc *desc, const ttrnn_rnn_worksp
                               float *d_params, float *d_x, float *d_h0, float *d_c0,
                               void *scratch, void *stream, float *dh_log, float *dc_log);
 int ttrnn_step_norms(const float *v, int64_t B, int32_t T, int32_t H, float *out, void *stream);
+
+/* Inter-layer dropout, the `dropout` argument of torch.nn.LSTM / GRU: the output sequence of every layer but the last is
+ * multiplied by mask / (1 - p) before the next layer reads it; mask is Bernoulli(1 - p) per element.  The final states
+ * are never masked.  The mask is a pure function of (seed, offset, boundary k = the layer whose output it masks, GLOBAL
+ * batch row b, t, feature j): Philox4x32-10 with key = seed and counter = (e / 4 as 64 bits with k in bits 48..63,
+ * offset), e = (b * T + t) * F + j, element e kept when its 32-bit word is below (1 - p) * 2^32.  So it does not depend on
+ * row groups, time chunks, rows per CTA or streams, and the backward regenerates it from (seed, offset): nothing of the
+ * mask is stored.  p must be in [0, 1]; p = 1 zeroes the input of the layers above the first (and its gradient).
+ *
+ * ttrnn_rnn_forward_dropout / ttrnn_rnn_backward_dropout: ttrnn_rnn_forward / _backward with the mask applied between
+ * the layers.  The plan must carry TTRNN_WS_DROPOUT when dp->p > 0 (a plan with it also runs p = 0: the mask keeps every
+ * element); a forward and its backward take the same `dp`.
+ *
+ * ttrnn_dropout_apply: the mask of boundary `boundary` over a (B, T, F) block whose first row is global row `row0`.
+ *   backward == 0: y = x * mask / (1 - p); unless y_rev is NULL also y_rev[b,t] = y[b,T-1-t] (the input of a
+ *                  bidirectional layer's reverse direction).  y may alias x.
+ *   backward != 0: y = (x + rev(y_rev)) * mask / (1 - p), y_rev read as the gradient of the reversed copy (NULL = zero):
+ *                  the adjoint of the forward.  y may alias x, not y_rev.
+ * Multiplying a ones block gives the mask / (1 - p) itself. */
+typedef struct ttrnn_dropout {
+    float p;              /* drop probability, 0 <= p <= 1          */
+    int32_t reserved;     /* 0                                      */
+    uint64_t seed;        /* Philox key                             */
+    uint64_t offset;      /* Philox counter words 2-3               */
+} ttrnn_dropout;
+int ttrnn_rnn_forward_dropout(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
+                              const float *x, const float *h0, const float *c0,
+                              const float *params, float *out, float *hT, float *cT,
+                              void *saved, void *scratch, void *stream, const ttrnn_dropout *dp);
+int ttrnn_rnn_backward_dropout(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
+                               const float *x, const float *h0, const float *c0,
+                               const float *params, const float *out, const void *saved,
+                               const float *d_out, const float *d_hT, const float *d_cT,
+                               float *d_params, float *d_x, float *d_h0, float *d_c0,
+                               void *scratch, void *stream, const ttrnn_dropout *dp);
+int ttrnn_dropout_apply(int64_t B, int32_t T, int32_t F, int64_t row0, int32_t boundary, int32_t backward,
+                        const ttrnn_dropout *dp, const float *x, float *y, float *y_rev, void *stream);
 
 /* Bidirectional stacks (the contract of torch.nn.LSTM(bidirectional=True)).  The library has no whole-stack
  * bidirectional call: the reverse direction of a layer is the ordinary one-layer ttrnn_rnn_forward / _backward (or

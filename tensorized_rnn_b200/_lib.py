@@ -16,6 +16,7 @@ MAX_LAYERS = 8
 PLAN_WORDS = 24
 WS_WHOLE_BATCH = 1
 WS_LAYER_STATES = 2      # per-layer (L, B, H) initial / final states and their gradients
+WS_DROPOUT = 4           # inter-layer dropout: saved keeps the masked inputs of layers 1 .. L-1
 CELL_LSTM, CELL_GRU = 0, 1
 
 _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc", "libttrnn_b200.so")
@@ -48,6 +49,10 @@ class RnnWorkspace(C.Structure):
                 ("plan", C.c_int64 * PLAN_WORDS)]
 
 
+class Dropout(C.Structure):
+    _fields_ = [("p", C.c_float), ("reserved", C.c_int32), ("seed", C.c_uint64), ("offset", C.c_uint64)]
+
+
 # every symbol include/ttrnn_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -64,6 +69,11 @@ SYMBOLS = {
     "ttrnn_bidir_join": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "ttrnn_rnn_forward": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 10),
     "ttrnn_rnn_backward": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 15),
+    "ttrnn_rnn_forward_dropout": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 10 + [C.POINTER(Dropout)]),
+    "ttrnn_rnn_backward_dropout": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 15 +
+                                   [C.POINTER(Dropout)]),
+    "ttrnn_dropout_apply": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.POINTER(Dropout),
+                                      _P, _P, _P, _P]),
     "ttrnn_ttlinear_param_count": (C.c_int64, [C.POINTER(TTShape)]),
     "ttrnn_ttlinear_workspace_bytes": (C.c_int64, [C.POINTER(TTShape), C.c_int64]),
     "ttrnn_ttlinear_forward": (C.c_int, [C.POINTER(TTShape), C.c_int64] + [_P] * 6),

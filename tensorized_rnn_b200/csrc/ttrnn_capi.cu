@@ -16,6 +16,7 @@
 #include "tt_ge2e.cuh"
 #include "tt_dense.cuh"
 #include "tt_bidir.cuh"
+#include "tt_dropout.cuh"
 #include "tt_static.cuh"
 #include "tt_static_api.h"
 
@@ -79,9 +80,11 @@ struct Opts {
 constexpr int kOptFields = sizeof(Opts) / sizeof(long long);
 constexpr long long kPlanMagic = 0x7474726E6E706C36LL;          // "ttrnnpl6"
 // plan words: [0] magic, [1 .. kOptFields] options, then the row-group split (group count, rows of group 0), then 1 when
-// the state buffers are per layer (TTRNN_WS_LAYER_STATES)
-constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2, kPlanLayerStates = kOptFields + 3;
-static_assert(kOptFields + 4 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
+// the state buffers are per layer (TTRNN_WS_LAYER_STATES), then 1 when `saved` keeps the masked layer inputs of the
+// dropout entry points (TTRNN_WS_DROPOUT)
+constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2, kPlanLayerStates = kOptFields + 3,
+              kPlanDropout = kOptFields + 4;
+static_assert(kOptFields + 5 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
 thread_local Opts t_opt;
 inline int merge_fwd() { return t_opt.merge_cores >= 2 ? 1 : 0; }    // contracted forward variants (merge_cores = 2)
 inline int merge_bwd() { return t_opt.merge_cores >= 1 ? 1 : 0; }    // contracted dX-only BPTT variants (merge_cores >= 1)
@@ -566,9 +569,13 @@ struct RnnLayout {
     // kept gate activations (static kernels, within the save_u_bytes budget): per layer flag and offset into `saved`
     bool kept[TTRNN_MAX_LAYERS] = {};
     long long sv_u[TTRNN_MAX_LAYERS] = {};
+    // inter-layer dropout (TTRNN_WS_DROPOUT, L > 1): masked inputs of layers 1 .. L-1 at the end of `saved` (training),
+    // one (B, T, H) block at the end of the forward scratch (inference)
+    bool masked = false;
+    long long sv_drop = 0, f_drop = 0;
 };
 
-int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, RnnLayout *lo) {
+int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, RnnLayout *lo, bool keep_masked) {
     const long long B = d->batch, T = d->seq_len, H = d->hidden_size, L = d->num_layers;
     const long long GH = (long long)rp.G * H;
     lo->BTH = B * T * H;
@@ -608,6 +615,8 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
         lo->kept[l] = keep_all && can_keep[l];
         if (lo->kept[l]) { lo->sv_u[l] = lo->sv_total; lo->sv_total += r4(B * T * 4 * H); }
     }
+    lo->masked = keep_masked && L > 1;
+    if (lo->masked) { lo->sv_drop = lo->sv_total; lo->sv_total += r4((L - 1) * lo->BTH); }
     // forward scratch
     long long o = 0;
     lo->f_xg = o; o += lo->xg_floats;
@@ -622,6 +631,7 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
             if (dense_bwd_floats(rp.layer[l].ih) > dbw) dbw = dense_bwd_floats(rp.layer[l].ih);
         }
     lo->f_dense = o; o += dfw;
+    lo->f_drop = o; o += lo->masked ? r4(lo->BTH) : 0;
     lo->f_total = o;
     // backward scratch
     long long maxp = 0;
@@ -674,11 +684,44 @@ struct CallPlan {
     const ttrnn_rnn_desc *d() const { return &eff.d; }
 };
 
-int plan_call(const ttrnn_rnn_desc *d_in, const DevInfo &dv, CallPlan *cp) {
+// keep_masked: the plan carries TTRNN_WS_DROPOUT
+int plan_call(const ttrnn_rnn_desc *d_in, const DevInfo &dv, CallPlan *cp, bool keep_masked = false) {
     cp->dv = dv;
     if (build_rnn_plan(d_in, &cp->rp) || make_eff_desc(d_in, &dv, &cp->eff)) return 1;
     if (cp->eff.padded && build_rnn_plan(&cp->eff.d, &cp->rp)) return 1;
-    return build_layout(&cp->eff.d, cp->rp, dv, &cp->lo);
+    return build_layout(&cp->eff.d, cp->rp, dv, &cp->lo, keep_masked);
+}
+
+// ---- inter-layer dropout (tt_dropout.cuh) --------------------------------------------------------------------------
+// the mask of one call: nullptr = no dropout; row0 = global batch row of the row group's first row
+struct DropCall {
+    float p;
+    uint64_t seed, offset;
+    long long row0;
+};
+static ttdrop::Mask drop_mask(const DropCall &dc, long long row0, int boundary) {
+    ttdrop::Mask m;
+    m.seed = dc.seed; m.offset = dc.offset; m.row0 = row0; m.boundary = (unsigned)boundary;
+    const double keep = 1.0 - (double)dc.p;
+    m.thr = (unsigned long long)(keep * 4294967296.0);
+    m.scale = keep > 0.0 ? (float)(1.0 / keep) : 0.f;
+    return m;
+}
+static bool aligned16(const void *p) { return ((uintptr_t)p & 15) == 0; }
+// y = (x + rev(xr)) * mask / (1 - p) over (B, T, F), rows from row0; yr (optional) receives y reversed in time
+static int launch_dropout(const DevInfo &dv, long long B, int T, int F, const DropCall &dc, long long row0, int boundary,
+                          const float *x, const float *xr, float *y, float *yr, cudaStream_t st) {
+    const ttdrop::Mask m = drop_mask(dc, row0, boundary);
+    if (F % 4 == 0 && aligned16(x) && aligned16(xr) && aligned16(y) && aligned16(yr)) {
+        const long long n = B * (long long)T * (F / 4);
+        ttdrop::k_dropout_4<<<ttdrop::grid_for(n, dv.sms), ttdrop::NT, 0, st>>>(x, xr, y, yr, n, T, F / 4, m);
+    } else {
+        const long long n = B * (long long)T * F;
+        ttdrop::k_dropout_1<<<ttdrop::grid_for(n, dv.sms), ttdrop::NT, 0, st>>>(x, xr, y, yr, n, T, F, m);
+    }
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
 }
 
 // ---- launch helpers ------------------------------------------------------------------------
@@ -1333,10 +1376,10 @@ int64_t ttrnn_rnn_param_count(const ttrnn_rnn_desc *desc) {
 }
 
 // byte sizes of ONE row group (the whole batch when the plan has a single group), under the calling thread's options
-static int workspace_one(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *ws) {
+static int workspace_one(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *ws, bool keep_masked) {
     DevInfo dv;
     CallPlan cp;
-    if (get_dev(&dv) || plan_call(desc, dv, &cp)) return 1;
+    if (get_dev(&dv) || plan_call(desc, dv, &cp, keep_masked)) return 1;
     ws->saved_bytes = cp.lo.sv_total * 4;
     ws->fwd_scratch_bytes = (cp.lo.f_total + cp.eff.pad_floats) * 4;       // + the rank-padded parameter blob
     ws->bwd_scratch_bytes = (cp.lo.b_total + 2 * cp.eff.pad_floats) * 4;   // + padded parameters and padded gradients
@@ -1353,8 +1396,9 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
     if (flags & TTRNN_WS_WHOLE_BATCH) t_opt.row_groups = 0;
     GroupPlan gp;
     if (plan_row_groups(desc, &gp)) return 1;
+    const bool masked = (flags & TTRNN_WS_DROPOUT) != 0;
     if (gp.n == 1) {
-        if (workspace_one(desc, ws)) return 1;
+        if (workspace_one(desc, ws, masked)) return 1;
     } else {
         // one region per group in every buffer (256-byte aligned), + the gradient blob of every group but the first
         const int64_t pf = ttrnn_rnn_param_count(desc);
@@ -1363,7 +1407,7 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
             ttrnn_rnn_desc dg = *desc;
             dg.batch = gp.rows[g];
             ttrnn_rnn_workspace wg;
-            if (workspace_one(&dg, &wg)) return 1;
+            if (workspace_one(&dg, &wg, masked)) return 1;
             ws->saved_bytes += a256(wg.saved_bytes);
             ws->fwd_scratch_bytes += a256(wg.fwd_scratch_bytes);
             ws->bwd_scratch_bytes += a256(wg.bwd_scratch_bytes) + (g > 0 ? a256(pf * 4) : 0);
@@ -1374,17 +1418,19 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
     ws->plan[kPlanGroups] = gp.n;
     ws->plan[kPlanRows0] = gp.rows[0];
     ws->plan[kPlanLayerStates] = (flags & TTRNN_WS_LAYER_STATES) ? 1 : 0;
+    ws->plan[kPlanDropout] = masked ? 1 : 0;
     return 0;
 }
 
 // forward of ONE row group on stream `stream`; `ws` carries the byte sizes of this group, t_opt is already loaded
+// `dc`: inter-layer dropout (nullptr = none; the plan then has no masked buffers)
 static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
                        const float *h0, const float *c0, const float *params_in, float *out, float *hT, float *cT, void *saved,
-                       void *scratch, void *stream) {
+                       void *scratch, void *stream, const DropCall *dc) {
     if (!x || !params_in || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     DevInfo dv;
     CallPlan cp;
-    if (get_dev(&dv) || plan_call(d_in, dv, &cp)) return 1;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp, ws->plan[kPlanDropout] != 0)) return 1;
     const ttrnn_rnn_desc *d = cp.d();
     const RnnPlan &rp = cp.rp;
     const RnnLayout &lo = cp.lo;
@@ -1418,6 +1464,12 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
         const float *lin;       // input of this layer (B, T, nin)
         if (l == 0) lin = x;
         else lin = sv ? sv + lo.sv_hs + (long long)(l - 1) * lo.BTH : sc + lo.f_hs + ((l - 1) & 1) * r4(lo.BTH);
+        if (l > 0 && dc) {
+            // dropout: layer l reads the masked output of layer l - 1 (kept for the backward in training)
+            float *masked = sv ? sv + lo.sv_drop + (long long)(l - 1) * lo.BTH : sc + lo.f_drop;
+            if (launch_dropout(dv, B, T, H, *dc, dc->row0, l - 1, lin, nullptr, masked, nullptr, st)) return 1;
+            lin = masked;
+        }
         float *lout;            // output of this layer (B, T, H)
         if (l == L - 1) lout = out;
         else lout = sv ? sv + lo.sv_hs + (long long)l * lo.BTH : sc + lo.f_hs + (l & 1) * r4(lo.BTH);
@@ -1573,16 +1625,16 @@ static SideCtx *side_ctx() {
 static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float *x, const float *h0, const float *c0,
                              const float *params, const float *out, const void *saved, const float *d_out, const float *d_hT,
                              const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch,
-                             cudaStream_t st);
+                             cudaStream_t st, const DropCall *dc);
 
 static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
                         const float *h0, const float *c0, const float *params, const float *out, const void *saved,
                         const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0,
-                        float *d_c0, void *scratch, void *stream) {
+                        float *d_c0, void *scratch, void *stream, const DropCall *dc) {
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     DevInfo dv;
     CallPlan cp;
-    if (get_dev(&dv) || plan_call(d_in, dv, &cp)) return 1;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp, ws->plan[kPlanDropout] != 0)) return 1;
     const RnnLayout &lo = cp.lo;
     const EffDesc &eff = cp.eff;
     if ((lo.b_total + 2 * eff.pad_floats) * 4 != ws->bwd_scratch_bytes || lo.sv_total * 4 != ws->saved_bytes)
@@ -1591,13 +1643,13 @@ static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
     cudaStream_t st = (cudaStream_t)stream;
     if (!eff.padded)
         return rnn_backward_impl(cp, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
-                                 st);
+                                 st, dc);
     float *pp = (float *)scratch + lo.b_total, *dpp = pp + eff.pad_floats;
     CU_CHECK(cudaMemsetAsync(pp, 0, (size_t)eff.pad_floats * 4, st));
     k_pad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, params, pp);
     ++g_launches;
     CU_CHECK(cudaGetLastError());
-    if (rnn_backward_impl(cp, sm, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st)) return 1;
+    if (rnn_backward_impl(cp, sm, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st, dc)) return 1;
     // the gradient wrt a real core is the matching block of the padded core's gradient
     k_unpad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, dpp, d_params);
     ++g_launches;
@@ -1608,7 +1660,7 @@ static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
 static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float *x, const float *h0, const float *c0,
                              const float *params, const float *out, const void *saved, const float *d_out, const float *d_hT,
                              const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch,
-                             cudaStream_t st) {
+                             cudaStream_t st, const DropCall *dc) {
     const ttrnn_rnn_desc *d = cp.d();
     const RnnPlan &rp = cp.rp;
     const RnnLayout &lo = cp.lo;
@@ -1618,6 +1670,7 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
     const int GH = G * H;
     const bool lstm = d->cell == TTRNN_CELL_LSTM;
     if ((L > 1 || lstm) && !saved) return fail("backward needs the `saved` buffer written by a training forward");
+    if (dc && L > 1 && !lo.masked) return fail("internal: dropout backward without the masked layer inputs");
     float *sc = (float *)scratch;
     const float *sv = (const float *)saved;
     float *sdh = sc + lo.b_sdh, *sdc = sc + lo.b_sdc;
@@ -1647,12 +1700,19 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
         float *part_hh = ss + lo.b_part_hh, *part_ih = ss + lo.b_part_ih;
         cudaStream_t ws = st;                                 // stream of the weight-gradient work of this layer
         DevInfo dvw = dv;                                     // ... and the SMs it may plan for
-        const float *lin = (l == 0) ? x : sv + lo.sv_hs + (long long)(l - 1) * lo.BTH;
+        // dropout: layers >= 1 read the masked output of the layer below, which the forward kept
+        const float *lin = (l == 0) ? x : sv + (dc ? lo.sv_drop : lo.sv_hs) + (long long)(l - 1) * lo.BTH;
         const float *lout = (l == L - 1) ? out : sv + lo.sv_hs + (long long)l * lo.BTH;
         const float *lcs = lstm ? sv + lo.sv_cs + (long long)l * lo.BTH : nullptr;
         // gradient wrt this layer's outputs / wrt its inputs
         const float *dhs = (l == L - 1) ? d_out : sc + lo.b_dhs + ((l + 1) & 1) * r4(lo.BTH);
         float *dlin = (l == 0) ? d_x : sc + lo.b_dhs + (l & 1) * r4(lo.BTH);
+        if (l < L - 1 && dc) {
+            // dropout: the gradient wrt the masked input of layer l + 1 (its dX, written on this stream also under the
+            // backward overlap) times mask / (1 - p) is the gradient wrt this layer's output; in place
+            float *g = sc + lo.b_dhs + ((l + 1) & 1) * r4(lo.BTH);
+            if (launch_dropout(dv, B, T, H, *dc, dc->row0, l, g, nullptr, g, nullptr, st)) return 1;
+        }
         const float *b_ih = d->has_bias ? params + lp.off_ih_bias : nullptr;
         const float *b_hh = d->has_bias ? params + lp.off_hh_bias : nullptr;
         // this layer's initial state and the upstream gradient of its final state (enters its last step)
@@ -2046,7 +2106,7 @@ static int group_slices(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
         gs->row0[g] = g ? rows0 : 0;
         gs->d[g] = *d_in;
         gs->d[g].batch = g ? d_in->batch - rows0 : rows0;
-        if (workspace_one(&gs->d[g], &gs->w[g])) return 1;
+        if (workspace_one(&gs->d[g], &gs->w[g], ws->plan[kPlanDropout] != 0)) return 1;
         memcpy(gs->w[g].plan, ws->plan, sizeof ws->plan);
         gs->sv_off[g] = sv; sv += a256(gs->w[g].saved_bytes);
         gs->f_off[g] = f;   f += a256(gs->w[g].fwd_scratch_bytes);
@@ -2060,14 +2120,37 @@ static int group_slices(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
     return 0;
 }
 
-int ttrnn_rnn_forward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
-                      const float *c0, const float *params, float *out, float *hT, float *cT, void *saved, void *scratch,
-                      void *stream) {
+// the mask of a dropout entry point: nullptr when there is none to apply (no dp, or a one-layer stack).  `who` names the
+// entry point in errors; dp_given: the call is a dropout entry point (which requires dp)
+static int drop_call(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, bool dp_given,
+                     const ttrnn_dropout *dp, DropCall *dc, const DropCall **out) {
+    *out = nullptr;
+    if (!dp_given) {
+        if (ws->plan[kPlanDropout])
+            return fail("%s: the plan was sized with TTRNN_WS_DROPOUT; run it with the _dropout entry points", who);
+        return 0;
+    }
+    if (!dp) return fail("%s: dp must be non-null", who);
+    if (!(dp->p >= 0.f && dp->p <= 1.f)) return fail("%s: dropout p must be in [0, 1], got %g", who, (double)dp->p);
+    if (dp->p > 0.f && !ws->plan[kPlanDropout])
+        return fail("%s: dropout p > 0 needs a plan sized with TTRNN_WS_DROPOUT", who);
+    if (d_in->num_layers < 2 || !ws->plan[kPlanDropout]) return 0;       // nothing between layers / p = 0 without buffers
+    dc->p = dp->p; dc->seed = dp->seed; dc->offset = dp->offset; dc->row0 = 0;
+    *out = dc;
+    return 0;
+}
+
+static int rnn_forward_entry(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x,
+                             const float *h0, const float *c0, const float *params, float *out, float *hT, float *cT,
+                             void *saved, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp) {
     if (!ws || !plan_load(ws->plan, &t_opt))
-        return fail("ttrnn_rnn_forward: `ws` must be the struct filled by ttrnn_rnn_workspace_bytes() for this descriptor");
+        return fail("%s: `ws` must be the struct filled by ttrnn_rnn_workspace_bytes() for this descriptor", who);
     if (!d_in) return fail("null descriptor");
+    DropCall dcs;
+    const DropCall *dc = nullptr;
+    if (drop_call(who, d_in, ws, dp_given, dp, &dcs, &dc)) return 1;
     const StateMap sm = state_map(d_in, ws);
-    if (ws->plan[kPlanGroups] <= 1) return forward_one(d_in, ws, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream);
+    if (ws->plan[kPlanGroups] <= 1) return forward_one(d_in, ws, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream, dc);
     if (!x || !params || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_forward")) return 1;
@@ -2084,10 +2167,11 @@ int ttrnn_rnn_forward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws,
     for (int g = 0; g < gs.n && !rc; ++g) {
         const long long r0 = gs.row0[g];
         t_group = g;
+        if (dc) dcs.row0 = r0;                  // the mask is indexed by global rows
         rc = forward_one(&gs.d[g], &gs.w[g], sm, x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
                          out + r0 * T * H, hT ? hT + r0 * H : nullptr, cT ? cT + r0 * H : nullptr,
                          saved ? (char *)saved + gs.sv_off[g] : nullptr, (char *)scratch + gs.f_off[g],
-                         (g == 0 || serial) ? (void *)st : (void *)gc->s);
+                         (g == 0 || serial) ? (void *)st : (void *)gc->s, dc);
     }
     t_group = 0;
     if (!serial) {       // also on the error path: the caller's stream must not run ahead of the group stream
@@ -2097,17 +2181,34 @@ int ttrnn_rnn_forward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws,
     return rc;
 }
 
-int ttrnn_rnn_backward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
-                       const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
-                       const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
-                       void *scratch, void *stream) {
+int ttrnn_rnn_forward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                      const float *c0, const float *params, float *out, float *hT, float *cT, void *saved, void *scratch,
+                      void *stream) {
+    return rnn_forward_entry("ttrnn_rnn_forward", d_in, ws, x, h0, c0, params, out, hT, cT, saved, scratch, stream, false,
+                             nullptr);
+}
+
+int ttrnn_rnn_forward_dropout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                              const float *c0, const float *params, float *out, float *hT, float *cT, void *saved,
+                              void *scratch, void *stream, const ttrnn_dropout *dp) {
+    return rnn_forward_entry("ttrnn_rnn_forward_dropout", d_in, ws, x, h0, c0, params, out, hT, cT, saved, scratch, stream,
+                             true, dp);
+}
+
+static int rnn_backward_entry(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x,
+                              const float *h0, const float *c0, const float *params, const float *out, const void *saved,
+                              const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x,
+                              float *d_h0, float *d_c0, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp) {
     if (!ws || !plan_load(ws->plan, &t_opt))
-        return fail("ttrnn_rnn_backward: `ws` must be the struct the matching forward ran with");
+        return fail("%s: `ws` must be the struct the matching forward ran with", who);
     if (!d_in) return fail("null descriptor");
+    DropCall dcs;
+    const DropCall *dc = nullptr;
+    if (drop_call(who, d_in, ws, dp_given, dp, &dcs, &dc)) return 1;
     const StateMap sm = state_map(d_in, ws);
     if (ws->plan[kPlanGroups] <= 1)
         return backward_one(d_in, ws, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
-                            stream);
+                            stream, dc);
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_backward")) return 1;
@@ -2126,11 +2227,12 @@ int ttrnn_rnn_backward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
         const long long r0 = gs.row0[g];
         float *dp = g == 0 ? d_params : (float *)((char *)scratch + gs.dp_off[g]);
         t_group = g;
+        if (dc) dcs.row0 = r0;
         rc = backward_one(&gs.d[g], &gs.w[g], sm, x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
                           out + r0 * T * H, saved ? (const char *)saved + gs.sv_off[g] : nullptr,
                           d_out ? d_out + r0 * T * H : nullptr, d_hT ? d_hT + r0 * H : nullptr, d_cT ? d_cT + r0 * H : nullptr, dp,
                           d_x ? d_x + r0 * T * I : nullptr, d_h0 ? d_h0 + r0 * H : nullptr, d_c0 ? d_c0 + r0 * H : nullptr,
-                          (char *)scratch + gs.b_off[g], (g == 0 || serial) ? (void *)st : (void *)gc->s);
+                          (char *)scratch + gs.b_off[g], (g == 0 || serial) ? (void *)st : (void *)gc->s, dc);
     }
     t_group = 0;
     if (!serial) {
@@ -2144,12 +2246,46 @@ int ttrnn_rnn_backward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
     return 0;
 }
 
+int ttrnn_rnn_backward(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                       const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
+                       const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
+                       void *scratch, void *stream) {
+    return rnn_backward_entry("ttrnn_rnn_backward", d_in, ws, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x,
+                              d_h0, d_c0, scratch, stream, false, nullptr);
+}
+
+int ttrnn_rnn_backward_dropout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                               const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
+                               const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
+                               void *scratch, void *stream, const ttrnn_dropout *dp) {
+    return rnn_backward_entry("ttrnn_rnn_backward_dropout", d_in, ws, x, h0, c0, params, out, saved, d_out, d_hT, d_cT,
+                              d_params, d_x, d_h0, d_c0, scratch, stream, true, dp);
+}
+
+int ttrnn_dropout_apply(int64_t B, int32_t T, int32_t F, int64_t row0, int32_t boundary, int32_t backward,
+                        const ttrnn_dropout *dp, const float *x, float *y, float *y_rev, void *stream) {
+    if (B < 1 || T < 1 || F < 1 || row0 < 0) return fail("ttrnn_dropout_apply: B, T, F must be >= 1 and row0 >= 0 (got %lld, %d, %d, %lld)",
+                                                         (long long)B, T, F, (long long)row0);
+    if (boundary < 0 || boundary >= TTRNN_MAX_LAYERS) return fail("ttrnn_dropout_apply: boundary %d out of range", boundary);
+    if (!dp) return fail("ttrnn_dropout_apply: dp must be non-null");
+    if (!(dp->p >= 0.f && dp->p <= 1.f)) return fail("ttrnn_dropout_apply: dropout p must be in [0, 1], got %g", (double)dp->p);
+    if (!x || !y) return fail("ttrnn_dropout_apply: x and y must be non-null");
+    if (y_rev && (y_rev == y || y_rev == x)) return fail("ttrnn_dropout_apply: y_rev must not alias x or y");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    DropCall dc;
+    dc.p = dp->p; dc.seed = dp->seed; dc.offset = dp->offset; dc.row0 = row0;
+    if (backward) return launch_dropout(dv, B, T, F, dc, row0, boundary, x, y_rev, y, nullptr, (cudaStream_t)stream);
+    return launch_dropout(dv, B, T, F, dc, row0, boundary, x, nullptr, y, y_rev, (cudaStream_t)stream);
+}
+
 int ttrnn_rnn_backward_logged(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
                               const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
                               const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
                               void *scratch, void *stream, float *dh_log, float *dc_log) {
     if (!d_in || !ws) return fail("null descriptor / workspace struct");
     if (!dh_log) return fail("ttrnn_rnn_backward_logged: dh_log must be non-null");
+    if (ws->plan[kPlanDropout]) return fail("ttrnn_rnn_backward_logged: the plan was sized with TTRNN_WS_DROPOUT");
     if (ws->plan[kPlanGroups] > 1)
         return fail("ttrnn_rnn_backward_logged needs a whole-batch plan: size the call with "
                     "ttrnn_rnn_workspace_bytes_ex(desc, TTRNN_WS_WHOLE_BATCH, ws)");
@@ -2169,7 +2305,7 @@ int ttrnn_rnn_saved_layout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace
     if (!hs_off || !cs_off) return fail("hs_off and cs_off must be non-null");
     DevInfo dv;
     CallPlan cp;
-    if (get_dev(&dv) || plan_call(d_in, dv, &cp)) return 1;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp, ws->plan[kPlanDropout] != 0)) return 1;
     if (layer < 0 || layer >= d_in->num_layers) return fail("layer %d out of range", layer);
     *hs_off = (layer == d_in->num_layers - 1) ? -1 : cp.lo.sv_hs + (long long)layer * cp.lo.BTH;
     *cs_off = (d_in->cell == TTRNN_CELL_LSTM) ? cp.lo.sv_cs + (long long)layer * cp.lo.BTH : -1;
@@ -2185,7 +2321,6 @@ int ttrnn_step_norms(const float *v, int64_t B, int32_t T, int32_t H, float *out
 }
 
 // ---- bidirectional stacks: time-reversed moves around the one-layer calls (tt_bidir.cuh) ---------------------------
-static bool aligned16(const void *p) { return ((uintptr_t)p & 15) == 0; }
 
 int ttrnn_time_reverse_add(int64_t B, int32_t T, int32_t F, const float *a, const float *r, float *y, void *stream) {
     if (B < 1 || T < 1 || F < 1) return fail("ttrnn_time_reverse_add: B, T and F must be >= 1 (got %lld, %d, %d)",

@@ -9,6 +9,8 @@ modules `pmnist_test.py` builds without `--tt` and `SpeakerEncoder` builds with 
 paper's dense-vs-TT comparison runs on the same device path (C ABI `ttrnn_dense_rnn_*`, csrc/tt_dense.cuh).
 `bidirectional=True` adds `cell{i}_reverse` per layer and runs the stack as one-layer calls per (layer, direction), as the TT
 modules do (functional.bidirectional_stack, DESIGN.md §4.17).
+`dropout=p` masks the output of every layer but the last in training mode, as torch.nn.LSTM(dropout=p) does; a stack with
+active dropout runs as one-layer calls with the mask kernel between them (DESIGN.md §4.18).
 """
 from __future__ import annotations
 
@@ -19,8 +21,9 @@ import torch
 from torch import nn
 
 from . import _lib
-from .functional import _bytes_to_floats, _dense16, _ptr, _require_cuda_f32, bidirectional_stack, \
+from .functional import _bytes_to_floats, _dense16, _ptr, _require_cuda_f32, bidirectional_stack, layer_dropout, \
     shared_bidirectional_state
+from .rnn import active_dropout, check_dropout
 
 
 class _DenseRnnFunction(torch.autograd.Function):
@@ -151,11 +154,14 @@ class _DenseRnnBase(nn.Module):
     cell_kind = ""
     cell_cls = None
 
-    def __init__(self, input_size, hidden_size, num_layers, device, bias=True, log_grads=False, bidirectional=False):
+    def __init__(self, input_size, hidden_size, num_layers, device, bias=True, log_grads=False, bidirectional=False,
+                 dropout=0.0):
+        dropout = check_dropout(dropout, num_layers)
         super().__init__()
         self.input_size, self.hidden_size, self.num_layers = input_size, hidden_size, num_layers
         self.bias, self.device, self.log_grads = bias, device, log_grads
         self.bidirectional = bool(bidirectional)
+        self.dropout = dropout
         if log_grads:
             raise NotImplementedError("log_grads=True is implemented for the TT modules (TTLSTM / TTGRU); the dense baselines "
                                       "run as one fused sequence call and expose no per-step hooks")
@@ -179,8 +185,32 @@ class _DenseRnnBase(nn.Module):
             raise NameError("name 'x' is not defined")       # the reference fails the same way on T = 0 (lstm.py:135)
         if self.bidirectional:
             return self._run_bidirectional(input, h0, c0, layer_states)
+        dropout = active_dropout(self, input.device)
+        if dropout is not None:
+            return self._run_layers(input, h0, c0, layer_states, dropout)
         return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.num_layers, bool(self.bias), layer_states, input,
                                        h0, c0, *self.flat_parameters())
+
+    def _run_layers(self, input, h0, c0, layer_states, dropout):
+        """A unidirectional stack with inter-layer dropout: one one-layer sequence call per layer, the mask kernel between
+        them (functional.layer_dropout).  layer_states: h0 / c0 (L, B, H), every layer's final states returned; else one
+        (B, H) state seeds every layer and the last layer's final states come back."""
+        states = [h0, c0] if self.cell_kind == "lstm" else [h0]
+        shape = (self.num_layers, input.size(0), self.hidden_size)
+        if layer_states:
+            for s in states:
+                if s is not None and tuple(s.shape) != shape:
+                    raise ValueError("per-layer states must have shape %s, got %s" % (shape, tuple(s.shape)))
+        inp, fins = input, []
+        for l, cell in enumerate(self._all_layers):
+            st = [None if s is None else (s[l] if layer_states else s) for s in states]
+            res = _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, 1, bool(self.bias), False, inp, *st,
+                                          *([None] if self.cell_kind == "gru" else []), *cell.flat_parameters())
+            inp = res[0] if l == self.num_layers - 1 else layer_dropout(res[0], dropout, l)
+            fins.append(res[1:])
+        if layer_states:
+            return (inp, *[torch.stack([f[k] for f in fins]) for k in range(len(states))])
+        return (inp, *fins[-1])
 
     def _run_bidirectional(self, input, h0, c0, layer_states):
         """Every (layer, direction) is a one-layer sequence call (functional.bidirectional_stack).  layer_states: h0 / c0
@@ -194,7 +224,8 @@ class _DenseRnnBase(nn.Module):
         states = [h0, c0] if self.cell_kind == "lstm" else [h0]
         if not layer_states:
             states = [shared_bidirectional_state(s, self.num_layers, input.size(0), self.hidden_size) for s in states]
-        out, fin = bidirectional_stack(input, states, self.num_layers, self.hidden_size, run)
+        out, fin = bidirectional_stack(input, states, self.num_layers, self.hidden_size, run,
+                                       dropout=active_dropout(self, input.device))
         if not layer_states:
             fin = [f[-2:] for f in fin]
         return (out, *fin)

@@ -87,15 +87,84 @@ def _step_stats(lib, v: torch.Tensor, stream) -> torch.Tensor:
     return out
 
 
+def dropout_draw(device: torch.device) -> Tuple[int, int]:
+    """(seed, offset) of one dropout mask from the device's default CUDA generator, which advances by 4 per draw: so
+    torch.manual_seed / torch.cuda.manual_seed reproduce a run and two successive calls draw different masks.  The
+    generator's offset is host state that a replayed CUDA graph would not advance, so drawing under stream capture is an
+    error."""
+    if torch.cuda.is_current_stream_capturing():
+        raise RuntimeError("tensorized_rnn_b200: dropout draws its mask offset from the CUDA generator on the host, which "
+                           "is not graph-safe; capture the module in eval mode or with dropout=0")
+    idx = device.index if device.index is not None else torch.cuda.current_device()
+    gen = torch.cuda.default_generators[idx]
+    seed, offset = int(gen.initial_seed()), int(gen.get_offset())
+    gen.set_offset(offset + 4)
+    return seed, offset
+
+
+def _dropout_struct(dropout) -> _lib.Dropout:
+    p, seed, offset = dropout
+    d = _lib.Dropout()
+    d.p, d.reserved, d.seed, d.offset = float(p), 0, int(seed) & (2 ** 64 - 1), int(offset) & (2 ** 64 - 1)
+    return d
+
+
+class _DropoutFunction(torch.autograd.Function):
+    """y = x * mask / (1 - p) of one layer boundary (ttrnn_dropout_apply), `dropout` = (p, seed, offset).  With `rev`
+    also y reversed in time (the next bidirectional layer's reverse-direction input); the backward forms
+    d_x = (dy + reverse(dy_rev)) * mask / (1 - p) in the same kernel, regenerating the mask."""
+
+    @staticmethod
+    def forward(ctx, dropout, boundary: int, rev: bool, x):
+        lib = _lib.load()
+        _require_cuda_f32("input", x)
+        x = _dense16(x)
+        B, T, F = x.shape
+        dp = _dropout_struct(dropout)
+        with torch.cuda.device(x.device):
+            y = torch.empty_like(x)
+            y_rev = torch.empty_like(x) if rev else None
+            _lib.check(lib.ttrnn_dropout_apply(B, T, F, 0, boundary, 0, C.byref(dp), _ptr(x), _ptr(y), _ptr(y_rev),
+                                               torch.cuda.current_stream(x.device).cuda_stream), "ttrnn_dropout_apply")
+        ctx.dropout, ctx.boundary = dropout, boundary
+        ctx.set_materialize_grads(False)
+        return (y, y_rev) if rev else y
+
+    @staticmethod
+    def backward(ctx, dy, dy_rev=None):
+        if dy is None and dy_rev is None:
+            return None, None, None, None
+        lib = _lib.load()
+        dy, dy_rev = _dense16(dy), _dense16(dy_rev)
+        like = dy if dy is not None else dy_rev
+        B, T, F = like.shape
+        dp = _dropout_struct(ctx.dropout)
+        with torch.cuda.device(like.device):
+            d_x = torch.empty_like(like)
+            src = dy if dy is not None else torch.zeros_like(like)
+            _lib.check(lib.ttrnn_dropout_apply(B, T, F, 0, ctx.boundary, 1, C.byref(dp), _ptr(src), _ptr(d_x), _ptr(dy_rev),
+                                               torch.cuda.current_stream(like.device).cuda_stream), "ttrnn_dropout_apply")
+        return None, None, None, d_x
+
+
+def layer_dropout(x: torch.Tensor, dropout, boundary: int, rev: bool = False):
+    """The inter-layer dropout of a stack composed of one-layer calls: the output x (B, T, F) of layer `boundary` times
+    mask / (1 - p), the mask drawn from `dropout` = (p, seed, offset) as the whole-stack call draws it (DESIGN.md
+    §4.18).  rev: returns (y, y reversed in time)."""
+    return _DropoutFunction.apply(dropout, int(boundary), bool(rev), x)
+
+
 class _RnnFunction(torch.autograd.Function):
     """`step_log` (None or an object with .activations(layer, var, stats) / .gradients(layer, var, stats)): fused
     log_grads.  The training forward reports the per-step statistics of every layer's h_t / c_t sequence, the
     backward those of the total gradients reaching them, (2, T) tensors each (reference rnn_utils.py:127-172).
     `layer_states`: h0 / c0 and the returned final states are (L, B, H), one block per layer (TTRNN_WS_LAYER_STATES);
-    else (B, H), shared by every layer on the way in and the last layer's on the way out."""
+    else (B, H), shared by every layer on the way in and the last layer's on the way out.
+    `dropout`: None, or (p, seed, offset) of the inter-layer dropout (ttrnn_rnn_forward_dropout, TTRNN_WS_DROPOUT); the
+    backward regenerates the same mask from them."""
 
     @staticmethod
-    def forward(ctx, spec: RnnSpec, grad_enabled: bool, step_log, layer_states: bool, x, h0, c0, *params):
+    def forward(ctx, spec: RnnSpec, grad_enabled: bool, step_log, layer_states: bool, dropout, x, h0, c0, *params):
         lib = _lib.load()
         _require_cuda_f32("input", x)
         for i, p in enumerate(params):
@@ -124,11 +193,12 @@ class _RnnFunction(torch.autograd.Function):
             if want != blob.numel():
                 raise RuntimeError("parameter blob has %d floats, descriptor expects %d" % (blob.numel(), want))
             ws = _lib.RnnWorkspace()
-            flags = (_lib.WS_WHOLE_BATCH if step_log is not None else 0) | (_lib.WS_LAYER_STATES if layer_states else 0)
+            flags = (_lib.WS_WHOLE_BATCH if step_log is not None else 0) | (_lib.WS_LAYER_STATES if layer_states else 0) | \
+                (_lib.WS_DROPOUT if dropout is not None else 0)
             _lib.check(lib.ttrnn_rnn_workspace_bytes_ex(C.byref(desc), flags, C.byref(ws)), "ttrnn_rnn_workspace_bytes")
             # grad mode is always off inside Function.forward and needs_input_grad stays True for nn.Parameters under
             # torch.no_grad(): the caller captures torch.is_grad_enabled() before .apply (ADVICE r1)
-            training = bool(grad_enabled) and any(ctx.needs_input_grad[4:])
+            training = bool(grad_enabled) and any(ctx.needs_input_grad[5:])
             if step_log is not None and not training:
                 raise RuntimeError("fused per-step logging needs a training forward (it reads the kept h_t / c_t sequences)")
             out = torch.empty((B, T, H), device=x.device, dtype=torch.float32)
@@ -138,9 +208,13 @@ class _RnnFunction(torch.autograd.Function):
                 if training else None
             scratch = torch.empty(_bytes_to_floats(ws.fwd_scratch_bytes), device=x.device, dtype=torch.float32)
             stream = torch.cuda.current_stream(x.device).cuda_stream
-            _lib.check(lib.ttrnn_rnn_forward(C.byref(desc), C.byref(ws), _ptr(x), _ptr(h0c), _ptr(c0c), _ptr(blob), _ptr(out),
-                                             _ptr(hT), _ptr(cT), _ptr(saved), _ptr(scratch), stream),
-                       "ttrnn_rnn_forward")
+            args = (C.byref(desc), C.byref(ws), _ptr(x), _ptr(h0c), _ptr(c0c), _ptr(blob), _ptr(out), _ptr(hT), _ptr(cT),
+                    _ptr(saved), _ptr(scratch), stream)
+            if dropout is None:
+                _lib.check(lib.ttrnn_rnn_forward(*args), "ttrnn_rnn_forward")
+            else:
+                _lib.check(lib.ttrnn_rnn_forward_dropout(*(args + (C.byref(_dropout_struct(dropout)),))),
+                           "ttrnn_rnn_forward_dropout")
             if step_log is not None:
                 hs_off, cs_off = C.c_int64(), C.c_int64()
                 for l in range(spec.num_layers):
@@ -153,6 +227,7 @@ class _RnnFunction(torch.autograd.Function):
         if training:
             ctx.spec = spec
             ctx.step_log = step_log
+            ctx.dropout = dropout
             ctx.shapes = [tuple(p.shape) for p in params]
             ctx.ws = ws                    # sizes + execution plan: backward runs from the same plan as this forward
             ctx.bwd_floats = _bytes_to_floats(ws.bwd_scratch_bytes)
@@ -180,17 +255,20 @@ class _RnnFunction(torch.autograd.Function):
         d_cT = _dense16(d_cT)
         with torch.cuda.device(x.device):
             d_blob = torch.empty_like(blob)
-            d_x = torch.empty_like(x) if ctx.needs_input_grad[4] else None
+            d_x = torch.empty_like(x) if ctx.needs_input_grad[5] else None
             d_h0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
-                if (ctx.has_h0 and ctx.needs_input_grad[5]) else None
+                if (ctx.has_h0 and ctx.needs_input_grad[6]) else None
             d_c0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
-                if (spec.cell == "lstm" and ctx.has_c0 and ctx.needs_input_grad[6]) else None
+                if (spec.cell == "lstm" and ctx.has_c0 and ctx.needs_input_grad[7]) else None
             scratch = torch.empty(ctx.bwd_floats, device=x.device, dtype=torch.float32)
             stream = torch.cuda.current_stream(x.device).cuda_stream
             args = (C.byref(desc), C.byref(ctx.ws), _ptr(x), _ptr(h0), _ptr(c0), _ptr(blob), _ptr(out),
                     _ptr(saved), _ptr(d_out), _ptr(d_hT), _ptr(d_cT), _ptr(d_blob),
                     _ptr(d_x), _ptr(d_h0), _ptr(d_c0), _ptr(scratch), stream)
-            if ctx.step_log is None:
+            if ctx.dropout is not None:
+                _lib.check(lib.ttrnn_rnn_backward_dropout(*(args + (C.byref(_dropout_struct(ctx.dropout)),))),
+                           "ttrnn_rnn_backward_dropout")
+            elif ctx.step_log is None:
                 _lib.check(lib.ttrnn_rnn_backward(*args), "ttrnn_rnn_backward")
             else:
                 L = spec.num_layers
@@ -207,19 +285,23 @@ class _RnnFunction(torch.autograd.Function):
             n = 1
             for v in shp:
                 n *= v
-            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[7 + i] else None)
+            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[8 + i] else None)
             off += n
-        return (None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
+        return (None, None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
 
 
 def rnn_sequence(spec: RnnSpec, x: torch.Tensor, h0: Optional[torch.Tensor], c0: Optional[torch.Tensor],
-                 params: Sequence[torch.Tensor], step_log=None, layer_states: bool = False):
+                 params: Sequence[torch.Tensor], step_log=None, layer_states: bool = False, dropout=None):
     """Run the whole stack over the whole sequence.  Returns (out, hT[, cT]).  `step_log`: see _RnnFunction.
     `layer_states=True`: h0 / c0 and the returned hT / cT are (num_layers, batch, hidden), one state per layer, so that
-    the final states of one call can seed the next call over the rest of the sequence."""
+    the final states of one call can seed the next call over the rest of the sequence.
+    `dropout`: None, or (p, seed, offset) (dropout_draw): the output of every layer but the last is multiplied by
+    mask / (1 - p) before the next layer reads it (DESIGN.md §4.18)."""
     if x.dim() != 3:
         raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
-    return _RnnFunction.apply(spec, torch.is_grad_enabled(), step_log, bool(layer_states), x, h0, c0, *params)
+    if dropout is not None and step_log is not None:
+        raise NotImplementedError("inter-layer dropout has no fused per-step logging form")
+    return _RnnFunction.apply(spec, torch.is_grad_enabled(), step_log, bool(layer_states), dropout, x, h0, c0, *params)
 
 
 # ---- bidirectional stacks (DESIGN.md §4.17) --------------------------------------------------------------------------
@@ -313,7 +395,7 @@ def shared_bidirectional_state(state: Optional[torch.Tensor], num_layers: int, b
 
 
 def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]], num_layers: int, hidden_size: int,
-                        run):
+                        run, dropout=None):
     """A bidirectional stack composed of one-layer calls, the contract of torch.nn.LSTM / GRU(bidirectional=True).
 
     `run(layer, direction, x, *states)` runs direction 0 (forward) or 1 (reverse) of one layer over x (B, T, F) from its
@@ -326,7 +408,10 @@ def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]
     direction is issued on a side stream forked from the caller's current stream and joined back into it with events,
     so that the two directions of a layer run concurrently.  Autograd runs each backward on the stream of its forward,
     so the two directions' backward passes overlap as well, and it synchronises (and records) the gradients it hands
-    from one stream to the other; the forward's own cross-stream tensors are recorded here."""
+    from one stream to the other; the forward's own cross-stream tensors are recorded here.
+    `dropout`: None, or (p, seed, offset): the joined (B, T, 2H) output of every layer but the last is masked (boundary =
+    layer index) before the next layer's two directions read it; the reverse direction sees the masked values reversed
+    in time."""
     if x.dim() != 3:
         raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
     _require_cuda_f32("input", x)
@@ -360,6 +445,8 @@ def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]
             last = l == num_layers - 1
             if last:
                 out = _BidirJoinFunction.apply(True, res_f[0], res_r[0])
+            elif dropout is not None:
+                inp_f, inp_r = layer_dropout(_BidirJoinFunction.apply(True, res_f[0], res_r[0]), dropout, l, rev=True)
             else:
                 inp_f, inp_r = _BidirJoinFunction.apply(False, res_f[0], res_r[0])
             finals.append((res_f[1:], res_r[1:]))

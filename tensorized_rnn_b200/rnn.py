@@ -25,19 +25,47 @@ Two execution modes, chosen per module:
 `bidirectional=True` (no reference counterpart; the contract of torch.nn.LSTM(bidirectional=True)) adds a reverse cell
 per layer, `cell{i}_reverse`, and runs every (layer, direction) as a one-layer sequence call, the two directions of a
 layer on two streams (functional.bidirectional_stack, DESIGN.md §4.17).  It needs the fused mode.
+
+`dropout=p` (no reference counterpart; the contract of torch.nn.LSTM(dropout=p)): in training mode the output sequence of
+every layer but the last is multiplied by a Bernoulli(1 - p) mask / (1 - p) before the next layer reads it, inside the
+stack call (DESIGN.md §4.18).  It needs the fused mode as well.
 """
 from __future__ import annotations
 
+import numbers
+import warnings
 from typing import List, Optional
 
 import torch
 from torch import nn
 
-from .functional import RnnSpec, bidirectional_stack, rnn_sequence, shared_bidirectional_state
+from .functional import RnnSpec, bidirectional_stack, dropout_draw, rnn_sequence, shared_bidirectional_state
 from .functional import cell_step
 from .layers import TTLinear, TTLinearSet
 from .rnn_utils import ActivGradLogger
 from .shapes import tt_shape
+
+
+def check_dropout(dropout, num_layers: int) -> float:
+    """torch.nn.LSTM's validation of `dropout`: a number in [0, 1], with a warning when there is no layer boundary."""
+    if isinstance(dropout, bool) or not isinstance(dropout, numbers.Number) or not 0 <= dropout <= 1:
+        raise ValueError("dropout should be a number in range [0, 1] representing the probability of an element being "
+                         "zeroed, got %r" % (dropout,))
+    if dropout > 0 and num_layers == 1:
+        warnings.warn("dropout option adds dropout after all but last recurrent layer, so non-zero dropout expects "
+                      "num_layers greater than 1, but got dropout=%s and num_layers=%d" % (dropout, num_layers))
+    return float(dropout)
+
+
+def active_dropout(module: nn.Module, device: torch.device):
+    """(p, seed, offset) of this call's inter-layer dropout, or None: dropout > 0, training mode (also under no_grad, as
+    torch.nn.LSTM), more than one layer.  Draws the mask from the device's CUDA generator."""
+    if module.dropout > 0 and module.training and module.num_layers > 1:
+        if device.type != "cuda":
+            return (module.dropout, 0, 0)          # the engine rejects the CPU tensors itself
+        seed, offset = dropout_draw(device)
+        return (module.dropout, seed, offset)
+    return None
 
 
 class _StepLogSink(object):
@@ -166,11 +194,15 @@ class _TTRNNBase(nn.Module):
     cell_kind = ""
 
     def __init__(self, input_size, hidden_size, num_layers, device, n_cores, tt_rank, bias=True,
-                 is_naive=False, log_grads=False, new_core=None, bidirectional=False):
+                 is_naive=False, log_grads=False, new_core=None, bidirectional=False, dropout=0.0):
         assert new_core in [None, 'first', 'last']
         if bidirectional and (is_naive or log_grads):
             raise NotImplementedError("bidirectional=True runs on the sequence kernels only; is_naive=True and "
                                       "log_grads=True need the cell-step mode, which has no bidirectional form")
+        dropout = check_dropout(dropout, num_layers)
+        if dropout > 0 and (is_naive or log_grads):
+            raise NotImplementedError("dropout > 0 runs on the sequence kernels only; is_naive=True and log_grads=True "
+                                      "need the cell-step mode, which has no dropout form")
         super().__init__()
         self.n_cores = n_cores
         self.tt_rank = tt_rank
@@ -183,6 +215,7 @@ class _TTRNNBase(nn.Module):
         self.device = device
         self.log_grads = log_grads
         self.bidirectional = bool(bidirectional)
+        self.dropout = dropout
         self._all_layers = []
         for i in range(self.num_layers):
             cell = self._create_first_layer_cell() if i == 0 else self._create_other_layer_cell()
@@ -279,7 +312,8 @@ class _TTRNNBase(nn.Module):
             cell = self._all_layers[2 * layer + direction]
             return rnn_sequence(cell._single_step_spec(), x, h0, c0, cell.flat_parameters())
 
-        return bidirectional_stack(input, states, self.num_layers, self.hidden_size, run)
+        return bidirectional_stack(input, states, self.num_layers, self.hidden_size, run,
+                                   dropout=active_dropout(self, input.device))
 
     def _shared_to_bidirectional(self, input, state):
         return shared_bidirectional_state(state, self.num_layers, input.size(0), self.hidden_size)
@@ -323,7 +357,8 @@ class TTLSTM(_TTRNNBase):
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, init_states)
         h0, c0 = (None, None) if init_states is None else init_states
-        out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink)
+        out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink,
+                                 dropout=active_dropout(self, input.device))
         return out, (h, c)
 
     def forward_states(self, input, states=None):
@@ -341,7 +376,8 @@ class TTLSTM(_TTRNNBase):
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, states, layer_states=True)
         h0, c0 = (None, None) if states is None else states
-        out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink, layer_states=True)
+        out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink, layer_states=True,
+                                 dropout=active_dropout(self, input.device))
         return out, (h, c)
 
     def _forward_cell_steps(self, input, init_states, layer_states=False):
@@ -390,7 +426,8 @@ class TTGRU(_TTRNNBase):
         sink = self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, init_states)
-        out, h = rnn_sequence(self.spec(), input, init_states, None, self.flat_parameters(), step_log=sink)
+        out, h = rnn_sequence(self.spec(), input, init_states, None, self.flat_parameters(), step_log=sink,
+                              dropout=active_dropout(self, input.device))
         return out, h
 
     def forward_states(self, input, states=None):
@@ -404,7 +441,8 @@ class TTGRU(_TTRNNBase):
         sink = self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, states, layer_states=True)
-        return rnn_sequence(self.spec(), input, states, None, self.flat_parameters(), step_log=sink, layer_states=True)
+        return rnn_sequence(self.spec(), input, states, None, self.flat_parameters(), step_log=sink, layer_states=True,
+                            dropout=active_dropout(self, input.device))
 
     def _forward_cell_steps(self, input, init_states, layer_states=False):
         """The reference's own loop (gru.py:119-136); `layer_states` as for TTLSTM."""
