@@ -38,7 +38,10 @@ extern "C" {
                                  Still 4 with bidirectional stacks: two new symbols (ttrnn_time_reverse_add,
                                  ttrnn_bidir_join), nothing existing changes.  Still 4 with inter-layer dropout: one more
                                  flag value (TTRNN_WS_DROPOUT), one struct and three new symbols (ttrnn_rnn_forward_dropout,
-                                 ttrnn_rnn_backward_dropout, ttrnn_dropout_apply) */
+                                 ttrnn_rnn_backward_dropout, ttrnn_dropout_apply).  Still 4 with projected LSTM stacks:
+                                 one more flag value (TTRNN_WS_PROJ), one struct and four new symbols
+                                 (ttrnn_rnn_param_count_proj, ttrnn_rnn_workspace_bytes_proj, ttrnn_rnn_forward_proj,
+                                 ttrnn_rnn_backward_proj) */
 #define TTRNN_MAX_CORES   6
 #define TTRNN_MAX_LAYERS  8
 
@@ -193,6 +196,44 @@ int ttrnn_rnn_backward_dropout(const ttrnn_rnn_desc *desc, const ttrnn_rnn_works
                                void *scratch, void *stream, const ttrnn_dropout *dp);
 int ttrnn_dropout_apply(int64_t B, int32_t T, int32_t F, int64_t row0, int32_t boundary, int32_t backward,
                         const ttrnn_dropout *dp, const float *x, float *y, float *y_rev, void *stream);
+
+/* Projected LSTM stacks (LSTMP), the `proj_size` of torch.nn.LSTM: each layer computes m_t = o_t * tanh(c_t) (H wide) and
+ * outputs h_t = W_hr m_t (P < H wide), which is also the next step's hh input.  W_hr of layer l is a TT matrix P x H
+ * without bias; the recurrent kernels contract it between the gate math of one step and the hh chain of the next.
+ *
+ *   - desc->cell must be TTRNN_CELL_LSTM; desc->hh[l] is 4H x P, desc->ih[l] for l >= 1 is 4H x P.
+ *   - Parameter blob, per layer: [ih cores][ih bias][hh cores][hh bias][hr cores], the order of the state_dict keys
+ *     ..., cell{l}.hidden_weights.bias, cell{l}.projection_weights.parameters.{k}.
+ *   - Every h-state buffer is P wide: out (B, T, P), h0, hT, d_hT, d_h0 (B, P).  The c-state buffers c0, cT, d_cT, d_c0
+ *     stay (B, H).  Under TTRNN_WS_LAYER_STATES the layer stride is B * P for the h states and B * H for the c states.
+ *   - The plan comes from ttrnn_rnn_workspace_bytes_proj (flags as for ttrnn_rnn_workspace_bytes_ex; TTRNN_WS_PROJ is
+ *     implied, TTRNN_WS_WHOLE_BATCH has no effect: a projected plan is always one row group).  ttrnn_rnn_forward /
+ *     _backward / _forward_dropout / _backward_dropout / _backward_logged / ttrnn_rnn_saved_layout refuse such a plan, and
+ *     ttrnn_rnn_workspace_bytes_ex refuses the flag; the _proj calls refuse a plan without it, a GRU descriptor, a NULL
+ *     `pj` and hr shapes that are not P x H.
+ *   - `dp` may be NULL (no dropout).  With TTRNN_WS_DROPOUT the masked layer inputs kept in `saved` take
+ *     (L-1) * B * T * P floats and the mask covers the P-wide layer output.
+ *   - Projected layers run on the runtime-shape recurrent kernels (k_rnn_fwd_proj / k_rnn_bwd_proj); no statically
+ *     specialised kernel and no rank padding applies to them. */
+#define TTRNN_WS_PROJ 8
+typedef struct ttrnn_rnn_proj {
+    int32_t proj_size;                   /* P >= 1, P < hidden_size; desc->cell must be TTRNN_CELL_LSTM */
+    int32_t reserved;                    /* 0                                                           */
+    ttrnn_tt_shape hr[TTRNN_MAX_LAYERS]; /* W_hr of layer l: P x H                                      */
+} ttrnn_rnn_proj;
+int64_t ttrnn_rnn_param_count_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_proj *pj);
+int ttrnn_rnn_workspace_bytes_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_proj *pj, int32_t flags,
+                                   ttrnn_rnn_workspace *ws);
+int ttrnn_rnn_forward_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
+                           const float *x, const float *h0, const float *c0,
+                           const float *params, float *out, float *hT, float *cT,
+                           void *saved, void *scratch, void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp);
+int ttrnn_rnn_backward_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
+                            const float *x, const float *h0, const float *c0,
+                            const float *params, const float *out, const void *saved,
+                            const float *d_out, const float *d_hT, const float *d_cT,
+                            float *d_params, float *d_x, float *d_h0, float *d_c0,
+                            void *scratch, void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp);
 
 /* Bidirectional stacks (the contract of torch.nn.LSTM(bidirectional=True)).  The library has no whole-stack
  * bidirectional call: the reverse direction of a layer is the ordinary one-layer ttrnn_rnn_forward / _backward (or

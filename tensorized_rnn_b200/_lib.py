@@ -17,6 +17,7 @@ PLAN_WORDS = 24
 WS_WHOLE_BATCH = 1
 WS_LAYER_STATES = 2      # per-layer (L, B, H) initial / final states and their gradients
 WS_DROPOUT = 4           # inter-layer dropout: saved keeps the masked inputs of layers 1 .. L-1
+WS_PROJ = 8              # projected LSTM (proj_size): the plan of the _proj entry points
 CELL_LSTM, CELL_GRU = 0, 1
 
 _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc", "libttrnn_b200.so")
@@ -53,6 +54,10 @@ class Dropout(C.Structure):
     _fields_ = [("p", C.c_float), ("reserved", C.c_int32), ("seed", C.c_uint64), ("offset", C.c_uint64)]
 
 
+class RnnProj(C.Structure):
+    _fields_ = [("proj_size", C.c_int32), ("reserved", C.c_int32), ("hr", TTShape * MAX_LAYERS)]
+
+
 # every symbol include/ttrnn_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -72,6 +77,12 @@ SYMBOLS = {
     "ttrnn_rnn_forward_dropout": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 10 + [C.POINTER(Dropout)]),
     "ttrnn_rnn_backward_dropout": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 15 +
                                    [C.POINTER(Dropout)]),
+    "ttrnn_rnn_param_count_proj": (C.c_int64, [C.POINTER(RnnDesc), C.POINTER(RnnProj)]),
+    "ttrnn_rnn_workspace_bytes_proj": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnProj), C.c_int32, C.POINTER(RnnWorkspace)]),
+    "ttrnn_rnn_forward_proj": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 10 +
+                               [C.POINTER(RnnProj), C.POINTER(Dropout)]),
+    "ttrnn_rnn_backward_proj": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 15 +
+                                [C.POINTER(RnnProj), C.POINTER(Dropout)]),
     "ttrnn_dropout_apply": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.POINTER(Dropout),
                                       _P, _P, _P, _P]),
     "ttrnn_ttlinear_param_count": (C.c_int64, [C.POINTER(TTShape)]),

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "tt_kernels.cuh"
+#include "tt_proj.cuh"
 #include "tt_cell.cuh"
 #include "tt_gemm.cuh"
 #include "tt_tc.cuh"
@@ -81,10 +82,10 @@ constexpr int kOptFields = sizeof(Opts) / sizeof(long long);
 constexpr long long kPlanMagic = 0x7474726E6E706C36LL;          // "ttrnnpl6"
 // plan words: [0] magic, [1 .. kOptFields] options, then the row-group split (group count, rows of group 0), then 1 when
 // the state buffers are per layer (TTRNN_WS_LAYER_STATES), then 1 when `saved` keeps the masked layer inputs of the
-// dropout entry points (TTRNN_WS_DROPOUT)
+// dropout entry points (TTRNN_WS_DROPOUT), then 1 when the plan is for the projected entry points (TTRNN_WS_PROJ)
 constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2, kPlanLayerStates = kOptFields + 3,
-              kPlanDropout = kOptFields + 4;
-static_assert(kOptFields + 5 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
+              kPlanDropout = kOptFields + 4, kPlanProj = kOptFields + 5;
+static_assert(kOptFields + 6 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
 thread_local Opts t_opt;
 inline int merge_fwd() { return t_opt.merge_cores >= 2 ? 1 : 0; }    // contracted forward variants (merge_cores = 2)
 inline int merge_bwd() { return t_opt.merge_cores >= 1 ? 1 : 0; }    // contracted dX-only BPTT variants (merge_cores >= 1)
@@ -184,12 +185,16 @@ int get_dev(DevInfo *d) {
 // (lstm.py:120-121,135): one (B, H) block seeds every layer, only the last layer's final state comes back and takes an
 // upstream gradient, and d_h0 / d_c0 receive the sum over layers.  stride > 0 (TTRNN_WS_LAYER_STATES): every state buffer
 // is (L, B, H) and layer l's block starts l * stride floats in.  The stride is the FULL batch's B * H, also inside a row
-// group, whose pointers the entry points have already moved to the group's first row.
+// group, whose pointers the entry points have already moved to the group's first row.  With a projection the h-state
+// blocks are B * P and the c-state blocks B * H: `c` selects the c-state stride.
 struct StateMap {
-    long long stride = 0;
-    template <class P> P init(P p, int l) const { return (p && stride) ? p + l * stride : p; }               // h0, c0, d_h0, d_c0
-    template <class P> P fin(P p, int l, int L) const {                                                       // hT, cT, d_hT, d_cT
-        if (stride) return p ? p + l * stride : p;
+    long long stride = 0, cstride = 0;
+    template <class P> P init(P p, int l, bool c = false) const {                                             // h0, c0, d_h0, d_c0
+        const long long s = c ? cstride : stride;
+        return (p && s) ? p + l * s : p;
+    }
+    template <class P> P fin(P p, int l, int L, bool c = false) const {                                       // hT, cT, d_hT, d_cT
+        if (stride) return p ? p + l * (c ? cstride : stride) : p;
         return l == L - 1 ? p : nullptr;
     }
 };
@@ -297,6 +302,53 @@ int plan_bwd(const ChainPlan &base, Fixed fixed_floats, const DevInfo &dv, long 
     return 0;
 }
 
+// projected LSTM: footprints of k_rnn_fwd_proj / k_rnn_bwd_proj (tt_proj.cuh), hh chain p and projection chain q
+long long smem_rnn_fwd_proj(const ChainPlan &p, const ChainPlan &q, int R, int H) {
+    const long long pp0 = p.pp_floats[0] > q.pp_floats[0] ? p.pp_floats[0] : q.pp_floats[0];
+    const long long pp1 = p.pp_floats[1] > q.pp_floats[1] ? p.pp_floats[1] : q.pp_floats[1];
+    return p.w_floats + q.w_floats + r4((long long)R * H) + r4((long long)R * 4 * H) +
+           (long long)R * (p.g_BS + p.in_BS + q.in_BS + q.g_BS + pp0 + pp1);
+}
+long long smem_rnn_bwd_proj_fixed(const ChainPlan &p, const ChainPlan &q, int R, int H, int P) {
+    return 2LL * (p.w_floats + q.w_floats) + (long long)R * (p.g_BS + q.g_BS + p.in_BS) + r4((long long)R * 4 * H) +
+           r4((long long)R * P) + 2 * r4((long long)R * H);
+}
+struct BwdProjCfg {
+    ChainPlan p, q;         // plans with the slot placement applied
+    int R = 0;
+    size_t smem = 0;        // bytes
+    long long spill = 0;    // floats of global spill per CTA (both chains)
+};
+// plan_bwd for the two chains of k_rnn_bwd_proj: when their kept X_k slots do not fit one row per CTA, the projection
+// chain's largest slots move to the spill area first, then the hh chain's
+int plan_bwd_proj(const ChainPlan &p, const ChainPlan &q, int H, int P, const DevInfo &dv, long long units, BwdProjCfg *c) {
+    c->p = p;
+    c->q = q;
+    auto fixed = [&](int r) { return smem_rnn_bwd_proj_fixed(p, q, r, H, P); };
+    auto total = [&](int r) { return fixed(r) + (long long)r * (p.all_floats + q.all_floats); };
+    int R = pick_rows(total, dv.smem_optin, 8, units, dv.sms, 2);
+    if (R > 0) {
+        c->R = R;
+        c->smem = (size_t)total(R) * 4;
+        c->spill = 0;
+        return 0;
+    }
+    const long long budget = dv.smem_optin / 4 - fixed(1);
+    if (budget < 0)
+        return fail("projected hh backward: cores alone need %lld bytes of shared memory (limit %d): unsupported TT shape",
+                    fixed(1) * 4, dv.smem_optin);
+    if (budget >= p.all_floats) {
+        tt_place_slots(&c->q, budget - p.all_floats);
+    } else {
+        tt_place_slots(&c->q, 0);
+        tt_place_slots(&c->p, budget);
+    }
+    c->R = 1;
+    c->smem = (size_t)(fixed(1) + c->p.all_floats + c->q.all_floats) * 4;
+    c->spill = c->p.spill_floats + c->q.spill_floats;
+    return 0;
+}
+
 template <class K>
 int grid_for(K kernel, size_t smem_bytes, long long ntiles, const DevInfo &dv, int *grid) {
     CU_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
@@ -314,15 +366,20 @@ constexpr int kMaxSlotsPerSM = 4;
 // ---- descriptor validation / parameter blob layout -----------------------------------------
 struct LayerPlan {
     ChainPlan ih, hh;
+    ChainPlan hr;                                                     // projection W_hr (H -> P), when P > 0
     long long off_ih_cores, off_ih_bias, off_hh_cores, off_hh_bias;   // floats into the blob
+    long long off_hr_cores;
 };
 struct RnnPlan {
     int G = 0;
+    int P = 0;               // projection size (TTRNN_WS_PROJ); 0 = none, the layer output is H wide
     long long param_floats = 0;
     LayerPlan layer[TTRNN_MAX_LAYERS];
+    int out_width(const ttrnn_rnn_desc *d) const { return P ? P : d->hidden_size; }
 };
 
-int build_rnn_plan(const ttrnn_rnn_desc *d, RnnPlan *rp) {
+// pj: the projection of the _proj entry points, or nullptr
+int build_rnn_plan(const ttrnn_rnn_desc *d, RnnPlan *rp, const ttrnn_rnn_proj *pj = nullptr) {
     if (!d) return fail("null descriptor");
     if (d->cell != TTRNN_CELL_LSTM && d->cell != TTRNN_CELL_GRU) return fail("unknown cell kind %d", d->cell);
     if (d->num_layers < 1 || d->num_layers > TTRNN_MAX_LAYERS)
@@ -330,7 +387,14 @@ int build_rnn_plan(const ttrnn_rnn_desc *d, RnnPlan *rp) {
     if (d->input_size < 1 || d->hidden_size < 1) return fail("input_size / hidden_size must be positive");
     if (d->batch < 1 || d->seq_len < 1) return fail("batch and seq_len must be >= 1 (got %lld, %d)", (long long)d->batch, d->seq_len);
     rp->G = gates_of(d->cell);
-    const int GH = rp->G * d->hidden_size;
+    rp->P = 0;
+    if (pj) {
+        if (d->cell != TTRNN_CELL_LSTM) return fail("a projection (proj_size) needs an LSTM descriptor");
+        if (pj->proj_size < 1 || pj->proj_size >= d->hidden_size)
+            return fail("proj_size %d out of range [1, hidden_size %d)", pj->proj_size, d->hidden_size);
+        rp->P = pj->proj_size;
+    }
+    const int GH = rp->G * d->hidden_size, W = rp->out_width(d);
     long long off = 0;
     for (int l = 0; l < d->num_layers; ++l) {
         LayerPlan &lp = rp->layer[l];
@@ -338,15 +402,24 @@ int build_rnn_plan(const ttrnn_rnn_desc *d, RnnPlan *rp) {
         if (rc) return fail("layer %d: malformed ih TT shape (code %d)", l, rc);
         rc = tt_build_plan(&d->hh[l], &lp.hh);
         if (rc) return fail("layer %d: malformed hh TT shape (code %d)", l, rc);
-        const int want_in = (l == 0) ? d->input_size : d->hidden_size;
+        const int want_in = (l == 0) ? d->input_size : W;
         if (lp.ih.n_in != want_in || lp.ih.n_out != GH)
             return fail("layer %d: ih TT matrix is %d x %d, expected %d x %d", l, lp.ih.n_out, lp.ih.n_in, GH, want_in);
-        if (lp.hh.n_in != d->hidden_size || lp.hh.n_out != GH)
-            return fail("layer %d: hh TT matrix is %d x %d, expected %d x %d", l, lp.hh.n_out, lp.hh.n_in, GH, d->hidden_size);
+        if (lp.hh.n_in != W || lp.hh.n_out != GH)
+            return fail("layer %d: hh TT matrix is %d x %d, expected %d x %d", l, lp.hh.n_out, lp.hh.n_in, GH, W);
         lp.off_ih_cores = off; off += lp.ih.core_floats;
         lp.off_ih_bias = off;  if (d->has_bias) off += GH;
         lp.off_hh_cores = off; off += lp.hh.core_floats;
         lp.off_hh_bias = off;  if (d->has_bias) off += GH;
+        lp.off_hr_cores = off;
+        if (rp->P) {
+            rc = tt_build_plan(&pj->hr[l], &lp.hr);
+            if (rc) return fail("layer %d: malformed hr TT shape (code %d)", l, rc);
+            if (lp.hr.n_in != d->hidden_size || lp.hr.n_out != rp->P)
+                return fail("layer %d: hr TT matrix is %d x %d, expected %d x %d", l, lp.hr.n_out, lp.hr.n_in, rp->P,
+                            d->hidden_size);
+            off += lp.hr.core_floats;
+        }
     }
     rp->param_floats = off;
     return 0;
@@ -361,9 +434,10 @@ inline int layer_mode(const ttrnn_rnn_desc *d, int l) {
     return (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
 }
 
-// statically specialised forward kernel of layer l at B rows on `sms` SMs, or nullptr (runtime-shape kernel)
-const TtsRnnFwdEntry *fwd_route(const ttrnn_rnn_desc *d, int l, long long B, int sms) {
-    if (!t_opt.stat) return nullptr;
+// statically specialised forward kernel of layer l at B rows on `sms` SMs, or nullptr (runtime-shape kernel).  A projected
+// layer has none: its chains run on the runtime-shape kernels k_rnn_fwd_proj / k_rnn_bwd_proj.
+const TtsRnnFwdEntry *fwd_route(const ttrnn_rnn_desc *d, const RnnPlan &rp, int l, long long B, int sms) {
+    if (!t_opt.stat || rp.P) return nullptr;
     return tts_find_rnn_fwd(&d->hh[l], d->cell, layer_mode(d, l), B, sms, (int)t_opt.srows_fwd, merge_fwd());
 }
 
@@ -401,17 +475,22 @@ __global__ void __launch_bounds__(256) k_unpad_cores(const __grid_constant__ Pad
 
 struct EffDesc {
     ttrnn_rnn_desc d;          // descriptor the kernels run on (padded ranks when `padded`)
+    bool proj = false;         // + the projection `pj` (TTRNN_WS_PROJ)
+    ttrnn_rnn_proj pj;
     bool padded = false;
     PadTable tab;
     long long pad_floats = 0;  // floats of the padded parameter blob
 };
 
-int make_eff_desc(const ttrnn_rnn_desc *d, const DevInfo *dv, EffDesc *e) {
+// pj: a projected stack is never padded (no static kernel would take it)
+int make_eff_desc(const ttrnn_rnn_desc *d, const ttrnn_rnn_proj *pj, const DevInfo *dv, EffDesc *e) {
     e->d = *d;
     e->padded = false;
     e->pad_floats = 0;
     e->tab.n = 0;
-    if (!t_opt.stat || !t_opt.rank_pad || !dv) return 0;
+    e->proj = pj != nullptr;
+    if (pj) e->pj = *pj;
+    if (!t_opt.stat || !t_opt.rank_pad || !dv || pj) return 0;
     RnnPlan real;
     if (build_rnn_plan(d, &real)) return 1;
     bool any = false;
@@ -426,7 +505,7 @@ int make_eff_desc(const ttrnn_rnn_desc *d, const DevInfo *dv, EffDesc *e) {
         }
     if (!any) return 0;
     for (int l = 0; l < d->num_layers; ++l)
-        if (!fwd_route(&p, l, d->batch, dv->sms)) return 0;     // padding would not reach a static kernel
+        if (!fwd_route(&p, real, l, d->batch, dv->sms)) return 0;     // padding would not reach a static kernel
     RnnPlan pad;
     if (build_rnn_plan(&p, &pad)) return 0;
     const int GH = real.G * d->hidden_size;
@@ -501,7 +580,7 @@ struct BwdRoute {
 int bwd_route(const ttrnn_rnn_desc *d, const RnnPlan &rp, int l, int mode, long long B, int sms, bool kept, long long Tc,
               BwdRoute *r) {
     *r = BwdRoute();
-    if (!t_opt.stat) return 0;
+    if (!t_opt.stat || rp.P) return 0;
     const ttrnn_tt_shape *hh = &d->hh[l];
     const int srows = (int)t_opt.srows_bwd;
     const TtsRnnBwdEntry *be = tts_find_rnn_bwd(hh, d->cell, mode, B, sms, srows, 0, 0, merge_bwd());
@@ -554,6 +633,7 @@ long long dense_bwd_floats(const ChainPlan &ih) {
 struct RnnLayout {
     int Tc = 0;                 // timesteps per chunk
     long long BTH = 0, BH = 0;
+    long long BTW = 0, BW = 0;  // the same for a layer's output width W: P with a projection (h_t, its gradients), else H
     long long xg_floats = 0;
     // saved (floats)
     long long sv_hs = 0, sv_cs = 0, sv_total = 0;
@@ -577,9 +657,11 @@ struct RnnLayout {
 
 int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, RnnLayout *lo, bool keep_masked) {
     const long long B = d->batch, T = d->seq_len, H = d->hidden_size, L = d->num_layers;
-    const long long GH = (long long)rp.G * H;
+    const long long GH = (long long)rp.G * H, W = rp.out_width(d);
     lo->BTH = B * T * H;
     lo->BH = B * H;
+    lo->BTW = B * T * W;
+    lo->BW = B * W;
     long long tc = t_opt.chunk;
     if (tc <= 0) {
         tc = t_opt.chunk_bytes / (B * GH * 4);
@@ -591,7 +673,7 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
     const bool lstm = d->cell == TTRNN_CELL_LSTM;
     // saved: inner-layer outputs, then cell states of every layer
     lo->sv_hs = 0;
-    lo->sv_cs = r4((L - 1) * lo->BTH);
+    lo->sv_cs = r4((L - 1) * lo->BTW);
     lo->sv_total = lo->sv_cs + (lstm ? r4(L * lo->BTH) : 0);
     // kept gate activations of the static recurrent kernels ("save_u_bytes" budget, default 16 GiB): 4*H floats per row
     // and step (LSTM i,f,g,o; GRU r,z,n,u_n) -- backward skips the final stage of the recompute and all gate math.  Every
@@ -605,7 +687,7 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
             if (bwd_route(d, rp, l, layer_mode(d, l), B, dv.sms, false, tc, &recompute) ||
                 bwd_route(d, rp, l, layer_mode(d, l), B, dv.sms, true, tc, &keep))
                 return 1;
-            can_keep[l] = keep.kept && fwd_route(d, l, B, dv.sms);
+            can_keep[l] = keep.kept && fwd_route(d, rp, l, B, dv.sms);
             if (can_keep[l]) kept_floats += r4(B * T * 4 * H);
             if ((recompute.dense_hh || keep.dense_hh) && dense_bwd_floats(rp.layer[l].hh) > dhh)
                 dhh = dense_bwd_floats(rp.layer[l].hh);
@@ -616,13 +698,13 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
         if (lo->kept[l]) { lo->sv_u[l] = lo->sv_total; lo->sv_total += r4(B * T * 4 * H); }
     }
     lo->masked = keep_masked && L > 1;
-    if (lo->masked) { lo->sv_drop = lo->sv_total; lo->sv_total += r4((L - 1) * lo->BTH); }
+    if (lo->masked) { lo->sv_drop = lo->sv_total; lo->sv_total += r4((L - 1) * lo->BTW); }
     // forward scratch
     long long o = 0;
     lo->f_xg = o; o += lo->xg_floats;
-    lo->f_sh = o; o += r4(lo->BH);
+    lo->f_sh = o; o += r4(lo->BW);
     lo->f_sc = o; o += r4(lo->BH);
-    lo->f_hs = o; o += (L > 1 ? 2 * r4(lo->BTH) : 0);     // used only when nothing is saved
+    lo->f_hs = o; o += (L > 1 ? 2 * r4(lo->BTW) : 0);     // used only when nothing is saved
     lo->f_aux = o; o += r4(GH) + 4;                       // rank-one input mode: dense W_ih column + a 1.0f
     long long dfw = 0, dbw = 0;                           // dense ih route: identity, W^T (+ W, dW^T, split partials)
     for (int l = 0; l < L; ++l)
@@ -631,20 +713,21 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
             if (dense_bwd_floats(rp.layer[l].ih) > dbw) dbw = dense_bwd_floats(rp.layer[l].ih);
         }
     lo->f_dense = o; o += dfw;
-    lo->f_drop = o; o += lo->masked ? r4(lo->BTH) : 0;
+    lo->f_drop = o; o += lo->masked ? r4(lo->BTW) : 0;
     lo->f_total = o;
     // backward scratch
     long long maxp = 0;
     for (int l = 0; l < L; ++l) {
         long long a = rp.layer[l].ih.core_floats + GH, b = rp.layer[l].hh.core_floats + 3 * GH;
+        if (rp.P) b += rp.layer[l].hr.core_floats;
         if (a > maxp) maxp = a;
         if (b > maxp) maxp = b;
     }
     lo->part_stride = r4(maxp);
     lo->nslots = dv.sms * kMaxSlotsPerSM;
     o = 0;
-    lo->b_dhs = o; o += (L > 1 ? 2 * r4(lo->BTH) : 0);
-    lo->b_sdh = o; o += r4(lo->BH);
+    lo->b_dhs = o; o += (L > 1 ? 2 * r4(lo->BTW) : 0);
+    lo->b_sdh = o; o += r4(lo->BW);
     lo->b_sdc = o; o += r4(lo->BH);
     const long long set_base = o;                         // per-layer buffers from here on
     lo->b_xg = o; o += lo->xg_floats;
@@ -656,8 +739,14 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
         BwdCfg c;
         const ChainPlan &hh = rp.layer[l].hh, &ih = rp.layer[l].ih;
         const int Hh = (int)H, Gg = rp.G;
-        if (plan_bwd(hh, [&](int r) { return smem_rnn_bwd_fixed(hh, r, Hh, Gg); }, dv, B, &c, "hh backward")) return 1;
-        if (c.spill > spill) spill = c.spill;
+        if (rp.P) {
+            BwdProjCfg cq;
+            if (plan_bwd_proj(hh, rp.layer[l].hr, Hh, rp.P, dv, B, &cq)) return 1;
+            if (cq.spill > spill) spill = cq.spill;
+        } else {
+            if (plan_bwd(hh, [&](int r) { return smem_rnn_bwd_fixed(hh, r, Hh, Gg); }, dv, B, &c, "hh backward")) return 1;
+            if (c.spill > spill) spill = c.spill;
+        }
         if (plan_bwd(ih, [&](int r) { return smem_ttlin_bwd_fixed(ih, r); }, dv, B * tc, &c, "ih backward")) return 1;
         if (c.spill > spill) spill = c.spill;
     }
@@ -682,12 +771,15 @@ struct CallPlan {
     RnnPlan rp;         // of eff.d
     RnnLayout lo;
     const ttrnn_rnn_desc *d() const { return &eff.d; }
+    const ttrnn_rnn_proj *pj() const { return eff.proj ? &eff.pj : nullptr; }
 };
 
-// keep_masked: the plan carries TTRNN_WS_DROPOUT
-int plan_call(const ttrnn_rnn_desc *d_in, const DevInfo &dv, CallPlan *cp, bool keep_masked = false) {
+// keep_masked: the plan carries TTRNN_WS_DROPOUT; pj: the projection of the _proj entry points (TTRNN_WS_PROJ) or nullptr.
+// The effective descriptor carries the projection from here on.
+int plan_call(const ttrnn_rnn_desc *d_in, const DevInfo &dv, CallPlan *cp, bool keep_masked = false,
+              const ttrnn_rnn_proj *pj = nullptr) {
     cp->dv = dv;
-    if (build_rnn_plan(d_in, &cp->rp) || make_eff_desc(d_in, &dv, &cp->eff)) return 1;
+    if (build_rnn_plan(d_in, &cp->rp, pj) || make_eff_desc(d_in, pj, &dv, &cp->eff)) return 1;
     if (cp->eff.padded && build_rnn_plan(&cp->eff.d, &cp->rp)) return 1;
     return build_layout(&cp->eff.d, cp->rp, dv, &cp->lo, keep_masked);
 }
@@ -1073,7 +1165,7 @@ bool group_launches(const CallPlan &cp, long long Bg, std::vector<SimLaunch> *fq
         q->push_back({(int)(tiles < sms ? tiles : sms), (double)waves * (kFloor + R)});
     };
     for (int l = 0; l < d->num_layers; ++l) {
-        const TtsRnnFwdEntry *se = fwd_route(d, l, Bg, sms);
+        const TtsRnnFwdEntry *se = fwd_route(d, cp.rp, l, Bg, sms);
         if (!se) return false;
         push(fq, Bg, se->R);
     }
@@ -1347,7 +1439,7 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
         const char *route = rank1 ? "rank_one" : (dense ? "dense" : "tt_chain");
         const bool tc_f = dense && tc_rows_use(B * (long long)lo.Tc, lp.ih.n_in, GH, false);
         const bool tc_r = dense && t_opt.tc_gemm && ttc::tc_red_ok(B * (long long)lo.Tc, lp.ih.n_in, GH);
-        const TtsRnnFwdEntry *se = fwd_route(d, l, B, dv.sms);
+        const TtsRnnFwdEntry *se = fwd_route(d, rp, l, B, dv.sms);
         // save_mode 2 = kept gate activations, 0 = recompute
         put("layer=%d ih_route=%s ih_fwd_tc=%d ih_dw_tc=%d fwd_kernel=%s fwd_rows=%d save_mode=%d", l, route, (int)tc_f, (int)tc_r,
             se ? tok(se->name).c_str() : "runtime", se ? se->R : 0, lo.kept[l] ? 2 : 0);
@@ -1375,11 +1467,19 @@ int64_t ttrnn_rnn_param_count(const ttrnn_rnn_desc *desc) {
     return rp.param_floats;
 }
 
+int64_t ttrnn_rnn_param_count_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_proj *pj) {
+    if (!pj) { fail("ttrnn_rnn_param_count_proj: pj must be non-null"); return -1; }
+    RnnPlan rp;
+    if (build_rnn_plan(desc, &rp, pj)) return -1;
+    return rp.param_floats;
+}
+
 // byte sizes of ONE row group (the whole batch when the plan has a single group), under the calling thread's options
-static int workspace_one(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *ws, bool keep_masked) {
+static int workspace_one(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *ws, bool keep_masked,
+                         const ttrnn_rnn_proj *pj = nullptr) {
     DevInfo dv;
     CallPlan cp;
-    if (get_dev(&dv) || plan_call(desc, dv, &cp, keep_masked)) return 1;
+    if (get_dev(&dv) || plan_call(desc, dv, &cp, keep_masked, pj)) return 1;
     ws->saved_bytes = cp.lo.sv_total * 4;
     ws->fwd_scratch_bytes = (cp.lo.f_total + cp.eff.pad_floats) * 4;       // + the rank-padded parameter blob
     ws->bwd_scratch_bytes = (cp.lo.b_total + 2 * cp.eff.pad_floats) * 4;   // + padded parameters and padded gradients
@@ -1392,6 +1492,7 @@ int ttrnn_rnn_workspace_bytes(const ttrnn_rnn_desc *desc, ttrnn_rnn_workspace *w
 
 int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrnn_rnn_workspace *ws) {
     if (!ws) return fail("null workspace struct");
+    if (flags & TTRNN_WS_PROJ) return fail("TTRNN_WS_PROJ: size the plan with ttrnn_rnn_workspace_bytes_proj");
     t_opt = snapshot_options();
     if (flags & TTRNN_WS_WHOLE_BATCH) t_opt.row_groups = 0;
     GroupPlan gp;
@@ -1422,15 +1523,37 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
     return 0;
 }
 
+// a projected stack runs as one row group: the group split is planned from the static kernels, which it has none of
+int ttrnn_rnn_workspace_bytes_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_proj *pj, int32_t flags,
+                                   ttrnn_rnn_workspace *ws) {
+    if (!ws) return fail("null workspace struct");
+    if (!pj) return fail("ttrnn_rnn_workspace_bytes_proj: pj must be non-null");
+    if (!desc) return fail("null descriptor");
+    if (desc->cell != TTRNN_CELL_LSTM) return fail("ttrnn_rnn_workspace_bytes_proj: a projection needs an LSTM descriptor");
+    t_opt = snapshot_options();
+    t_opt.row_groups = 0;
+    const bool masked = (flags & TTRNN_WS_DROPOUT) != 0;
+    if (workspace_one(desc, ws, masked, pj)) return 1;
+    memset(ws->plan, 0, sizeof ws->plan);
+    plan_store(t_opt, ws->plan);
+    ws->plan[kPlanGroups] = 1;
+    ws->plan[kPlanRows0] = desc->batch;
+    ws->plan[kPlanLayerStates] = (flags & TTRNN_WS_LAYER_STATES) ? 1 : 0;
+    ws->plan[kPlanDropout] = masked ? 1 : 0;
+    ws->plan[kPlanProj] = 1;
+    return 0;
+}
+
 // forward of ONE row group on stream `stream`; `ws` carries the byte sizes of this group, t_opt is already loaded
 // `dc`: inter-layer dropout (nullptr = none; the plan then has no masked buffers)
+// `pj`: the projection (nullptr = none)
 static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
                        const float *h0, const float *c0, const float *params_in, float *out, float *hT, float *cT, void *saved,
-                       void *scratch, void *stream, const DropCall *dc) {
+                       void *scratch, void *stream, const DropCall *dc, const ttrnn_rnn_proj *pj) {
     if (!x || !params_in || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     DevInfo dv;
     CallPlan cp;
-    if (get_dev(&dv) || plan_call(d_in, dv, &cp, ws->plan[kPlanDropout] != 0)) return 1;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp, ws->plan[kPlanDropout] != 0, pj)) return 1;
     const ttrnn_rnn_desc *d = cp.d();
     const RnnPlan &rp = cp.rp;
     const RnnLayout &lo = cp.lo;
@@ -1451,7 +1574,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
     }
     const long long B = d->batch;
     const int T = d->seq_len, H = d->hidden_size, L = d->num_layers, G = rp.G;
-    const int GH = G * H;
+    const int GH = G * H, W = rp.out_width(d);       // W: width of a layer's output and h state
     const bool lstm = d->cell == TTRNN_CELL_LSTM;
     float *sc = (float *)scratch;
     float *sv = (float *)saved;
@@ -1463,22 +1586,22 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
         const int nin = lp.ih.n_in;
         const float *lin;       // input of this layer (B, T, nin)
         if (l == 0) lin = x;
-        else lin = sv ? sv + lo.sv_hs + (long long)(l - 1) * lo.BTH : sc + lo.f_hs + ((l - 1) & 1) * r4(lo.BTH);
+        else lin = sv ? sv + lo.sv_hs + (long long)(l - 1) * lo.BTW : sc + lo.f_hs + ((l - 1) & 1) * r4(lo.BTW);
         if (l > 0 && dc) {
             // dropout: layer l reads the masked output of layer l - 1 (kept for the backward in training)
-            float *masked = sv ? sv + lo.sv_drop + (long long)(l - 1) * lo.BTH : sc + lo.f_drop;
-            if (launch_dropout(dv, B, T, H, *dc, dc->row0, l - 1, lin, nullptr, masked, nullptr, st)) return 1;
+            float *masked = sv ? sv + lo.sv_drop + (long long)(l - 1) * lo.BTW : sc + lo.f_drop;
+            if (launch_dropout(dv, B, T, W, *dc, dc->row0, l - 1, lin, nullptr, masked, nullptr, st)) return 1;
             lin = masked;
         }
-        float *lout;            // output of this layer (B, T, H)
+        float *lout;            // output of this layer (B, T, W)
         if (l == L - 1) lout = out;
-        else lout = sv ? sv + lo.sv_hs + (long long)l * lo.BTH : sc + lo.f_hs + (l & 1) * r4(lo.BTH);
+        else lout = sv ? sv + lo.sv_hs + (long long)l * lo.BTW : sc + lo.f_hs + (l & 1) * r4(lo.BTW);
         float *csave = (sv && lstm) ? sv + lo.sv_cs + (long long)l * lo.BTH : nullptr;
         const float *b_ih = d->has_bias ? params + lp.off_ih_bias : nullptr;
         const float *b_hh = d->has_bias ? params + lp.off_hh_bias : nullptr;
         // this layer's initial state, read by its first chunk, and where its last chunk leaves the final state
-        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
-        float *hTl = sm.fin(hT, l, L), *cTl = sm.fin(cT, l, L);
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l, true);
+        float *hTl = sm.fin(hT, l, L), *cTl = sm.fin(cT, l, L, true);
 
         // ---- batched ih projection of one time chunk: xg[b, t, :] = W_ih x[b, t0+t, :] + b_ih (+ b_hh for LSTM),
         // through the TT chain or, when that is the cheaper contraction order, through dense W_ih^T
@@ -1501,7 +1624,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
         };
 
         // ---- statically specialised kernel for this hh shape, if one is registered -------------------
-        const TtsRnnFwdEntry *se = fwd_route(d, l, B, dv.sms);
+        const TtsRnnFwdEntry *se = fwd_route(d, rp, l, B, dv.sms);
         if (se) {
             int occ = 0;
             int rc = se->prepare(&occ);
@@ -1553,6 +1676,48 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                 }
                 ++g_launches;
                 if (rc) return fail("static kernel %s launch failed: %s", se->name, cudaGetErrorString((cudaError_t)rc));
+            }
+            continue;
+        }
+
+        if (rp.P) {
+            // projected LSTM: the projection chain runs inside the recurrent kernel after the gate math of every step
+            RnnFwdProjArgs a;
+            memset(&a, 0, sizeof a);
+            a.p = lp.hh;
+            a.q = lp.hr;
+            const int R = pick_rows([&](int r) { return smem_rnn_fwd_proj(lp.hh, lp.hr, r, H); }, dv.smem_optin, 8, B,
+                                    dv.sms, 2);
+            if (R == 0)
+                return fail("layer %d: projected hh / hr TT shapes need %lld bytes of shared memory per CTA (limit %d): "
+                            "unsupported", l, smem_rnn_fwd_proj(lp.hh, lp.hr, 1, H) * 4, dv.smem_optin);
+            a.R = R;
+            fill_tiles(lp.hh, R, a.tile, nullptr, nullptr);
+            fill_tiles(lp.hr, R, a.tile_q, nullptr, nullptr);
+            a.H = H; a.P = W; a.B = B;
+            a.cores = params + lp.off_hh_cores;
+            a.cores_q = params + lp.off_hr_cores;
+            const size_t smem = (size_t)smem_rnn_fwd_proj(lp.hh, lp.hr, R, H) * 4;
+            int grid = 0;
+            if (grid_for(k_rnn_fwd_proj, smem, (B + R - 1) / R, dv, &grid)) return 1;
+            for (int t0 = 0; t0 < T; t0 += lo.Tc) {
+                const int tc = (T - t0 < lo.Tc) ? T - t0 : lo.Tc;
+                if (project(t0, tc)) return 1;
+                const bool first = (t0 == 0), last = (t0 + tc == T);
+                a.steps = tc;
+                a.xg = xg; a.xg_bstride = (long long)tc * GH;
+                a.h_in = first ? h0l : st_h;
+                a.c_in = first ? c0l : st_c;
+                a.out = lout + (long long)t0 * W; a.out_bstride = (long long)T * W;
+                a.c_save = csave ? csave + (long long)t0 * H : nullptr; a.c_bstride = (long long)T * H;
+                a.h_out = (last && hTl) ? hTl : st_h;
+                a.c_out = (last && cTl) ? cTl : st_c;
+                {
+                    KernelTimer tm(TTRNN_K_RNN_FWD, st, R, grid, B, tc);
+                    k_rnn_fwd_proj<<<grid, TT_NTHREADS, smem, st>>>(a);
+                }
+                ++g_launches;
+                CU_CHECK(cudaGetLastError());
             }
             continue;
         }
@@ -1630,11 +1795,11 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
 static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
                         const float *h0, const float *c0, const float *params, const float *out, const void *saved,
                         const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0,
-                        float *d_c0, void *scratch, void *stream, const DropCall *dc) {
+                        float *d_c0, void *scratch, void *stream, const DropCall *dc, const ttrnn_rnn_proj *pj) {
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     DevInfo dv;
     CallPlan cp;
-    if (get_dev(&dv) || plan_call(d_in, dv, &cp, ws->plan[kPlanDropout] != 0)) return 1;
+    if (get_dev(&dv) || plan_call(d_in, dv, &cp, ws->plan[kPlanDropout] != 0, pj)) return 1;
     const RnnLayout &lo = cp.lo;
     const EffDesc &eff = cp.eff;
     if ((lo.b_total + 2 * eff.pad_floats) * 4 != ws->bwd_scratch_bytes || lo.sv_total * 4 != ws->saved_bytes)
@@ -1667,7 +1832,7 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
     const DevInfo &dv = cp.dv;
     const long long B = d->batch;
     const int T = d->seq_len, H = d->hidden_size, L = d->num_layers, G = rp.G;
-    const int GH = G * H;
+    const int GH = G * H, W = rp.out_width(d);       // W: width of a layer's output and h state
     const bool lstm = d->cell == TTRNN_CELL_LSTM;
     if ((L > 1 || lstm) && !saved) return fail("backward needs the `saved` buffer written by a training forward");
     if (dc && L > 1 && !lo.masked) return fail("internal: dropout backward without the masked layer inputs");
@@ -1701,23 +1866,23 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
         cudaStream_t ws = st;                                 // stream of the weight-gradient work of this layer
         DevInfo dvw = dv;                                     // ... and the SMs it may plan for
         // dropout: layers >= 1 read the masked output of the layer below, which the forward kept
-        const float *lin = (l == 0) ? x : sv + (dc ? lo.sv_drop : lo.sv_hs) + (long long)(l - 1) * lo.BTH;
-        const float *lout = (l == L - 1) ? out : sv + lo.sv_hs + (long long)l * lo.BTH;
+        const float *lin = (l == 0) ? x : sv + (dc ? lo.sv_drop : lo.sv_hs) + (long long)(l - 1) * lo.BTW;
+        const float *lout = (l == L - 1) ? out : sv + lo.sv_hs + (long long)l * lo.BTW;
         const float *lcs = lstm ? sv + lo.sv_cs + (long long)l * lo.BTH : nullptr;
         // gradient wrt this layer's outputs / wrt its inputs
-        const float *dhs = (l == L - 1) ? d_out : sc + lo.b_dhs + ((l + 1) & 1) * r4(lo.BTH);
-        float *dlin = (l == 0) ? d_x : sc + lo.b_dhs + (l & 1) * r4(lo.BTH);
+        const float *dhs = (l == L - 1) ? d_out : sc + lo.b_dhs + ((l + 1) & 1) * r4(lo.BTW);
+        float *dlin = (l == 0) ? d_x : sc + lo.b_dhs + (l & 1) * r4(lo.BTW);
         if (l < L - 1 && dc) {
             // dropout: the gradient wrt the masked input of layer l + 1 (its dX, written on this stream also under the
             // backward overlap) times mask / (1 - p) is the gradient wrt this layer's output; in place
-            float *g = sc + lo.b_dhs + ((l + 1) & 1) * r4(lo.BTH);
-            if (launch_dropout(dv, B, T, H, *dc, dc->row0, l, g, nullptr, g, nullptr, st)) return 1;
+            float *g = sc + lo.b_dhs + ((l + 1) & 1) * r4(lo.BTW);
+            if (launch_dropout(dv, B, T, W, *dc, dc->row0, l, g, nullptr, g, nullptr, st)) return 1;
         }
         const float *b_ih = d->has_bias ? params + lp.off_ih_bias : nullptr;
         const float *b_hh = d->has_bias ? params + lp.off_hh_bias : nullptr;
         // this layer's initial state and the upstream gradient of its final state (enters its last step)
-        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
-        const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L);
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l, true);
+        const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L, true);
 
         // ---- ih projection (recompute) and its backward per time chunk: TT chain or dense route ---------
         // a rank-one layer 0 whose input gradient is wanted runs the projected-input kernels (delta_ih feeds dX)
@@ -1995,7 +2160,71 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
                 set_busy[set] = true;
             }
             if (d_h0 && axpy1(sdh, sm.init(d_h0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
-            if (lstm && d_c0 && axpy1(sdc, sm.init(d_c0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
+            if (lstm && d_c0 && axpy1(sdc, sm.init(d_c0, l, true), lo.BH, !sm.stride && l != L - 1, st)) return 1;
+            continue;
+        }
+
+        if (rp.P) {
+            // projected LSTM: k_rnn_bwd_proj runs the projection chain forward and backward inside every BPTT step; the
+            // per-CTA slots hold the hh core gradients, then the hr core gradients
+            RnnBwdProjArgs a;
+            memset(&a, 0, sizeof a);
+            BwdProjCfg cfg;
+            if (plan_bwd_proj(lp.hh, lp.hr, H, W, dv, B, &cfg)) return 1;
+            a.p = cfg.p;
+            a.q = cfg.q;
+            const int R = cfg.R;
+            a.R = R;
+            a.spill = cfg.spill > 0 ? ss + lo.b_spill : nullptr;
+            fill_tiles(cfg.p, R, a.tile, a.tile_bd, a.mg);
+            fill_tiles(cfg.q, R, a.tile_q, a.tile_bd_q, a.mg_q);
+            a.H = H; a.P = W; a.B = B; a.T = T;
+            a.cores = params + lp.off_hh_cores;
+            a.cores_q = params + lp.off_hr_cores;
+            a.hs = lout; a.cs = lcs; a.h0 = h0l; a.c0 = c0l; a.dhs = dhs;
+            int grid = 0;
+            if (grid_for(k_rnn_bwd_proj, cfg.smem, (B + R - 1) / R, dv, &grid)) return 1;
+            if (grid > lo.nslots) grid = lo.nslots;
+            const long long hh_slot = lp.hh.core_floats + lp.hr.core_floats;
+            const long long ih_slot = lp.ih.core_floats + GH;
+            CU_CHECK(cudaMemsetAsync(part_hh, 0, (size_t)hh_slot * grid * 4, st));
+            CU_CHECK(cudaMemsetAsync(part_ih, 0, (size_t)ih_slot * lo.nslots * 4, st));
+            a.partial = part_hh;
+            int ih_slots_used = 0;
+            const int nchunks = (T + lo.Tc - 1) / lo.Tc;
+            for (int ci = nchunks - 1; ci >= 0; --ci) {
+                const int t0 = ci * lo.Tc;
+                const int tc = (T - t0 < lo.Tc) ? T - t0 : lo.Tc;
+                const bool last = (t0 + tc == T);
+                if (project(t0, tc)) return 1;
+                a.t0 = t0; a.steps = tc;
+                a.xg = xg; a.xg_bstride = (long long)tc * GH;
+                a.dh_in = last ? dhTl : sdh;
+                a.dc_in = last ? dcTl : sdc;
+                a.dh_out = sdh; a.dc_out = sdc;
+                {
+                    KernelTimer tm(TTRNN_K_RNN_BWD, st, R, grid, B, tc);
+                    k_rnn_bwd_proj<<<grid, TT_NTHREADS, cfg.smem, st>>>(a);
+                }
+                ++g_launches;
+                CU_CHECK(cudaGetLastError());
+                if (project_bwd(t0, tc, &ih_slots_used)) return 1;
+            }
+            if (project_finish(&ih_slots_used)) return 1;
+            if (reduce_partials(part_hh, grid, hh_slot, 0, lp.hh.core_floats, d_params + lp.off_hh_cores, st)) return 1;
+            if (reduce_partials(part_hh, grid, hh_slot, lp.hh.core_floats, lp.hr.core_floats, d_params + lp.off_hr_cores, st))
+                return 1;
+            if (reduce_partials(part_ih, ih_slots_used, ih_slot, 0, lp.ih.core_floats, d_params + lp.off_ih_cores, st)) return 1;
+            if (d->has_bias) {
+                if (dense) {
+                    if (axpy1(D.dbias, d_params + lp.off_ih_bias, GH, 0, st)) return 1;
+                } else if (reduce_partials(part_ih, ih_slots_used, ih_slot, lp.ih.core_floats, GH, d_params + lp.off_ih_bias, st)) {
+                    return 1;
+                }
+                if (axpy1(d_params + lp.off_ih_bias, d_params + lp.off_hh_bias, GH, 0, st)) return 1;
+            }
+            if (d_h0 && axpy1(sdh, sm.init(d_h0, l), lo.BW, !sm.stride && l != L - 1, st)) return 1;
+            if (d_c0 && axpy1(sdc, sm.init(d_c0, l, true), lo.BH, !sm.stride && l != L - 1, st)) return 1;
             continue;
         }
 
@@ -2067,17 +2296,35 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
         }
         // (5) gradient wrt the initial state: this layer's own block, or the sum over layers when the state is shared
         if (d_h0 && axpy1(sdh, sm.init(d_h0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
-        if (lstm && d_c0 && axpy1(sdc, sm.init(d_c0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
+        if (lstm && d_c0 && axpy1(sdc, sm.init(d_c0, l, true), lo.BH, !sm.stride && l != L - 1, st)) return 1;
     }
     return 0;
 }
 
 // per-layer state buffers (TTRNN_WS_LAYER_STATES in the plan) are strided by the full batch's B * H, so that a row group
 // reaches layer l's rows from a pointer moved to its first row
-static StateMap state_map(const ttrnn_rnn_desc *d_full, const ttrnn_rnn_workspace *ws) {
+static StateMap state_map(const ttrnn_rnn_desc *d_full, const ttrnn_rnn_workspace *ws, const ttrnn_rnn_proj *pj) {
     StateMap sm;
-    if (ws->plan[kPlanLayerStates]) sm.stride = (long long)d_full->batch * d_full->hidden_size;
+    if (ws->plan[kPlanLayerStates]) {
+        sm.cstride = (long long)d_full->batch * d_full->hidden_size;
+        sm.stride = pj ? (long long)d_full->batch * pj->proj_size : sm.cstride;
+    }
     return sm;
+}
+
+// the projection of an entry point: proj_given = the call is a _proj entry point (which requires pj and a plan sized
+// with TTRNN_WS_PROJ); every other entry point refuses such a plan
+static int proj_call(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, bool proj_given,
+                     const ttrnn_rnn_proj *pj) {
+    if (!proj_given) {
+        if (ws->plan[kPlanProj])
+            return fail("%s: the plan was sized with TTRNN_WS_PROJ; run it with the _proj entry points", who);
+        return 0;
+    }
+    if (!ws->plan[kPlanProj]) return fail("%s: the plan was not sized with TTRNN_WS_PROJ (ttrnn_rnn_workspace_bytes_proj)", who);
+    if (!pj) return fail("%s: pj must be non-null", who);
+    if (d_in->cell != TTRNN_CELL_LSTM) return fail("%s: a projection needs an LSTM descriptor", who);
+    return 0;
 }
 
 // ---- public entry points: one call of the single-group path per row group ---------------------------------------
@@ -2142,15 +2389,18 @@ static int drop_call(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rn
 
 static int rnn_forward_entry(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x,
                              const float *h0, const float *c0, const float *params, float *out, float *hT, float *cT,
-                             void *saved, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp) {
+                             void *saved, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp,
+                             bool proj_given = false, const ttrnn_rnn_proj *pj = nullptr) {
     if (!ws || !plan_load(ws->plan, &t_opt))
         return fail("%s: `ws` must be the struct filled by ttrnn_rnn_workspace_bytes() for this descriptor", who);
     if (!d_in) return fail("null descriptor");
+    if (proj_call(who, d_in, ws, proj_given, pj)) return 1;
     DropCall dcs;
     const DropCall *dc = nullptr;
     if (drop_call(who, d_in, ws, dp_given, dp, &dcs, &dc)) return 1;
-    const StateMap sm = state_map(d_in, ws);
-    if (ws->plan[kPlanGroups] <= 1) return forward_one(d_in, ws, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream, dc);
+    const StateMap sm = state_map(d_in, ws, pj);
+    if (ws->plan[kPlanGroups] <= 1)
+        return forward_one(d_in, ws, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream, dc, pj);
     if (!x || !params || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_forward")) return 1;
@@ -2171,7 +2421,7 @@ static int rnn_forward_entry(const char *who, const ttrnn_rnn_desc *d_in, const 
         rc = forward_one(&gs.d[g], &gs.w[g], sm, x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
                          out + r0 * T * H, hT ? hT + r0 * H : nullptr, cT ? cT + r0 * H : nullptr,
                          saved ? (char *)saved + gs.sv_off[g] : nullptr, (char *)scratch + gs.f_off[g],
-                         (g == 0 || serial) ? (void *)st : (void *)gc->s, dc);
+                         (g == 0 || serial) ? (void *)st : (void *)gc->s, dc, nullptr);
     }
     t_group = 0;
     if (!serial) {       // also on the error path: the caller's stream must not run ahead of the group stream
@@ -2198,17 +2448,19 @@ int ttrnn_rnn_forward_dropout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_worksp
 static int rnn_backward_entry(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x,
                               const float *h0, const float *c0, const float *params, const float *out, const void *saved,
                               const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x,
-                              float *d_h0, float *d_c0, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp) {
+                              float *d_h0, float *d_c0, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp,
+                              bool proj_given = false, const ttrnn_rnn_proj *pj = nullptr) {
     if (!ws || !plan_load(ws->plan, &t_opt))
         return fail("%s: `ws` must be the struct the matching forward ran with", who);
     if (!d_in) return fail("null descriptor");
+    if (proj_call(who, d_in, ws, proj_given, pj)) return 1;
     DropCall dcs;
     const DropCall *dc = nullptr;
     if (drop_call(who, d_in, ws, dp_given, dp, &dcs, &dc)) return 1;
-    const StateMap sm = state_map(d_in, ws);
+    const StateMap sm = state_map(d_in, ws, pj);
     if (ws->plan[kPlanGroups] <= 1)
         return backward_one(d_in, ws, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
-                            stream, dc);
+                            stream, dc, pj);
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_backward")) return 1;
@@ -2232,7 +2484,7 @@ static int rnn_backward_entry(const char *who, const ttrnn_rnn_desc *d_in, const
                           out + r0 * T * H, saved ? (const char *)saved + gs.sv_off[g] : nullptr,
                           d_out ? d_out + r0 * T * H : nullptr, d_hT ? d_hT + r0 * H : nullptr, d_cT ? d_cT + r0 * H : nullptr, dp,
                           d_x ? d_x + r0 * T * I : nullptr, d_h0 ? d_h0 + r0 * H : nullptr, d_c0 ? d_c0 + r0 * H : nullptr,
-                          (char *)scratch + gs.b_off[g], (g == 0 || serial) ? (void *)st : (void *)gc->s, dc);
+                          (char *)scratch + gs.b_off[g], (g == 0 || serial) ? (void *)st : (void *)gc->s, dc, nullptr);
     }
     t_group = 0;
     if (!serial) {
@@ -2262,6 +2514,21 @@ int ttrnn_rnn_backward_dropout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_works
                               d_params, d_x, d_h0, d_c0, scratch, stream, true, dp);
 }
 
+int ttrnn_rnn_forward_proj(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                           const float *c0, const float *params, float *out, float *hT, float *cT, void *saved, void *scratch,
+                           void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp) {
+    return rnn_forward_entry("ttrnn_rnn_forward_proj", d_in, ws, x, h0, c0, params, out, hT, cT, saved, scratch, stream,
+                             dp != nullptr, dp, true, pj);
+}
+
+int ttrnn_rnn_backward_proj(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                            const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
+                            const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
+                            void *scratch, void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp) {
+    return rnn_backward_entry("ttrnn_rnn_backward_proj", d_in, ws, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params,
+                              d_x, d_h0, d_c0, scratch, stream, dp != nullptr, dp, true, pj);
+}
+
 int ttrnn_dropout_apply(int64_t B, int32_t T, int32_t F, int64_t row0, int32_t boundary, int32_t backward,
                         const ttrnn_dropout *dp, const float *x, float *y, float *y_rev, void *stream) {
     if (B < 1 || T < 1 || F < 1 || row0 < 0) return fail("ttrnn_dropout_apply: B, T, F must be >= 1 and row0 >= 0 (got %lld, %d, %d, %lld)",
@@ -2286,6 +2553,7 @@ int ttrnn_rnn_backward_logged(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_worksp
     if (!d_in || !ws) return fail("null descriptor / workspace struct");
     if (!dh_log) return fail("ttrnn_rnn_backward_logged: dh_log must be non-null");
     if (ws->plan[kPlanDropout]) return fail("ttrnn_rnn_backward_logged: the plan was sized with TTRNN_WS_DROPOUT");
+    if (ws->plan[kPlanProj]) return fail("ttrnn_rnn_backward_logged: the plan was sized with TTRNN_WS_PROJ");
     if (ws->plan[kPlanGroups] > 1)
         return fail("ttrnn_rnn_backward_logged needs a whole-batch plan: size the call with "
                     "ttrnn_rnn_workspace_bytes_ex(desc, TTRNN_WS_WHOLE_BATCH, ws)");
@@ -2302,6 +2570,7 @@ int ttrnn_rnn_saved_layout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace
                            int64_t *cs_off) {
     if (!ws || !plan_load(ws->plan, &t_opt)) return fail("ttrnn_rnn_saved_layout: `ws` must come from ttrnn_rnn_workspace_bytes()");
     if (ws->plan[kPlanGroups] > 1) return fail("ttrnn_rnn_saved_layout needs a whole-batch plan (TTRNN_WS_WHOLE_BATCH)");
+    if (ws->plan[kPlanProj]) return fail("ttrnn_rnn_saved_layout: the plan was sized with TTRNN_WS_PROJ");
     if (!hs_off || !cs_off) return fail("hs_off and cs_off must be non-null");
     DevInfo dv;
     CallPlan cp;

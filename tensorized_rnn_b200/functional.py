@@ -30,11 +30,14 @@ def _require_cuda_f32(name: str, t: torch.Tensor) -> None:
 
 
 class RnnSpec(object):
-    """Static description of a TT-RNN stack: cell kind, sizes and the TT shape of every weight."""
+    """Static description of a TT-RNN stack: cell kind, sizes and the TT shape of every weight.  `proj_size` > 0 (LSTM
+    only) with `hr_shapes`: the projected LSTM, whose layers output h_t = W_hr m_t of width proj_size (DESIGN.md §4.19)."""
 
     def __init__(self, cell: str, input_size: int, hidden_size: int, has_bias: bool,
                  ih_shapes: Sequence[Tuple[Sequence[int], Sequence[int], Sequence[int]]],
-                 hh_shapes: Sequence[Tuple[Sequence[int], Sequence[int], Sequence[int]]]):
+                 hh_shapes: Sequence[Tuple[Sequence[int], Sequence[int], Sequence[int]]],
+                 proj_size: int = 0,
+                 hr_shapes: Optional[Sequence[Tuple[Sequence[int], Sequence[int], Sequence[int]]]] = None):
         assert cell in ("lstm", "gru")
         self.cell = cell
         self.n_gates = 4 if cell == "lstm" else 3
@@ -44,7 +47,24 @@ class RnnSpec(object):
             raise ValueError("at most %d layers are supported" % _lib.MAX_LAYERS)
         self.ih_shapes = [tuple(list(map(int, v)) for v in s) for s in ih_shapes]   # (in_modes, out_modes, ranks)
         self.hh_shapes = [tuple(list(map(int, v)) for v in s) for s in hh_shapes]
+        self.proj_size = int(proj_size)
+        self.hr_shapes = [tuple(list(map(int, v)) for v in s) for s in hr_shapes] if self.proj_size else []
+        assert not self.proj_size or (cell == "lstm" and len(self.hr_shapes) == self.num_layers)
+        self.output_size = self.proj_size or self.hidden_size       # width of h_t and of every layer's output
+        self._proj = None
         self._cache = {}
+
+    def proj(self) -> Optional[_lib.RnnProj]:
+        """The ttrnn_rnn_proj of a projected stack, else None."""
+        if not self.proj_size:
+            return None
+        if self._proj is None:
+            pj = _lib.RnnProj()
+            pj.proj_size, pj.reserved = self.proj_size, 0
+            for l in range(self.num_layers):
+                pj.hr[l] = _lib.make_tt_shape(*self.hr_shapes[l])
+            self._proj = pj
+        return self._proj
 
     def desc(self, batch: int, seq_len: int) -> _lib.RnnDesc:
         key = (batch, seq_len)
@@ -161,7 +181,8 @@ class _RnnFunction(torch.autograd.Function):
     `layer_states`: h0 / c0 and the returned final states are (L, B, H), one block per layer (TTRNN_WS_LAYER_STATES);
     else (B, H), shared by every layer on the way in and the last layer's on the way out.
     `dropout`: None, or (p, seed, offset) of the inter-layer dropout (ttrnn_rnn_forward_dropout, TTRNN_WS_DROPOUT); the
-    backward regenerates the same mask from them."""
+    backward regenerates the same mask from them.
+    A projected spec (proj_size P > 0) runs the _proj entry points: out and the h states are P wide, the c states H."""
 
     @staticmethod
     def forward(ctx, spec: RnnSpec, grad_enabled: bool, step_log, layer_states: bool, dropout, x, h0, c0, *params):
@@ -172,22 +193,25 @@ class _RnnFunction(torch.autograd.Function):
             if p.device != x.device:
                 raise RuntimeError("parameter %d is on %s but the input is on %s" % (i, p.device, x.device))
         B, T, I = x.shape
-        H = spec.hidden_size
+        H, W = spec.hidden_size, spec.output_size
         if I != spec.input_size:
             raise ValueError("input has %d features, the module was built for %d" % (I, spec.input_size))
-        state_shape = (spec.num_layers, B, H) if layer_states else (B, H)
-        for name, s in (("h0", h0), ("c0", c0)):
+        lead = (spec.num_layers, B) if layer_states else (B,)
+        state_shape, h_shape = lead + (H,), lead + (W,)
+        for name, s, shp in (("h0", h0, h_shape), ("c0", c0, state_shape)):
             if s is not None:
                 _require_cuda_f32(name, s)
-                if tuple(s.shape) != state_shape:
-                    raise ValueError("%s must have shape %s, got %s" % (name, state_shape, tuple(s.shape)))
+                if tuple(s.shape) != shp:
+                    raise ValueError("%s must have shape %s, got %s" % (name, shp, tuple(s.shape)))
         x = _dense16(x)
         h0c = _dense16(h0)
         c0c = _dense16(c0)
         desc = spec.desc(B, T)
         with torch.cuda.device(x.device):
             blob = torch.cat([p.detach().reshape(-1) for p in params])
-            want = lib.ttrnn_rnn_param_count(C.byref(desc))
+            pj = spec.proj()
+            want = lib.ttrnn_rnn_param_count(C.byref(desc)) if pj is None else \
+                lib.ttrnn_rnn_param_count_proj(C.byref(desc), C.byref(pj))
             if want < 0:
                 raise RuntimeError("ttrnn_rnn_param_count failed: " + _lib.last_error())
             if want != blob.numel():
@@ -195,14 +219,18 @@ class _RnnFunction(torch.autograd.Function):
             ws = _lib.RnnWorkspace()
             flags = (_lib.WS_WHOLE_BATCH if step_log is not None else 0) | (_lib.WS_LAYER_STATES if layer_states else 0) | \
                 (_lib.WS_DROPOUT if dropout is not None else 0)
-            _lib.check(lib.ttrnn_rnn_workspace_bytes_ex(C.byref(desc), flags, C.byref(ws)), "ttrnn_rnn_workspace_bytes")
+            if pj is None:
+                _lib.check(lib.ttrnn_rnn_workspace_bytes_ex(C.byref(desc), flags, C.byref(ws)), "ttrnn_rnn_workspace_bytes")
+            else:
+                _lib.check(lib.ttrnn_rnn_workspace_bytes_proj(C.byref(desc), C.byref(pj), flags | _lib.WS_PROJ, C.byref(ws)),
+                           "ttrnn_rnn_workspace_bytes_proj")
             # grad mode is always off inside Function.forward and needs_input_grad stays True for nn.Parameters under
             # torch.no_grad(): the caller captures torch.is_grad_enabled() before .apply (ADVICE r1)
             training = bool(grad_enabled) and any(ctx.needs_input_grad[5:])
             if step_log is not None and not training:
                 raise RuntimeError("fused per-step logging needs a training forward (it reads the kept h_t / c_t sequences)")
-            out = torch.empty((B, T, H), device=x.device, dtype=torch.float32)
-            hT = torch.empty(state_shape, device=x.device, dtype=torch.float32)
+            out = torch.empty((B, T, W), device=x.device, dtype=torch.float32)
+            hT = torch.empty(h_shape, device=x.device, dtype=torch.float32)
             cT = torch.empty(state_shape, device=x.device, dtype=torch.float32) if spec.cell == "lstm" else None
             saved = torch.empty(_bytes_to_floats(ws.saved_bytes), device=x.device, dtype=torch.float32) \
                 if training else None
@@ -210,7 +238,10 @@ class _RnnFunction(torch.autograd.Function):
             stream = torch.cuda.current_stream(x.device).cuda_stream
             args = (C.byref(desc), C.byref(ws), _ptr(x), _ptr(h0c), _ptr(c0c), _ptr(blob), _ptr(out), _ptr(hT), _ptr(cT),
                     _ptr(saved), _ptr(scratch), stream)
-            if dropout is None:
+            if pj is not None:
+                dp = None if dropout is None else C.byref(_dropout_struct(dropout))
+                _lib.check(lib.ttrnn_rnn_forward_proj(*(args + (C.byref(pj), dp))), "ttrnn_rnn_forward_proj")
+            elif dropout is None:
                 _lib.check(lib.ttrnn_rnn_forward(*args), "ttrnn_rnn_forward")
             else:
                 _lib.check(lib.ttrnn_rnn_forward_dropout(*(args + (C.byref(_dropout_struct(dropout)),))),
@@ -232,7 +263,7 @@ class _RnnFunction(torch.autograd.Function):
             ctx.ws = ws                    # sizes + execution plan: backward runs from the same plan as this forward
             ctx.bwd_floats = _bytes_to_floats(ws.bwd_scratch_bytes)
             ctx.has_h0, ctx.has_c0 = h0 is not None, c0 is not None
-            ctx.state_shape = state_shape
+            ctx.state_shape, ctx.h_shape = state_shape, h_shape
             ctx.set_materialize_grads(False)
             ctx.save_for_backward(x, h0c, c0c, blob, out, saved)
         if spec.cell == "lstm":
@@ -256,7 +287,7 @@ class _RnnFunction(torch.autograd.Function):
         with torch.cuda.device(x.device):
             d_blob = torch.empty_like(blob)
             d_x = torch.empty_like(x) if ctx.needs_input_grad[5] else None
-            d_h0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
+            d_h0 = torch.empty(ctx.h_shape, device=x.device, dtype=torch.float32) \
                 if (ctx.has_h0 and ctx.needs_input_grad[6]) else None
             d_c0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
                 if (spec.cell == "lstm" and ctx.has_c0 and ctx.needs_input_grad[7]) else None
@@ -265,7 +296,10 @@ class _RnnFunction(torch.autograd.Function):
             args = (C.byref(desc), C.byref(ctx.ws), _ptr(x), _ptr(h0), _ptr(c0), _ptr(blob), _ptr(out),
                     _ptr(saved), _ptr(d_out), _ptr(d_hT), _ptr(d_cT), _ptr(d_blob),
                     _ptr(d_x), _ptr(d_h0), _ptr(d_c0), _ptr(scratch), stream)
-            if ctx.dropout is not None:
+            if spec.proj_size:
+                dp = None if ctx.dropout is None else C.byref(_dropout_struct(ctx.dropout))
+                _lib.check(lib.ttrnn_rnn_backward_proj(*(args + (C.byref(spec.proj()), dp))), "ttrnn_rnn_backward_proj")
+            elif ctx.dropout is not None:
                 _lib.check(lib.ttrnn_rnn_backward_dropout(*(args + (C.byref(_dropout_struct(ctx.dropout)),))),
                            "ttrnn_rnn_backward_dropout")
             elif ctx.step_log is None:
@@ -385,23 +419,26 @@ def _side_stream(device: torch.device) -> torch.cuda.Stream:
     return s
 
 
-def shared_bidirectional_state(state: Optional[torch.Tensor], num_layers: int, batch: int, hidden_size: int):
-    """forward()'s one (B, H) initial state, which seeds every layer and both directions, as (2L, B, H) views of it."""
+def shared_bidirectional_state(state: Optional[torch.Tensor], num_layers: int, batch: int, width: int):
+    """forward()'s one (B, width) initial state, which seeds every layer and both directions, as (2L, B, width) views of
+    it.  width: the size of that state variable (the hidden size; the projection size for a projected LSTM's h)."""
     if state is None:
         return None
-    if tuple(state.shape) != (batch, hidden_size):
-        raise ValueError("init_states must have shape %s, got %s" % ((batch, hidden_size), tuple(state.shape)))
-    return state.unsqueeze(0).expand(2 * num_layers, batch, hidden_size)
+    if tuple(state.shape) != (batch, width):
+        raise ValueError("init_states must have shape %s, got %s" % ((batch, width), tuple(state.shape)))
+    return state.unsqueeze(0).expand(2 * num_layers, batch, width)
 
 
 def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]], num_layers: int, hidden_size: int,
-                        run, dropout=None):
+                        run, dropout=None, output_size: Optional[int] = None):
     """A bidirectional stack composed of one-layer calls, the contract of torch.nn.LSTM / GRU(bidirectional=True).
 
     `run(layer, direction, x, *states)` runs direction 0 (forward) or 1 (reverse) of one layer over x (B, T, F) from its
-    (B, H) initial states (None = zeros) with the existing one-layer call and returns (out (B, T, H), *final states).
-    `states`: one entry per state variable (h, and c for an LSTM), each (2L, B, H) with direction d of layer l at
-    2l + d, or None (zeros).  Returns (out (B, T, 2H), [final states, each (2L, B, H) in the same order]).
+    initial states (None = zeros) with the existing one-layer call and returns (out (B, T, W), *final states).
+    W = output_size (the projection size of a projected LSTM), default hidden_size: the width of the output and of the
+    h state; every other state (c) is hidden_size wide.
+    `states`: one entry per state variable (h, and c for an LSTM), each (2L, B, width) with direction d of layer l at
+    2l + d, or None (zeros).  Returns (out (B, T, 2W), [final states, each (2L, B, width) in the same order]).
 
     The reverse direction of a layer sees its input reversed in time and returns its outputs reversed in time; the join
     kernel writes the next layer's input and, for its reverse direction, the same tensor reversed.  The reverse
@@ -416,12 +453,12 @@ def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]
         raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
     _require_cuda_f32("input", x)
     B = x.shape[0]
-    shape = (2 * num_layers, B, hidden_size)
-    for s in states:
+    for k, s in enumerate(states):
         if s is not None:
+            shape = (2 * num_layers, B, (output_size or hidden_size) if k == 0 else hidden_size)
             _require_cuda_f32("state", s)
             if tuple(s.shape) != shape:
-                raise ValueError("bidirectional states must have shape %s (2 * num_layers, batch, hidden), got %s"
+                raise ValueError("bidirectional states must have shape %s (2 * num_layers, batch, width), got %s"
                                  % (shape, tuple(s.shape)))
     dev = x.device
     with torch.cuda.device(dev):

@@ -29,6 +29,10 @@ layer on two streams (functional.bidirectional_stack, DESIGN.md §4.17).  It nee
 `dropout=p` (no reference counterpart; the contract of torch.nn.LSTM(dropout=p)): in training mode the output sequence of
 every layer but the last is multiplied by a Bernoulli(1 - p) mask / (1 - p) before the next layer reads it, inside the
 stack call (DESIGN.md §4.18).  It needs the fused mode as well.
+
+`proj_size=P` (TTLSTM only; the contract of torch.nn.LSTM(proj_size=P)): each cell gets `projection_weights`, a TTLinear
+H -> P without bias created after `hidden_weights`, and outputs h_t = W_hr (o_t * tanh(c_t)), which is also the next
+step's hh input.  The recurrent kernels contract W_hr inside every step (DESIGN.md §4.19).  It needs the fused mode.
 """
 from __future__ import annotations
 
@@ -55,6 +59,16 @@ def check_dropout(dropout, num_layers: int) -> float:
         warnings.warn("dropout option adds dropout after all but last recurrent layer, so non-zero dropout expects "
                       "num_layers greater than 1, but got dropout=%s and num_layers=%d" % (dropout, num_layers))
     return float(dropout)
+
+
+def check_proj_size(proj_size, hidden_size: int) -> int:
+    """torch.nn.LSTM's validation of `proj_size`: an int in [0, hidden_size)."""
+    if isinstance(proj_size, bool) or not isinstance(proj_size, numbers.Integral) or proj_size < 0:
+        raise ValueError("proj_size should be a positive integer or zero to disable projections, got %r" % (proj_size,))
+    if proj_size >= hidden_size:
+        raise ValueError("proj_size has to be smaller than hidden_size, got proj_size=%d, hidden_size=%d"
+                         % (proj_size, hidden_size))
+    return int(proj_size)
 
 
 def active_dropout(module: nn.Module, device: torch.device):
@@ -99,11 +113,12 @@ class _TTCellBase(nn.Module):
     n_gate = 0
     cell_kind = ""
 
-    def __init__(self, input_size, hidden_size, bias, device, n_cores, tt_rank, is_naive=False, new_core=None):
+    def __init__(self, input_size, hidden_size, bias, device, n_cores, tt_rank, is_naive=False, new_core=None, proj_size=0):
         super().__init__()
         assert new_core in [None, 'first', 'last']
         self.input_size = input_size
         self.hidden_size = hidden_size
+        self.proj_size = proj_size
         self.bias = bias
         self.device = device
         self.n_cores = n_cores
@@ -113,6 +128,11 @@ class _TTCellBase(nn.Module):
         # creation order (ih before hh) fixes the RNG stream, as in reference lstm.py:14-15
         self.input_weights = self._create_input_hidden_weights()
         self.hidden_weights = self._create_hidden_hidden_weights()
+        if proj_size:
+            # W_hr (H -> P, no bias), created last so that proj_size = 0 consumes the RNG as before.  new_core concerns
+            # the gate axis, which the projection does not have
+            self.projection_weights = TTLinear(out_features=proj_size, shape=tt_shape(hidden_size, proj_size, n_cores, 1),
+                                               bias=False, auto_shapes=False, d=n_cores, tt_rank=tt_rank).to(device)
 
     # bias of the per-gate TTLinears of the naive form: the reference gives the TT-LSTM gates none
     # (tt_lstm.py:20,33) and the TT-GRU gates `self.bias` (gru.py:152,165)
@@ -131,23 +151,27 @@ class _TTCellBase(nn.Module):
         return self._tt_linear(self.input_size)
 
     def _create_hidden_hidden_weights(self):
-        return self._tt_linear(self.hidden_size)
+        return self._tt_linear(self.proj_size or self.hidden_size)
 
     def flat_parameters(self) -> List[torch.Tensor]:
-        """Parameters in C-ABI blob order: ih cores, ih bias, hh cores, hh bias (naive form: gate by gate)."""
+        """Parameters in C-ABI blob order: ih cores, ih bias, hh cores, hh bias (naive form: gate by gate), hr cores."""
         out: List[torch.Tensor] = []
         for w in (self.input_weights, self.hidden_weights):
             for lin in (list(w.gates) if self.is_naive else [w]):
                 out += list(lin.weight_t.tt_cores)
                 if lin.bias is not None:
                     out.append(lin.bias)
+        if self.proj_size:
+            out += list(self.projection_weights.weight_t.tt_cores)
         return out
 
     def _single_step_spec(self) -> RnnSpec:
         if getattr(self, "_step_spec", None) is None:
             self._step_spec = RnnSpec(self.cell_kind, self.input_size, self.hidden_size,
                                       self.input_weights.bias is not None,
-                                      [self.input_weights.tt_modes()], [self.hidden_weights.tt_modes()])
+                                      [self.input_weights.tt_modes()], [self.hidden_weights.tt_modes()],
+                                      proj_size=self.proj_size,
+                                      hr_shapes=[self.projection_weights.tt_modes()] if self.proj_size else None)
         return self._step_spec
 
 
@@ -157,6 +181,7 @@ class TTLSTMCell(_TTCellBase):
     cell_kind = "lstm"
 
     def forward(self, input, hx, cx):
+        """One step: (h (B, P or H), c (B, H))."""
         hooked = hasattr(self, '_h_backward_hook')
         if self.is_naive or hooked:
             # two projections + the fused gate kernel.  The c_t hook of log_grads (reference lstm.py:35-39)
@@ -194,8 +219,14 @@ class _TTRNNBase(nn.Module):
     cell_kind = ""
 
     def __init__(self, input_size, hidden_size, num_layers, device, n_cores, tt_rank, bias=True,
-                 is_naive=False, log_grads=False, new_core=None, bidirectional=False, dropout=0.0):
+                 is_naive=False, log_grads=False, new_core=None, bidirectional=False, dropout=0.0, proj_size=0):
         assert new_core in [None, 'first', 'last']
+        if proj_size != 0 and self.cell_kind != "lstm":
+            raise ValueError("proj_size argument is only supported for LSTM, not GRU")
+        proj_size = check_proj_size(proj_size, hidden_size)
+        if proj_size > 0 and (is_naive or log_grads):
+            raise NotImplementedError("proj_size > 0 runs on the sequence kernels only; is_naive=True and log_grads=True "
+                                      "need the cell-step mode, which has no projected form")
         if bidirectional and (is_naive or log_grads):
             raise NotImplementedError("bidirectional=True runs on the sequence kernels only; is_naive=True and "
                                       "log_grads=True need the cell-step mode, which has no bidirectional form")
@@ -216,6 +247,7 @@ class _TTRNNBase(nn.Module):
         self.log_grads = log_grads
         self.bidirectional = bool(bidirectional)
         self.dropout = dropout
+        self.proj_size = proj_size
         self._all_layers = []
         for i in range(self.num_layers):
             cell = self._create_first_layer_cell() if i == 0 else self._create_other_layer_cell()
@@ -264,20 +296,27 @@ class _TTRNNBase(nn.Module):
         return bool(self.is_naive or self.log_grads)
 
     def _make_cell(self, in_size):
+        extra = {"proj_size": self.proj_size} if self.proj_size else {}
         return self.cell_cls(in_size, self.hidden_size, self.bias, self.device, n_cores=self.n_cores,
-                             tt_rank=self.tt_rank, is_naive=self.is_naive, new_core=self.new_core)
+                             tt_rank=self.tt_rank, is_naive=self.is_naive, new_core=self.new_core, **extra)
+
+    @property
+    def output_size(self) -> int:
+        """Width of every layer's output and of h: proj_size when projected, else hidden_size."""
+        return self.proj_size or self.hidden_size
 
     def _create_first_layer_cell(self):
         return self._make_cell(self.input_size)
 
     def _create_other_layer_cell(self):
-        return self._make_cell(2 * self.hidden_size if self.bidirectional else self.hidden_size)
+        return self._make_cell(2 * self.output_size if self.bidirectional else self.output_size)
 
     def param_count(self):
         total = 0
         for cell in self._all_layers:
-            for attr in ('input_weights', 'hidden_weights'):
-                total += param_count(getattr(cell, attr))
+            for attr in ('input_weights', 'hidden_weights', 'projection_weights'):
+                if hasattr(cell, attr):
+                    total += param_count(getattr(cell, attr))
         return total
 
     def spec(self) -> RnnSpec:
@@ -287,7 +326,10 @@ class _TTRNNBase(nn.Module):
         if self._spec is None:
             self._spec = RnnSpec(self.cell_kind, self.input_size, self.hidden_size, bool(self.bias),
                                  [c.input_weights.tt_modes() for c in self._all_layers],
-                                 [c.hidden_weights.tt_modes() for c in self._all_layers])
+                                 [c.hidden_weights.tt_modes() for c in self._all_layers],
+                                 proj_size=self.proj_size,
+                                 hr_shapes=[c.projection_weights.tt_modes() for c in self._all_layers] if self.proj_size
+                                 else None)
         return self._spec
 
     def flat_parameters(self) -> List[torch.Tensor]:
@@ -313,10 +355,10 @@ class _TTRNNBase(nn.Module):
             return rnn_sequence(cell._single_step_spec(), x, h0, c0, cell.flat_parameters())
 
         return bidirectional_stack(input, states, self.num_layers, self.hidden_size, run,
-                                   dropout=active_dropout(self, input.device))
+                                   dropout=active_dropout(self, input.device), output_size=self.output_size)
 
-    def _shared_to_bidirectional(self, input, state):
-        return shared_bidirectional_state(state, self.num_layers, input.size(0), self.hidden_size)
+    def _shared_to_bidirectional(self, input, state, width=None):
+        return shared_bidirectional_state(state, self.num_layers, input.size(0), width or self.hidden_size)
 
     def _layer_states_in(self, input, states):
         """Per-layer initial states of the cell-step loop: a list of num_layers (batch, hidden) tensors per state
@@ -337,21 +379,29 @@ class TTLSTM(_TTRNNBase):
     cell_cls = TTLSTMCell
     cell_kind = "lstm"
 
+    def __init__(self, input_size, hidden_size, num_layers, device, n_cores, tt_rank, bias=True, is_naive=False,
+                 log_grads=False, new_core=None, bidirectional=False, dropout=0.0, proj_size=0):
+        super().__init__(input_size, hidden_size, num_layers, device, n_cores, tt_rank, bias=bias, is_naive=is_naive,
+                         log_grads=log_grads, new_core=new_core, bidirectional=bidirectional, dropout=dropout,
+                         proj_size=proj_size)
+
     def init_hidden(self, batch_size):
-        h = torch.zeros(batch_size, self.hidden_size).to(self.device)
+        h = torch.zeros(batch_size, self.output_size).to(self.device)
         c = torch.zeros(batch_size, self.hidden_size).to(self.device)
         return h, c
 
     def forward(self, input, init_states=None):
         """input (batch, seq_len, input_size) -> outputs (batch, seq_len, hidden), (h_T, c_T) of the last layer.
         `init_states` = (h0, c0), each (batch, hidden), shared by every layer; None = zeros.
+        proj_size = P > 0: outputs and h are P wide, c stays hidden wide.
         bidirectional: outputs (batch, seq_len, 2 * hidden); (h0, c0) seed every layer and both directions; h_T, c_T
         are (2, batch, hidden): the last layer's forward direction after the last step, then its reverse direction
         after the first step."""
         self._check_input(input)
         if self.bidirectional:
             h0, c0 = (None, None) if init_states is None else init_states
-            out, (h, c) = self._run_bidirectional(input, [self._shared_to_bidirectional(input, s) for s in (h0, c0)])
+            out, (h, c) = self._run_bidirectional(input, [self._shared_to_bidirectional(input, h0, self.output_size),
+                                                          self._shared_to_bidirectional(input, c0)])
             return out, (h[-2:], c[-2:])
         sink = self._fused_step_log()
         if self.cell_step_mode and sink is None:
@@ -365,7 +415,7 @@ class TTLSTM(_TTRNNBase):
         """Per-layer states, the contract of torch.nn.LSTM: `states` = (h, c), each (num_layers, batch, hidden), or None
         (zeros).  Returns (outputs (batch, seq_len, hidden), (h_n, c_n)) with every layer's final state, each
         (num_layers, batch, hidden): feeding them to the next call continues the sequence exactly where this one
-        stopped (streaming inference, truncated BPTT).
+        stopped (streaming inference, truncated BPTT).  proj_size = P > 0: h and the outputs are P wide (as torch).
         bidirectional: the states are (2 * num_layers, batch, hidden), direction d of layer l at 2l + d, in and out, as
         torch.nn.LSTM(bidirectional=True) takes them; outputs are (batch, seq_len, 2 * hidden)."""
         self._check_input(input)
