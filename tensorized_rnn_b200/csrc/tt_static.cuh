@@ -11,6 +11,7 @@
 #include <cuda_runtime.h>
 #include <type_traits>
 #include "tt_plan.h"
+#include "tt_umma.cuh"
 
 namespace tts {
 
@@ -822,14 +823,16 @@ template <class S, int k> struct WTOff { static constexpr int v = WTOff<S, k - 1
 template <class S> struct WTOff<S, 0> { static constexpr int v = 0; };
 template <class S> constexpr int wt_floats() { return WTOff<S, S::D - 1>::v + StT<S, S::D - 1>::FLOATS; }
 
-template <class S, int k>
+// wt points at WT_{K0}: stages below K0 are not staged (BwdSmem::WT0)
+template <class S, int k, int K0 = 0>
 TTS_DEV void stage_weights_t(const float *__restrict__ cores, float *__restrict__ wt, int tid) {
     using T = St<S, k>;
     using TT_ = StT<S, k>;
     constexpr int I0p = T::PACK ? T::I / (T::PACK ? S::G : 1) : 1;
     constexpr bool ZERO = (k == 0 && S::G == 3) || (T::K != T::Kraw);
+    constexpr int OFF = WTOff<S, k>::v - WTOff<S, K0>::v;
     if (ZERO)
-        for (int e = tid; e < TT_::FLOATS; e += NTHR) wt[WTOff<S, k>::v + e] = 0.f;
+        for (int e = tid; e < TT_::FLOATS; e += NTHR) wt[OFF + e] = 0.f;
     if (ZERO) __syncthreads();
     for (int e = tid; e < T::CORE; e += NTHR) {
         const int ap = e % T::rn;
@@ -839,9 +842,9 @@ TTS_DEV void stage_weights_t(const float *__restrict__ cores, float *__restrict_
         const int i = t % T::I;
         const int a = t / T::I;
         const int row = (k == 0 && T::PACK) ? gate_col<S>(i % I0p, i / I0p) : i * T::r + a;
-        wt[WTOff<S, k>::v + row * TT_::KST + j * T::rn + ap] = core_elem<S, k>(cores, e);
+        wt[OFF + row * TT_::KST + j * T::rn + ap] = core_elem<S, k>(cores, e);
     }
-    if constexpr (k + 1 < S::D) stage_weights_t<S, k + 1>(cores, wt, tid);
+    if constexpr (k + 1 < S::D) stage_weights_t<S, k + 1, K0>(cores, wt, tid);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1151,6 +1154,106 @@ TTS_DEV void flush_dw(f32x2 (&acc2)[TK][2], float *__restrict__ stg, float *__re
     __syncthreads();
 }
 
+// ---------------------------------------------------------------------------------------------
+// Tensor-core stage 0 of the contracted dX-only backward (Merge01 chains, LSTM):
+//   dX_0[b][mr][kappa] = sum_n W01[kappa][n] dY_0[b][mr][n]      (kappa < 256; n = i0'*4 + g < 64; mr < Mrow_0)
+// is one product per step with a weight that is fixed for the launch, run as D[kappa][(b, mr)] = A[kappa][n] B[(b, mr)][n]
+// with tcgen05.mma kind::tf32 and the 3xTF32 split of tt_tc.cuh (hi*hi' into the main accumulator, lo*hi' + hi*lo' into
+// a second one), so it holds the FP32 tolerances of the FFMA reference:
+//   A = W01: M = 256 = two 128-lane M-tiles, K = 64; contracted (core_elem) and split into hi / lo once per launch and
+//       kept in TMEM: columns [t*128, t*128 + 64) hi and [t*128 + 64, t*128 + 128) lo of M-tile t
+//   B = dY_0: N = 16 R rows (b, mr), K-major SWIZZLE_128B, one hi and one lo buffer in shared memory, written by the gate
+//       phase (lo = delta - hi left unrounded, as in the gradient GEMMs)
+//   D: columns 256 + t*NR (main) and 256 + (2 + t)*NR (small terms) of M-tile t; 448 columns at R = 3, 512 at R = 4
+// ---------------------------------------------------------------------------------------------
+template <class S, int R>
+struct TcStage0 {
+    using T = St<S, 0>;
+    static constexpr int NK = T::NW;                  // MMA K: the gate-packed columns of dY_0
+    static constexpr int NR = R * T::Mrow;            // MMA N: the rows (b, mr)
+    static_assert(SrcOf<S>::merged && S::G == 4 && T::K == 256 && T::r == 1 && NK % 32 == 0 && NK <= 64,
+                  "tensor-core stage 0: contracted LSTM chain with K_0 = 256 and at most 64 gate columns");
+    static_assert(NR % 16 == 0 && NR <= 64, "N of an M = 128 MMA; four accumulators of NR columns after the 256 A columns");
+    static constexpr int KB_BYTES = NR * 128;         // one k-block of 32 n: NR rows of 128 B
+    static constexpr int BUF_BYTES = (NK / 32) * KB_BYTES;
+    static constexpr int SMEM_BYTES = 2 * BUF_BYTES + 1024 /*alignment slack*/ + 16 /*mbarrier, TMEM address*/;
+    static constexpr uint32_t TCOLS = 512, ACC = 256;
+    // byte offset of the 16-byte chunk n..n+3 (n % 4 == 0) of row `row` in a K-major SWIZZLE_128B buffer
+    TTS_DEV static uint32_t b_off(int row, int n) {
+        return (uint32_t)((n / 32) * KB_BYTES + (row / 8) * 1024 + (row % 8) * 128 + ((((n % 32) / 4) ^ (row % 8)) * 16));
+    }
+    // A hi / lo -> TMEM.  Warp w writes lane quarter w % 4 of M-tile w / 4: thread = one kappa, 2 NK columns.
+    TTS_DEV static void stage_a(const float *__restrict__ cores, uint32_t tb, int tid) {
+        const int warp = tid >> 5, lane = tid & 31;
+        const int mt = warp / 4, q = warp % 4;
+        const int kap = mt * 128 + q * 32 + lane;
+        const int j = kap / T::rn, ap = kap % T::rn;
+        constexpr int I0p = T::I / S::G;
+        const uint32_t ta = tb + ((uint32_t)(q * 32) << 16) + mt * 128;
+#pragma unroll 1
+        for (int c = 0; c < NK / 32; ++c) {
+            float hi[32], lo[32];
+#pragma unroll
+            for (int e = 0; e < 32; ++e) {
+                const int n = c * 32 + e;
+                const int i = (n % 4) * I0p + n / 4;   // n = gate_col(i0', g) = i0'*4 + g, i = g*I0' + i0'
+                const float v = core_elem<S, 0>(cores, (i * T::J + j) * T::rn + ap);
+                hi[e] = ttc::tf32_rna(v);
+                lo[e] = ttc::tf32_rna(v - hi[e]);
+            }
+            ttc::tmem_st32(ta + c * 32, hi);
+            ttc::tmem_st32(ta + NK + c * 32, lo);
+        }
+        ttc::tmem_wait_st();
+    }
+    // 2 M-tiles x NK/8 k-slices x 3 products, then a commit to `bar`; one thread
+    TTS_DEV static void issue(uint32_t tb, uint32_t bhi, uint32_t blo, uint32_t bar) {
+        constexpr uint32_t idesc = ttc::umma_idesc_tf32(128, NR);
+        const uint64_t dh = ttc::umma_desc_sw128(bhi), dl = ttc::umma_desc_sw128(blo);
+#pragma unroll
+        for (int t = 0; t < 2; ++t) {
+            const uint32_t a = tb + t * 128, dm = tb + ACC + t * NR, ds = tb + ACC + (2 + t) * NR;
+            // grouped by accumulator: a change of accumulator between two MMAs costs extra issue time (tt_tc.cuh)
+#pragma unroll
+            for (int ks = 0; ks < NK / 8; ++ks) {
+                const uint64_t o = (uint64_t)((ks / 4) * (KB_BYTES >> 4) + (ks % 4) * 2);
+                ttc::umma_tf32_ts(dm, a + ks * 8, dh + o, idesc, ks > 0 ? 1u : 0u);
+            }
+#pragma unroll
+            for (int ks = 0; ks < NK / 8; ++ks) {
+                const uint64_t o = (uint64_t)((ks / 4) * (KB_BYTES >> 4) + (ks % 4) * 2);
+                ttc::umma_tf32_ts(ds, a + NK + ks * 8, dh + o, idesc, ks > 0 ? 1u : 0u);
+                ttc::umma_tf32_ts(ds, a + ks * 8, dl + o, idesc, 1u);
+            }
+        }
+        ttc::umma_commit(bar);
+    }
+    // D -> dX_0 in the X_0 slot: warp w reads lane quarter w % 4 of M-tile w / 4, thread = one kappa, all NR rows
+    TTS_DEV static void drain(uint32_t tb, float *__restrict__ dX, int tid) {
+        const int warp = tid >> 5, lane = tid & 31;
+        const int mt = warp / 4, q = warp % 4;
+        const int kap = mt * 128 + q * 32 + lane;
+        const uint32_t tl = tb + ((uint32_t)(q * 32) << 16);
+#pragma unroll
+        for (int c0 = 0; c0 < NR; c0 += 16) {
+            uint32_t m[16], s[16];
+            ttc::tmem_ld16(tl + ACC + mt * NR + c0, m);
+            ttc::tmem_ld16(tl + ACC + (2 + mt) * NR + c0, s);
+            ttc::tmem_wait_ld();
+#pragma unroll
+            for (int e = 0; e < 16; ++e) {
+                const int row = c0 + e, b = row / T::Mrow, mr = row % T::Mrow;
+                dX[b * T::BS + T::roff(mr) + kap] = __uint_as_float(m[e]) + __uint_as_float(s[e]);
+            }
+        }
+    }
+};
+
+template <class S, int R> constexpr int tc_stage0_bytes() {
+    if constexpr (SrcOf<S>::merged) return TcStage0<S, R>::SMEM_BYTES;
+    else return 0;
+}
+
 // ---- backward tuning: forward tiles (recompute) + bwd-data tiles + bwd-weight tiles -------------
 // BTM[k] rows per thread of the bwd-data stage k, BSP = split of the last bwd-data stage, WTK[k] = TK
 template <class FT, int BTM0, int BTM1, int BTM2, int BTM3, int BSP_, int WTK0, int WTK1, int WTK2, int WTK3>
@@ -1172,7 +1275,10 @@ struct BwdSmem {
     using FM = FinMap<S, R, TU::FTMr, TU::FTI, TU::FSK>;
     // forward-layout cores are only staged by the kernels that recompute (part of) the chain
     static constexpr int W = (!DWI && SV != 0) ? 0 : w_floats<S>();
-    static constexpr int WT = wt_floats<S>();
+    // contracted chains run bwd-data stage 0 on the tensor cores (TcStage0): W_0^T and dY_0 are not staged
+    static constexpr bool TC = SrcOf<S>::merged;
+    static constexpr int WT0 = TC ? StT<S, 0>::FLOATS : 0;
+    static constexpr int WT = wt_floats<S>() - WT0;
     static constexpr int stage_bs(int k) { return slot_floats_of<S>(k); }
     static constexpr int HS0 = cr4(R * stage_bs(S::D - 1));
     static constexpr int xoff(int k) {
@@ -1186,14 +1292,16 @@ struct BwdSmem {
     }
     template <int k> struct XOff { static constexpr int v = xoff(k); };
     static constexpr int XALL = DWI ? xoff(0) + cr4(R * stage_bs(0)) : HS0 + PPSlots<S, R>::P + PPSlots<S, R>::Q;
-    static constexpr int DY = cr4(R * DY0<S>::BS);
+    static constexpr int DY = TC ? 0 : cr4(R * DY0<S>::BS);
     static constexpr int DHC = cr4(R * St<S, D - 1>::BS);
     static constexpr int XCH = cmax(FM::XCH_FLOATS, BdMap<S, D - 1, R, TB::BTM[D - 1], TB::BSP>::XCH_FLOATS);
     static constexpr int H2 = cr4(R * St<S, D - 1>::BS);          // second h_{t-1} slot (cp.async double buffer)
     static constexpr int X1W = (SV != 0) ? 2 * R * XW : 0;        // rank-one input windows (kept-gates kernels)
     static constexpr int DHO = (SV != 0) ? cr4(R * n_in<S>()) : 0; // upstream-gradient tile dOut[:, t, :] (kept-gates kernels)
-    static constexpr int TOTAL = W + WT + XALL + DY + DHC + XCH + H2 + X1W + DHO;
-    static constexpr size_t BYTES = (size_t)TOTAL * 4;
+    static constexpr int TCS = tc_stage0_bytes<S, R>() / 4;          // B operand buffers, mbarrier, TMEM address
+    static constexpr int TOTAL = W + WT + XALL + DY + DHC + XCH + H2 + X1W + DHO + TCS;
+    // a TMEM-allocating kernel requests more than half of the SM's shared memory (co-residence rule, tt_umma.cuh)
+    static constexpr size_t BYTES = TC ? cmax(TOTAL * 4, ttc::TMEM_EXCLUSIVE_SMEM) : (size_t)TOTAL * 4;
 };
 
 struct RnnBwdSArgs {
@@ -1249,14 +1357,14 @@ TTS_DEV void bwd_chain(float *xs, float *hcur, float *dy0, float *dhc, const flo
     if constexpr (DWI && k == 3) bwd_weight_stage<S, 3, R, TB::WTK[3]>(X, dY, dw.a3, tid);
     if constexpr (k == S::D - 1) {
         // last stage: dX goes to the dh slot (no aliasing with X_k); split reduction
-        if constexpr (WANT_DX) bwd_data_stage<S, k, R, TB::BTM[k], TB::BSP>(dY, wt + WTOff<S, k>::v, dhc, xch, tid);
+        if constexpr (WANT_DX) bwd_data_stage<S, k, R, TB::BTM[k], TB::BSP>(dY, wt + WTOff<S, k>::v - SM::WT0, dhc, xch, tid);
         // the cp.async tiles of the NEXT step (h_{t-2}, dOut[:, t-1]) were issued at least one stage ago: waiting for them
         // here lets this barrier also publish them, so the step loop needs no barrier of its own at the top
         cp_async_wait_all();
         __syncthreads();
     } else {
         if constexpr (DWI) __syncthreads();               // X_k is overwritten in place by dX_k
-        bwd_data_stage<S, k, R, TB::BTM[k], 1>(dY, wt + WTOff<S, k>::v, X, xch, tid);
+        bwd_data_stage<S, k, R, TB::BTM[k], 1>(dY, wt + WTOff<S, k>::v - SM::WT0, X, xch, tid);
         __syncthreads();
         bwd_chain<S, R, TB, k + 1, WANT_DX, DWI>(xs, hcur, dy0, dhc, wt, xch, dw, tid);
     }
@@ -1297,6 +1405,7 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
     constexpr int G = S::G, H = n_in<S>(), GH = G * H;
     constexpr int NE = FM::NE;
     constexpr bool LSTM = (CELL == TTRNN_CELL_LSTM);
+    constexpr bool TC = SM::TC;                                  // bwd-data stage 0 on the tensor cores
     const int tid = threadIdx.x;
     float *wsm = smem;
     float *wt = wsm + SM::W;
@@ -1309,10 +1418,31 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
     constexpr int HOFF1 = SM::W + SM::WT + SM::XALL + SM::DY + SM::DHC + SM::XCH;
     float *xw1 = smem + HOFF1 + SM::H2;
     float *dho_s = xw1 + SM::X1W;
-
-    if constexpr (SM::W > 0) stage_weights_k<S, 0>(a.cores, wsm, tid);
-    stage_weights_t<S, 0>(a.cores, wt, tid);
-    for (int e = tid; e < SM::DY; e += NTHR) dy0[e] = 0.f;       // padded gate column stays zero
+    // tensor-core stage 0: B operand buffers (1024-byte aligned), the mbarrier of the MMA commit, the TMEM address
+    uint32_t tc_hi = 0, tc_lo = 0, tc_bar = 0, tmem = 0, tc_phase = 0;
+    char *tc_hi_p = nullptr, *tc_lo_p = nullptr;
+    if constexpr (TC) {
+        using TC0 = TcStage0<S, R>;
+        tc_hi = (ttc::smem_u32(dho_s + SM::DHO) + 1023u) & ~1023u;
+        tc_lo = tc_hi + TC0::BUF_BYTES;
+        tc_bar = tc_lo + TC0::BUF_BYTES;
+        const uint32_t tc_slot = tc_bar + 8;
+        tc_hi_p = reinterpret_cast<char *>(smem) + (tc_hi - ttc::smem_u32(smem));
+        tc_lo_p = tc_hi_p + TC0::BUF_BYTES;
+        if (tid == 0) { ttc::mbar_init(tc_bar, 1); ttc::fence_barrier_init(); }
+        if (tid < 32) ttc::tmem_alloc(tc_slot, TC0::TCOLS);
+        ttc::tc_fence_before();
+        __syncthreads();
+        ttc::tc_fence_after();
+        tmem = *reinterpret_cast<volatile uint32_t *>(reinterpret_cast<char *>(smem) + (tc_slot - ttc::smem_u32(smem)));
+        TC0::stage_a(a.cores, tmem, tid);
+        ttc::tc_fence_before();                                  // ordered before the first MMA by the step barriers
+        stage_weights_t<S, 1, 1>(a.cores, wt, tid);
+    } else {
+        if constexpr (SM::W > 0) stage_weights_k<S, 0>(a.cores, wsm, tid);
+        stage_weights_t<S, 0>(a.cores, wt, tid);
+        for (int e = tid; e < SM::DY; e += NTHR) dy0[e] = 0.f;   // padded gate column stays zero
+    }
 
     int mt, itg, kh;
     FM::coords(tid, mt, itg, kh);
@@ -1564,7 +1694,14 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
                     // delta_hh -> dY_0 [b][mr][i0'*4 + g]
                     const int mr = h % T0::Mrow, i0p = h / T0::Mrow;
                     float *dyr = dy0 + b * DY0<S>::BS + mr * DY0<S>::DS;
-                    if (G == 4) {
+                    if constexpr (TC) {                   // hi / lo rows of the B operand
+                        using TC0 = TcStage0<S, R>;
+                        float4 dhi, dlo;
+                        ttc::split4_trunc(make_float4(d_hh[0], d_hh[1], d_hh[2], d_hh[3]), dhi, dlo);
+                        const uint32_t off = TC0::b_off(b * T0::Mrow + mr, i0p * 4);
+                        *reinterpret_cast<float4 *>(tc_hi_p + off) = dhi;
+                        *reinterpret_cast<float4 *>(tc_lo_p + off) = dlo;
+                    } else if (G == 4) {
                         st4(dyr + i0p * 4, make_float4(d_hh[0], d_hh[1], d_hh[2], d_hh[3]));
                     } else {
                         *reinterpret_cast<float2 *>(dyr + gate_col<S>(i0p, 0)) = make_float2(d_hh[0], d_hh[1]);
@@ -1582,12 +1719,29 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
                         g_bhh[n][g] += d_hh[g];
                     }
                 }
+            if constexpr (TC) ttc::fence_proxy_async();   // the B operand is read by the tensor core
             __syncthreads();
             if constexpr (SAVEU) {
                 if (t > 0) fetch_dho(tg - 1);             // the tile of this step has been consumed by every thread
             }
             // ---- backward chain: core gradients (register tiles) and dh_{t-1}
-            bwd_chain<S, R, TB, 0, true, DWI>(xs, hcur, dy0, dhc, wt, xch, dw, tid);
+            if constexpr (TC) {
+                using TC0 = TcStage0<S, R>;
+                if (tid < 32) {
+                    ttc::tc_fence_after();
+                    if (ttc::elect_one()) TC0::issue(tmem, tc_hi, tc_lo, tc_bar);
+                    __syncwarp();
+                }
+                ttc::mbar_wait(tc_bar, tc_phase);
+                tc_phase ^= 1u;
+                ttc::tc_fence_after();
+                TC0::drain(tmem, xs + SM::template XOff<0>::v, tid);
+                ttc::tc_fence_before();                   // the next step's MMAs overwrite the accumulators
+                __syncthreads();
+                bwd_chain<S, R, TB, 1, true, DWI>(xs, hcur, dy0, dhc, wt, xch, dw, tid);
+            } else {
+                bwd_chain<S, R, TB, 0, true, DWI>(xs, hcur, dy0, dhc, wt, xch, dw, tid);
+            }
             cp_async_wait_all();
         }
         __syncthreads();
@@ -1600,6 +1754,11 @@ __global__ void __launch_bounds__(NTHR, MINB) k_rnn_bwd_s(const __grid_constant_
                     a.dh_out[(row0 + b) * H + h] = dhd[b][n] + dhc[b * TL::BS + (h / TL::K) * TL::KS + (h % TL::K)];
                     if (LSTM) a.dc_out[(row0 + b) * H + h] = dcs[b][n];
                 }
+    }
+    if constexpr (TC) {
+        ttc::tc_fence_before();
+        __syncthreads();
+        if (tid < 32) ttc::tmem_dealloc(tmem, TcStage0<S, R>::TCOLS);
     }
     // ---- flush gradients of this CTA into its slot
     if (!a.partial) return;

@@ -170,9 +170,9 @@ using TB_d3_split_R3 = TuneB<Tune<1, 1, 1, 1, 8, 1, 8>, 2, 2, 1, 1, 8, 4, 8, 4, 
 // H = 768 d2 r4: dX-only kernel with kept gates (the fused variant's core-gradient tiles do not divide 256 threads)
 using TB_h768_split = TuneB<Tune<1, 3, 1, 1, 8>, 1, 1, 1, 1, 2, 8, 8, 8, 8>;
 using TB_d4r16_split = TuneB<Tune<4, 1, 4, 8, 8, 8, 8, 4, 8>, 8, 8, 4, 1, 4, 4, 4, 4, 4>;
-// contracted d3 r8 chain, dX only: bwd-data stage 0 (K = 256, 64 gate rows) two rows per thread, stage 1 as stage 2 of
-// the three-core chain (split 8 ways); the forward tile only sets the ownership of hidden units (one per thread)
-using TB_m01_split = TuneB<Tune<1, 1, 1, 1, 8>, 2, 1, 1, 1, 8, 4, 8, 4, 4>;
+// contracted d3 r8 chain, dX only: bwd-data stage 0 runs on the tensor cores (tts::TcStage0, no FFMA tile), stage 1 as
+// stage 2 of the three-core chain (split 8 ways); the forward tile only sets the ownership of hidden units (one per thread)
+using TB_m01_split = TuneB<Tune<1, 1, 1, 1, 8>, 1, 1, 1, 1, 8, 4, 8, 4, 4>;
 const TtsRnnBwdEntry kBwd[] = {
     TTS_BWD(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_RANK1, TB_d2),
     TTS_BWD(HH_H256_d2r4_lstm, TTRNN_CELL_LSTM, 4, tts::MODE_RANK1, TB_d2),
@@ -218,7 +218,7 @@ const TtsRnnBwdEntry kBwd[] = {
     TTS_BWD_SPLIT_SAVEU(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, TB_d3_split_R2),
     TTS_BWD_SPLIT_SAVEU(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_XG, TB_d3_split_R2),
     TTS_BWD_SPLIT_SAVEU(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 3, tts::MODE_XG, TB_d3_split_R3),
-    // four rows fit once the contracted chain drops the second X_k slot (209 KB; 246 KB for the three-core chain)
+    // contracted chain: stage 0 of the backward on the tensor cores, one CTA per SM at every R (TMEM co-residence rule)
     TTS_BWD_SPLIT_SAVEU_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 1, tts::MODE_XG, TB_m01_split),
     TTS_BWD_SPLIT_SAVEU_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 2, tts::MODE_XG, TB_m01_split),
     TTS_BWD_SPLIT_SAVEU_M01(HH_H256_d3r8_lstm, TTRNN_CELL_LSTM, 3, tts::MODE_XG, TB_m01_split),

@@ -34,6 +34,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "tt_umma.cuh"
+
 namespace ttc {
 
 // -DTC_PROBE (tools/tc_gemm_test only): clock64 around every wait of the MMA issuer of one CTA
@@ -64,161 +66,6 @@ inline RagBox make_ragbox(long long rpb, long long nb, int cap) {
     else { g.rb = (int)rpb; g.nbx = (int)(cap / rpb); g.tpb = 1; }
     g.nboxes = ((nb + g.nbx - 1) / g.nbx) * g.tpb;
     return g;
-}
-
-// ---- PTX wrappers ----------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-// bounded wait: a protocol bug must abort the kernel, not hang the GPU
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    if (mbar_try(bar, parity)) return;
-    const long long t0 = clock64();
-    while (!mbar_try(bar, parity))
-        if (clock64() - t0 > 8000000000LL) __trap();
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap *map) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t slot_smem, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot_smem), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-// D[tmem] (+)= A[smem desc] * B[smem desc]^T, TF32 inputs, FP32 accumulate; issued by ONE thread
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// D[tmem] (+)= A[tmem] * B[smem desc]^T: the A operand (128 rows x 8 k, one 32-bit column per k value) read from TMEM
-__device__ __forceinline__ void umma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// 32 lanes x 16 consecutive columns: thread l of the warp writes row (lane base + l)
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const float (&v)[16]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-        ::"r"(taddr), "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
-          "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7])),
-          "r"(__float_as_uint(v[8])), "r"(__float_as_uint(v[9])), "r"(__float_as_uint(v[10])), "r"(__float_as_uint(v[11])),
-          "r"(__float_as_uint(v[12])), "r"(__float_as_uint(v[13])), "r"(__float_as_uint(v[14])), "r"(__float_as_uint(v[15]))
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const float (&v)[32]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-        ::"r"(taddr), "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
-          "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7])),
-          "r"(__float_as_uint(v[8])), "r"(__float_as_uint(v[9])), "r"(__float_as_uint(v[10])), "r"(__float_as_uint(v[11])),
-          "r"(__float_as_uint(v[12])), "r"(__float_as_uint(v[13])), "r"(__float_as_uint(v[14])), "r"(__float_as_uint(v[15])),
-          "r"(__float_as_uint(v[16])), "r"(__float_as_uint(v[17])), "r"(__float_as_uint(v[18])), "r"(__float_as_uint(v[19])),
-          "r"(__float_as_uint(v[20])), "r"(__float_as_uint(v[21])), "r"(__float_as_uint(v[22])), "r"(__float_as_uint(v[23])),
-          "r"(__float_as_uint(v[24])), "r"(__float_as_uint(v[25])), "r"(__float_as_uint(v[26])), "r"(__float_as_uint(v[27])),
-          "r"(__float_as_uint(v[28])), "r"(__float_as_uint(v[29])), "r"(__float_as_uint(v[30])), "r"(__float_as_uint(v[31]))
-        : "memory");
-}
-__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// arrive on an mbarrier once every MMA issued so far by this thread has completed
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// 32 lanes x 32 consecutive columns: thread l of the warp gets row (lane base + l), v[j] = column j
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-    uint32_t r[32];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr)
-        : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
-}
-
-// K-major SWIZZLE_128B shared-memory matrix descriptor (tile base 1024-byte aligned):
-// start address >> 4 | LBO (ignored for swizzled K-major) = 1 | SBO = 1024 B (8-row group pitch) | version 1 | layout 2
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
-    return (uint64_t)((smem_addr >> 4) & 0x3FFF) | (1ull << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
-}
-// instruction descriptor: D = F32, A = B = TF32, both K-major, M x N
-__host__ __device__ constexpr uint32_t umma_idesc_tf32(int M, int N) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-// one lane of a fully converged warp (elect.sync).  The MMA issuer must be selected THIS way: under `if (lane == 0)` ptxas
-// wraps every UTCHMMA in a per-lane ELECT / BRA.U.ANY loop (it cannot prove the branch selects one lane), which costs ~100
-// clk of issue time per MMA on a shared scheduler -- more than the 64 clk the tensor core needs for it (measured, round 2)
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred = 0;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "elect.sync _|p, 0xffffffff;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(pred));
-    return pred != 0;
-}
-
-__device__ __forceinline__ float tf32_rna(float x) {
-    uint32_t u;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));
-    return __uint_as_float(u);
-}
-__device__ __forceinline__ void split4(const float4 v, float4 &hi, float4 &lo) {
-    hi.x = tf32_rna(v.x); hi.y = tf32_rna(v.y); hi.z = tf32_rna(v.z); hi.w = tf32_rna(v.w);
-    lo.x = tf32_rna(v.x - hi.x); lo.y = tf32_rna(v.y - hi.y); lo.z = tf32_rna(v.z - hi.z); lo.w = tf32_rna(v.w - hi.w);
-}
-
-// gradient kernels: lo = x - hi left unrounded (the tensor core truncates it to TF32: error <= 2^-21 |x|, two ALU ops fewer)
-__device__ __forceinline__ void split4_trunc(const float4 v, float4 &hi, float4 &lo) {
-    hi.x = tf32_rna(v.x); hi.y = tf32_rna(v.y); hi.z = tf32_rna(v.z); hi.w = tf32_rna(v.w);
-    lo.x = v.x - hi.x; lo.y = v.y - hi.y; lo.z = v.z - hi.z; lo.w = v.w - hi.w;
 }
 
 // one k-block (BK = 32 k-values, `nks` slices of 8) of the compensated product: hi*hi' into the main accumulator,
@@ -276,6 +123,7 @@ constexpr int ROWS_STAGES = 3;
 constexpr int ROWS_NT = 448;                     // 14 warps
 constexpr int ROWS_STAGE_BYTES = 4 * TILE_BYTES;             // A hi (raw lands here), A lo, Bt hi, Bt lo
 constexpr int ROWS_SMEM = ROWS_STAGES * ROWS_STAGE_BYTES + 1024 /*alignment slack*/ + 256 /*barriers*/;
+static_assert(ROWS_SMEM >= TMEM_EXCLUSIVE_SMEM, "TMEM co-residence rule");
 
 struct TcRowsArgs {
     RagBox g;                // row tiles (cap 128)
@@ -455,6 +303,7 @@ constexpr int RWT_STAGES = 4;
 constexpr int RWT_NT = 576;
 constexpr int RWT_STAGE_BYTES = 3 * TILE_BYTES;              // raw A, Bt hi, Bt lo
 constexpr int RWT_SMEM = RWT_STAGES * RWT_STAGE_BYTES + 1024 + 256;
+static_assert(RWT_SMEM >= TMEM_EXCLUSIVE_SMEM, "TMEM co-residence rule");
 
 template <bool GRAD>
 __global__ void __launch_bounds__(RWT_NT, 1)
@@ -677,6 +526,7 @@ constexpr int RED_RAW_STAGES = 3, RED_OP_STAGES = 2;
 constexpr int RED_RAW_BYTES = 2 * TILE_BYTES;                // raw A [32][128], raw B [32][128]
 constexpr int RED_OP_BYTES = 4 * TILE_BYTES;                 // A hi, A lo, B hi, B lo
 constexpr int RED_SMEM = RED_RAW_STAGES * RED_RAW_BYTES + RED_OP_STAGES * RED_OP_BYTES + 1024 + 256 + 2 * 128 * 4;
+static_assert(RED_SMEM >= TMEM_EXCLUSIVE_SMEM, "TMEM co-residence rule");
 
 struct TcRedArgs {
     RagBox g;                // k-blocks of the row dimension (cap 32)
@@ -876,6 +726,7 @@ k_tc_red(const __grid_constant__ TcRedArgs g, const __grid_constant__ CUtensorMa
 constexpr int RTS_RAW_STAGES = 5, RTS_OP_STAGES = 2;
 constexpr int RTS_OP_BYTES = 2 * TILE_BYTES;                 // B hi, B lo
 constexpr int RTS_SMEM = RTS_RAW_STAGES * RED_RAW_BYTES + RTS_OP_STAGES * RTS_OP_BYTES + 1024 + 256;
+static_assert(RTS_SMEM >= TMEM_EXCLUSIVE_SMEM, "TMEM co-residence rule");
 
 __global__ void __launch_bounds__(RED_NT, 1)
 k_tc_red_ts(const __grid_constant__ TcRedArgs g, const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB) {

@@ -1,9 +1,12 @@
-// Micro-benchmark: cycles per tcgen05.mma kind::tf32 dispatch on sm_100a, for the issue patterns of csrc/tt_tc.cuh.
+// Micro-benchmark: cycles per tcgen05.mma kind::tf32 dispatch on sm_100a, for the issue patterns of csrc/tt_tc.cuh,
+// and the per-step round trip of the tensor-core stage 0 of the contracted BPTT kernel (tts::TcStage0).
 // One CTA per SM, operands are whatever shared memory / TMEM holds (timing only).  Build:
-//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 tools/mma_rate_probe.cu -o tools/mma_rate_probe
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 --expt-relaxed-constexpr tools/mma_rate_probe.cu -o tools/mma_rate_probe
 #include <cstdio>
 #include <cstdlib>
 
+#include "../tensorized_rnn_b200/csrc/tt_plan.h"
+#include "../tensorized_rnn_b200/csrc/tt_static.cuh"
 #include "../tensorized_rnn_b200/csrc/tt_tc.cuh"
 
 using namespace ttc;
@@ -139,9 +142,105 @@ __global__ void __launch_bounds__(256, 1) k_probe(int mode, int N, int iters, lo
     if (threadIdx.x < 32) tmem_dealloc(tb, 512);
 }
 
-int main() {
+// Round trip of one step of the tensor-core stage 0 at R rows per CTA, as k_rnn_bwd_s runs it: every thread writes the
+// hi / lo parts of its R gate-gradient chunks into the B buffers -> proxy fence + barrier -> 48 MMAs with A from TMEM ->
+// commit -> mbarrier wait -> tcgen05.ld of 2 x 16R columns per thread -> stores into the X_0 slot -> barrier.
+struct HH_d3r8 {
+    static constexpr int D = 3, G = 4;
+    static constexpr int J[7] = {4, 8, 8}, I[7] = {8, 8, 16}, RK[7] = {1, 8, 8, 1};
+};
+template <int R>
+__global__ void __launch_bounds__(256, 1) k_step_probe(const float *cores, int steps, long long *out) {
+    using S = tts::Merge01<HH_d3r8>;
+    using TC0 = tts::TcStage0<S, R>;
+    using T0 = tts::St<S, 0>;
+    extern __shared__ __align__(16) float smem[];
+    const int tid = threadIdx.x;
+    float *x0 = smem;
+    const uint32_t hi = (smem_u32(smem + R * T0::BS) + 1023u) & ~1023u, lo = hi + TC0::BUF_BYTES;
+    const uint32_t bar = lo + TC0::BUF_BYTES, slot = bar + 8;
+    char *hi_p = reinterpret_cast<char *>(smem) + (hi - smem_u32(smem)), *lo_p = hi_p + TC0::BUF_BYTES;
+    if (tid == 0) { mbar_init(bar, 1); fence_barrier_init(); }
+    if (tid < 32) tmem_alloc(slot, TC0::TCOLS);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tb = *reinterpret_cast<volatile uint32_t *>(reinterpret_cast<char *>(smem) + (slot - smem_u32(smem)));
+    TC0::stage_a(cores, tb, tid);
+    tc_fence_before();
+    __syncthreads();
+    const int mr = tid % T0::Mrow, i0p = tid / T0::Mrow;          // the hidden unit of the gate phase (one per thread)
+    uint32_t phase = 0;
+    const long long t0 = clock64();
+    for (int t = 0; t < steps; ++t) {
+#pragma unroll
+        for (int b = 0; b < R; ++b) {
+            const float v = x0[b * T0::BS + T0::roff(mr) + tid] * 0.5f + (float)(t + b);
+            float4 h, l;
+            split4_trunc(make_float4(v, v + 1.f, v + 2.f, v + 3.f), h, l);
+            const uint32_t off = TC0::b_off(b * T0::Mrow + mr, i0p * 4);
+            *reinterpret_cast<float4 *>(hi_p + off) = h;
+            *reinterpret_cast<float4 *>(lo_p + off) = l;
+        }
+        fence_proxy_async();
+        __syncthreads();
+        if (tid < 32) {
+            tc_fence_after();
+            if (elect_one()) TC0::issue(tb, hi, lo, bar);
+            __syncwarp();
+        }
+        mbar_wait(bar, phase);
+        phase ^= 1u;
+        tc_fence_after();
+        TC0::drain(tb, x0, tid);
+        tc_fence_before();
+        __syncthreads();
+    }
+    const long long t1 = clock64();
+    if (tid == 0) out[blockIdx.x] = t1 - t0;
+    if (tid < 32) tmem_dealloc(tb, TC0::TCOLS);
+}
+
+template <int R>
+void step_probe(const float *cores, long long *d) {
+    using S = tts::Merge01<HH_d3r8>;
+    static_assert(R * tts::St<S, 0>::BS * 4 + tts::TcStage0<S, R>::SMEM_BYTES <= ttc::TMEM_EXCLUSIVE_SMEM, "probe smem");
+    cudaFuncSetAttribute(k_step_probe<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, ttc::TMEM_EXCLUSIVE_SMEM);
+    const int steps = 160, reps = 20;
+    k_step_probe<R><<<148, 256, ttc::TMEM_EXCLUSIVE_SMEM>>>(cores, steps, d);
+    cudaEvent_t e0, e1;
+    cudaEventCreate(&e0);
+    cudaEventCreate(&e1);
+    cudaEventRecord(e0);
+    for (int i = 0; i < reps; ++i) k_step_probe<R><<<148, 256, ttc::TMEM_EXCLUSIVE_SMEM>>>(cores, steps, d);
+    cudaEventRecord(e1);
+    cudaError_t e = cudaDeviceSynchronize();
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, e0, e1);
+    long long c[148];
+    cudaMemcpy(c, d, sizeof(c), cudaMemcpyDeviceToHost);
+    long long cmax = 0;
+    double csum = 0;
+    for (int i = 0; i < 148; ++i) { csum += c[i]; if (c[i] > cmax) cmax = c[i]; }
+    printf("stage-0 round trip R=%d (N=%d, 148 CTAs, %d steps): %s  %.0f clk per step (mean over CTAs, max %.0f);  "
+           "%.3f us per step (launch time / steps, incl. TMEM set-up)\n",
+           R, 16 * R, steps, cudaGetErrorString(e), csum / 148 / steps, (double)cmax / steps, 1e3 * ms / reps / steps);
+}
+
+int main(int argc, char **argv) {
     long long *d;
-    cudaMalloc(&d, 64);
+    cudaMalloc(&d, 148 * 8);
+    if (argc > 1 && argv[1][0] == 's') {                     // "step": the stage-0 round trip only
+        float *cores;
+        const int n = tts::core_floats<HH_d3r8>();
+        cudaMalloc(&cores, n * 4);
+        cudaMemset(cores, 0, n * 4);
+        step_probe<1>(cores, d);
+        step_probe<2>(cores, d);
+        step_probe<3>(cores, d);
+        step_probe<4>(cores, d);
+        return 0;
+    }
     const int smem = 6 * TILE_BYTES + 2048 + 96 * 16 * 16 + 1024;
     cudaFuncSetAttribute(k_probe, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     const int iters = 2000;
