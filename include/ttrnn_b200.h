@@ -368,7 +368,8 @@ int ttrnn_kernel_timing(int32_t enable);
 int ttrnn_kernel_times(double *ms /*[TTRNN_K_KINDS]*/, int64_t *count /*[TTRNN_K_KINDS]*/);
 /* Per-launch records of the last ttrnn_kernel_times() call: 6 doubles per record = {kind, rows per CTA, grid size (CTAs),
  * batch rows of the launch, timesteps of the launch, milliseconds}; all but kind and milliseconds are 0 for the kinds
- * that are not recurrent kernels.
+ * that are not recurrent kernels, except that a statically specialised TT-matvec kernel (kinds 0 and 3) reports its rows
+ * per CTA, grid and rows (batch rows x timesteps of the chunk).
  * Returns the number of records (buf NULL: just the count).  bench.py reports the recurrent kernels per variant from it. */
 int64_t ttrnn_kernel_launch_records(double *buf, int64_t cap_records);
 
@@ -397,6 +398,16 @@ int64_t ttrnn_tc_launch_count(int32_t reset);
  * kernel "kind|name|rows_per_cta|shared_memory_bytes|fits" (fits = 1 when it is within the 227 KB opt-in limit
  * and can be selected).  Returns the number of characters written, < 0 on a bad buffer. */
 int ttrnn_static_kernel_table(char *buf, int32_t cap);
+/* Host-only: the same kernels in the same order, one line per kernel with the key that identifies it:
+ * "kind|name|rows_per_cta|cell|mode|saved|split|merged" (cell = TTRNN_CELL_*, mode = input mode 0 projected /
+ * 1 rank-one, saved = 2 when the BPTT kernel consumes kept gate activations, split = 1 for dX-only BPTT kernels and for
+ * the TT-matvec backward kernels without dX, merged = 1 for the chain with cores 0 and 1 contracted; -1 where a column
+ * does not apply to the TT-matvec kernels).  Returns the number of characters written, < 0 on a bad buffer. */
+int ttrnn_static_kernel_keys(char *buf, int32_t cap);
+/* Host-only: launches of every statically specialised kernel since the last reset, one counter per line of
+ * ttrnn_static_kernel_table (and ttrnn_static_kernel_keys) in their order; copies min(cap, entries) counters into
+ * counts (may be NULL), zeroes them when reset != 0.  Returns the number of entries. */
+int ttrnn_static_kernel_launches(int64_t *counts, int32_t cap, int32_t reset);
 
 /* Tuning knobs (process-wide; also read from the environment at load time):
  *   "rows_per_cta"  batch rows owned by one CTA of the recurrent kernels (0 = auto)

@@ -104,8 +104,10 @@ SYMBOLS = {
     "ttrnn_ge2e_loss_backward": (C.c_int, [C.c_int32, C.c_int32, C.c_int32] + [_P] * 7),
     "ttrnn_rnn_ih_route": (C.c_int, [C.POINTER(RnnDesc), C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "ttrnn_static_kernel_table": (C.c_int, [C.c_char_p, C.c_int32]),
+    "ttrnn_static_kernel_keys": (C.c_int, [C.c_char_p, C.c_int32]),
     "ttrnn_rnn_describe": (C.c_int, [C.POINTER(RnnDesc), C.c_int32, C.c_char_p, C.c_int32]),
     "ttrnn_tc_launch_count": (C.c_int64, [C.c_int32]),
+    "ttrnn_static_kernel_launches": (C.c_int, [C.POINTER(C.c_int64), C.c_int32, C.c_int32]),
     "ttrnn_rnn_row_groups": (C.c_int, [C.POINTER(RnnDesc), C.c_int32, C.POINTER(C.c_int64)]),
     "ttrnn_ffma_probe": (C.c_int, [C.c_int32, _P, C.POINTER(C.c_double), _P]),
     "ttrnn_launch_count": (C.c_int64, [C.c_int32]),

@@ -70,3 +70,13 @@ const TtsTtlBwdEntry *tts_find_ttl_bwd(const ttrnn_tt_shape *s, long long rows, 
 
 // text table of the registry (kind|name|R|smem bytes|fits 227 KB), returns the number of characters written
 int tts_dump_entries(char *buf, int cap);
+// the registry's keys in the same order (kind|name|R|cell|mode|saved|split|merged), returns the characters written
+int tts_dump_keys(char *buf, int cap);
+
+// launch counters per registry entry (table order of tts_dump_entries / tts_dump_keys): every call site of an entry's `launch` counts it
+void tts_count_launch(const TtsRnnFwdEntry *e);
+void tts_count_launch(const TtsRnnBwdEntry *e);
+void tts_count_launch(const TtsTtlFwdEntry *e);
+void tts_count_launch(const TtsTtlBwdEntry *e);
+// copies min(cap, entries) counters into counts (may be null), zeroes them all when reset != 0; returns the entry count
+int tts_entry_launches(long long *counts, int cap, int reset);

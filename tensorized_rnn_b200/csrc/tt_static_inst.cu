@@ -2,6 +2,7 @@
 // lookup used by the C ABI.  Adding a shape = one TTS_SHAPE line + one TTS_FWD line per variant.
 #include "tt_static.cuh"
 #include "tt_static_api.h"
+#include <atomic>
 #include <cstdio>
 
 namespace {
@@ -284,7 +285,7 @@ const TtsTtlBwdEntry kTtlBwd[] = {
 
 }  // namespace
 
-// text table of every registered static kernel: "kind name R smem_bytes fits\n" (tests assert that all fit)
+// text table of every registered static kernel: "kind|name|R|smem_bytes|fits\n" (tests assert that all fit)
 int tts_dump_entries(char *buf, int cap) {
     int n = 0;
     auto put = [&](const char *kind, const char *name, int R, size_t smem) {
@@ -295,6 +296,42 @@ int tts_dump_entries(char *buf, int cap) {
     for (const auto &e : kTtlFwd) put("ttl_fwd", e.name, e.R, e.smem);
     for (const auto &e : kTtlBwd) put("ttl_bwd", e.name, e.R, e.smem);
     return n;
+}
+
+// the same entries in the same order, each with its full key: "kind|name|R|cell|mode|saved|split|merged\n".
+// (kind, name, R) alone is not unique (d2 r4 has rank-one and projected-input kernels under one name).  The TT-matvec
+// kernels (ttl_*) have no cell, mode or saved gates (-1); a ttl_bwd entry with split = 1 computes the core gradients
+// only (no dX).
+int tts_dump_keys(char *buf, int cap) {
+    int n = 0;
+    auto put = [&](const char *kind, const char *name, int R, int cell, int mode, int saved, int split, int merged) {
+        if (n < cap)
+            n += snprintf(buf + n, cap - n, "%s|%s|%d|%d|%d|%d|%d|%d\n", kind, name, R, cell, mode, saved, split, merged);
+    };
+    for (const auto &e : kFwd) put("rnn_fwd", e.name, e.R, e.cell, e.mode, 0, 0, e.merged);
+    for (const auto &e : kBwd) put("rnn_bwd", e.name, e.R, e.cell, e.mode, e.saved, e.split, e.merged);
+    for (const auto &e : kTtlFwd) put("ttl_fwd", e.name, e.R, -1, -1, -1, 0, 0);
+    for (const auto &e : kTtlBwd) put("ttl_bwd", e.name, e.R, -1, -1, -1, e.want_dx ? 0 : 1, 0);
+    return n;
+}
+
+// launches per registry entry, indexed in the order of tts_dump_entries / tts_dump_keys (host counters, bumped by the launch sites)
+namespace {
+constexpr int kNFwd = sizeof kFwd / sizeof kFwd[0], kNBwd = sizeof kBwd / sizeof kBwd[0];
+constexpr int kNTtlFwd = sizeof kTtlFwd / sizeof kTtlFwd[0], kNTtlBwd = sizeof kTtlBwd / sizeof kTtlBwd[0];
+constexpr int kNEntries = kNFwd + kNBwd + kNTtlFwd + kNTtlBwd;
+std::atomic<long long> g_entry_launches[kNEntries];
+}  // namespace
+void tts_count_launch(const TtsRnnFwdEntry *e) { ++g_entry_launches[e - kFwd]; }
+void tts_count_launch(const TtsRnnBwdEntry *e) { ++g_entry_launches[kNFwd + (e - kBwd)]; }
+void tts_count_launch(const TtsTtlFwdEntry *e) { ++g_entry_launches[kNFwd + kNBwd + (e - kTtlFwd)]; }
+void tts_count_launch(const TtsTtlBwdEntry *e) { ++g_entry_launches[kNFwd + kNBwd + kNTtlFwd + (e - kTtlBwd)]; }
+int tts_entry_launches(long long *counts, int cap, int reset) {
+    for (int i = 0; i < kNEntries; ++i) {
+        const long long v = reset ? g_entry_launches[i].exchange(0) : g_entry_launches[i].load();
+        if (counts && i < cap) counts[i] = v;
+    }
+    return kNEntries;
 }
 
 const TtsTtlFwdEntry *tts_find_ttl_fwd(const ttrnn_tt_shape *s, long long rows) {

@@ -434,6 +434,15 @@ inline int layer_mode(const ttrnn_rnn_desc *d, int l) {
     return (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
 }
 
+// input modes the BPTT of layer l may run: the layer's own, and for a rank-one layer 0 also MODE_XG, which the backward
+// takes when the input gradient is requested (buffers are sized before it is known whether it will be).  Returns the count.
+inline int bwd_modes(const ttrnn_rnn_desc *d, int l, int modes[2]) {
+    modes[0] = layer_mode(d, l);
+    if (modes[0] != tts::MODE_RANK1) return 1;
+    modes[1] = tts::MODE_XG;
+    return 2;
+}
+
 // statically specialised forward kernel of layer l at B rows on `sms` SMs, or nullptr (runtime-shape kernel).  A projected
 // layer has none: its chains run on the runtime-shape kernels k_rnn_fwd_proj / k_rnn_bwd_proj.
 const TtsRnnFwdEntry *fwd_route(const ttrnn_rnn_desc *d, const RnnPlan &rp, int l, long long B, int sms) {
@@ -678,19 +687,27 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
     // kept gate activations of the static recurrent kernels ("save_u_bytes" budget, default 16 GiB): 4*H floats per row
     // and step (LSTM i,f,g,o; GRU r,z,n,u_n) -- backward skips the final stage of the recompute and all gate math.  Every
     // layer whose forward and kept-gates backward are static keeps them, or none does.  The dense accumulation of the hh
-    // core gradients is sized for a split backward with or without kept gates.
+    // core gradients is sized for a split backward with or without kept gates.  Both hold for every input mode the
+    // layer's backward may run (bwd_modes): a rank-one layer 0 keeps its gates only when the projected-input route with
+    // dX has a kept-gates kernel too, and that route's split kernels need the dense buffer also where the rank-one split
+    // route does not apply (chunked plans).
     bool can_keep[TTRNN_MAX_LAYERS] = {};
     long long kept_floats = 0, dhh = 0;
     if (t_opt.stat)
         for (int l = 0; l < L; ++l) {
-            BwdRoute recompute, keep;
-            if (bwd_route(d, rp, l, layer_mode(d, l), B, dv.sms, false, tc, &recompute) ||
-                bwd_route(d, rp, l, layer_mode(d, l), B, dv.sms, true, tc, &keep))
-                return 1;
-            can_keep[l] = keep.kept && fwd_route(d, rp, l, B, dv.sms);
+            int modes[2];
+            const int nm = bwd_modes(d, l, modes);
+            can_keep[l] = fwd_route(d, rp, l, B, dv.sms) != nullptr;
+            for (int k = 0; k < nm; ++k) {
+                BwdRoute recompute, keep;
+                if (bwd_route(d, rp, l, modes[k], B, dv.sms, false, tc, &recompute) ||
+                    bwd_route(d, rp, l, modes[k], B, dv.sms, true, tc, &keep))
+                    return 1;
+                can_keep[l] = can_keep[l] && keep.kept;
+                if ((recompute.dense_hh || keep.dense_hh) && dense_bwd_floats(rp.layer[l].hh) > dhh)
+                    dhh = dense_bwd_floats(rp.layer[l].hh);
+            }
             if (can_keep[l]) kept_floats += r4(B * T * 4 * H);
-            if ((recompute.dense_hh || keep.dense_hh) && dense_bwd_floats(rp.layer[l].hh) > dhh)
-                dhh = dense_bwd_floats(rp.layer[l].hh);
         }
     const bool keep_all = kept_floats > 0 && kept_floats * 4 <= t_opt.save_u_bytes;
     for (int l = 0; l < L; ++l) {
@@ -833,9 +850,10 @@ int launch_ttlinear_fwd(const ChainPlan &p, const DevInfo &dv, long long rows, i
             sa.rows = rows; sa.rows_per_b = rows_per_b; sa.x_bstride = x_bstride; sa.y_bstride = y_bstride;
             sa.x = x; sa.cores = cores; sa.bias = bias; sa.bias2 = bias2; sa.y = y;
             {
-                KernelTimer tm(TTRNN_K_TTLINEAR_FWD, st);
+                KernelTimer tm(TTRNN_K_TTLINEAR_FWD, st, e->R, (int)g, rows);
                 rc = e->launch(&sa, (int)g, st);
             }
+            tts_count_launch(e);
             ++g_launches;
             if (rc) return fail("static kernel %s launch failed: %s", e->name, cudaGetErrorString((cudaError_t)rc));
             return 0;
@@ -883,9 +901,10 @@ int launch_ttlinear_bwd(const ChainPlan &p0, const DevInfo &dv, long long rows, 
             sa.x_bstride = x_bstride; sa.dy_bstride = dy_bstride; sa.dx_bstride = dx_bstride;
             sa.x = x; sa.cores = cores; sa.dy = dy; sa.dx = dx; sa.partial = partial; sa.want_dbias = want_dbias;
             {
-                KernelTimer tm(TTRNN_K_TTLINEAR_BWD, st);
+                KernelTimer tm(TTRNN_K_TTLINEAR_BWD, st, e->R, (int)g, rows);
                 rc = e->launch(&sa, (int)g, st);
             }
+            tts_count_launch(e);
             ++g_launches;
             if (rc) return fail("static kernel %s launch failed: %s", e->name, cudaGetErrorString((cudaError_t)rc));
             if (slots_used && (int)g > *slots_used) *slots_used = (int)g;
@@ -1348,6 +1367,11 @@ int ttrnn_static_kernel_table(char *buf, int32_t cap) {
     return tts_dump_entries(buf, cap);
 }
 
+int ttrnn_static_kernel_keys(char *buf, int32_t cap) {
+    if (!buf || cap < 1) return -1;
+    return tts_dump_keys(buf, cap);
+}
+
 int ttrnn_rnn_ih_route(const ttrnn_rnn_desc *desc, int32_t layer, int64_t *chain_macs_per_row, int64_t *dense_macs_per_row) {
     t_opt = snapshot_options();
     RnnPlan rp;
@@ -1382,6 +1406,14 @@ int64_t ttrnn_tc_launch_count(int32_t reset) {
     long long v = g_tc_launches.load();
     if (reset) g_tc_launches.store(0);
     return v;
+}
+
+int ttrnn_static_kernel_launches(int64_t *counts, int32_t cap, int32_t reset) {
+    std::vector<long long> v(cap > 0 ? cap : 0);
+    const int n = tts_entry_launches(counts && cap > 0 ? v.data() : nullptr, cap, reset);
+    if (counts)
+        for (int i = 0; i < n && i < cap; ++i) counts[i] = v[i];
+    return n;
 }
 
 int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf, int32_t cap) {
@@ -1454,6 +1486,14 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
                     put(" bwd_kernel2=%s bwd_rows2=%d bwd_phase_rows2=%lld", tok(br.e[1]->name).c_str(), br.e[1]->R, br.rows[1]);
                 put(" hh_dw=%s hh_dw_tc=%d", br.split ? (br.dense_hh ? "dense" : "tt_chain") : "fused",
                     (int)(br.dense_hh && t_opt.tc_gemm && ttc::tc_red_ok(B * (long long)lo.Tc, d->hidden_size, GH)));
+            }
+            // a rank-one layer 0 whose input gradient is requested runs the projected-input route (bwd_modes)
+            int modes[2];
+            if (bwd_modes(d, l, modes) == 2) {
+                BwdRoute bx;
+                if (bwd_route(d, rp, l, modes[1], B, dv.sms, lo.kept[l], lo.Tc, &bx)) return -1;
+                if (!bx.nph) put(" bwd_kernel_dx=runtime bwd_rows_dx=0");
+                else put(" bwd_kernel_dx=%s bwd_rows_dx=%d", tok(bx.e[0]->name).c_str(), bx.e[0]->R);
             }
         }
         put("\n");
@@ -1674,6 +1714,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                     KernelTimer tm(TTRNN_K_RNN_FWD, st, se->R, (int)g, B, tc);
                     rc = se->launch(&sa, (int)g, st);
                 }
+                tts_count_launch(se);
                 ++g_launches;
                 if (rc) return fail("static kernel %s launch failed: %s", se->name, cudaGetErrorString((cudaError_t)rc));
             }
@@ -1981,6 +2022,7 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
                         KernelTimer tm(TTRNN_K_RNN_BWD, st, br.e[q]->R, ph_grid[q], br.rows[q], a2.steps);
                         e = br.e[q]->launch(&a2, ph_grid[q], st);
                     }
+                    tts_count_launch(br.e[q]);
                     ++g_launches;
                     if (e) return fail("static kernel %s launch failed: %s", br.e[q]->name, cudaGetErrorString((cudaError_t)e));
                 }
@@ -2007,6 +2049,12 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
             DenseIh DH;
             int hh_dense_calls = 0;
             if (dense_hh) {
+                // the dense buffers end inside this layer's scratch set (build_layout sizes them for every route of bwd_modes)
+                const long long set_end = lo.overlap ? lo.b_xg + lo.set_stride : lo.b_total;
+                if (lo.b_dense_hh + dense_bwd_floats(lp.hh) > set_end)
+                    return fail("internal: layer %d: the dense hh-gradient buffers of %s (%lld floats from %lld) overrun the "
+                                "backward scratch set (%lld floats)", l, br.e[0]->name, dense_bwd_floats(lp.hh),
+                                lo.b_dense_hh, set_end);
                 dense_carve(ss + lo.b_dense_hh, lp.hh, true, &DH);
                 ttg::k_eye<<<1024, 256, 0, st>>>(DH.eye, H);
                 ++g_launches;
