@@ -41,7 +41,9 @@ extern "C" {
                                  ttrnn_rnn_backward_dropout, ttrnn_dropout_apply).  Still 4 with projected LSTM stacks:
                                  one more flag value (TTRNN_WS_PROJ), one struct and four new symbols
                                  (ttrnn_rnn_param_count_proj, ttrnn_rnn_workspace_bytes_proj, ttrnn_rnn_forward_proj,
-                                 ttrnn_rnn_backward_proj) */
+                                 ttrnn_rnn_backward_proj).  Still 4 with projected dense LSTM stacks: four new symbols
+                                 (ttrnn_dense_rnn_param_count_proj, ttrnn_dense_rnn_workspace_bytes_proj,
+                                 ttrnn_dense_rnn_forward_proj, ttrnn_dense_rnn_backward_proj); nothing existing changes */
 #define TTRNN_MAX_CORES   6
 #define TTRNN_MAX_LAYERS  8
 
@@ -323,6 +325,30 @@ int ttrnn_dense_rnn_backward_ex(const ttrnn_dense_desc *desc, const float *x, co
                                 const float *d_out, const float *d_hT, const float *d_cT,
                                 float *d_params, float *d_x, float *d_h0, float *d_c0,
                                 void *scratch, void *stream, int32_t flags);
+/* Projected dense LSTM stacks (LSTMP), the `proj_size` of torch.nn.LSTM: each layer computes m_t = o_t * tanh(c_t) (H wide)
+ * and outputs h_t = W_hr m_t (P < H wide, no bias), which is also the next step's hh input.  Each call takes the arguments
+ * of its counterpart above (the _ex form for forward / backward) plus proj_size = P.
+ *   - desc->cell must be TTRNN_CELL_LSTM; 1 <= P < hidden_size and P % 128 == 0 (P is N of the per-step projection GEMM
+ *     and of the dh carry GEMM).  proj_size = 0 is refused: that is the unprojected stack of the calls above.
+ *   - Parameter blob, per layer: [W_ih (4H x in)] [W_hh (4H x P)] [b_hh (4H) with bias] [W_hr (P x H)], the state_dict
+ *     order; `in` is P for layers >= 1 (torch.nn.LSTM: weight_ih_l{l}, weight_hh_l{l}, bias_hh_l{l}, weight_hr_l{l}, with
+ *     bias_ih_l{l} = 0).
+ *   - Every h-state buffer is P wide: out (B, T, P), h0, hT, d_hT, d_h0 (B, P).  The c-state buffers c0, cT, d_cT, d_c0
+ *     stay (B, H).  Under TTRNN_WS_LAYER_STATES the layer stride is B * P for the h states and B * H for the c states.
+ *   - Per step, the forward runs the hh GEMM (K = P), the gate kernel (writes c_t and m_t) and h_t = m_t W_hr^T; the
+ *     backward forms dh_t, runs dm_t = dh_t W_hr, the gate backward and the carry du_t W_hh.  dW_hr = sum_t dh_t^T m_t
+ *     is one GEMM over all B * T rows after the loop. */
+int64_t ttrnn_dense_rnn_param_count_proj(const ttrnn_dense_desc *desc, int32_t proj_size);
+int ttrnn_dense_rnn_workspace_bytes_proj(const ttrnn_dense_desc *desc, int64_t *saved_bytes, int64_t *scratch_bytes,
+                                         int32_t proj_size);
+int ttrnn_dense_rnn_forward_proj(const ttrnn_dense_desc *desc, const float *x, const float *h0, const float *c0,
+                                 const float *params, float *out, float *hT, float *cT,
+                                 void *saved, void *scratch, void *stream, int32_t flags, int32_t proj_size);
+int ttrnn_dense_rnn_backward_proj(const ttrnn_dense_desc *desc, const float *x, const float *h0, const float *c0,
+                                  const float *params, const float *out, void *saved,
+                                  const float *d_out, const float *d_hT, const float *d_cT,
+                                  float *d_params, float *d_x, float *d_h0, float *d_c0,
+                                  void *scratch, void *stream, int32_t flags, int32_t proj_size);
 
 /* GE2E head on the device (SURVEY.md 8f-4): the part of the speaker-encoder training step the reference runs on the CPU
  * after every RNN pass (experiments/speaker_verification/encoder/main.py:279-280 moves the embeddings to `loss_device`).

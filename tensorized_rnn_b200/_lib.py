@@ -97,6 +97,11 @@ SYMBOLS = {
     "ttrnn_dense_rnn_backward": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 15),
     "ttrnn_dense_rnn_forward_ex": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 10 + [C.c_int32]),
     "ttrnn_dense_rnn_backward_ex": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 15 + [C.c_int32]),
+    "ttrnn_dense_rnn_param_count_proj": (C.c_int64, [C.POINTER(DenseDesc), C.c_int32]),
+    "ttrnn_dense_rnn_workspace_bytes_proj": (C.c_int, [C.POINTER(DenseDesc), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
+                                                       C.c_int32]),
+    "ttrnn_dense_rnn_forward_proj": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 10 + [C.c_int32, C.c_int32]),
+    "ttrnn_dense_rnn_backward_proj": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 15 + [C.c_int32, C.c_int32]),
     "ttrnn_embed_forward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 4),
     "ttrnn_embed_backward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 6),
     "ttrnn_ge2e_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),

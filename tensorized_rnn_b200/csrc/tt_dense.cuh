@@ -173,6 +173,17 @@ __global__ void __launch_bounds__(128) k_smallk_dw_part(const float *__restrict_
     part[((long long)s * N + n) * K + k] = a0 + a1;
 }
 
+// Projected LSTM backward, step t: dh_t = dOut[:, t, :] + carry (du_{t+1} W_hh, or the upstream d_hT at t = T-1), P wide,
+// written into the (B, T, P) buffer that the dm_t GEMM reads now and the dW_hr GEMM reads after the loop.  dout and
+// carry may be null (zero); carry is (B, P) contiguous.  One CTA per batch row (grid-stride over rows), threads over j.
+__global__ void __launch_bounds__(128) k_dense_proj_dh(const float *__restrict__ dout, long long lddo,
+                                                       const float *__restrict__ carry, float *__restrict__ dh, long long lddh,
+                                                       long long B, int P) {
+    for (long long b = blockIdx.x; b < B; b += gridDim.x)
+        for (int j = threadIdx.x; j < P; j += blockDim.x)
+            dh[b * lddh + j] = (dout ? dout[b * lddo + j] : 0.f) + (carry ? carry[b * P + j] : 0.f);
+}
+
 // out[e] = a[e] + (b ? b[e] : 0)
 __global__ void __launch_bounds__(256) k_add2(const float *__restrict__ a, const float *__restrict__ b, float *__restrict__ out,
                                               long long n) {

@@ -2790,58 +2790,77 @@ int ttrnn_cell_backward(int32_t cell, int64_t B, int32_t H, const float *a, cons
 
 // ---- dense LSTM / GRU baselines (SURVEY.md 8f-3) -----------------------------------------------------------------
 namespace {
-struct DenseLayerOff { long long w_ih, b_ih, w_hh, b_hh; int nin; bool has_bih, has_bhh; };
+struct DenseLayerOff { long long w_ih, b_ih, w_hh, b_hh, w_hr; int nin; bool has_bih, has_bhh; };
 struct DensePlan {
     int G = 0;
+    int P = 0;          // projected LSTM (the _proj entry points): proj_size, else 0
+    int W = 0;          // width of h_t and of every layer's output: P when projected, else hidden_size
     long long param_floats = 0;
     DenseLayerOff layer[TTRNN_MAX_LAYERS];
 };
 // parameter blob, per layer: [W_ih (G*H x I)] [b_ih (G*H): GRU with bias only] [W_hh (G*H x H)] [b_hh (G*H) with bias]
-// (LSTMCell: input_weights has no bias, lstm.py:17-21; GRUCell: both carry `bias`, gru.py:19-23)
-int build_dense_plan(const ttrnn_dense_desc *d, DensePlan *dp) {
+// (LSTMCell: input_weights has no bias, lstm.py:17-21; GRUCell: both carry `bias`, gru.py:19-23).
+// proj_size P > 0 (LSTM): W_hh is 4H x P, W_ih of layers >= 1 is 4H x P, and [W_hr (P x H)] follows b_hh.
+int build_dense_plan(const ttrnn_dense_desc *d, int P, DensePlan *dp) {
     if (!d) return fail("null descriptor");
     if (d->cell != TTRNN_CELL_LSTM && d->cell != TTRNN_CELL_GRU) return fail("unknown cell kind %d", d->cell);
     if (d->num_layers < 1 || d->num_layers > TTRNN_MAX_LAYERS) return fail("num_layers %d out of range", d->num_layers);
     if (d->input_size < 1 || d->hidden_size < 1 || d->batch < 1 || d->seq_len < 1) return fail("sizes must be positive");
     if (d->hidden_size % 128 != 0)
         return fail("dense cells: hidden_size must be a multiple of 128 (the GEMM tiles are 128 columns wide), got %d", d->hidden_size);
+    if (P) {
+        if (d->cell != TTRNN_CELL_LSTM) return fail("dense cells: proj_size needs an LSTM descriptor (torch.nn.GRU has no projection)");
+        if (P < 1 || P >= d->hidden_size)
+            return fail("dense cells: proj_size must be in [1, hidden_size), got %d with hidden_size %d", P, d->hidden_size);
+        // P is N of the per-step projection GEMM and of the dh carry GEMM
+        if (P % 128 != 0)
+            return fail("dense cells: proj_size must be a multiple of 128 (the GEMM tiles are 128 columns wide), got %d", P);
+    }
     dp->G = gates_of(d->cell);
+    dp->P = P;
+    dp->W = P ? P : d->hidden_size;
     const long long GH = (long long)dp->G * d->hidden_size;
     long long off = 0;
     for (int l = 0; l < d->num_layers; ++l) {
         DenseLayerOff &o = dp->layer[l];
-        o.nin = l == 0 ? d->input_size : d->hidden_size;
+        o.nin = l == 0 ? d->input_size : dp->W;
         o.has_bih = d->has_bias && d->cell == TTRNN_CELL_GRU;
         o.has_bhh = d->has_bias != 0;
         o.w_ih = off; off += GH * o.nin;
         o.b_ih = off; if (o.has_bih) off += GH;
-        o.w_hh = off; off += GH * d->hidden_size;
+        o.w_hh = off; off += GH * dp->W;
         o.b_hh = off; if (o.has_bhh) off += GH;
+        o.w_hr = off; off += (long long)P * d->hidden_size;
     }
     dp->param_floats = off;
     return 0;
 }
 struct DenseLayout {
-    long long BTH, BTG, BH;
-    long long sv_hs, sv_cs, sv_a, sv_u, sv_total;      // saved: inner-layer outputs, c states, a = W_ih x, u = W_hh h (per layer)
-    long long s_w, s_dh, s_part, s_total;              // scratch: weight splits / transposes, dh carries, reduction partials
+    long long BTH, BTW, BTG, BH;
+    long long sv_hs, sv_cs, sv_a, sv_u, sv_ms, sv_total;  // saved: inner-layer outputs, c states, a = W_ih x, u = W_hh h,
+                                                          // projected: m_t = o_t * tanh(c_t) (per layer)
+    long long s_w, s_dh, s_part, s_hr, s_dhs, s_total;    // scratch: weight splits / transposes, dh carries, reduction
+                                                          // partials; projected: W_hr forms, dh_t of every step
     long long wmax;
 };
 void build_dense_layout(const ttrnn_dense_desc *d, const DensePlan &dp, DenseLayout *lo) {
     const long long B = d->batch, T = d->seq_len, H = d->hidden_size, L = d->num_layers, GH = (long long)dp.G * H;
     const long long Imax = d->input_size > H ? d->input_size : H;
-    lo->BTH = B * T * H; lo->BTG = B * T * GH; lo->BH = B * H;
+    lo->BTH = B * T * H; lo->BTW = B * T * dp.W; lo->BTG = B * T * GH; lo->BH = B * H;
     long long o = 0;
-    lo->sv_hs = o; o += r4((L - 1) * lo->BTH);
+    lo->sv_hs = o; o += r4((L - 1) * lo->BTW);
     lo->sv_cs = o; o += (d->cell == TTRNN_CELL_LSTM) ? r4(L * lo->BTH) : 0;
     lo->sv_a = o; o += r4(L * lo->BTG);
     lo->sv_u = o; o += r4(L * lo->BTG);
+    lo->sv_ms = o; o += dp.P ? r4(L * lo->BTH) : 0;
     lo->sv_total = o;
     lo->wmax = r4(GH * Imax);
     o = 0;
     lo->s_w = o; o += 8 * lo->wmax;                    // W_ih hi/lo, W_hh hi/lo, W^T + hi/lo (one side at a time), dW^T
     lo->s_dh = o; o += 6 * r4(lo->BH);                 // dh_gemm, dh_direct x 2 (ping-pong), dc, h zero pad, spare
     lo->s_part = o; o += kDenseMaxSplit * (lo->wmax + r4(GH)) + 2 * r4(GH);
+    lo->s_hr = o; o += dp.P ? 3 * r4((long long)dp.P * H) : 0;   // W_hr or W_hr^T as the GEMM operand: plain, hi, lo
+    lo->s_dhs = o; o += dp.P ? r4(lo->BTW) : 0;
     lo->s_total = o;
 }
 // y = x W^T (+ bias): rows GEMM on the tensor cores when it fits, else FFMA (needs W^T as K x N)
@@ -2875,13 +2894,13 @@ int transpose_to(const float *src, float *dst, int rows, int cols, cudaStream_t 
 
 int64_t ttrnn_dense_rnn_param_count(const ttrnn_dense_desc *desc) {
     DensePlan dp;
-    if (build_dense_plan(desc, &dp)) return -1;
+    if (build_dense_plan(desc, 0, &dp)) return -1;
     return dp.param_floats;
 }
 
-int ttrnn_dense_rnn_workspace_bytes(const ttrnn_dense_desc *desc, int64_t *saved_bytes, int64_t *scratch_bytes) {
+static int dense_workspace_bytes(const ttrnn_dense_desc *desc, int P, int64_t *saved_bytes, int64_t *scratch_bytes) {
     DensePlan dp;
-    if (build_dense_plan(desc, &dp)) return 1;
+    if (build_dense_plan(desc, P, &dp)) return 1;
     if (!saved_bytes || !scratch_bytes) return fail("null output pointer");
     DenseLayout lo;
     build_dense_layout(desc, dp, &lo);
@@ -2889,12 +2908,17 @@ int ttrnn_dense_rnn_workspace_bytes(const ttrnn_dense_desc *desc, int64_t *saved
     *scratch_bytes = lo.s_total * 4;
     return 0;
 }
+int ttrnn_dense_rnn_workspace_bytes(const ttrnn_dense_desc *desc, int64_t *saved_bytes, int64_t *scratch_bytes) {
+    return dense_workspace_bytes(desc, 0, saved_bytes, scratch_bytes);
+}
 
-static int dense_forward(const ttrnn_dense_desc *d, const StateMap &sm, const float *x, const float *h0, const float *c0,
+// Projected LSTM (P > 0), step t: u_t = h_{t-1} W_hh^T + b_hh (K = P), the gate kernel writes c_t and m_t, then
+// h_t = m_t W_hr^T (N = P) into the layer output: three launches per step where the unprojected stack has two.
+static int dense_forward(const ttrnn_dense_desc *d, int P, const StateMap &sm, const float *x, const float *h0, const float *c0,
                          const float *params, float *out, float *hT, float *cT, void *saved, void *scratch, void *stream) {
     t_opt = snapshot_options();
     DensePlan dp;
-    if (build_dense_plan(d, &dp)) return 1;
+    if (build_dense_plan(d, P, &dp)) return 1;
     if (!x || !params || !out || !saved || !scratch) return fail("x, params, out, saved and scratch must be non-null");
     DevInfo dv;
     if (get_dev(&dv)) return 1;
@@ -2902,24 +2926,28 @@ static int dense_forward(const ttrnn_dense_desc *d, const StateMap &sm, const fl
     build_dense_layout(d, dp, &lo);
     cudaStream_t st = (cudaStream_t)stream;
     const long long B = d->batch;
-    const int T = d->seq_len, H = d->hidden_size, L = d->num_layers, G = dp.G, GH = G * H;
+    const int T = d->seq_len, H = d->hidden_size, L = d->num_layers, G = dp.G, GH = G * H, W = dp.W;
     const bool lstm = d->cell == TTRNN_CELL_LSTM;
     float *sv = (float *)saved, *sc = (float *)scratch;
     float *w_ih_hi = sc + lo.s_w, *w_ih_lo = w_ih_hi + lo.wmax, *w_hh_hi = w_ih_lo + lo.wmax, *w_hh_lo = w_hh_hi + lo.wmax;
     float *wt_ih = w_hh_lo + lo.wmax, *wt_hh = wt_ih + lo.wmax;
+    const long long nhr = r4((long long)P * H);
+    float *wt_hr = sc + lo.s_hr, *w_hr_hi = wt_hr + nhr, *w_hr_lo = w_hr_hi + nhr;
     long long blocks = (B * (long long)H + 255) / 256;
     if (blocks > (long long)dv.sms * 8) blocks = (long long)dv.sms * 8;
     for (int l = 0; l < L; ++l) {
         const DenseLayerOff &o = dp.layer[l];
-        const float *lin = l == 0 ? x : sv + lo.sv_hs + (long long)(l - 1) * lo.BTH;
-        float *lout = l == L - 1 ? out : sv + lo.sv_hs + (long long)l * lo.BTH;
+        const float *lin = l == 0 ? x : sv + lo.sv_hs + (long long)(l - 1) * lo.BTW;
+        float *lout = l == L - 1 ? out : sv + lo.sv_hs + (long long)l * lo.BTW;
         float *cs = lstm ? sv + lo.sv_cs + (long long)l * lo.BTH : nullptr;
+        float *ms = P ? sv + lo.sv_ms + (long long)l * lo.BTH : nullptr;
         float *ab = sv + lo.sv_a + (long long)l * lo.BTG, *ub = sv + lo.sv_u + (long long)l * lo.BTG;
-        const float *W_ih = params + o.w_ih, *W_hh = params + o.w_hh;
-        const long long nih = (long long)GH * o.nin, nhh = (long long)GH * H;
+        const float *W_ih = params + o.w_ih, *W_hh = params + o.w_hh, *W_hr = params + o.w_hr;
+        const long long nih = (long long)GH * o.nin, nhh = (long long)GH * W;
         // both operand forms: TF32 hi / lo split of W (tensor cores) and W^T as K x N (FFMA fallback)
         if (o.nin % 4 == 0 && (split_tf32(W_ih, w_ih_hi, w_ih_lo, r4(nih), st) || transpose_to(W_ih, wt_ih, GH, o.nin, st))) return 1;
-        if (split_tf32(W_hh, w_hh_hi, w_hh_lo, r4(nhh), st) || transpose_to(W_hh, wt_hh, GH, H, st)) return 1;
+        if (split_tf32(W_hh, w_hh_hi, w_hh_lo, r4(nhh), st) || transpose_to(W_hh, wt_hh, GH, W, st)) return 1;
+        if (P && (split_tf32(W_hr, w_hr_hi, w_hr_lo, nhr, st) || transpose_to(W_hr, wt_hr, P, H, st))) return 1;
         // a = X W_ih^T (+ b_ih) for every timestep at once
         if (o.nin % 4 != 0) {
             long long gb = (B * (long long)T * GH + 255) / 256;
@@ -2929,13 +2957,13 @@ static int dense_forward(const ttrnn_dense_desc *d, const StateMap &sm, const fl
         } else if (dense_linear(dv, B * (long long)T, T, lin, (long long)T * o.nin, o.nin, w_ih_hi, w_ih_lo, wt_ih, GH,
                          o.has_bih ? params + o.b_ih : nullptr, ab, (long long)T * GH, false, st))
             return 1;
-        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l, true);
         for (int t = 0; t < T; ++t) {
-            const float *hp = t == 0 ? h0l : lout + (long long)(t - 1) * H;
-            const long long ldhp = t == 0 ? H : (long long)T * H;
+            const float *hp = t == 0 ? h0l : lout + (long long)(t - 1) * W;
+            const long long ldhp = t == 0 ? W : (long long)T * W;
             // u_t = h_{t-1} W_hh^T + b_hh  (h_{-1} = 0: u_0 = b_hh)
             if (hp) {
-                if (dense_linear(dv, B, 1, hp, ldhp, H, w_hh_hi, w_hh_lo, wt_hh, GH,
+                if (dense_linear(dv, B, 1, hp, ldhp, W, w_hh_hi, w_hh_lo, wt_hh, GH,
                                  o.has_bhh ? params + o.b_hh : nullptr, ub + (long long)t * GH, (long long)T * GH, false, st))
                     return 1;
             } else {
@@ -2950,7 +2978,7 @@ static int dense_forward(const ttrnn_dense_desc *d, const StateMap &sm, const fl
             a.u = ub + (long long)t * GH; a.ldu = (long long)T * GH;
             a.h_prev = hp; a.ldhp = ldhp;
             a.c_prev = t == 0 ? c0l : cs + (long long)(t - 1) * H; a.ldcp = t == 0 ? H : (long long)T * H;
-            a.h = lout + (long long)t * H; a.ldh = (long long)T * H;
+            a.h = (P ? ms : lout) + (long long)t * H; a.ldh = (long long)T * H;      // projected: m_t
             a.c = lstm ? cs + (long long)t * H : nullptr; a.ldc = (long long)T * H;
             {
                 KernelTimer tm(TTRNN_K_RNN_FWD, st);
@@ -2958,10 +2986,14 @@ static int dense_forward(const ttrnn_dense_desc *d, const StateMap &sm, const fl
                 else ttd::k_dense_cell_fwd<false><<<(unsigned)blocks, 256, 0, st>>>(a);
             }
             ++g_launches;
+            // projected: h_t = m_t W_hr^T
+            if (P && dense_linear(dv, B, 1, ms + (long long)t * H, (long long)T * H, H, w_hr_hi, w_hr_lo, wt_hr, P, nullptr,
+                                  lout + (long long)t * P, (long long)T * P, false, st))
+                return 1;
         }
         CU_CHECK(cudaGetLastError());
-        float *hTl = sm.fin(hT, l, L), *cTl = sm.fin(cT, l, L);
-        if (hTl) CU_CHECK(cudaMemcpy2DAsync(hTl, (size_t)H * 4, lout + (long long)(T - 1) * H, (size_t)T * H * 4, (size_t)H * 4, B,
+        float *hTl = sm.fin(hT, l, L), *cTl = sm.fin(cT, l, L, true);
+        if (hTl) CU_CHECK(cudaMemcpy2DAsync(hTl, (size_t)W * 4, lout + (long long)(T - 1) * W, (size_t)T * W * 4, (size_t)W * 4, B,
                                             cudaMemcpyDeviceToDevice, st));
         if (lstm && cTl) CU_CHECK(cudaMemcpy2DAsync(cTl, (size_t)H * 4, cs + (long long)(T - 1) * H, (size_t)T * H * 4, (size_t)H * 4,
                                                     B, cudaMemcpyDeviceToDevice, st));
@@ -2969,12 +3001,15 @@ static int dense_forward(const ttrnn_dense_desc *d, const StateMap &sm, const fl
     return 0;
 }
 
-static int dense_backward(const ttrnn_dense_desc *d, const StateMap &sm, const float *x, const float *h0, const float *c0,
+// Projected LSTM (P > 0), step t in reverse: dh_t = d_out_t + the carry (k_dense_proj_dh, kept in a (B, T, P) buffer),
+// dm_t = dh_t W_hr (N = H), the gate backward with dm_t as its dh, then the carry du_t W_hh (N = P): four launches per
+// step where the unprojected stack has two.  dW_hr = sum_t dh_t^T m_t after the loop, batched over B*T.
+static int dense_backward(const ttrnn_dense_desc *d, int P, const StateMap &sm, const float *x, const float *h0, const float *c0,
                           const float *params, const float *out, void *saved, const float *d_out, const float *d_hT,
                           const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream) {
     t_opt = snapshot_options();
     DensePlan dp;
-    if (build_dense_plan(d, &dp)) return 1;
+    if (build_dense_plan(d, P, &dp)) return 1;
     if (!x || !params || !out || !saved || !scratch || !d_params) return fail("x, params, out, saved, scratch, d_params must be non-null");
     DevInfo dv;
     if (get_dev(&dv)) return 1;
@@ -2982,47 +3017,64 @@ static int dense_backward(const ttrnn_dense_desc *d, const StateMap &sm, const f
     build_dense_layout(d, dp, &lo);
     cudaStream_t st = (cudaStream_t)stream;
     const long long B = d->batch;
-    const int T = d->seq_len, H = d->hidden_size, L = d->num_layers, G = dp.G, GH = G * H;
+    const int T = d->seq_len, H = d->hidden_size, L = d->num_layers, G = dp.G, GH = G * H, W = dp.W;
     const bool lstm = d->cell == TTRNN_CELL_LSTM;
     float *sv = (float *)saved, *sc = (float *)scratch;
     float *wT_hi = sc + lo.s_w, *wT_lo = wT_hi + lo.wmax, *wT = wT_lo + lo.wmax, *wplain_t = wT + lo.wmax, *dwt = wplain_t + lo.wmax;
     float *dh_gemm = sc + lo.s_dh, *dhd[2] = {dh_gemm + r4(lo.BH), dh_gemm + 2 * r4(lo.BH)}, *dcc = dh_gemm + 3 * r4(lo.BH);
     float *part = sc + lo.s_part, *pbias = part + kDenseMaxSplit * lo.wmax, *dbias = pbias + kDenseMaxSplit * r4(GH);
+    // projected: W_hr^T (H x P) and its hi / lo split (the dm_t GEMM's Bt), dh_t of every step; dm_t (B, H) takes the
+    // first direct-term buffer, which the LSTM does not use
+    const long long nhr = r4((long long)P * H);
+    float *wt_hr = sc + lo.s_hr, *wt_hr_hi = wt_hr + nhr, *wt_hr_lo = wt_hr_hi + nhr, *dhsb = sc + lo.s_dhs, *dm = dhd[0];
     long long blocks = (B * (long long)H + 255) / 256;
     if (blocks > (long long)dv.sms * 8) blocks = (long long)dv.sms * 8;
+    const unsigned prow_blocks = (unsigned)(B < (long long)dv.sms * 8 ? B : (long long)dv.sms * 8);
     // dW^T (K x GH) = sum over rows of A^T Bm, then transposed into the parameter layout (GH x K); db = column sums of Bm
     DenseIh D;
     memset(&D, 0, sizeof D);
     D.part = part; D.pbias = pbias; D.dwt = dwt; D.dbias = dbias;
     for (int l = L - 1; l >= 0; --l) {
         const DenseLayerOff &o = dp.layer[l];
-        const float *lin = l == 0 ? x : sv + lo.sv_hs + (long long)(l - 1) * lo.BTH;
-        const float *lout = l == L - 1 ? out : sv + lo.sv_hs + (long long)l * lo.BTH;
+        const float *lin = l == 0 ? x : sv + lo.sv_hs + (long long)(l - 1) * lo.BTW;
+        const float *lout = l == L - 1 ? out : sv + lo.sv_hs + (long long)l * lo.BTW;
         const float *cs = lstm ? sv + lo.sv_cs + (long long)l * lo.BTH : nullptr;
+        const float *ms = P ? sv + lo.sv_ms + (long long)l * lo.BTH : nullptr;
         float *ab = sv + lo.sv_a + (long long)l * lo.BTG, *ub = sv + lo.sv_u + (long long)l * lo.BTG;
         // gradient wrt this layer's outputs: the caller's d_out for the last layer; for an inner layer the dX of the layer
-        // above, which that layer wrote over its own (by then dead) `u` buffer, packed (B, T, H) at the front
+        // above, which that layer wrote over its own (by then dead) `u` buffer, packed (B, T, W) at the front
         const float *dhs = l == L - 1 ? d_out : sv + lo.sv_u + (long long)(l + 1) * lo.BTG;
-        const float *W_ih = params + o.w_ih, *W_hh = params + o.w_hh;
-        const long long nhh = (long long)GH * H;
-        // dh_{t-1} += du_t W_hh : rows GEMM with Bt = W_hh^T (H x GH)
-        if (transpose_to(W_hh, wT, GH, H, st)) return 1;                         // wT = W_hh^T (H x GH)
+        const float *W_ih = params + o.w_ih, *W_hh = params + o.w_hh, *W_hr = params + o.w_hr;
+        const long long nhh = (long long)GH * W;
+        // dh_{t-1} += du_t W_hh : rows GEMM with Bt = W_hh^T (W x GH)
+        if (transpose_to(W_hh, wT, GH, W, st)) return 1;                         // wT = W_hh^T (W x GH)
         if (split_tf32(wT, wT_hi, wT_lo, r4(nhh), st)) return 1;
-        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l);
-        const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L);
+        if (P && (transpose_to(W_hr, wt_hr, P, H, st) || split_tf32(wt_hr, wt_hr_hi, wt_hr_lo, nhr, st))) return 1;
+        const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l, true);
+        const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L, true);
         for (int t = T - 1; t >= 0; --t) {
             ttd::DenseStepArgs a;
             memset(&a, 0, sizeof a);
             a.B = B; a.H = H;
             a.a = ab + (long long)t * GH; a.lda = (long long)T * GH;
             a.u = ub + (long long)t * GH; a.ldu = (long long)T * GH;
-            a.h_prev = t == 0 ? h0l : lout + (long long)(t - 1) * H; a.ldhp = t == 0 ? H : (long long)T * H;
+            a.h_prev = t == 0 ? h0l : lout + (long long)(t - 1) * W; a.ldhp = t == 0 ? W : (long long)T * W;
             a.c_prev = t == 0 ? c0l : (lstm ? cs + (long long)(t - 1) * H : nullptr); a.ldcp = t == 0 ? H : (long long)T * H;
-            a.dout = dhs ? dhs + (long long)t * H : nullptr; a.lddo = (long long)T * H;
             a.first = t == T - 1;
-            a.dh_gemm = a.first ? nullptr : dh_gemm;
+            if (P) {
+                // dh_t, then dm_t = dh_t W_hr: the gate backward's only dh term
+                float *dht = dhsb + (long long)t * P;
+                ttd::k_dense_proj_dh<<<prow_blocks, 128, 0, st>>>(dhs ? dhs + (long long)t * P : nullptr, (long long)T * P,
+                                                                  a.first ? dhTl : dh_gemm, dht, (long long)T * P, B, P);
+                ++g_launches;
+                if (dense_linear(dv, B, 1, dht, (long long)T * P, P, wt_hr_hi, wt_hr_lo, W_hr, H, nullptr, dm, H, true, st)) return 1;
+                a.dout = dm; a.lddo = H;
+            } else {
+                a.dout = dhs ? dhs + (long long)t * H : nullptr; a.lddo = (long long)T * H;
+                a.dh_gemm = a.first ? nullptr : dh_gemm;
+                a.dh_T = a.first ? dhTl : nullptr;
+            }
             a.dh_direct = (a.first || lstm) ? nullptr : dhd[(t + 1) & 1];
-            a.dh_T = a.first ? dhTl : nullptr;
             a.dc_T = a.first ? dcTl : nullptr;
             a.da = ab + (long long)t * GH; a.ldda = (long long)T * GH;
             a.du = ub + (long long)t * GH; a.lddu = (long long)T * GH;
@@ -3036,37 +3088,44 @@ static int dense_backward(const ttrnn_dense_desc *d, const StateMap &sm, const f
             ++g_launches;
             if (t > 0 || (d_h0 && h0l)) {
                 // dh_gemm = du_t W_hh
-                if (dense_linear(dv, B, 1, ub + (long long)t * GH, (long long)T * GH, GH, wT_hi, wT_lo, W_hh, H, nullptr,
-                                 dh_gemm, H, true, st))
+                if (dense_linear(dv, B, 1, ub + (long long)t * GH, (long long)T * GH, GH, wT_hi, wT_lo, W_hh, W, nullptr,
+                                 dh_gemm, W, true, st))
                     return 1;
             }
         }
         CU_CHECK(cudaGetLastError());
         // gradient wrt the initial state: this layer's own block, or the sum over layers when the state is shared
+        const long long BW = B * (long long)W;
         if (d_h0 && h0l) {
-            ttd::k_add2<<<(unsigned)blocks, 256, 0, st>>>(dh_gemm, lstm ? nullptr : dhd[0], sc + lo.s_dh + 4 * r4(lo.BH), lo.BH);
+            ttd::k_add2<<<(unsigned)blocks, 256, 0, st>>>(dh_gemm, lstm ? nullptr : dhd[0], sc + lo.s_dh + 4 * r4(lo.BH), BW);
             ++g_launches;
-            if (axpy1(sc + lo.s_dh + 4 * r4(lo.BH), sm.init(d_h0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
+            if (axpy1(sc + lo.s_dh + 4 * r4(lo.BH), sm.init(d_h0, l), BW, !sm.stride && l != L - 1, st)) return 1;
         }
-        if (lstm && d_c0 && c0l && axpy1(dcc, sm.init(d_c0, l), lo.BH, !sm.stride && l != L - 1, st)) return 1;
-        // dW_hh^T (H x GH) = sum_t h_{t-1}^T du_t ; db_hh = column sums of du (all T steps)
+        if (lstm && d_c0 && c0l && axpy1(dcc, sm.init(d_c0, l, true), lo.BH, !sm.stride && l != L - 1, st)) return 1;
+        // dW_hh^T (W x GH) = sum_t h_{t-1}^T du_t ; db_hh = column sums of du (all T steps)
         {
             bool acc = false;
             if (T > 1) {
-                if (dense_dw(dv, B * (long long)(T - 1), T - 1, lout, (long long)T * H, H, ub + GH, (long long)T * GH, GH, D, false, false, st))
+                if (dense_dw(dv, B * (long long)(T - 1), T - 1, lout, (long long)T * W, W, ub + GH, (long long)T * GH, GH, D, false, false, st))
                     return 1;
                 acc = true;
             }
             if (h0l) {
-                if (dense_dw(dv, B, 1, h0l, H, H, ub, (long long)T * GH, GH, D, acc, false, st)) return 1;
+                if (dense_dw(dv, B, 1, h0l, W, W, ub, (long long)T * GH, GH, D, acc, false, st)) return 1;
                 acc = true;
             }
             if (acc) {
-                if (transpose_to(dwt, d_params + o.w_hh, H, GH, st)) return 1;
+                if (transpose_to(dwt, d_params + o.w_hh, W, GH, st)) return 1;
             } else {
                 CU_CHECK(cudaMemsetAsync(d_params + o.w_hh, 0, (size_t)nhh * 4, st));
             }
             if (o.has_bhh && dense_colsum(dv, ub, B * (long long)T, GH, part, d_params + o.b_hh, st)) return 1;
+        }
+        // projected: dW_hr (P x H) = sum_t dh_t^T m_t, which is already the parameter layout
+        if (P) {
+            DenseIh DR = D;
+            DR.dwt = d_params + o.w_hr;
+            if (dense_dw(dv, B * (long long)T, T, dhsb, (long long)T * P, P, ms, (long long)T * H, H, DR, false, false, st)) return 1;
         }
         // dW_ih^T (I x GH) = X^T da ; db_ih = column sums of da
         if (o.nin % 4 != 0) {
@@ -3087,7 +3146,7 @@ static int dense_backward(const ttrnn_dense_desc *d, const StateMap &sm, const f
         }
         if (o.has_bih && dense_colsum(dv, ab, B * (long long)T, GH, part, d_params + o.b_ih, st)) return 1;
         // dX = da W_ih (B, T, I): for l > 0 it is the upstream gradient of the layer below, written over this layer's dead
-        // `u` buffer (packed (B, T, H) at its front); for l == 0 into the caller's d_x (if requested)
+        // `u` buffer (packed (B, T, W) at its front); for l == 0 into the caller's d_x (if requested)
         float *dxl = l == 0 ? d_x : ub;
         if (dxl) {
             if (o.nin % 128 != 0)
@@ -3105,32 +3164,67 @@ static int dense_backward(const ttrnn_dense_desc *d, const StateMap &sm, const f
 // ---- GE2E head (SURVEY.md 8f-4) ------------------------------------------------------------------------------------
 int ttrnn_dense_rnn_forward(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
                             float *out, float *hT, float *cT, void *saved, void *scratch, void *stream) {
-    return dense_forward(d, StateMap(), x, h0, c0, params, out, hT, cT, saved, scratch, stream);
+    return dense_forward(d, 0, StateMap(), x, h0, c0, params, out, hT, cT, saved, scratch, stream);
 }
 int ttrnn_dense_rnn_backward(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
                              const float *out, void *saved, const float *d_out, const float *d_hT, const float *d_cT,
                              float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream) {
-    return dense_backward(d, StateMap(), x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
+    return dense_backward(d, 0, StateMap(), x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
                           stream);
 }
-static int dense_state_map(const ttrnn_dense_desc *d, int32_t flags, StateMap *sm) {
+// per-layer states: h blocks are B x (P or H), c blocks B x H
+static int dense_state_map(const ttrnn_dense_desc *d, int P, int32_t flags, StateMap *sm) {
     if (!d) return fail("null descriptor");
     if (flags & ~TTRNN_WS_LAYER_STATES) return fail("dense cells: unknown flags 0x%x (only TTRNN_WS_LAYER_STATES applies)", flags);
-    if (flags & TTRNN_WS_LAYER_STATES) sm->stride = d->batch * (long long)d->hidden_size;
+    if (flags & TTRNN_WS_LAYER_STATES) {
+        sm->stride = d->batch * (long long)(P ? P : d->hidden_size);
+        sm->cstride = d->batch * (long long)d->hidden_size;
+    }
     return 0;
 }
 int ttrnn_dense_rnn_forward_ex(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
                                float *out, float *hT, float *cT, void *saved, void *scratch, void *stream, int32_t flags) {
     StateMap sm;
-    if (dense_state_map(d, flags, &sm)) return 1;
-    return dense_forward(d, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream);
+    if (dense_state_map(d, 0, flags, &sm)) return 1;
+    return dense_forward(d, 0, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream);
 }
 int ttrnn_dense_rnn_backward_ex(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
                                 const float *out, void *saved, const float *d_out, const float *d_hT, const float *d_cT,
                                 float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream, int32_t flags) {
     StateMap sm;
-    if (dense_state_map(d, flags, &sm)) return 1;
-    return dense_backward(d, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch, stream);
+    if (dense_state_map(d, 0, flags, &sm)) return 1;
+    return dense_backward(d, 0, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch, stream);
+}
+
+// projected LSTM: proj_size 0 is the unprojected stack of the entry points above, which these calls do not run
+static int dense_proj_arg(int32_t proj_size) {
+    return proj_size < 1 ? fail("dense cells: the _proj calls need proj_size >= 1, got %d", proj_size) : 0;
+}
+int64_t ttrnn_dense_rnn_param_count_proj(const ttrnn_dense_desc *desc, int32_t proj_size) {
+    DensePlan dp;
+    if (dense_proj_arg(proj_size) || build_dense_plan(desc, proj_size, &dp)) return -1;
+    return dp.param_floats;
+}
+int ttrnn_dense_rnn_workspace_bytes_proj(const ttrnn_dense_desc *desc, int64_t *saved_bytes, int64_t *scratch_bytes,
+                                         int32_t proj_size) {
+    if (dense_proj_arg(proj_size)) return 1;
+    return dense_workspace_bytes(desc, proj_size, saved_bytes, scratch_bytes);
+}
+int ttrnn_dense_rnn_forward_proj(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
+                                 float *out, float *hT, float *cT, void *saved, void *scratch, void *stream, int32_t flags,
+                                 int32_t proj_size) {
+    StateMap sm;
+    if (dense_proj_arg(proj_size) || dense_state_map(d, proj_size, flags, &sm)) return 1;
+    return dense_forward(d, proj_size, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream);
+}
+int ttrnn_dense_rnn_backward_proj(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0, const float *params,
+                                  const float *out, void *saved, const float *d_out, const float *d_hT, const float *d_cT,
+                                  float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream, int32_t flags,
+                                  int32_t proj_size) {
+    StateMap sm;
+    if (dense_proj_arg(proj_size) || dense_state_map(d, proj_size, flags, &sm)) return 1;
+    return dense_backward(d, proj_size, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
+                          stream);
 }
 
 int ttrnn_embed_forward(int64_t rows, int32_t E, const float *x, float *y, float *inv_norm, void *stream) {

@@ -8,6 +8,9 @@ accepted and ignored (the reference moves the embeddings to the CPU for the loss
 in the CUDA library, ge2e.py); the EER, which the reference computes with scikit-learn on the CPU and does not backpropagate
 (speaker_encoder.py:158-169), is computed the same way from a host copy of the similarity matrix only when `compute_eer=True`;
 the evaluation form of `similarity_matrix` (`enrollment_embeds` given) is not provided by the CUDA head and raises.
+`proj_size=P` (appended to the reference signature; LSTM only, the GRU modules refuse it) builds the LSTM with a recurrent
+projection of the GE2E paper (LSTMP) on either side, `compression=None` (dense `LSTM`) or `'tt'` (`TTLSTM`); the embedding
+`linear` then reads the P-wide final state.
 """
 from __future__ import annotations
 
@@ -23,23 +26,25 @@ from .rnn import TTGRU, TTLSTM
 
 class SpeakerEncoder(nn.Module):
     def __init__(self, mel_n_channels, model_hidden_size, model_num_layers, model_embedding_size, device, loss_device=None,
-                 compression=None, n_cores=3, rank=8, clip=3, use_gru=False):
+                 compression=None, n_cores=3, rank=8, clip=3, use_gru=False, proj_size=0):
         super().__init__()
+        state_size = proj_size or model_hidden_size
         self.loss_device = loss_device
         self.clip = clip
         self.use_gru = use_gru
         if compression is None:
             cls = GRU if use_gru else LSTM
-            self.rnn = cls(mel_n_channels, model_hidden_size, model_num_layers, device)
-            self.linear = nn.Linear(in_features=model_hidden_size, out_features=model_embedding_size).to(device)
+            self.rnn = cls(mel_n_channels, model_hidden_size, model_num_layers, device, proj_size=proj_size)
+            self.linear = nn.Linear(in_features=state_size, out_features=model_embedding_size).to(device)
         elif compression == 'tt':
             print("Encoding linear layer as a tensor-train...")
             if not use_gru:
-                self.rnn = TTLSTM(mel_n_channels, model_hidden_size, model_num_layers, device, n_cores=n_cores, tt_rank=rank)
+                self.rnn = TTLSTM(mel_n_channels, model_hidden_size, model_num_layers, device, n_cores=n_cores, tt_rank=rank,
+                                  proj_size=proj_size)
             else:
                 self.rnn = TTGRU(mel_n_channels, model_hidden_size, model_num_layers, device, bias=True, n_cores=n_cores,
-                                 tt_rank=rank)
-            self.linear = TTLinear(in_features=model_hidden_size, out_features=model_embedding_size, bias=True,
+                                 tt_rank=rank, proj_size=proj_size)
+            self.linear = TTLinear(in_features=state_size, out_features=model_embedding_size, bias=True,
                                    auto_shapes=True, d=n_cores, tt_rank=rank).to(device)
         else:
             raise ValueError("Unknown compression type: '{}'".format(compression))
