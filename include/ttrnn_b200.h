@@ -370,6 +370,28 @@ int ttrnn_ge2e_loss_forward(int32_t S, int32_t U, int32_t E, const float *embeds
 int ttrnn_ge2e_loss_backward(int32_t S, int32_t U, int32_t E, const float *embeds, const float *wb,
                              const float *dloss, void *workspace, float *d_embeds, float *d_wb, void *stream);
 
+/* Utterance-level embeddings (SpeakerEncoder.embed_utterances, DESIGN.md §4.21): every fixed-length window of every utterance
+ * goes through one stack call; these two steps surround it.  All pointers are device pointers.
+ *
+ * ttrnn_partials_gather: builds the window block out (W, P, F) from the packed frames (total_frames, F) of the utterances
+ * concatenated in order.  Window w copies the rows win_first[w] .. win_first[w] + win_valid[w] - 1 to out[w, 0 .. valid-1, :]
+ * and writes zeros to out[w, valid .. P-1, :].  A pure copy (bit-exact).
+ * PRECONDITION, not checked on the device: for every w, 0 <= win_first[w], 1 <= win_valid[w] <= P and
+ * win_first[w] + win_valid[w] <= total_frames.
+ *
+ * ttrnn_segment_mean_normalize_forward: rows x (R, E) in n_seg consecutive segments, seg_off (n_seg + 1, int64) with
+ * seg_off[0] = 0 and seg_off[n_seg] = R.  y (n_seg, E): y[s] = m / ||m||_2 with m the mean of rows seg_off[s] ..
+ * seg_off[s+1] - 1; inv_norm (n_seg) = 1 / ||m||_2, kept for the backward.  ttrnn_segment_mean_normalize_backward writes
+ * dx (R, E): dx[r] = (dy[s] - y[s] (y[s] . dy[s])) * inv_norm[s] / count_s for every row r of segment s.
+ * PRECONDITION, not checked on the device: seg_off non-decreasing; a segment is empty when two offsets are equal, and then
+ * its y row is NaN (0 / 0).  Sums run in a fixed order without atomics: two calls are bit-identical. */
+int ttrnn_partials_gather(int64_t W, int32_t P, int32_t F, const float *frames, int64_t total_frames,
+                          const int64_t *win_first, const int32_t *win_valid, float *out, void *stream);
+int ttrnn_segment_mean_normalize_forward(int64_t n_seg, int32_t E, const float *x, const int64_t *seg_off,
+                                         float *y, float *inv_norm, void *stream);
+int ttrnn_segment_mean_normalize_backward(int64_t n_seg, int32_t E, const int64_t *seg_off, const float *y,
+                                          const float *inv_norm, const float *dy, float *dx, void *stream);
+
 /* Measurement helpers (bench.py only).
  * ttrnn_ffma_probe: dependent-chain-free FP32 FFMA loop on every SM; writes the
  * number of FLOPs executed to *flops_out (host) and leaves a checksum in sink

@@ -107,6 +107,9 @@ SYMBOLS = {
     "ttrnn_ge2e_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
     "ttrnn_ge2e_loss_forward": (C.c_int, [C.c_int32, C.c_int32, C.c_int32] + [_P] * 6),
     "ttrnn_ge2e_loss_backward": (C.c_int, [C.c_int32, C.c_int32, C.c_int32] + [_P] * 7),
+    "ttrnn_partials_gather": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, _P, C.c_int64, _P, _P, _P, _P]),
+    "ttrnn_segment_mean_normalize_forward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 5),
+    "ttrnn_segment_mean_normalize_backward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 6),
     "ttrnn_rnn_ih_route": (C.c_int, [C.POINTER(RnnDesc), C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "ttrnn_static_kernel_table": (C.c_int, [C.c_char_p, C.c_int32]),
     "ttrnn_static_kernel_keys": (C.c_int, [C.c_char_p, C.c_int32]),

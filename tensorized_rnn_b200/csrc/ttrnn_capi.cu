@@ -18,6 +18,7 @@
 #include "tt_dense.cuh"
 #include "tt_bidir.cuh"
 #include "tt_dropout.cuh"
+#include "tt_utter.cuh"
 #include "tt_static.cuh"
 #include "tt_static_api.h"
 
@@ -3245,6 +3246,52 @@ int ttrnn_embed_backward(int64_t rows, int32_t E, const float *x, const float *y
     DevInfo dv;
     if (get_dev(&dv)) return 1;
     ge2e::k_embed_bwd<<<(unsigned)((rows + 7) / 8), ge2e::NT, 0, (cudaStream_t)stream>>>(x, y, inv_norm, dy, dx, (int)rows, E);
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int ttrnn_partials_gather(int64_t W, int32_t P, int32_t F, const float *frames, int64_t total_frames,
+                          const int64_t *win_first, const int32_t *win_valid, float *out, void *stream) {
+    if (W < 1 || P < 1 || F < 1 || total_frames < 1)
+        return fail("ttrnn_partials_gather: W, P, F and total_frames must be >= 1 (got %lld, %d, %d, %lld)", (long long)W, P, F,
+                    (long long)total_frames);
+    if (!frames || !win_first || !win_valid || !out) return fail("ttrnn_partials_gather: null operand");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    const unsigned grid = utter::grid_for(W, dv.sms);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (F % 4 == 0 && ((uintptr_t)frames | (uintptr_t)out) % 16 == 0)
+        utter::k_partials_gather<float4><<<grid, utter::NT, 0, st>>>((const float4 *)frames, win_first, win_valid, (float4 *)out, W,
+                                                                    P, F / 4);
+    else
+        utter::k_partials_gather<float><<<grid, utter::NT, 0, st>>>(frames, win_first, win_valid, out, W, P, F);
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int ttrnn_segment_mean_normalize_forward(int64_t n_seg, int32_t E, const float *x, const int64_t *seg_off, float *y,
+                                         float *inv_norm, void *stream) {
+    if (n_seg < 1 || E < 1) return fail("ttrnn_segment_mean_normalize_forward: n_seg and E must be >= 1");
+    if (!x || !seg_off || !y || !inv_norm) return fail("ttrnn_segment_mean_normalize_forward: null operand");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    utter::k_segment_mean_norm_fwd<<<utter::grid_for(n_seg, dv.sms), utter::NT, 0, (cudaStream_t)stream>>>(x, seg_off, y, inv_norm,
+                                                                                                          n_seg, E);
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int ttrnn_segment_mean_normalize_backward(int64_t n_seg, int32_t E, const int64_t *seg_off, const float *y, const float *inv_norm,
+                                          const float *dy, float *dx, void *stream) {
+    if (n_seg < 1 || E < 1) return fail("ttrnn_segment_mean_normalize_backward: n_seg and E must be >= 1");
+    if (!seg_off || !y || !inv_norm || !dy || !dx) return fail("ttrnn_segment_mean_normalize_backward: null operand");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    utter::k_segment_mean_norm_bwd<<<utter::grid_for(n_seg, dv.sms), utter::NT, 0, (cudaStream_t)stream>>>(seg_off, y, inv_norm, dy,
+                                                                                                          dx, n_seg, E);
     ++g_launches;
     CU_CHECK(cudaGetLastError());
     return 0;

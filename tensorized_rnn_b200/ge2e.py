@@ -7,12 +7,17 @@ reference moves the embeddings to the CPU for this (encoder/main.py:279-280); he
 library (`ttrnn_embed_*`, `ttrnn_ge2e_loss_*`), with hand-written backward kernels.  Under data parallelism the loss
 couples every speaker of the global batch: `ge2e_loss(..., group=...)` all-gathers the embeddings (NCCL), every
 rank evaluates the full loss and keeps the gradient rows of its own utterances.
+
+Utterance-level embeddings (DESIGN.md §4.21): `partial_windows` cuts utterances of any length into the fixed-length windows
+the encoder trains on, `gather_partials` builds the window block on the device and `segment_mean_normalize` averages and
+L2-normalises the window embeddings of each utterance (or the d-vectors of each speaker).
 """
 from __future__ import annotations
 
 import ctypes as C
 from typing import Optional
 
+import numpy as np
 import torch
 from torch import nn
 
@@ -127,6 +132,117 @@ def ge2e_loss(embeds: torch.Tensor, similarity_weight: torch.Tensor, similarity_
     wb = torch.cat([similarity_weight.reshape(1), similarity_bias.reshape(1)])
     loss, sim = _Ge2eLoss.apply(embeds, wb, bool(return_similarity))
     return (loss, sim) if return_similarity else loss
+
+
+def _counts(v, what: str) -> np.ndarray:
+    """A 1-D host sequence of ints >= 1 (a list, a numpy array or a CPU tensor) as int64."""
+    a = np.asarray(v.tolist() if isinstance(v, torch.Tensor) else v)
+    if a.ndim != 1 or a.size == 0 or a.dtype.kind not in "iu":
+        raise ValueError("%s must be a non-empty 1-D sequence of ints, got %r" % (what, v))
+    if (a < 1).any():
+        raise ValueError("every entry of %s must be >= 1, got %r" % (what, v))
+    return a.astype(np.int64)
+
+
+def partial_windows(lengths, partial_frames: int = 160, overlap: float = 0.5, min_coverage: float = 0.75):
+    """Window table of `compute_partial_slices` (Real-Time-Voice-Cloning, encoder/inference.py), in frames.
+
+    For an utterance of n >= 1 frames and P = partial_frames: step = max(round_half_even(P * (1 - overlap)), 1); the
+    window starts are range(0, max(1, n - P + step + 1), step); when there is more than one window and
+    (n - last_start) / P < min_coverage, the last window is dropped.  The utterances are packed in order, so window w
+    covers packed rows first[w] .. first[w] + valid[w] - 1 and is zero past them (valid = min(P, n - start)).
+
+    Host only.  Returns (first int64, valid int32, windows per utterance int64), numpy arrays."""
+    if isinstance(partial_frames, bool) or not isinstance(partial_frames, (int, np.integer)) or partial_frames < 1:
+        raise ValueError("partial_frames must be an int >= 1, got %r" % (partial_frames,))
+    if not 0.0 <= overlap < 1.0:
+        raise ValueError("overlap must be in [0, 1), got %r" % (overlap,))
+    if not 0.0 < min_coverage <= 1.0:
+        raise ValueError("min_coverage must be in (0, 1], got %r" % (min_coverage,))
+    n = _counts(lengths, "lengths")
+    P = int(partial_frames)
+    step = max(int(np.round(P * (1 - overlap))), 1)
+    k = (np.maximum(1, n - P + step + 1) + step - 1) // step
+    k -= (k > 1) & ((n - (k - 1) * step) / P < min_coverage)
+    utt = np.repeat(np.arange(n.size), k)
+    start = (np.arange(int(k.sum())) - np.repeat(np.cumsum(k) - k, k)) * step
+    first = (np.cumsum(n) - n)[utt] + start
+    valid = np.minimum(P, n[utt] - start)
+    assert (valid >= 1).all()
+    return first.astype(np.int64), valid.astype(np.int32), k
+
+
+def gather_partials(frames: torch.Tensor, first, valid, partial_frames: int) -> torch.Tensor:
+    """(W, partial_frames, F) window block from the packed frames (total_frames, F) and a window table (`partial_windows`):
+    window w holds rows first[w] .. first[w] + valid[w] - 1 and zeros after them.  A copy on the device
+    (`ttrnn_partials_gather`), without autograd: the frames are model inputs."""
+    if frames.requires_grad:
+        raise NotImplementedError("gather_partials has no backward: the frames must not require grad")
+    first, valid = np.asarray(first), np.asarray(valid)
+    if first.ndim != 1 or first.size == 0 or first.shape != valid.shape or first.dtype.kind not in "iu" \
+            or valid.dtype.kind not in "iu":
+        raise ValueError("first / valid must be two non-empty 1-D int arrays of one length")
+    if frames.dim() != 2:
+        raise ValueError("frames must be (total_frames, features), got %s" % (tuple(frames.shape),))
+    P = int(partial_frames)
+    total, F = frames.shape
+    if P < 1 or (valid < 1).any() or (valid > P).any() or (first < 0).any() or (first + valid > total).any():
+        raise ValueError("window table out of range: need 1 <= valid <= partial_frames and first + valid <= %d" % total)
+    lib = _lib.load()
+    _require_cuda_f32("frames", frames)
+    frames = _dense16(frames)
+    W = first.size
+    with torch.cuda.device(frames.device):
+        out = torch.empty((W, P, F), device=frames.device, dtype=torch.float32)
+        first_d = torch.from_numpy(first.astype(np.int64)).to(frames.device)
+        valid_d = torch.from_numpy(valid.astype(np.int32)).to(frames.device)
+        stream = torch.cuda.current_stream(frames.device).cuda_stream
+        _lib.check(lib.ttrnn_partials_gather(W, P, F, _ptr(frames), total, _ptr(first_d), _ptr(valid_d), _ptr(out), stream),
+                   "ttrnn_partials_gather")
+    return out
+
+
+class _SegmentMeanNormalize(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, off):
+        lib = _lib.load()
+        x = _dense16(x)
+        n_seg, (rows, E) = off.numel() - 1, x.shape
+        with torch.cuda.device(x.device):
+            y = torch.empty((n_seg, E), device=x.device, dtype=torch.float32)
+            inv = torch.empty(n_seg, device=x.device, dtype=torch.float32)
+            stream = torch.cuda.current_stream(x.device).cuda_stream
+            _lib.check(lib.ttrnn_segment_mean_normalize_forward(n_seg, E, _ptr(x), _ptr(off), _ptr(y), _ptr(inv), stream),
+                       "ttrnn_segment_mean_normalize_forward")
+        ctx.save_for_backward(off, y, inv)
+        ctx.rows = rows
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        lib = _lib.load()
+        off, y, inv = ctx.saved_tensors
+        dy = _dense16(dy)
+        n_seg, E = y.shape
+        with torch.cuda.device(y.device):
+            dx = torch.empty((ctx.rows, E), device=y.device, dtype=torch.float32)
+            stream = torch.cuda.current_stream(y.device).cuda_stream
+            _lib.check(lib.ttrnn_segment_mean_normalize_backward(n_seg, E, _ptr(off), _ptr(y), _ptr(inv), _ptr(dy), _ptr(dx),
+                                                                 stream), "ttrnn_segment_mean_normalize_backward")
+        return dx, None
+
+
+def segment_mean_normalize(x: torch.Tensor, counts) -> torch.Tensor:
+    """L2-normalised means of consecutive row groups: x (R, E), counts (S,) of ints >= 1 summing to R -> (S, E), row s the
+    normalised mean of the counts[s] rows after the first sum(counts[:s]).  Differentiable (`ttrnn_segment_mean_normalize_*`)."""
+    c = _counts(counts, "counts")
+    if x.dim() != 2:
+        raise ValueError("x must be (rows, features), got %s" % (tuple(x.shape),))
+    if int(c.sum()) != x.shape[0]:
+        raise ValueError("counts sum to %d, but x has %d rows" % (int(c.sum()), x.shape[0]))
+    _require_cuda_f32("x", x)
+    off = torch.from_numpy(np.concatenate([[0], np.cumsum(c)])).to(x.device)
+    return _SegmentMeanNormalize.apply(x, off)
 
 
 class GE2EHead(nn.Module):

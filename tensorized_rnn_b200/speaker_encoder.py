@@ -10,7 +10,8 @@ in the CUDA library, ge2e.py); the EER, which the reference computes with scikit
 the evaluation form of `similarity_matrix` (`enrollment_embeds` given) is not provided by the CUDA head and raises.
 `proj_size=P` (appended to the reference signature; LSTM only, the GRU modules refuse it) builds the LSTM with a recurrent
 projection of the GE2E paper (LSTMP) on either side, `compression=None` (dense `LSTM`) or `'tt'` (`TTLSTM`); the embedding
-`linear` then reads the P-wide final state.
+`linear` then reads the P-wide final state.  `embed_utterances` / `embed_speakers` (appended) give the utterance and speaker
+embeddings of enrollment and verification: sliding-window partials, embedded in one stack call and averaged (DESIGN.md §4.21).
 """
 from __future__ import annotations
 
@@ -19,7 +20,7 @@ import torch
 from torch import nn
 
 from .dense import GRU, LSTM
-from .ge2e import embed_normalize, ge2e_loss
+from .ge2e import _counts, embed_normalize, gather_partials, ge2e_loss, partial_windows, segment_mean_normalize
 from .layers import TTLinear
 from .rnn import TTGRU, TTLSTM
 
@@ -63,6 +64,24 @@ class SpeakerEncoder(nn.Module):
         else:
             out, last_hidden = self.rnn(utterances)
         return embed_normalize(self.linear(last_hidden))            # relu + L2 norm (speaker_encoder.py:86-89)
+
+    def embed_utterances(self, frames, lengths, partial_frames=160, overlap=0.5, min_coverage=0.75):
+        """Utterance d-vectors (N, E) of N utterances of any length, as GE2E and Real-Time-Voice-Cloning's `embed_utterance`
+        define them: each utterance is cut into overlapping windows of `partial_frames` frames (`partial_windows`), every
+        window is embedded by `forward`, and the window embeddings are averaged and L2-normalised.
+
+        frames: the utterances' frames packed in order, a CUDA float32 (sum(lengths), mel_n_channels) block (for a list of
+        (n_i, mel) tensors: `torch.cat(utts)` with `[u.size(0) for u in utts]`); lengths: ints >= 1.  All windows of all
+        utterances go through one gather, one `forward` and one segment mean; the call is differentiable in the parameters."""
+        n = _counts(lengths, "lengths")
+        if frames.dim() != 2 or frames.shape[0] != int(n.sum()):
+            raise ValueError("frames must be (sum(lengths) = %d, mel_n_channels), got %s" % (int(n.sum()), tuple(frames.shape)))
+        first, valid, n_windows = partial_windows(n, partial_frames, overlap, min_coverage)
+        return segment_mean_normalize(self(gather_partials(frames, first, valid, partial_frames)), n_windows)
+
+    def embed_speakers(self, d_vectors, counts):
+        """Speaker embeddings (S, E): the L2-normalised mean of each group of `counts[s]` consecutive d-vector rows."""
+        return segment_mean_normalize(d_vectors, counts)
 
     def similarity_matrix(self, verification_embeds, enrollment_embeds=None):
         if enrollment_embeds is not None:
