@@ -43,7 +43,12 @@ extern "C" {
                                  (ttrnn_rnn_param_count_proj, ttrnn_rnn_workspace_bytes_proj, ttrnn_rnn_forward_proj,
                                  ttrnn_rnn_backward_proj).  Still 4 with projected dense LSTM stacks: four new symbols
                                  (ttrnn_dense_rnn_param_count_proj, ttrnn_dense_rnn_workspace_bytes_proj,
-                                 ttrnn_dense_rnn_forward_proj, ttrnn_dense_rnn_backward_proj); nothing existing changes */
+                                 ttrnn_dense_rnn_forward_proj, ttrnn_dense_rnn_backward_proj); nothing existing changes.
+                                 Still 4 with variable-length rows: one more flag value (TTRNN_WS_LENGTHS) and seven new
+                                 symbols (ttrnn_rnn_forward_lengths, ttrnn_rnn_backward_lengths,
+                                 ttrnn_dense_rnn_forward_lengths, ttrnn_dense_rnn_backward_lengths,
+                                 ttrnn_time_reverse_add_lengths, ttrnn_bidir_join_lengths, ttrnn_rnn_describe_ex); nothing
+                                 existing changes */
 #define TTRNN_MAX_CORES   6
 #define TTRNN_MAX_LAYERS  8
 
@@ -259,6 +264,51 @@ int ttrnn_time_reverse_add(int64_t B, int32_t T, int32_t F, const float *a, cons
 int ttrnn_bidir_join(int64_t B, int32_t T, int32_t H, int32_t backward, const float *p, const float *q, float *u,
                      float *v, void *stream);
 
+/* Variable-length rows (DESIGN.md §4.22), the PackedSequence input of torch.nn.LSTM / GRU in its padded form: row b of a
+ * (B, T, .) batch is len_b steps long, 1 <= len_b <= T.  `lengths` is a DEVICE array of B int32.
+ * PRECONDITION, not checked on the device: 1 <= lengths[b] <= T for every b; and the padded inputs x[b, t >= len_b] must be
+ * finite (their products with zero gate gradients enter dW_ih).
+ *
+ * No recurrent kernel sees the lengths.  After every write of the ih projection (forward and backward recompute) the gate
+ * pre-activations of each padded (b, t) are overwritten so that the row is frozen: LSTM i = -inf, f = +inf, g = o = 0
+ * (c_t = c_{t-1} exactly), GRU z = +inf, r = n = 0 (h_t = h_{t-1} exactly).  So every route that reads a materialised ih
+ * projection runs unchanged; the rank-one input mode (I = 1, layer 0) builds its projection inside the kernel and is not
+ * taken under lengths.  What the calls return, torch's contract:
+ *   - out[b, t] = 0 for t >= len_b; the caller's d_out there is ignored (never written);
+ *   - h_n of every layer (hT, also per layer under TTRNN_WS_LAYER_STATES) is the state after step len_b - 1, and c_n (LSTM)
+ *     likewise; their gradients enter at that step;
+ *   - d_x[b, t] = 0 for t >= len_b.
+ *
+ * TTRNN_WS_LENGTHS: the plan is for ttrnn_rnn_forward_lengths / ttrnn_rnn_backward_lengths (it combines with the other
+ * flags of ttrnn_rnn_workspace_bytes_ex and ttrnn_rnn_workspace_bytes_proj).  The backward scratch grows by one (B, T, W)
+ * block, W the output width; every other entry point refuses such a plan, and the _lengths calls refuse a plan without it.
+ * There is no logged (log_grads) form.
+ *
+ * ttrnn_rnn_forward_lengths / _backward_lengths: the arguments of the _proj calls with `pj` optional (NULL = unprojected;
+ * it must be given exactly when the plan was sized with TTRNN_WS_PROJ), `dp` optional (NULL = no dropout), then lengths.
+ * ttrnn_dense_rnn_forward_lengths / _backward_lengths: the arguments of the dense _proj calls, proj_size 0 = unprojected,
+ * then lengths; flags as for the dense _ex calls (TTRNN_WS_LENGTHS may be passed and changes nothing); the workspace
+ * sizes are those of ttrnn_dense_rnn_workspace_bytes (_proj with proj_size > 0).
+ * ttrnn_time_reverse_add_lengths / ttrnn_bidir_join_lengths: ttrnn_time_reverse_add / ttrnn_bidir_join with every row
+ * reversed over its own length, x'[b, t] = x[b, len_b - 1 - t] for t < len_b; every output position t >= len_b is 0. */
+#define TTRNN_WS_LENGTHS 16
+int ttrnn_rnn_forward_lengths(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
+                              const float *x, const float *h0, const float *c0,
+                              const float *params, float *out, float *hT, float *cT,
+                              void *saved, void *scratch, void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp,
+                              const int32_t *lengths);
+int ttrnn_rnn_backward_lengths(const ttrnn_rnn_desc *desc, const ttrnn_rnn_workspace *ws,
+                               const float *x, const float *h0, const float *c0,
+                               const float *params, const float *out, const void *saved,
+                               const float *d_out, const float *d_hT, const float *d_cT,
+                               float *d_params, float *d_x, float *d_h0, float *d_c0,
+                               void *scratch, void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp,
+                               const int32_t *lengths);
+int ttrnn_time_reverse_add_lengths(int64_t B, int32_t T, int32_t F, const float *a, const float *r, float *y,
+                                   const int32_t *lengths, void *stream);
+int ttrnn_bidir_join_lengths(int64_t B, int32_t T, int32_t H, int32_t backward, const float *p, const float *q, float *u,
+                             float *v, const int32_t *lengths, void *stream);
+
 /* Stand-alone TT linear map y = x W^T + bias over `rows` rows:
  * replaces TTLinear.forward (t3nsor/layers.py:121-127) -> tt_dense_matmul
  * (t3nsor/ops.py:54-93).  bias may be NULL. */
@@ -349,6 +399,16 @@ int ttrnn_dense_rnn_backward_proj(const ttrnn_dense_desc *desc, const float *x, 
                                   const float *d_out, const float *d_hT, const float *d_cT,
                                   float *d_params, float *d_x, float *d_h0, float *d_c0,
                                   void *scratch, void *stream, int32_t flags, int32_t proj_size);
+/* Variable-length rows of a dense stack: see TTRNN_WS_LENGTHS above. */
+int ttrnn_dense_rnn_forward_lengths(const ttrnn_dense_desc *desc, const float *x, const float *h0, const float *c0,
+                                    const float *params, float *out, float *hT, float *cT,
+                                    void *saved, void *scratch, void *stream, int32_t flags, int32_t proj_size,
+                                    const int32_t *lengths);
+int ttrnn_dense_rnn_backward_lengths(const ttrnn_dense_desc *desc, const float *x, const float *h0, const float *c0,
+                                     const float *params, const float *out, void *saved,
+                                     const float *d_out, const float *d_hT, const float *d_cT,
+                                     float *d_params, float *d_x, float *d_h0, float *d_c0,
+                                     void *scratch, void *stream, int32_t flags, int32_t proj_size, const int32_t *lengths);
 
 /* GE2E head on the device (SURVEY.md 8f-4): the part of the speaker-encoder training step the reference runs on the CPU
  * after every RNN pass (experiments/speaker_verification/encoder/main.py:279-280 moves the embeddings to `loss_device`).
@@ -433,6 +493,10 @@ int ttrnn_rnn_ih_route(const ttrnn_rnn_desc *desc, int32_t layer, int64_t *chain
  * batch rows per CTA, save_mode = 2 with kept gate activations else 0, and with training != 0: bwd_kernel, bwd_rows, bwd_phase_rows, optional second phase,
  * hh_dw, hh_dw_tc).  Needs a CUDA device (the plan depends on its SM count).  Returns characters written, < 0 on error. */
 int ttrnn_rnn_describe(const ttrnn_rnn_desc *desc, int32_t training, char *buf, int32_t cap);
+/* The same for the plan that ttrnn_rnn_workspace_bytes_ex(desc, flags, .) would size: TTRNN_WS_WHOLE_BATCH plans one row group
+ * and TTRNN_WS_LENGTHS leaves out the rank-one input mode (I = 1), which variable-length rows do not take; the other flags
+ * change no route.  TTRNN_WS_PROJ is refused (projected stacks run on the runtime-shape kernels only). */
+int ttrnn_rnn_describe_ex(const ttrnn_rnn_desc *desc, int32_t flags, int32_t training, char *buf, int32_t cap);
 /* Row-group split of `desc` under the current options (round 2, "row_groups"): multi-layer stacks whose batch does not
  * fill whole waves of CTAs are cut into two independent row groups that run the stack on two streams, so that the SMs
  * a layer-pass of one group leaves idle run the next layer of the other (the reference has no counterpart: its layer

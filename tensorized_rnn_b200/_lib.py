@@ -18,6 +18,7 @@ WS_WHOLE_BATCH = 1
 WS_LAYER_STATES = 2      # per-layer (L, B, H) initial / final states and their gradients
 WS_DROPOUT = 4           # inter-layer dropout: saved keeps the masked inputs of layers 1 .. L-1
 WS_PROJ = 8              # projected LSTM (proj_size): the plan of the _proj entry points
+WS_LENGTHS = 16          # variable-length rows: the plan of the _lengths entry points
 CELL_LSTM, CELL_GRU = 0, 1
 
 _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc", "libttrnn_b200.so")
@@ -83,6 +84,12 @@ SYMBOLS = {
                                [C.POINTER(RnnProj), C.POINTER(Dropout)]),
     "ttrnn_rnn_backward_proj": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 15 +
                                 [C.POINTER(RnnProj), C.POINTER(Dropout)]),
+    "ttrnn_rnn_forward_lengths": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 10 +
+                                  [C.POINTER(RnnProj), C.POINTER(Dropout), _P]),
+    "ttrnn_rnn_backward_lengths": (C.c_int, [C.POINTER(RnnDesc), C.POINTER(RnnWorkspace)] + [_P] * 15 +
+                                   [C.POINTER(RnnProj), C.POINTER(Dropout), _P]),
+    "ttrnn_time_reverse_add_lengths": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    "ttrnn_bidir_join_lengths": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "ttrnn_dropout_apply": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.POINTER(Dropout),
                                       _P, _P, _P, _P]),
     "ttrnn_ttlinear_param_count": (C.c_int64, [C.POINTER(TTShape)]),
@@ -102,6 +109,8 @@ SYMBOLS = {
                                                        C.c_int32]),
     "ttrnn_dense_rnn_forward_proj": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 10 + [C.c_int32, C.c_int32]),
     "ttrnn_dense_rnn_backward_proj": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 15 + [C.c_int32, C.c_int32]),
+    "ttrnn_dense_rnn_forward_lengths": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 10 + [C.c_int32, C.c_int32, _P]),
+    "ttrnn_dense_rnn_backward_lengths": (C.c_int, [C.POINTER(DenseDesc)] + [_P] * 15 + [C.c_int32, C.c_int32, _P]),
     "ttrnn_embed_forward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 4),
     "ttrnn_embed_backward": (C.c_int, [C.c_int64, C.c_int32] + [_P] * 6),
     "ttrnn_ge2e_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
@@ -114,6 +123,7 @@ SYMBOLS = {
     "ttrnn_static_kernel_table": (C.c_int, [C.c_char_p, C.c_int32]),
     "ttrnn_static_kernel_keys": (C.c_int, [C.c_char_p, C.c_int32]),
     "ttrnn_rnn_describe": (C.c_int, [C.POINTER(RnnDesc), C.c_int32, C.c_char_p, C.c_int32]),
+    "ttrnn_rnn_describe_ex": (C.c_int, [C.POINTER(RnnDesc), C.c_int32, C.c_int32, C.c_char_p, C.c_int32]),
     "ttrnn_tc_launch_count": (C.c_int64, [C.c_int32]),
     "ttrnn_static_kernel_launches": (C.c_int, [C.POINTER(C.c_int64), C.c_int32, C.c_int32]),
     "ttrnn_rnn_row_groups": (C.c_int, [C.POINTER(RnnDesc), C.c_int32, C.POINTER(C.c_int64)]),
@@ -161,11 +171,15 @@ def load() -> C.CDLL:
     return lib
 
 
-def describe_plan(desc: "RnnDesc", training: bool = True) -> list:
-    """Execution plan of a descriptor (ttrnn_rnn_describe) as a list of dicts: [header, layer 0, layer 1, ...]."""
+def describe_plan(desc: "RnnDesc", training: bool = True, flags: int = 0) -> list:
+    """Execution plan of a descriptor (ttrnn_rnn_describe) as a list of dicts: [header, layer 0, layer 1, ...].
+    flags: the workspace flags of the plan (ttrnn_rnn_describe_ex), e.g. WS_LENGTHS."""
     lib = load()
     buf = C.create_string_buffer(8192)
-    n = lib.ttrnn_rnn_describe(C.byref(desc), 1 if training else 0, buf, 8192)
+    if flags:
+        n = lib.ttrnn_rnn_describe_ex(C.byref(desc), int(flags), 1 if training else 0, buf, 8192)
+    else:
+        n = lib.ttrnn_rnn_describe(C.byref(desc), 1 if training else 0, buf, 8192)
     if n < 0:
         raise RuntimeError("ttrnn_rnn_describe failed: " + last_error())
     out = []

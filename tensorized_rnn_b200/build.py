@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libttrnn_b200.so")
 SOURCES = ["ttrnn_capi.cu", "tt_static_inst.cu"]
-HEADERS = ["tt_plan.h", "tt_stage.cuh", "tt_kernels.cuh", "tt_proj.cuh", "tt_cell.cuh", "tt_gemm.cuh", "tt_umma.cuh", "tt_tc.cuh", "tt_ge2e.cuh", "tt_dense.cuh", "tt_bidir.cuh", "tt_dropout.cuh", "tt_utter.cuh", "tt_static.cuh", "tt_static_api.h",
+HEADERS = ["tt_plan.h", "tt_stage.cuh", "tt_kernels.cuh", "tt_proj.cuh", "tt_cell.cuh", "tt_gemm.cuh", "tt_umma.cuh", "tt_tc.cuh", "tt_ge2e.cuh", "tt_dense.cuh", "tt_bidir.cuh", "tt_dropout.cuh", "tt_utter.cuh", "tt_varlen.cuh", "tt_static.cuh", "tt_static_api.h",
            os.path.join("..", "..", "include", "ttrnn_b200.h")]
 
 NVCC_FLAGS = [

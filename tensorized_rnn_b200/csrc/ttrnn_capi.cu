@@ -19,6 +19,7 @@
 #include "tt_bidir.cuh"
 #include "tt_dropout.cuh"
 #include "tt_utter.cuh"
+#include "tt_varlen.cuh"
 #include "tt_static.cuh"
 #include "tt_static_api.h"
 
@@ -83,11 +84,18 @@ constexpr int kOptFields = sizeof(Opts) / sizeof(long long);
 constexpr long long kPlanMagic = 0x7474726E6E706C36LL;          // "ttrnnpl6"
 // plan words: [0] magic, [1 .. kOptFields] options, then the row-group split (group count, rows of group 0), then 1 when
 // the state buffers are per layer (TTRNN_WS_LAYER_STATES), then 1 when `saved` keeps the masked layer inputs of the
-// dropout entry points (TTRNN_WS_DROPOUT), then 1 when the plan is for the projected entry points (TTRNN_WS_PROJ)
+// dropout entry points (TTRNN_WS_DROPOUT), then the entry-point family: bit kEntryProj when the plan is for the projected
+// entry points (TTRNN_WS_PROJ), bit kEntryLengths when it is for the variable-length ones (TTRNN_WS_LENGTHS)
 constexpr int kPlanGroups = kOptFields + 1, kPlanRows0 = kOptFields + 2, kPlanLayerStates = kOptFields + 3,
-              kPlanDropout = kOptFields + 4, kPlanProj = kOptFields + 5;
+              kPlanDropout = kOptFields + 4, kPlanEntry = kOptFields + 5;
+constexpr int64_t kEntryProj = 1, kEntryLengths = 2;
 static_assert(kOptFields + 6 <= TTRNN_PLAN_WORDS, "plan does not fit ttrnn_rnn_workspace.plan");
 thread_local Opts t_opt;
+// the calling thread's current plan carries per-row lengths (TTRNN_WS_LENGTHS): every layer then reads a materialised ih
+// projection, which the lengths freeze (tt_varlen.cuh), so the rank-one input mode is not taken (layer_mode)
+thread_local bool t_varlen = false;
+inline bool plan_proj(const int64_t *plan) { return (plan[kPlanEntry] & kEntryProj) != 0; }
+inline bool plan_lengths(const int64_t *plan) { return (plan[kPlanEntry] & kEntryLengths) != 0; }
 inline int merge_fwd() { return t_opt.merge_cores >= 2 ? 1 : 0; }    // contracted forward variants (merge_cores = 2)
 inline int merge_bwd() { return t_opt.merge_cores >= 1 ? 1 : 0; }    // contracted dX-only BPTT variants (merge_cores >= 1)
 
@@ -100,6 +108,7 @@ Opts snapshot_options() {
     o.split_kept = g_opt_split_kept.load(); o.dense_ratio = g_opt_dense_ratio.load(); o.tc_gemm = g_opt_tc_gemm.load();
     o.rank_pad = g_opt_rank_pad.load(); o.bwd_overlap = g_opt_bwd_overlap.load(); o.row_groups = g_opt_row_groups.load();
     o.merge_cores = g_opt_merge_cores.load();
+    t_varlen = false;                  // a fresh snapshot plans without lengths; the callers that size one set it after
     return o;
 }
 void plan_store(const Opts &o, int64_t *plan) {
@@ -109,6 +118,7 @@ void plan_store(const Opts &o, int64_t *plan) {
 bool plan_load(const int64_t *plan, Opts *o) {
     if (!plan || plan[0] != kPlanMagic) return false;
     memcpy(o, plan + 1, sizeof *o);
+    t_varlen = plan_lengths(plan);
     return true;
 }
 
@@ -430,9 +440,10 @@ int build_rnn_plan(const ttrnn_rnn_desc *d, RnnPlan *rp, const ttrnn_rnn_proj *p
 // Every caller that needs to know which recurrent kernel a layer runs (workspace layout, row-group planner, describe,
 // the launch paths) asks these functions, so that the plan they report and model is the one that launches.
 
-// input mode of layer l: a single input feature (I = 1) is folded into the recurrent kernel as a rank-one term
+// input mode of layer l: a single input feature (I = 1) is folded into the recurrent kernel as a rank-one term, except
+// under per-row lengths, which need the materialised ih projection to freeze finished rows
 inline int layer_mode(const ttrnn_rnn_desc *d, int l) {
-    return (l == 0 && d->input_size == 1) ? tts::MODE_RANK1 : tts::MODE_XG;
+    return (l == 0 && d->input_size == 1 && !t_varlen) ? tts::MODE_RANK1 : tts::MODE_XG;
 }
 
 // input modes the BPTT of layer l may run: the layer's own, and for a rank-one layer 0 also MODE_XG, which the backward
@@ -650,7 +661,7 @@ struct RnnLayout {
     // fwd scratch (floats)
     long long f_xg = 0, f_sh = 0, f_sc = 0, f_hs = 0, f_aux = 0, f_dense = 0, f_total = 0;
     // bwd scratch (floats)
-    long long b_xg = 0, b_dhs = 0, b_sdh = 0, b_sdc = 0, b_part_hh = 0, b_part_ih = 0, b_spill = 0, b_aux = 0, b_dense = 0, b_dense_hh = 0, b_total = 0;
+    long long b_xg = 0, b_dhs = 0, b_sdh = 0, b_sdc = 0, b_dout = 0, b_part_hh = 0, b_part_ih = 0, b_spill = 0, b_aux = 0, b_dense = 0, b_dense_hh = 0, b_total = 0;
     long long part_stride = 0;  // floats per partial slot
     int nslots = 0;
     // backward overlap: the per-layer buffers (everything from b_xg on) exist twice, set (l & 1) at + set * set_stride
@@ -747,6 +758,7 @@ int build_layout(const ttrnn_rnn_desc *d, const RnnPlan &rp, const DevInfo &dv, 
     lo->b_dhs = o; o += (L > 1 ? 2 * r4(lo->BTW) : 0);
     lo->b_sdh = o; o += r4(lo->BW);
     lo->b_sdc = o; o += r4(lo->BH);
+    lo->b_dout = o; o += t_varlen ? r4(lo->BTW) : 0;     // lengths: the last layer's output gradient, zero past each row
     const long long set_base = o;                         // per-layer buffers from here on
     lo->b_xg = o; o += lo->xg_floats;
     lo->b_part_hh = o; o += lo->part_stride * lo->nslots;
@@ -829,6 +841,39 @@ static int launch_dropout(const DevInfo &dv, long long B, int T, int F, const Dr
         const long long n = B * (long long)T * F;
         ttdrop::k_dropout_1<<<ttdrop::grid_for(n, dv.sms), ttdrop::NT, 0, st>>>(x, xr, y, yr, n, T, F, m);
     }
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+// ---- variable-length rows (tt_varlen.cuh) ---------------------------------------------------------------------------
+// freeze the padded (b, t0 + t) of an ih-projection chunk xg (B, tc, G*H) at batch stride ld
+static int varlen_freeze(const DevInfo &dv, float *xg, long long ld, const int32_t *len, long long B, int tc, int t0, int H,
+                         int cell, cudaStream_t st) {
+    const int GH = gates_of(cell) * H;
+    const long long rows = B * tc;
+    varlen::k_varlen_freeze<<<varlen::grid_rows(rows, dv.sms), varlen::NT, 0, st>>>(xg, ld, len, rows, tc, t0, GH, H,
+                                                                                    cell == TTRNN_CELL_LSTM);
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+// dst (B, W) = src[b, len_b - 1] of a (B, T, W) block
+static int varlen_last(const DevInfo &dv, const float *src, const int32_t *len, long long B, int T, int W, float *dst,
+                       cudaStream_t st) {
+    const long long n = B * W;
+    varlen::k_varlen_last<<<varlen::grid_for(n, dv.sms), varlen::NT, 0, st>>>(src, (long long)T * W, len, dst, n, W);
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+// dst = src with every (b, t0 + t >= len_b) zeroed over (B, tn, F) blocks at batch strides ld_src / ld_dst, and dh[b]
+// (B, F; nullptr = none) added at t0 + t = len_b - 1
+static int varlen_mask(const DevInfo &dv, const float *src, long long ld_src, float *dst, long long ld_dst, const int32_t *len,
+                       long long B, int tn, int t0, int F, cudaStream_t st, const float *dh = nullptr) {
+    const long long rows = B * tn;
+    varlen::k_varlen_mask<<<varlen::grid_rows(rows, dv.sms), varlen::NT, 0, st>>>(src, ld_src, dst, ld_dst, len, dh, rows, tn,
+                                                                                   t0, F);
     ++g_launches;
     CU_CHECK(cudaGetLastError());
     return 0;
@@ -1207,6 +1252,7 @@ struct GroupCacheEntry {
     bool used = false;
     ttrnn_rnn_desc d;
     Opts o;
+    bool varlen = false;
     int sms = 0;
     GroupPlan gp;
 };
@@ -1229,14 +1275,14 @@ int plan_row_groups(const ttrnn_rnn_desc *d_in, GroupPlan *gp, const DevInfo *de
     thread_local GroupCacheEntry cache[kGroupCache];
     thread_local int cache_next = 0;
     for (const GroupCacheEntry &e : cache)
-        if (e.used && e.sms == dv.sms && !memcmp(&e.d, d_in, sizeof *d_in) && !memcmp(&e.o, &t_opt, sizeof t_opt)) {
+        if (e.used && e.sms == dv.sms && e.varlen == t_varlen && !memcmp(&e.d, d_in, sizeof *d_in) && !memcmp(&e.o, &t_opt, sizeof t_opt)) {
             *gp = e.gp;
             return 0;
         }
     auto remember = [&]() {
         GroupCacheEntry &e = cache[cache_next];
         cache_next = (cache_next + 1) % kGroupCache;
-        e.used = true; e.d = *d_in; e.o = t_opt; e.sms = dv.sms; e.gp = *gp;
+        e.used = true; e.d = *d_in; e.o = t_opt; e.varlen = t_varlen; e.sms = dv.sms; e.gp = *gp;
         return 0;
     };
     CallPlan cp;
@@ -1417,9 +1463,14 @@ int ttrnn_static_kernel_launches(int64_t *counts, int32_t cap, int32_t reset) {
     return n;
 }
 
-int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf, int32_t cap) {
+// flags: those of ttrnn_rnn_workspace_bytes_ex that decide a route: TTRNN_WS_WHOLE_BATCH (one row group) and
+// TTRNN_WS_LENGTHS (no rank-one input mode)
+static int describe_impl(const ttrnn_rnn_desc *d_full, int32_t flags, int32_t training, char *buf, int32_t cap) {
     if (!buf || cap < 1) return -1;
+    if (flags & TTRNN_WS_PROJ) { fail("ttrnn_rnn_describe_ex: projected stacks are not described"); return -1; }
     t_opt = snapshot_options();
+    t_varlen = (flags & TTRNN_WS_LENGTHS) != 0;
+    if (flags & TTRNN_WS_WHOLE_BATCH) t_opt.row_groups = 0;
     // with two row groups the layer lines describe group 0 (the full waves); the header names the split and the
     // rows per CTA the remainder group runs at
     DevInfo dv;
@@ -1502,6 +1553,14 @@ int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf
     return n;
 }
 
+int ttrnn_rnn_describe(const ttrnn_rnn_desc *d_full, int32_t training, char *buf, int32_t cap) {
+    return describe_impl(d_full, 0, training, buf, cap);
+}
+
+int ttrnn_rnn_describe_ex(const ttrnn_rnn_desc *d_full, int32_t flags, int32_t training, char *buf, int32_t cap) {
+    return describe_impl(d_full, flags, training, buf, cap);
+}
+
 int64_t ttrnn_rnn_param_count(const ttrnn_rnn_desc *desc) {
     RnnPlan rp;
     if (build_rnn_plan(desc, &rp)) return -1;
@@ -1535,6 +1594,7 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
     if (!ws) return fail("null workspace struct");
     if (flags & TTRNN_WS_PROJ) return fail("TTRNN_WS_PROJ: size the plan with ttrnn_rnn_workspace_bytes_proj");
     t_opt = snapshot_options();
+    t_varlen = (flags & TTRNN_WS_LENGTHS) != 0;
     if (flags & TTRNN_WS_WHOLE_BATCH) t_opt.row_groups = 0;
     GroupPlan gp;
     if (plan_row_groups(desc, &gp)) return 1;
@@ -1561,6 +1621,7 @@ int ttrnn_rnn_workspace_bytes_ex(const ttrnn_rnn_desc *desc, int32_t flags, ttrn
     ws->plan[kPlanRows0] = gp.rows[0];
     ws->plan[kPlanLayerStates] = (flags & TTRNN_WS_LAYER_STATES) ? 1 : 0;
     ws->plan[kPlanDropout] = masked ? 1 : 0;
+    ws->plan[kPlanEntry] = t_varlen ? kEntryLengths : 0;
     return 0;
 }
 
@@ -1573,6 +1634,7 @@ int ttrnn_rnn_workspace_bytes_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_p
     if (desc->cell != TTRNN_CELL_LSTM) return fail("ttrnn_rnn_workspace_bytes_proj: a projection needs an LSTM descriptor");
     t_opt = snapshot_options();
     t_opt.row_groups = 0;
+    t_varlen = (flags & TTRNN_WS_LENGTHS) != 0;
     const bool masked = (flags & TTRNN_WS_DROPOUT) != 0;
     if (workspace_one(desc, ws, masked, pj)) return 1;
     memset(ws->plan, 0, sizeof ws->plan);
@@ -1581,16 +1643,17 @@ int ttrnn_rnn_workspace_bytes_proj(const ttrnn_rnn_desc *desc, const ttrnn_rnn_p
     ws->plan[kPlanRows0] = desc->batch;
     ws->plan[kPlanLayerStates] = (flags & TTRNN_WS_LAYER_STATES) ? 1 : 0;
     ws->plan[kPlanDropout] = masked ? 1 : 0;
-    ws->plan[kPlanProj] = 1;
+    ws->plan[kPlanEntry] = kEntryProj | (t_varlen ? kEntryLengths : 0);
     return 0;
 }
 
 // forward of ONE row group on stream `stream`; `ws` carries the byte sizes of this group, t_opt is already loaded
 // `dc`: inter-layer dropout (nullptr = none; the plan then has no masked buffers)
 // `pj`: the projection (nullptr = none)
+// `lengths`: per-row lengths of a plan with TTRNN_WS_LENGTHS (nullptr = every row runs T steps)
 static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
                        const float *h0, const float *c0, const float *params_in, float *out, float *hT, float *cT, void *saved,
-                       void *scratch, void *stream, const DropCall *dc, const ttrnn_rnn_proj *pj) {
+                       void *scratch, void *stream, const DropCall *dc, const ttrnn_rnn_proj *pj, const int32_t *lengths) {
     if (!x || !params_in || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     DevInfo dv;
     CallPlan cp;
@@ -1655,13 +1718,21 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                               tc_rows_use(B * (long long)lo.Tc, nin, GH, false), false, st))
                 return 1;
         }
+        // with lengths, the padded steps of the chunk are frozen right after the projection wrote them
         auto project = [&](int t0, int tc) -> int {
-            if (dense)
-                return dense_rows_gemm(TTRNN_K_GEMM_FWD, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin, nin,
-                                       D.wt, D.w_hi, D.w_lo, GH, b_ih, lstm ? b_hh : nullptr, xg, (long long)tc * GH, false, st);
-            return launch_ttlinear_fwd(lp.ih, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin,
-                                       params + lp.off_ih_cores, b_ih, lstm ? b_hh : nullptr, xg, (long long)tc * GH, st,
-                                       &d->ih[l]);
+            const int rc = dense ? dense_rows_gemm(TTRNN_K_GEMM_FWD, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin,
+                                                   nin, D.wt, D.w_hi, D.w_lo, GH, b_ih, lstm ? b_hh : nullptr, xg,
+                                                   (long long)tc * GH, false, st)
+                                 : launch_ttlinear_fwd(lp.ih, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin,
+                                                       params + lp.off_ih_cores, b_ih, lstm ? b_hh : nullptr, xg,
+                                                       (long long)tc * GH, st, &d->ih[l]);
+            if (rc || !lengths) return rc;
+            return varlen_freeze(dv, xg, (long long)tc * GH, lengths, B, tc, t0, H, d->cell, st);
+        };
+        // with lengths, an LSTM layer's h_n is its output at step len_b - 1 (the kernel's h_T is that of step T - 1)
+        auto layer_done = [&]() -> int {
+            if (!lengths || !lstm || !hTl) return 0;
+            return varlen_last(dv, lout, lengths, B, T, W, hTl, st);
         };
 
         // ---- statically specialised kernel for this hh shape, if one is registered -------------------
@@ -1719,6 +1790,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                 ++g_launches;
                 if (rc) return fail("static kernel %s launch failed: %s", se->name, cudaGetErrorString((cudaError_t)rc));
             }
+            if (layer_done()) return 1;
             continue;
         }
 
@@ -1761,6 +1833,7 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
                 ++g_launches;
                 CU_CHECK(cudaGetLastError());
             }
+            if (layer_done()) return 1;
             continue;
         }
 
@@ -1802,7 +1875,10 @@ static int forward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws
             ++g_launches;
             CU_CHECK(cudaGetLastError());
         }
+        if (layer_done()) return 1;
     }
+    // with lengths, the output past each row's length is torch's padding value 0
+    if (lengths && varlen_mask(dv, out, (long long)T * W, out, (long long)T * W, lengths, B, T, 0, W, st)) return 1;
     return 0;
 }
 
@@ -1832,12 +1908,13 @@ static SideCtx *side_ctx() {
 static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float *x, const float *h0, const float *c0,
                              const float *params, const float *out, const void *saved, const float *d_out, const float *d_hT,
                              const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch,
-                             cudaStream_t st, const DropCall *dc);
+                             cudaStream_t st, const DropCall *dc, const int32_t *lengths);
 
 static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const StateMap &sm, const float *x,
                         const float *h0, const float *c0, const float *params, const float *out, const void *saved,
                         const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0,
-                        float *d_c0, void *scratch, void *stream, const DropCall *dc, const ttrnn_rnn_proj *pj) {
+                        float *d_c0, void *scratch, void *stream, const DropCall *dc, const ttrnn_rnn_proj *pj,
+                        const int32_t *lengths) {
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     DevInfo dv;
     CallPlan cp;
@@ -1850,13 +1927,14 @@ static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
     cudaStream_t st = (cudaStream_t)stream;
     if (!eff.padded)
         return rnn_backward_impl(cp, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
-                                 st, dc);
+                                 st, dc, lengths);
     float *pp = (float *)scratch + lo.b_total, *dpp = pp + eff.pad_floats;
     CU_CHECK(cudaMemsetAsync(pp, 0, (size_t)eff.pad_floats * 4, st));
     k_pad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, params, pp);
     ++g_launches;
     CU_CHECK(cudaGetLastError());
-    if (rnn_backward_impl(cp, sm, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st, dc)) return 1;
+    if (rnn_backward_impl(cp, sm, x, h0, c0, pp, out, saved, d_out, d_hT, d_cT, dpp, d_x, d_h0, d_c0, scratch, st, dc, lengths))
+        return 1;
     // the gradient wrt a real core is the matching block of the padded core's gradient
     k_unpad_cores<<<eff.tab.n, 256, 0, st>>>(eff.tab, dpp, d_params);
     ++g_launches;
@@ -1867,7 +1945,7 @@ static int backward_one(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *w
 static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float *x, const float *h0, const float *c0,
                              const float *params, const float *out, const void *saved, const float *d_out, const float *d_hT,
                              const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch,
-                             cudaStream_t st, const DropCall *dc) {
+                             cudaStream_t st, const DropCall *dc, const int32_t *lengths) {
     const ttrnn_rnn_desc *d = cp.d();
     const RnnPlan &rp = cp.rp;
     const RnnLayout &lo = cp.lo;
@@ -1925,6 +2003,18 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
         // this layer's initial state and the upstream gradient of its final state (enters its last step)
         const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l, true);
         const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L, true);
+        if (lengths) {
+            // the caller's output gradient past each row's length is ignored: the last layer reads a zeroed copy (an inner
+            // layer's is the dX of the layer above, exactly 0 there).  An LSTM h_n is the output at step len_b - 1, so its
+            // gradient enters there as an output gradient and the kernel's d_hT is 0 (DESIGN.md §4.22)
+            float *g = (l == L - 1) ? sc + lo.b_dout : sc + lo.b_dhs + ((l + 1) & 1) * r4(lo.BTW);
+            const float *dhn = lstm ? dhTl : nullptr;
+            if ((l == L - 1 || dhn) && varlen_mask(dv, l == L - 1 ? d_out : g, (long long)T * W, g, (long long)T * W, lengths,
+                                                   B, T, 0, W, st, dhn))
+                return 1;
+            dhs = g;
+            if (lstm) dhTl = nullptr;
+        }
 
         // ---- ih projection (recompute) and its backward per time chunk: TT chain or dense route ---------
         // a rank-one layer 0 whose input gradient is wanted runs the projected-input kernels (delta_ih feeds dX)
@@ -1939,13 +2029,16 @@ static int rnn_backward_impl(const CallPlan &cp, const StateMap &sm, const float
                 return 1;
         }
         bool dense_first = true;
+        // the recompute is frozen like the forward's projection
         auto project = [&](int t0, int tc) -> int {
-            if (dense)
-                return dense_rows_gemm(TTRNN_K_GEMM_FWD, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin, nin,
-                                       D.wt, D.w_hi, D.w_lo, GH, b_ih, lstm ? b_hh : nullptr, xg, (long long)tc * GH, false, st);
-            return launch_ttlinear_fwd(lp.ih, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin,
-                                       params + lp.off_ih_cores, b_ih, lstm ? b_hh : nullptr, xg, (long long)tc * GH, st,
-                                       &d->ih[l]);
+            const int rc = dense ? dense_rows_gemm(TTRNN_K_GEMM_FWD, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin,
+                                                   nin, D.wt, D.w_hi, D.w_lo, GH, b_ih, lstm ? b_hh : nullptr, xg,
+                                                   (long long)tc * GH, false, st)
+                                 : launch_ttlinear_fwd(lp.ih, dv, B * tc, tc, lin + (long long)t0 * nin, (long long)T * nin,
+                                                       params + lp.off_ih_cores, b_ih, lstm ? b_hh : nullptr, xg,
+                                                       (long long)tc * GH, st, &d->ih[l]);
+            if (rc || !lengths) return rc;
+            return varlen_freeze(dv, xg, (long long)tc * GH, lengths, B, tc, t0, H, d->cell, st);
         };
         // xg holds delta_ih of the chunk: core / bias gradients (accumulated over chunks) and dX
         auto project_dx = [&](int t0, int tc) -> int {       // dense route: dX = delta W on the caller's stream
@@ -2366,13 +2459,27 @@ static StateMap state_map(const ttrnn_rnn_desc *d_full, const ttrnn_rnn_workspac
 static int proj_call(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, bool proj_given,
                      const ttrnn_rnn_proj *pj) {
     if (!proj_given) {
-        if (ws->plan[kPlanProj])
+        if (plan_proj(ws->plan))
             return fail("%s: the plan was sized with TTRNN_WS_PROJ; run it with the _proj entry points", who);
         return 0;
     }
-    if (!ws->plan[kPlanProj]) return fail("%s: the plan was not sized with TTRNN_WS_PROJ (ttrnn_rnn_workspace_bytes_proj)", who);
+    if (!plan_proj(ws->plan)) return fail("%s: the plan was not sized with TTRNN_WS_PROJ (ttrnn_rnn_workspace_bytes_proj)", who);
     if (!pj) return fail("%s: pj must be non-null", who);
     if (d_in->cell != TTRNN_CELL_LSTM) return fail("%s: a projection needs an LSTM descriptor", who);
+    return 0;
+}
+
+// the lengths of an entry point: len_given = the call is a _lengths entry point (which requires them and a plan sized with
+// TTRNN_WS_LENGTHS); every other entry point refuses such a plan
+static int lengths_call(const char *who, const ttrnn_rnn_workspace *ws, bool len_given, const int32_t *lengths) {
+    if (!len_given) {
+        if (plan_lengths(ws->plan))
+            return fail("%s: the plan was sized with TTRNN_WS_LENGTHS; run it with the _lengths entry points", who);
+        return 0;
+    }
+    if (!plan_lengths(ws->plan))
+        return fail("%s: the plan was not sized with TTRNN_WS_LENGTHS (ttrnn_rnn_workspace_bytes_ex / _proj)", who);
+    if (!lengths) return fail("%s: lengths must be non-null", who);
     return 0;
 }
 
@@ -2439,17 +2546,18 @@ static int drop_call(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rn
 static int rnn_forward_entry(const char *who, const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x,
                              const float *h0, const float *c0, const float *params, float *out, float *hT, float *cT,
                              void *saved, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp,
-                             bool proj_given = false, const ttrnn_rnn_proj *pj = nullptr) {
+                             bool proj_given = false, const ttrnn_rnn_proj *pj = nullptr, bool len_given = false,
+                             const int32_t *lengths = nullptr) {
     if (!ws || !plan_load(ws->plan, &t_opt))
         return fail("%s: `ws` must be the struct filled by ttrnn_rnn_workspace_bytes() for this descriptor", who);
     if (!d_in) return fail("null descriptor");
-    if (proj_call(who, d_in, ws, proj_given, pj)) return 1;
+    if (lengths_call(who, ws, len_given, lengths) || proj_call(who, d_in, ws, proj_given, pj)) return 1;
     DropCall dcs;
     const DropCall *dc = nullptr;
     if (drop_call(who, d_in, ws, dp_given, dp, &dcs, &dc)) return 1;
     const StateMap sm = state_map(d_in, ws, pj);
     if (ws->plan[kPlanGroups] <= 1)
-        return forward_one(d_in, ws, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream, dc, pj);
+        return forward_one(d_in, ws, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream, dc, pj, lengths);
     if (!x || !params || !out || !scratch) return fail("x, params, out and scratch must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_forward")) return 1;
@@ -2470,7 +2578,7 @@ static int rnn_forward_entry(const char *who, const ttrnn_rnn_desc *d_in, const 
         rc = forward_one(&gs.d[g], &gs.w[g], sm, x + r0 * T * I, h0 ? h0 + r0 * H : nullptr, c0 ? c0 + r0 * H : nullptr, params,
                          out + r0 * T * H, hT ? hT + r0 * H : nullptr, cT ? cT + r0 * H : nullptr,
                          saved ? (char *)saved + gs.sv_off[g] : nullptr, (char *)scratch + gs.f_off[g],
-                         (g == 0 || serial) ? (void *)st : (void *)gc->s, dc, nullptr);
+                         (g == 0 || serial) ? (void *)st : (void *)gc->s, dc, nullptr, lengths ? lengths + r0 : nullptr);
     }
     t_group = 0;
     if (!serial) {       // also on the error path: the caller's stream must not run ahead of the group stream
@@ -2498,18 +2606,19 @@ static int rnn_backward_entry(const char *who, const ttrnn_rnn_desc *d_in, const
                               const float *h0, const float *c0, const float *params, const float *out, const void *saved,
                               const float *d_out, const float *d_hT, const float *d_cT, float *d_params, float *d_x,
                               float *d_h0, float *d_c0, void *scratch, void *stream, bool dp_given, const ttrnn_dropout *dp,
-                              bool proj_given = false, const ttrnn_rnn_proj *pj = nullptr) {
+                              bool proj_given = false, const ttrnn_rnn_proj *pj = nullptr, bool len_given = false,
+                              const int32_t *lengths = nullptr) {
     if (!ws || !plan_load(ws->plan, &t_opt))
         return fail("%s: `ws` must be the struct the matching forward ran with", who);
     if (!d_in) return fail("null descriptor");
-    if (proj_call(who, d_in, ws, proj_given, pj)) return 1;
+    if (lengths_call(who, ws, len_given, lengths) || proj_call(who, d_in, ws, proj_given, pj)) return 1;
     DropCall dcs;
     const DropCall *dc = nullptr;
     if (drop_call(who, d_in, ws, dp_given, dp, &dcs, &dc)) return 1;
     const StateMap sm = state_map(d_in, ws, pj);
     if (ws->plan[kPlanGroups] <= 1)
         return backward_one(d_in, ws, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
-                            stream, dc, pj);
+                            stream, dc, pj, lengths);
     if (!x || !params || !out || !scratch || !d_params) return fail("x, params, out, scratch, d_params must be non-null");
     GroupSlices gs;
     if (group_slices(d_in, ws, &gs, "ttrnn_rnn_backward")) return 1;
@@ -2533,7 +2642,8 @@ static int rnn_backward_entry(const char *who, const ttrnn_rnn_desc *d_in, const
                           out + r0 * T * H, saved ? (const char *)saved + gs.sv_off[g] : nullptr,
                           d_out ? d_out + r0 * T * H : nullptr, d_hT ? d_hT + r0 * H : nullptr, d_cT ? d_cT + r0 * H : nullptr, dp,
                           d_x ? d_x + r0 * T * I : nullptr, d_h0 ? d_h0 + r0 * H : nullptr, d_c0 ? d_c0 + r0 * H : nullptr,
-                          (char *)scratch + gs.b_off[g], (g == 0 || serial) ? (void *)st : (void *)gc->s, dc, nullptr);
+                          (char *)scratch + gs.b_off[g], (g == 0 || serial) ? (void *)st : (void *)gc->s, dc, nullptr,
+                          lengths ? lengths + r0 : nullptr);
     }
     t_group = 0;
     if (!serial) {
@@ -2578,6 +2688,27 @@ int ttrnn_rnn_backward_proj(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspac
                               d_x, d_h0, d_c0, scratch, stream, dp != nullptr, dp, true, pj);
 }
 
+int ttrnn_rnn_forward_lengths(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                              const float *c0, const float *params, float *out, float *hT, float *cT, void *saved,
+                              void *scratch, void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp,
+                              const int32_t *lengths) {
+    if (ws && plan_proj(ws->plan) != (pj != nullptr))
+        return fail("ttrnn_rnn_forward_lengths: pj must be given exactly when the plan was sized with TTRNN_WS_PROJ");
+    return rnn_forward_entry("ttrnn_rnn_forward_lengths", d_in, ws, x, h0, c0, params, out, hT, cT, saved, scratch, stream,
+                             dp != nullptr, dp, pj != nullptr, pj, true, lengths);
+}
+
+int ttrnn_rnn_backward_lengths(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace *ws, const float *x, const float *h0,
+                               const float *c0, const float *params, const float *out, const void *saved, const float *d_out,
+                               const float *d_hT, const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0,
+                               void *scratch, void *stream, const ttrnn_rnn_proj *pj, const ttrnn_dropout *dp,
+                               const int32_t *lengths) {
+    if (ws && plan_proj(ws->plan) != (pj != nullptr))
+        return fail("ttrnn_rnn_backward_lengths: pj must be given exactly when the plan was sized with TTRNN_WS_PROJ");
+    return rnn_backward_entry("ttrnn_rnn_backward_lengths", d_in, ws, x, h0, c0, params, out, saved, d_out, d_hT, d_cT,
+                              d_params, d_x, d_h0, d_c0, scratch, stream, dp != nullptr, dp, pj != nullptr, pj, true, lengths);
+}
+
 int ttrnn_dropout_apply(int64_t B, int32_t T, int32_t F, int64_t row0, int32_t boundary, int32_t backward,
                         const ttrnn_dropout *dp, const float *x, float *y, float *y_rev, void *stream) {
     if (B < 1 || T < 1 || F < 1 || row0 < 0) return fail("ttrnn_dropout_apply: B, T, F must be >= 1 and row0 >= 0 (got %lld, %d, %d, %lld)",
@@ -2602,7 +2733,8 @@ int ttrnn_rnn_backward_logged(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_worksp
     if (!d_in || !ws) return fail("null descriptor / workspace struct");
     if (!dh_log) return fail("ttrnn_rnn_backward_logged: dh_log must be non-null");
     if (ws->plan[kPlanDropout]) return fail("ttrnn_rnn_backward_logged: the plan was sized with TTRNN_WS_DROPOUT");
-    if (ws->plan[kPlanProj]) return fail("ttrnn_rnn_backward_logged: the plan was sized with TTRNN_WS_PROJ");
+    if (plan_proj(ws->plan)) return fail("ttrnn_rnn_backward_logged: the plan was sized with TTRNN_WS_PROJ");
+    if (plan_lengths(ws->plan)) return fail("ttrnn_rnn_backward_logged: the plan was sized with TTRNN_WS_LENGTHS");
     if (ws->plan[kPlanGroups] > 1)
         return fail("ttrnn_rnn_backward_logged needs a whole-batch plan: size the call with "
                     "ttrnn_rnn_workspace_bytes_ex(desc, TTRNN_WS_WHOLE_BATCH, ws)");
@@ -2619,7 +2751,8 @@ int ttrnn_rnn_saved_layout(const ttrnn_rnn_desc *d_in, const ttrnn_rnn_workspace
                            int64_t *cs_off) {
     if (!ws || !plan_load(ws->plan, &t_opt)) return fail("ttrnn_rnn_saved_layout: `ws` must come from ttrnn_rnn_workspace_bytes()");
     if (ws->plan[kPlanGroups] > 1) return fail("ttrnn_rnn_saved_layout needs a whole-batch plan (TTRNN_WS_WHOLE_BATCH)");
-    if (ws->plan[kPlanProj]) return fail("ttrnn_rnn_saved_layout: the plan was sized with TTRNN_WS_PROJ");
+    if (plan_proj(ws->plan)) return fail("ttrnn_rnn_saved_layout: the plan was sized with TTRNN_WS_PROJ");
+    if (plan_lengths(ws->plan)) return fail("ttrnn_rnn_saved_layout: the plan was sized with TTRNN_WS_LENGTHS");
     if (!hs_off || !cs_off) return fail("hs_off and cs_off must be non-null");
     DevInfo dv;
     CallPlan cp;
@@ -2679,6 +2812,38 @@ int ttrnn_bidir_join(int64_t B, int32_t T, int32_t H, int32_t backward, const fl
         if (vec) bidir::k_join_fwd<4><<<grid, bidir::NT, 0, st>>>(p, q, u, v, n, T, H / 4);
         else bidir::k_join_fwd<1><<<grid, bidir::NT, 0, st>>>(p, q, u, v, n, T, H);
     }
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int ttrnn_time_reverse_add_lengths(int64_t B, int32_t T, int32_t F, const float *a, const float *r, float *y,
+                                   const int32_t *lengths, void *stream) {
+    if (B < 1 || T < 1 || F < 1) return fail("ttrnn_time_reverse_add_lengths: B, T and F must be >= 1 (got %lld, %d, %d)",
+                                             (long long)B, T, F);
+    if (!y || !lengths) return fail("ttrnn_time_reverse_add_lengths: y and lengths must be non-null");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    const long long n = B * (long long)T * F;
+    varlen::k_varlen_reverse_add<<<varlen::grid_for(n, dv.sms), varlen::NT, 0, (cudaStream_t)stream>>>(a, r, y, lengths, n, T, F);
+    ++g_launches;
+    CU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int ttrnn_bidir_join_lengths(int64_t B, int32_t T, int32_t H, int32_t backward, const float *p, const float *q, float *u,
+                             float *v, const int32_t *lengths, void *stream) {
+    if (B < 1 || T < 1 || H < 1) return fail("ttrnn_bidir_join_lengths: B, T and H must be >= 1 (got %lld, %d, %d)",
+                                             (long long)B, T, H);
+    if (!u || (backward && !v) || !lengths) return fail("ttrnn_bidir_join_lengths: missing output or lengths");
+    if (!backward && (!p || !q)) return fail("ttrnn_bidir_join_lengths: the forward needs both directions' outputs");
+    DevInfo dv;
+    if (get_dev(&dv)) return 1;
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long n = B * (long long)T * H * (backward ? 1 : 2);
+    const unsigned grid = varlen::grid_for(n, dv.sms);
+    if (backward) varlen::k_varlen_join_bwd<<<grid, varlen::NT, 0, st>>>(p, q, u, v, lengths, n, T, H);
+    else varlen::k_varlen_join_fwd<<<grid, varlen::NT, 0, st>>>(p, q, u, v, lengths, n, T, H);
     ++g_launches;
     CU_CHECK(cudaGetLastError());
     return 0;
@@ -2915,8 +3080,11 @@ int ttrnn_dense_rnn_workspace_bytes(const ttrnn_dense_desc *desc, int64_t *saved
 
 // Projected LSTM (P > 0), step t: u_t = h_{t-1} W_hh^T + b_hh (K = P), the gate kernel writes c_t and m_t, then
 // h_t = m_t W_hr^T (N = P) into the layer output: three launches per step where the unprojected stack has two.
+// `lengths` (nullptr = none): the padded steps of `a` are frozen once it is written (tt_varlen.cuh), h_n is gathered from
+// step len_b - 1 and the output is zeroed past each row's length
 static int dense_forward(const ttrnn_dense_desc *d, int P, const StateMap &sm, const float *x, const float *h0, const float *c0,
-                         const float *params, float *out, float *hT, float *cT, void *saved, void *scratch, void *stream) {
+                         const float *params, float *out, float *hT, float *cT, void *saved, void *scratch, void *stream,
+                         const int32_t *lengths = nullptr) {
     t_opt = snapshot_options();
     DensePlan dp;
     if (build_dense_plan(d, P, &dp)) return 1;
@@ -2958,6 +3126,7 @@ static int dense_forward(const ttrnn_dense_desc *d, int P, const StateMap &sm, c
         } else if (dense_linear(dv, B * (long long)T, T, lin, (long long)T * o.nin, o.nin, w_ih_hi, w_ih_lo, wt_ih, GH,
                          o.has_bih ? params + o.b_ih : nullptr, ab, (long long)T * GH, false, st))
             return 1;
+        if (lengths && varlen_freeze(dv, ab, (long long)T * GH, lengths, B, T, 0, H, d->cell, st)) return 1;
         const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l, true);
         for (int t = 0; t < T; ++t) {
             const float *hp = t == 0 ? h0l : lout + (long long)(t - 1) * W;
@@ -2994,20 +3163,26 @@ static int dense_forward(const ttrnn_dense_desc *d, int P, const StateMap &sm, c
         }
         CU_CHECK(cudaGetLastError());
         float *hTl = sm.fin(hT, l, L), *cTl = sm.fin(cT, l, L, true);
-        if (hTl) CU_CHECK(cudaMemcpy2DAsync(hTl, (size_t)W * 4, lout + (long long)(T - 1) * W, (size_t)T * W * 4, (size_t)W * 4, B,
+        if (hTl && lengths) {
+            if (varlen_last(dv, lout, lengths, B, T, W, hTl, st)) return 1;
+        } else if (hTl) CU_CHECK(cudaMemcpy2DAsync(hTl, (size_t)W * 4, lout + (long long)(T - 1) * W, (size_t)T * W * 4, (size_t)W * 4, B,
                                             cudaMemcpyDeviceToDevice, st));
         if (lstm && cTl) CU_CHECK(cudaMemcpy2DAsync(cTl, (size_t)H * 4, cs + (long long)(T - 1) * H, (size_t)T * H * 4, (size_t)H * 4,
                                                     B, cudaMemcpyDeviceToDevice, st));
     }
+    if (lengths && varlen_mask(dv, out, (long long)T * W, out, (long long)T * W, lengths, B, T, 0, W, st)) return 1;
     return 0;
 }
 
 // Projected LSTM (P > 0), step t in reverse: dh_t = d_out_t + the carry (k_dense_proj_dh, kept in a (B, T, P) buffer),
 // dm_t = dh_t W_hr (N = H), the gate backward with dm_t as its dh, then the carry du_t W_hh (N = P): four launches per
 // step where the unprojected stack has two.  dW_hr = sum_t dh_t^T m_t after the loop, batched over B*T.
+// `lengths` (nullptr = none): step t reads its output gradient from a (B, W) copy zeroed past each row's length, into which
+// an LSTM layer's d_h_n is added at step len_b - 1 (the gate kernels then get no d_hT)
 static int dense_backward(const ttrnn_dense_desc *d, int P, const StateMap &sm, const float *x, const float *h0, const float *c0,
                           const float *params, const float *out, void *saved, const float *d_out, const float *d_hT,
-                          const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream) {
+                          const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch, void *stream,
+                          const int32_t *lengths = nullptr) {
     t_opt = snapshot_options();
     DensePlan dp;
     if (build_dense_plan(d, P, &dp)) return 1;
@@ -3053,7 +3228,17 @@ static int dense_backward(const ttrnn_dense_desc *d, int P, const StateMap &sm, 
         if (P && (transpose_to(W_hr, wt_hr, P, H, st) || split_tf32(wt_hr, wt_hr_hi, wt_hr_lo, nhr, st))) return 1;
         const float *h0l = sm.init(h0, l), *c0l = sm.init(c0, l, true);
         const float *dhTl = sm.fin(d_hT, l, L), *dcTl = sm.fin(d_cT, l, L, true);
+        const float *dhnl = (lengths && lstm) ? dhTl : nullptr;       // LSTM d_h_n: injected at step len_b - 1
+        if (dhnl) dhTl = nullptr;
+        float *dstep = sc + lo.s_dh + 5 * r4(lo.BH);                 // lengths: this step's output gradient (B, W)
         for (int t = T - 1; t >= 0; --t) {
+            const float *dhs_t = dhs ? dhs + (long long)t * W : nullptr;
+            long long ld_t = (long long)T * W;
+            if (lengths) {
+                if (varlen_mask(dv, dhs_t, ld_t, dstep, W, lengths, B, 1, t, W, st, dhnl)) return 1;
+                dhs_t = dstep;
+                ld_t = W;
+            }
             ttd::DenseStepArgs a;
             memset(&a, 0, sizeof a);
             a.B = B; a.H = H;
@@ -3065,13 +3250,12 @@ static int dense_backward(const ttrnn_dense_desc *d, int P, const StateMap &sm, 
             if (P) {
                 // dh_t, then dm_t = dh_t W_hr: the gate backward's only dh term
                 float *dht = dhsb + (long long)t * P;
-                ttd::k_dense_proj_dh<<<prow_blocks, 128, 0, st>>>(dhs ? dhs + (long long)t * P : nullptr, (long long)T * P,
-                                                                  a.first ? dhTl : dh_gemm, dht, (long long)T * P, B, P);
+                ttd::k_dense_proj_dh<<<prow_blocks, 128, 0, st>>>(dhs_t, ld_t, a.first ? dhTl : dh_gemm, dht, (long long)T * P, B, P);
                 ++g_launches;
                 if (dense_linear(dv, B, 1, dht, (long long)T * P, P, wt_hr_hi, wt_hr_lo, W_hr, H, nullptr, dm, H, true, st)) return 1;
                 a.dout = dm; a.lddo = H;
             } else {
-                a.dout = dhs ? dhs + (long long)t * H : nullptr; a.lddo = (long long)T * H;
+                a.dout = dhs_t; a.lddo = ld_t;
                 a.dh_gemm = a.first ? nullptr : dh_gemm;
                 a.dh_T = a.first ? dhTl : nullptr;
             }
@@ -3226,6 +3410,37 @@ int ttrnn_dense_rnn_backward_proj(const ttrnn_dense_desc *d, const float *x, con
     if (dense_proj_arg(proj_size) || dense_state_map(d, proj_size, flags, &sm)) return 1;
     return dense_backward(d, proj_size, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
                           stream);
+}
+
+// variable-length rows: the _proj arguments (proj_size 0 = unprojected) plus lengths; flags as for the _ex calls, and
+// TTRNN_WS_LENGTHS may be passed (the dense stack has no plan to stamp it into)
+static int dense_lengths_args(const char *who, const ttrnn_dense_desc *d, int32_t proj_size, int32_t *flags,
+                              const int32_t *lengths) {
+    if (!lengths) return fail("%s: lengths must be non-null", who);
+    if (proj_size < 0) return fail("%s: proj_size must be >= 0, got %d", who, proj_size);
+    if (!d) return fail("null descriptor");
+    *flags &= ~TTRNN_WS_LENGTHS;
+    return 0;
+}
+int ttrnn_dense_rnn_forward_lengths(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0,
+                                    const float *params, float *out, float *hT, float *cT, void *saved, void *scratch,
+                                    void *stream, int32_t flags, int32_t proj_size, const int32_t *lengths) {
+    StateMap sm;
+    if (dense_lengths_args("ttrnn_dense_rnn_forward_lengths", d, proj_size, &flags, lengths) ||
+        dense_state_map(d, proj_size, flags, &sm))
+        return 1;
+    return dense_forward(d, proj_size, sm, x, h0, c0, params, out, hT, cT, saved, scratch, stream, lengths);
+}
+int ttrnn_dense_rnn_backward_lengths(const ttrnn_dense_desc *d, const float *x, const float *h0, const float *c0,
+                                     const float *params, const float *out, void *saved, const float *d_out, const float *d_hT,
+                                     const float *d_cT, float *d_params, float *d_x, float *d_h0, float *d_c0, void *scratch,
+                                     void *stream, int32_t flags, int32_t proj_size, const int32_t *lengths) {
+    StateMap sm;
+    if (dense_lengths_args("ttrnn_dense_rnn_backward_lengths", d, proj_size, &flags, lengths) ||
+        dense_state_map(d, proj_size, flags, &sm))
+        return 1;
+    return dense_backward(d, proj_size, sm, x, h0, c0, params, out, saved, d_out, d_hT, d_cT, d_params, d_x, d_h0, d_c0, scratch,
+                          stream, lengths);
 }
 
 int ttrnn_embed_forward(int64_t rows, int32_t E, const float *x, float *y, float *inv_norm, void *stream) {

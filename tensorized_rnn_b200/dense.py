@@ -14,6 +14,8 @@ active dropout runs as one-layer calls with the mask kernel between them (DESIGN
 `proj_size=P` (LSTM only; the contract of torch.nn.LSTM(proj_size=P)): each cell gets `projection_weights`, an nn.Linear
 H -> P without bias; every layer outputs h_t = W_hr (o_t * tanh(c_t)), which is P wide and is the next step's hh input, so
 outputs and h states are P wide and c states stay H wide.  The engine runs P % 128 == 0 (DESIGN.md §4.20).
+`forward` / `forward_states` take a torch.nn.utils.rnn.PackedSequence as the TT modules do: one padded call with per-row
+lengths, a PackedSequence out (DESIGN.md §4.22).
 """
 from __future__ import annotations
 
@@ -24,18 +26,21 @@ import torch
 from torch import nn
 
 from . import _lib
-from .functional import _bytes_to_floats, _dense16, _ptr, _require_cuda_f32, bidirectional_stack, layer_dropout, \
-    shared_bidirectional_state
+from torch.nn.utils.rnn import PackedSequence
+
+from .functional import _bytes_to_floats, _dense16, _ptr, _require_cuda_f32, bidirectional_stack, check_lengths, \
+    layer_dropout, pack_like, shared_bidirectional_state, unpack_sequence
 from .rnn import active_dropout, check_dropout, check_proj_size
 
 
 class _DenseRnnFunction(torch.autograd.Function):
     """`layer_states`: h0 / c0 and the returned final states are (L, B, .), one block per layer (TTRNN_WS_LAYER_STATES).
-    `proj_size` P > 0 (LSTM): the _proj entry points; out and the h states are P wide, the c states H wide."""
+    `proj_size` P > 0 (LSTM): the _proj entry points; out and the h states are P wide, the c states H wide.
+    `lengths`: None, or host per-row lengths: the _lengths entry points."""
 
     @staticmethod
-    def forward(ctx, cell: str, hidden_size: int, proj_size: int, num_layers: int, has_bias: bool, layer_states: bool, x, h0,
-                c0, *params):
+    def forward(ctx, cell: str, hidden_size: int, proj_size: int, num_layers: int, has_bias: bool, layer_states: bool,
+                lengths, x, h0, c0, *params):
         lib = _lib.load()
         _require_cuda_f32("input", x)
         for i, p in enumerate(params):
@@ -54,6 +59,8 @@ class _DenseRnnFunction(torch.autograd.Function):
                 if tuple(s.shape) != shape:
                     raise ValueError("%s must have shape %s, got %s" % (name, shape, tuple(s.shape)))
         x, h0c, c0c = _dense16(x), _dense16(h0), _dense16(c0)
+        if lengths is not None:
+            lengths = check_lengths(lengths, B, T, x.device)
         desc = _lib.DenseDesc(_lib.CELL_LSTM if cell == "lstm" else _lib.CELL_GRU, num_layers, I, H, int(has_bias), T, B)
         with torch.cuda.device(x.device):
             blob = torch.cat([p.detach().reshape(-1) for p in params])
@@ -80,11 +87,13 @@ class _DenseRnnFunction(torch.autograd.Function):
             stream = torch.cuda.current_stream(x.device).cuda_stream
             args = (C.byref(desc), _ptr(x), _ptr(h0c), _ptr(c0c), _ptr(blob), _ptr(out), _ptr(hT), _ptr(cT), _ptr(saved),
                     _ptr(scratch), stream, flags)
-            if P:
+            if lengths is not None:
+                _lib.check(lib.ttrnn_dense_rnn_forward_lengths(*args, P, _ptr(lengths)), "ttrnn_dense_rnn_forward_lengths")
+            elif P:
                 _lib.check(lib.ttrnn_dense_rnn_forward_proj(*args, P), "ttrnn_dense_rnn_forward_proj")
             else:
                 _lib.check(lib.ttrnn_dense_rnn_forward_ex(*args), "ttrnn_dense_rnn_forward")
-        ctx.desc, ctx.cell, ctx.proj_size = desc, cell, P
+        ctx.desc, ctx.cell, ctx.proj_size, ctx.lengths = desc, cell, P, lengths
         ctx.flags, ctx.h_shape, ctx.c_shape = flags, h_shape, c_shape
         ctx.shapes = [tuple(p.shape) for p in params]
         ctx.scratch_floats = _bytes_to_floats(wb.value)
@@ -106,16 +115,19 @@ class _DenseRnnFunction(torch.autograd.Function):
         d_cT = _dense16(grads[2]) if lstm else None
         with torch.cuda.device(x.device):
             d_blob = torch.empty_like(blob)
-            d_x = torch.empty_like(x) if ctx.needs_input_grad[6] else None
+            d_x = torch.empty_like(x) if ctx.needs_input_grad[7] else None
             d_h0 = torch.empty(ctx.h_shape, device=x.device, dtype=torch.float32) \
-                if (ctx.has_h0 and ctx.needs_input_grad[7]) else None
+                if (ctx.has_h0 and ctx.needs_input_grad[8]) else None
             d_c0 = torch.empty(ctx.c_shape, device=x.device, dtype=torch.float32) \
-                if (lstm and ctx.has_c0 and ctx.needs_input_grad[8]) else None
+                if (lstm and ctx.has_c0 and ctx.needs_input_grad[9]) else None
             scratch = torch.empty(ctx.scratch_floats, device=x.device, dtype=torch.float32)
             stream = torch.cuda.current_stream(x.device).cuda_stream
             args = (C.byref(ctx.desc), _ptr(x), _ptr(h0), _ptr(c0), _ptr(blob), _ptr(out), _ptr(saved), _ptr(d_out), _ptr(d_hT),
                     _ptr(d_cT), _ptr(d_blob), _ptr(d_x), _ptr(d_h0), _ptr(d_c0), _ptr(scratch), stream, ctx.flags)
-            if ctx.proj_size:
+            if ctx.lengths is not None:
+                _lib.check(lib.ttrnn_dense_rnn_backward_lengths(*args, ctx.proj_size, _ptr(ctx.lengths)),
+                           "ttrnn_dense_rnn_backward_lengths")
+            elif ctx.proj_size:
                 _lib.check(lib.ttrnn_dense_rnn_backward_proj(*args, ctx.proj_size), "ttrnn_dense_rnn_backward_proj")
             else:
                 _lib.check(lib.ttrnn_dense_rnn_backward_ex(*args), "ttrnn_dense_rnn_backward")
@@ -124,9 +136,9 @@ class _DenseRnnFunction(torch.autograd.Function):
             n = 1
             for v in shp:
                 n *= v
-            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[9 + i] else None)
+            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[10 + i] else None)
             off += n
-        return (None, None, None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
+        return (None, None, None, None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
 
 
 class _DenseCell(nn.Module):
@@ -216,17 +228,25 @@ class _DenseRnnBase(nn.Module):
         return [p for c in self._all_layers for p in c.flat_parameters()]
 
     def _run(self, input, h0, c0, layer_states=False):
+        """A PackedSequence input runs padded with per-row lengths and comes back packed like the input."""
+        if isinstance(input, PackedSequence):
+            padded, lengths = unpack_sequence(input)
+            res = self._run_padded(padded, h0, c0, layer_states, lengths)
+            return (pack_like(res[0], lengths, input), *res[1:])
+        return self._run_padded(input, h0, c0, layer_states)
+
+    def _run_padded(self, input, h0, c0, layer_states, lengths=None):
         if input.shape[1] == 0:
             raise NameError("name 'x' is not defined")       # the reference fails the same way on T = 0 (lstm.py:135)
         if self.bidirectional:
-            return self._run_bidirectional(input, h0, c0, layer_states)
+            return self._run_bidirectional(input, h0, c0, layer_states, lengths)
         dropout = active_dropout(self, input.device)
         if dropout is not None:
-            return self._run_layers(input, h0, c0, layer_states, dropout)
+            return self._run_layers(input, h0, c0, layer_states, dropout, lengths)
         return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.proj_size, self.num_layers, bool(self.bias),
-                                       layer_states, input, h0, c0, *self.flat_parameters())
+                                       layer_states, lengths, input, h0, c0, *self.flat_parameters())
 
-    def _run_layers(self, input, h0, c0, layer_states, dropout):
+    def _run_layers(self, input, h0, c0, layer_states, dropout, lengths=None):
         """A unidirectional stack with inter-layer dropout: one one-layer sequence call per layer, the mask kernel between
         them (functional.layer_dropout).  layer_states: h0 / c0 (L, B, .), every layer's final states returned; else one
         (B, .) state seeds every layer and the last layer's final states come back."""
@@ -239,7 +259,8 @@ class _DenseRnnBase(nn.Module):
         inp, fins = input, []
         for l, cell in enumerate(self._all_layers):
             st = [None if s is None else (s[l] if layer_states else s) for s in states]
-            res = _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.proj_size, 1, bool(self.bias), False, inp, *st,
+            res = _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.proj_size, 1, bool(self.bias), False, lengths,
+                                          inp, *st,
                                           *([None] if self.cell_kind == "gru" else []), *cell.flat_parameters())
             inp = res[0] if l == self.num_layers - 1 else layer_dropout(res[0], dropout, l)
             fins.append(res[1:])
@@ -247,14 +268,14 @@ class _DenseRnnBase(nn.Module):
             return (inp, *[torch.stack([f[k] for f in fins]) for k in range(len(states))])
         return (inp, *fins[-1])
 
-    def _run_bidirectional(self, input, h0, c0, layer_states):
+    def _run_bidirectional(self, input, h0, c0, layer_states, lengths=None):
         """Every (layer, direction) is a one-layer sequence call (functional.bidirectional_stack).  layer_states: h0 / c0
         are (2L, B, H) and so are the returned final states; else one (B, H) state seeds every layer and both directions
         and the last layer's two directions' final states come back as (2, B, H)."""
         def run(layer, direction, x, h, c=None):
             cell = self._all_layers[2 * layer + direction]
-            return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.proj_size, 1, bool(self.bias), False, x, h,
-                                           c, *cell.flat_parameters())
+            return _DenseRnnFunction.apply(self.cell_kind, self.hidden_size, self.proj_size, 1, bool(self.bias), False, lengths,
+                                           x, h, c, *cell.flat_parameters())
 
         states = [h0, c0] if self.cell_kind == "lstm" else [h0]
         if not layer_states:
@@ -262,7 +283,8 @@ class _DenseRnnBase(nn.Module):
                                                  self.output_size if k == 0 else self.hidden_size)
                       for k, s in enumerate(states)]
         out, fin = bidirectional_stack(input, states, self.num_layers, self.hidden_size, run,
-                                       dropout=active_dropout(self, input.device), output_size=self.output_size)
+                                       dropout=active_dropout(self, input.device), output_size=self.output_size,
+                                       lengths=lengths)
         if not layer_states:
             fin = [f[-2:] for f in fin]
         return (out, *fin)
@@ -279,6 +301,12 @@ class LSTM(_DenseRnnBase):
     def forward(self, input, init_states=None):
         h0, c0 = init_states if init_states is not None else (None, None)
         out, h, c = self._run(input, h0, c0)
+        return out, (h, c)
+
+    def _forward_padded(self, input, init_states, lengths):
+        """forward() on a padded batch with optional per-row lengths (outputs zero past them)."""
+        h0, c0 = init_states if init_states is not None else (None, None)
+        out, h, c = self._run_padded(input, h0, c0, False, lengths)
         return out, (h, c)
 
     def forward_states(self, input, states=None):
@@ -300,6 +328,10 @@ class GRU(_DenseRnnBase):
     def forward(self, input, init_states=None):
         out, h = self._run(input, init_states, None)
         return out, h
+
+    def _forward_padded(self, input, init_states, lengths):
+        """forward() on a padded batch with optional per-row lengths (outputs zero past them)."""
+        return self._run_padded(input, init_states, None, False, lengths)
 
     def forward_states(self, input, states=None):
         """Per-layer states: `states` (num_layers, batch, hidden) or None (zeros) -> (outputs, h_n (num_layers, batch,

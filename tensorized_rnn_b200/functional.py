@@ -174,6 +174,34 @@ def layer_dropout(x: torch.Tensor, dropout, boundary: int, rev: bool = False):
     return _DropoutFunction.apply(dropout, int(boundary), bool(rev), x)
 
 
+def check_lengths(lengths, batch: int, seq_len: int, device: torch.device) -> torch.Tensor:
+    """Per-row lengths of a padded (batch, seq_len, .) input as the int32 device array the _lengths entry points take.
+    Checked on the host before the copy (1 <= len_b <= seq_len): the kernels trust them (DESIGN.md §4.22)."""
+    host = torch.as_tensor(lengths).detach().to("cpu")
+    if host.dtype.is_floating_point or host.dtype == torch.bool or host.dim() != 1 or host.numel() != batch:
+        raise ValueError("lengths must be %d integers (one per batch row), got %s of shape %s"
+                         % (batch, host.dtype, tuple(host.shape)))
+    if host.numel() and (int(host.min()) < 1 or int(host.max()) > seq_len):
+        raise ValueError("lengths must be in [1, %d] (the padded sequence length), got min %d, max %d"
+                         % (seq_len, int(host.min()), int(host.max())))
+    return host.to(torch.int32).to(device)
+
+
+def unpack_sequence(packed):
+    """A torch PackedSequence as (padded (B, T, F) zero-padded in the caller's batch order, lengths (B,) on the host)."""
+    return torch.nn.utils.rnn.pad_packed_sequence(packed, batch_first=True, padding_value=0.0)
+
+
+def pack_like(padded: torch.Tensor, lengths: torch.Tensor, like) -> "torch.nn.utils.rnn.PackedSequence":
+    """The (B, T, .) output of a padded run as a PackedSequence with the batch_sizes, sorted_indices and unsorted_indices
+    of the input `like` (rows are put in like's sorted order first, so that ties keep its order)."""
+    idx = like.sorted_indices
+    if idx is not None:
+        padded, lengths = padded.index_select(0, idx), lengths.index_select(0, idx.to(lengths.device))
+    data = torch.nn.utils.rnn.pack_padded_sequence(padded, lengths, batch_first=True, enforce_sorted=True).data
+    return torch.nn.utils.rnn.PackedSequence(data, like.batch_sizes, like.sorted_indices, like.unsorted_indices)
+
+
 class _RnnFunction(torch.autograd.Function):
     """`step_log` (None or an object with .activations(layer, var, stats) / .gradients(layer, var, stats)): fused
     log_grads.  The training forward reports the per-step statistics of every layer's h_t / c_t sequence, the
@@ -182,10 +210,11 @@ class _RnnFunction(torch.autograd.Function):
     else (B, H), shared by every layer on the way in and the last layer's on the way out.
     `dropout`: None, or (p, seed, offset) of the inter-layer dropout (ttrnn_rnn_forward_dropout, TTRNN_WS_DROPOUT); the
     backward regenerates the same mask from them.
-    A projected spec (proj_size P > 0) runs the _proj entry points: out and the h states are P wide, the c states H."""
+    A projected spec (proj_size P > 0) runs the _proj entry points: out and the h states are P wide, the c states H.
+    `lengths`: None, or the int32 device array of per-row lengths (check_lengths): the _lengths entry points."""
 
     @staticmethod
-    def forward(ctx, spec: RnnSpec, grad_enabled: bool, step_log, layer_states: bool, dropout, x, h0, c0, *params):
+    def forward(ctx, spec: RnnSpec, grad_enabled: bool, step_log, layer_states: bool, dropout, lengths, x, h0, c0, *params):
         lib = _lib.load()
         _require_cuda_f32("input", x)
         for i, p in enumerate(params):
@@ -218,7 +247,7 @@ class _RnnFunction(torch.autograd.Function):
                 raise RuntimeError("parameter blob has %d floats, descriptor expects %d" % (blob.numel(), want))
             ws = _lib.RnnWorkspace()
             flags = (_lib.WS_WHOLE_BATCH if step_log is not None else 0) | (_lib.WS_LAYER_STATES if layer_states else 0) | \
-                (_lib.WS_DROPOUT if dropout is not None else 0)
+                (_lib.WS_DROPOUT if dropout is not None else 0) | (_lib.WS_LENGTHS if lengths is not None else 0)
             if pj is None:
                 _lib.check(lib.ttrnn_rnn_workspace_bytes_ex(C.byref(desc), flags, C.byref(ws)), "ttrnn_rnn_workspace_bytes")
             else:
@@ -226,7 +255,7 @@ class _RnnFunction(torch.autograd.Function):
                            "ttrnn_rnn_workspace_bytes_proj")
             # grad mode is always off inside Function.forward and needs_input_grad stays True for nn.Parameters under
             # torch.no_grad(): the caller captures torch.is_grad_enabled() before .apply (ADVICE r1)
-            training = bool(grad_enabled) and any(ctx.needs_input_grad[5:])
+            training = bool(grad_enabled) and any(ctx.needs_input_grad[6:])
             if step_log is not None and not training:
                 raise RuntimeError("fused per-step logging needs a training forward (it reads the kept h_t / c_t sequences)")
             out = torch.empty((B, T, W), device=x.device, dtype=torch.float32)
@@ -238,7 +267,11 @@ class _RnnFunction(torch.autograd.Function):
             stream = torch.cuda.current_stream(x.device).cuda_stream
             args = (C.byref(desc), C.byref(ws), _ptr(x), _ptr(h0c), _ptr(c0c), _ptr(blob), _ptr(out), _ptr(hT), _ptr(cT),
                     _ptr(saved), _ptr(scratch), stream)
-            if pj is not None:
+            if lengths is not None:
+                dp = None if dropout is None else C.byref(_dropout_struct(dropout))
+                _lib.check(lib.ttrnn_rnn_forward_lengths(*(args + (None if pj is None else C.byref(pj), dp, _ptr(lengths)))),
+                           "ttrnn_rnn_forward_lengths")
+            elif pj is not None:
                 dp = None if dropout is None else C.byref(_dropout_struct(dropout))
                 _lib.check(lib.ttrnn_rnn_forward_proj(*(args + (C.byref(pj), dp))), "ttrnn_rnn_forward_proj")
             elif dropout is None:
@@ -259,6 +292,7 @@ class _RnnFunction(torch.autograd.Function):
             ctx.spec = spec
             ctx.step_log = step_log
             ctx.dropout = dropout
+            ctx.lengths = lengths
             ctx.shapes = [tuple(p.shape) for p in params]
             ctx.ws = ws                    # sizes + execution plan: backward runs from the same plan as this forward
             ctx.bwd_floats = _bytes_to_floats(ws.bwd_scratch_bytes)
@@ -286,17 +320,21 @@ class _RnnFunction(torch.autograd.Function):
         d_cT = _dense16(d_cT)
         with torch.cuda.device(x.device):
             d_blob = torch.empty_like(blob)
-            d_x = torch.empty_like(x) if ctx.needs_input_grad[5] else None
+            d_x = torch.empty_like(x) if ctx.needs_input_grad[6] else None
             d_h0 = torch.empty(ctx.h_shape, device=x.device, dtype=torch.float32) \
-                if (ctx.has_h0 and ctx.needs_input_grad[6]) else None
+                if (ctx.has_h0 and ctx.needs_input_grad[7]) else None
             d_c0 = torch.empty(ctx.state_shape, device=x.device, dtype=torch.float32) \
-                if (spec.cell == "lstm" and ctx.has_c0 and ctx.needs_input_grad[7]) else None
+                if (spec.cell == "lstm" and ctx.has_c0 and ctx.needs_input_grad[8]) else None
             scratch = torch.empty(ctx.bwd_floats, device=x.device, dtype=torch.float32)
             stream = torch.cuda.current_stream(x.device).cuda_stream
             args = (C.byref(desc), C.byref(ctx.ws), _ptr(x), _ptr(h0), _ptr(c0), _ptr(blob), _ptr(out),
                     _ptr(saved), _ptr(d_out), _ptr(d_hT), _ptr(d_cT), _ptr(d_blob),
                     _ptr(d_x), _ptr(d_h0), _ptr(d_c0), _ptr(scratch), stream)
-            if spec.proj_size:
+            if ctx.lengths is not None:
+                dp = None if ctx.dropout is None else C.byref(_dropout_struct(ctx.dropout))
+                pj = C.byref(spec.proj()) if spec.proj_size else None
+                _lib.check(lib.ttrnn_rnn_backward_lengths(*(args + (pj, dp, _ptr(ctx.lengths)))), "ttrnn_rnn_backward_lengths")
+            elif spec.proj_size:
                 dp = None if ctx.dropout is None else C.byref(_dropout_struct(ctx.dropout))
                 _lib.check(lib.ttrnn_rnn_backward_proj(*(args + (C.byref(spec.proj()), dp))), "ttrnn_rnn_backward_proj")
             elif ctx.dropout is not None:
@@ -319,92 +357,141 @@ class _RnnFunction(torch.autograd.Function):
             n = 1
             for v in shp:
                 n *= v
-            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[8 + i] else None)
+            d_params.append(d_blob[off:off + n].view(shp) if ctx.needs_input_grad[9 + i] else None)
             off += n
-        return (None, None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
+        return (None, None, None, None, None, None, d_x, d_h0, d_c0) + tuple(d_params)
 
 
 def rnn_sequence(spec: RnnSpec, x: torch.Tensor, h0: Optional[torch.Tensor], c0: Optional[torch.Tensor],
-                 params: Sequence[torch.Tensor], step_log=None, layer_states: bool = False, dropout=None):
+                 params: Sequence[torch.Tensor], step_log=None, layer_states: bool = False, dropout=None, lengths=None):
     """Run the whole stack over the whole sequence.  Returns (out, hT[, cT]).  `step_log`: see _RnnFunction.
     `layer_states=True`: h0 / c0 and the returned hT / cT are (num_layers, batch, hidden), one state per layer, so that
     the final states of one call can seed the next call over the rest of the sequence.
     `dropout`: None, or (p, seed, offset) (dropout_draw): the output of every layer but the last is multiplied by
-    mask / (1 - p) before the next layer reads it (DESIGN.md §4.18)."""
+    mask / (1 - p) before the next layer reads it (DESIGN.md §4.18).
+    `lengths`: None, or one length per batch row (1 <= len_b <= seq_len; a sequence or a tensor, checked on the host):
+    the padded form of torch's PackedSequence (DESIGN.md §4.22).  Row b runs len_b steps; out is 0 past
+    them, hT / cT are the states after step len_b - 1, and the output gradient past them is ignored.  Padded inputs
+    must be finite."""
     if x.dim() != 3:
         raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
     if dropout is not None and step_log is not None:
         raise NotImplementedError("inter-layer dropout has no fused per-step logging form")
-    return _RnnFunction.apply(spec, torch.is_grad_enabled(), step_log, bool(layer_states), dropout, x, h0, c0, *params)
+    if lengths is not None:
+        if step_log is not None:
+            raise NotImplementedError("variable-length rows have no fused per-step logging form")
+        lengths = check_lengths(lengths, x.shape[0], x.shape[1], x.device)
+    return _RnnFunction.apply(spec, torch.is_grad_enabled(), step_log, bool(layer_states), dropout, lengths, x, h0, c0,
+                              *params)
 
 
 # ---- bidirectional stacks (DESIGN.md §4.17) --------------------------------------------------------------------------
 class _BidirInputFunction(torch.autograd.Function):
     """Layer-0 input of a bidirectional stack: x for the forward direction, x reversed in time for the reverse one
     (ttrnn_time_reverse_add with a = NULL).  The backward forms d_x = d_x_forward + reverse(d_x_reverse) in the same
-    kernel, so the two directions' input gradients are summed by the library, not by autograd."""
+    kernel, so the two directions' input gradients are summed by the library, not by autograd.
+    `lengths` (check_lengths' device array or None): every row is reversed over its own length and zero past it
+    (ttrnn_time_reverse_add_lengths)."""
 
     @staticmethod
-    def forward(ctx, x):
+    def _reverse_add(lengths, B, T, F, a, r, y, stream):
         lib = _lib.load()
+        if lengths is None:
+            _lib.check(lib.ttrnn_time_reverse_add(B, T, F, _ptr(a), _ptr(r), _ptr(y), stream), "ttrnn_time_reverse_add")
+        else:
+            _lib.check(lib.ttrnn_time_reverse_add_lengths(B, T, F, _ptr(a), _ptr(r), _ptr(y), _ptr(lengths), stream),
+                       "ttrnn_time_reverse_add_lengths")
+
+    @staticmethod
+    def forward(ctx, lengths, x):
         _require_cuda_f32("input", x)
         B, T, F = x.shape
         x = _dense16(x)
         with torch.cuda.device(x.device):
             x_rev = torch.empty_like(x)
-            _lib.check(lib.ttrnn_time_reverse_add(B, T, F, None, _ptr(x), _ptr(x_rev),
-                                                  torch.cuda.current_stream(x.device).cuda_stream),
-                       "ttrnn_time_reverse_add")
+            _BidirInputFunction._reverse_add(lengths, B, T, F, None, x, x_rev, torch.cuda.current_stream(x.device).cuda_stream)
+        ctx.lengths = lengths
         ctx.set_materialize_grads(False)
         return x, x_rev
 
     @staticmethod
     def backward(ctx, d_x_f, d_x_r):
         if d_x_f is None and d_x_r is None:
-            return None
-        lib = _lib.load()
+            return None, None
         d_x_f, d_x_r = _dense16(d_x_f), _dense16(d_x_r)
         like = d_x_f if d_x_f is not None else d_x_r
         B, T, F = like.shape
         with torch.cuda.device(like.device):
             d_x = torch.empty_like(like)
-            _lib.check(lib.ttrnn_time_reverse_add(B, T, F, _ptr(d_x_f), _ptr(d_x_r), _ptr(d_x),
-                                                  torch.cuda.current_stream(like.device).cuda_stream),
-                       "ttrnn_time_reverse_add")
-        return d_x
+            _BidirInputFunction._reverse_add(ctx.lengths, B, T, F, d_x_f, d_x_r, d_x,
+                                             torch.cuda.current_stream(like.device).cuda_stream)
+        return None, d_x
+
+
+class _ReverseFunction(torch.autograd.Function):
+    """y reversed in time over each row's length (zero past it); its adjoint is the same reversal."""
+
+    @staticmethod
+    def forward(ctx, lengths, y):
+        y = _dense16(y)
+        B, T, F = y.shape
+        with torch.cuda.device(y.device):
+            y_rev = torch.empty_like(y)
+            _BidirInputFunction._reverse_add(lengths, B, T, F, None, y, y_rev, torch.cuda.current_stream(y.device).cuda_stream)
+        ctx.lengths = lengths
+        return y_rev
+
+    @staticmethod
+    def backward(ctx, d_rev):
+        d_rev = _dense16(d_rev)
+        B, T, F = d_rev.shape
+        with torch.cuda.device(d_rev.device):
+            d_y = torch.empty_like(d_rev)
+            _BidirInputFunction._reverse_add(ctx.lengths, B, T, F, None, d_rev, d_y,
+                                             torch.cuda.current_stream(d_rev.device).cuda_stream)
+        return None, d_y
 
 
 class _BidirJoinFunction(torch.autograd.Function):
     """Joins the two directions of one layer (ttrnn_bidir_join): y[b,t] = [out_f[b,t] | out_r[b,T-1-t]], the next
-    layer's (or the module's) output, and unless `last`, y reversed in time, the next layer's reverse-direction input."""
+    layer's (or the module's) output, and unless `last`, y reversed in time, the next layer's reverse-direction input.
+    `lengths` (device array or None): reversal over each row's length, zeros past it (ttrnn_bidir_join_lengths)."""
 
     @staticmethod
-    def forward(ctx, last: bool, out_f, out_r):
+    def _join(lengths, B, T, H, backward, p, q, u, v, stream):
         lib = _lib.load()
+        if lengths is None:
+            _lib.check(lib.ttrnn_bidir_join(B, T, H, backward, _ptr(p), _ptr(q), _ptr(u), _ptr(v), stream), "ttrnn_bidir_join")
+        else:
+            _lib.check(lib.ttrnn_bidir_join_lengths(B, T, H, backward, _ptr(p), _ptr(q), _ptr(u), _ptr(v), _ptr(lengths),
+                                                    stream), "ttrnn_bidir_join_lengths")
+
+    @staticmethod
+    def forward(ctx, last: bool, lengths, out_f, out_r):
         out_f, out_r = _dense16(out_f), _dense16(out_r)
         B, T, H = out_f.shape
         with torch.cuda.device(out_f.device):
             y = torch.empty((B, T, 2 * H), device=out_f.device, dtype=torch.float32)
             y_rev = None if last else torch.empty_like(y)
-            _lib.check(lib.ttrnn_bidir_join(B, T, H, 0, _ptr(out_f), _ptr(out_r), _ptr(y), _ptr(y_rev),
-                                            torch.cuda.current_stream(out_f.device).cuda_stream), "ttrnn_bidir_join")
+            _BidirJoinFunction._join(lengths, B, T, H, 0, out_f, out_r, y, y_rev,
+                                     torch.cuda.current_stream(out_f.device).cuda_stream)
+        ctx.lengths = lengths
         ctx.set_materialize_grads(False)
         return y if last else (y, y_rev)
 
     @staticmethod
     def backward(ctx, dy, dy_rev=None):
         if dy is None and dy_rev is None:
-            return None, None, None
-        lib = _lib.load()
+            return None, None, None, None
         dy, dy_rev = _dense16(dy), _dense16(dy_rev)
         like = dy if dy is not None else dy_rev
         B, T, H2 = like.shape
         with torch.cuda.device(like.device):
             d_f = torch.empty((B, T, H2 // 2), device=like.device, dtype=torch.float32)
             d_r = torch.empty_like(d_f)
-            _lib.check(lib.ttrnn_bidir_join(B, T, H2 // 2, 1, _ptr(dy), _ptr(dy_rev), _ptr(d_f), _ptr(d_r),
-                                            torch.cuda.current_stream(like.device).cuda_stream), "ttrnn_bidir_join")
-        return None, d_f, d_r
+            _BidirJoinFunction._join(ctx.lengths, B, T, H2 // 2, 1, dy, dy_rev, d_f, d_r,
+                                     torch.cuda.current_stream(like.device).cuda_stream)
+        return None, None, d_f, d_r
 
 
 _side_streams = {}
@@ -430,7 +517,7 @@ def shared_bidirectional_state(state: Optional[torch.Tensor], num_layers: int, b
 
 
 def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]], num_layers: int, hidden_size: int,
-                        run, dropout=None, output_size: Optional[int] = None):
+                        run, dropout=None, output_size: Optional[int] = None, lengths=None):
     """A bidirectional stack composed of one-layer calls, the contract of torch.nn.LSTM / GRU(bidirectional=True).
 
     `run(layer, direction, x, *states)` runs direction 0 (forward) or 1 (reverse) of one layer over x (B, T, F) from its
@@ -448,7 +535,9 @@ def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]
     from one stream to the other; the forward's own cross-stream tensors are recorded here.
     `dropout`: None, or (p, seed, offset): the joined (B, T, 2H) output of every layer but the last is masked (boundary =
     layer index) before the next layer's two directions read it; the reverse direction sees the masked values reversed
-    in time."""
+    in time.
+    `lengths`: None, or per-row lengths (DESIGN.md §4.22), which `run` must pass on to its one-layer calls: every row is
+    reversed over its own length, so the reverse direction starts at step len_b - 1; outputs are 0 past the length."""
     if x.dim() != 3:
         raise ValueError("input must be (batch, seq_len, input_size), got shape %s" % (tuple(x.shape),))
     _require_cuda_f32("input", x)
@@ -461,10 +550,12 @@ def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]
                 raise ValueError("bidirectional states must have shape %s (2 * num_layers, batch, width), got %s"
                                  % (shape, tuple(s.shape)))
     dev = x.device
+    if lengths is not None:
+        lengths = check_lengths(lengths, B, x.shape[1], dev)
     with torch.cuda.device(dev):
         main = torch.cuda.current_stream(dev)
         side = _side_stream(dev)
-        inp_f, inp_r = _BidirInputFunction.apply(x)
+        inp_f, inp_r = _BidirInputFunction.apply(lengths, x)
         finals = []
         for l in range(num_layers):
             st_f = [None if s is None else s[2 * l] for s in states]
@@ -481,11 +572,15 @@ def bidirectional_stack(x: torch.Tensor, states: Sequence[Optional[torch.Tensor]
                 t.record_stream(main)
             last = l == num_layers - 1
             if last:
-                out = _BidirJoinFunction.apply(True, res_f[0], res_r[0])
+                out = _BidirJoinFunction.apply(True, lengths, res_f[0], res_r[0])
+            elif dropout is not None and lengths is not None:
+                # the dropout kernel's own reversal spans all T steps: reverse over each row's length separately
+                inp_f = layer_dropout(_BidirJoinFunction.apply(True, lengths, res_f[0], res_r[0]), dropout, l)
+                inp_r = _ReverseFunction.apply(lengths, inp_f)
             elif dropout is not None:
-                inp_f, inp_r = layer_dropout(_BidirJoinFunction.apply(True, res_f[0], res_r[0]), dropout, l, rev=True)
+                inp_f, inp_r = layer_dropout(_BidirJoinFunction.apply(True, None, res_f[0], res_r[0]), dropout, l, rev=True)
             else:
-                inp_f, inp_r = _BidirJoinFunction.apply(False, res_f[0], res_r[0])
+                inp_f, inp_r = _BidirJoinFunction.apply(False, lengths, res_f[0], res_r[0])
             finals.append((res_f[1:], res_r[1:]))
     fin = [torch.stack([f[k] for pair in finals for f in pair]) for k in range(len(finals[0][0]))]
     return out, fin

@@ -33,6 +33,11 @@ stack call (DESIGN.md §4.18).  It needs the fused mode as well.
 `proj_size=P` (TTLSTM only; the contract of torch.nn.LSTM(proj_size=P)): each cell gets `projection_weights`, a TTLinear
 H -> P without bias created after `hidden_weights`, and outputs h_t = W_hr (o_t * tanh(c_t)), which is also the next
 step's hh input.  The recurrent kernels contract W_hr inside every step (DESIGN.md §4.19).  It needs the fused mode.
+
+`forward` / `forward_states` also take a torch.nn.utils.rnn.PackedSequence, with torch's contract: the output is a
+PackedSequence with the input's batch_sizes, sorted_indices and unsorted_indices, and the final states are those after
+each sequence's own last step, in the caller's batch order.  The batch runs as one padded call with per-row lengths
+(functional.rnn_sequence(lengths=...), DESIGN.md §4.22).  It needs the fused mode.
 """
 from __future__ import annotations
 
@@ -43,7 +48,10 @@ from typing import List, Optional
 import torch
 from torch import nn
 
-from .functional import RnnSpec, bidirectional_stack, dropout_draw, rnn_sequence, shared_bidirectional_state
+from torch.nn.utils.rnn import PackedSequence
+
+from .functional import RnnSpec, bidirectional_stack, dropout_draw, pack_like, rnn_sequence, shared_bidirectional_state, \
+    unpack_sequence
 from .functional import cell_step
 from .layers import TTLinear, TTLinearSet
 from .rnn_utils import ActivGradLogger
@@ -340,6 +348,15 @@ class _TTRNNBase(nn.Module):
             out += cell.flat_parameters()
         return out
 
+    def _unpack(self, input):
+        """(padded input, host lengths or None) of a forward input, which may be a PackedSequence."""
+        if not isinstance(input, PackedSequence):
+            return input, None
+        if self.cell_step_mode:
+            raise NotImplementedError("a PackedSequence runs on the sequence kernels only; is_naive=True and log_grads=True "
+                                      "need the cell-step mode, which has no variable-length form")
+        return unpack_sequence(input)
+
     def _check_input(self, input):
         if input.dim() != 3:
             raise ValueError("input must be (batch_size, seq_len, input_size)")
@@ -347,15 +364,16 @@ class _TTRNNBase(nn.Module):
             # the reference falls off its time loop with unbound locals (lstm.py:135 / gru.py:136)
             raise NameError("zero-length sequence: the reference raises NameError here and so does this module")
 
-    def _run_bidirectional(self, input, states):
+    def _run_bidirectional(self, input, states, lengths=None):
         """Bidirectional stack (functional.bidirectional_stack): every (layer, direction) is a one-layer sequence call.
         `states`: per state variable (2L, B, H) or None."""
         def run(layer, direction, x, h0, c0=None):
             cell = self._all_layers[2 * layer + direction]
-            return rnn_sequence(cell._single_step_spec(), x, h0, c0, cell.flat_parameters())
+            return rnn_sequence(cell._single_step_spec(), x, h0, c0, cell.flat_parameters(), lengths=lengths)
 
         return bidirectional_stack(input, states, self.num_layers, self.hidden_size, run,
-                                   dropout=active_dropout(self, input.device), output_size=self.output_size)
+                                   dropout=active_dropout(self, input.device), output_size=self.output_size,
+                                   lengths=lengths)
 
     def _shared_to_bidirectional(self, input, state, width=None):
         return shared_bidirectional_state(state, self.num_layers, input.size(0), width or self.hidden_size)
@@ -396,19 +414,27 @@ class TTLSTM(_TTRNNBase):
         proj_size = P > 0: outputs and h are P wide, c stays hidden wide.
         bidirectional: outputs (batch, seq_len, 2 * hidden); (h0, c0) seed every layer and both directions; h_T, c_T
         are (2, batch, hidden): the last layer's forward direction after the last step, then its reverse direction
-        after the first step."""
+        after the first step.
+        A PackedSequence input gives a PackedSequence output (see the module docstring)."""
+        padded, lengths = self._unpack(input)
+        out, st = self._forward_padded(padded, init_states, lengths)
+        return (out if lengths is None else pack_like(out, lengths, input)), st
+
+    def _forward_padded(self, input, init_states, lengths):
+        """forward() on a padded batch: lengths None, or one length per row (outputs zero past them, the final states
+        after each row's last step)."""
         self._check_input(input)
         if self.bidirectional:
             h0, c0 = (None, None) if init_states is None else init_states
             out, (h, c) = self._run_bidirectional(input, [self._shared_to_bidirectional(input, h0, self.output_size),
-                                                          self._shared_to_bidirectional(input, c0)])
+                                                          self._shared_to_bidirectional(input, c0)], lengths)
             return out, (h[-2:], c[-2:])
-        sink = self._fused_step_log()
+        sink = None if lengths is not None else self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, init_states)
         h0, c0 = (None, None) if init_states is None else init_states
         out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink,
-                                 dropout=active_dropout(self, input.device))
+                                 dropout=active_dropout(self, input.device), lengths=lengths)
         return out, (h, c)
 
     def forward_states(self, input, states=None):
@@ -417,18 +443,21 @@ class TTLSTM(_TTRNNBase):
         (num_layers, batch, hidden): feeding them to the next call continues the sequence exactly where this one
         stopped (streaming inference, truncated BPTT).  proj_size = P > 0: h and the outputs are P wide (as torch).
         bidirectional: the states are (2 * num_layers, batch, hidden), direction d of layer l at 2l + d, in and out, as
-        torch.nn.LSTM(bidirectional=True) takes them; outputs are (batch, seq_len, 2 * hidden)."""
+        torch.nn.LSTM(bidirectional=True) takes them; outputs are (batch, seq_len, 2 * hidden).
+        A PackedSequence input gives a PackedSequence output (see the module docstring)."""
+        packed = input
+        input, lengths = self._unpack(input)
         self._check_input(input)
         if self.bidirectional:
-            out, (h, c) = self._run_bidirectional(input, [None, None] if states is None else list(states))
-            return out, (h, c)
-        sink = self._fused_step_log()
+            out, (h, c) = self._run_bidirectional(input, [None, None] if states is None else list(states), lengths)
+            return (out if lengths is None else pack_like(out, lengths, packed)), (h, c)
+        sink = None if lengths is not None else self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, states, layer_states=True)
         h0, c0 = (None, None) if states is None else states
         out, h, c = rnn_sequence(self.spec(), input, h0, c0, self.flat_parameters(), step_log=sink, layer_states=True,
-                                 dropout=active_dropout(self, input.device))
-        return out, (h, c)
+                                 dropout=active_dropout(self, input.device), lengths=lengths)
+        return (out if lengths is None else pack_like(out, lengths, packed)), (h, c)
 
     def _forward_cell_steps(self, input, init_states, layer_states=False):
         """The reference's own loop (lstm.py:116-135): step-major, layer-minor, one shared initial state
@@ -468,31 +497,42 @@ class TTGRU(_TTRNNBase):
 
     def forward(self, input, init_states=None):
         """input (batch, seq_len, input_size) -> outputs (batch, seq_len, hidden), h_T of the last layer.
-        bidirectional: as for TTLSTM (outputs (batch, seq_len, 2 * hidden), h_T (2, batch, hidden))."""
+        bidirectional: as for TTLSTM (outputs (batch, seq_len, 2 * hidden), h_T (2, batch, hidden)).
+        A PackedSequence input gives a PackedSequence output (see the module docstring)."""
+        padded, lengths = self._unpack(input)
+        out, h = self._forward_padded(padded, init_states, lengths)
+        return (out if lengths is None else pack_like(out, lengths, input)), h
+
+    def _forward_padded(self, input, init_states, lengths):
+        """forward() on a padded batch with optional per-row lengths (see TTLSTM._forward_padded)."""
         self._check_input(input)
         if self.bidirectional:
-            out, (h,) = self._run_bidirectional(input, [self._shared_to_bidirectional(input, init_states)])
+            out, (h,) = self._run_bidirectional(input, [self._shared_to_bidirectional(input, init_states)], lengths)
             return out, h[-2:]
-        sink = self._fused_step_log()
+        sink = None if lengths is not None else self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, init_states)
         out, h = rnn_sequence(self.spec(), input, init_states, None, self.flat_parameters(), step_log=sink,
-                              dropout=active_dropout(self, input.device))
+                              dropout=active_dropout(self, input.device), lengths=lengths)
         return out, h
 
     def forward_states(self, input, states=None):
         """Per-layer states, the contract of torch.nn.GRU: `states` (num_layers, batch, hidden) or None (zeros).
         Returns (outputs (batch, seq_len, hidden), h_n (num_layers, batch, hidden)) with every layer's final state.
-        bidirectional: states (2 * num_layers, batch, hidden), outputs (batch, seq_len, 2 * hidden), as torch.nn.GRU."""
+        bidirectional: states (2 * num_layers, batch, hidden), outputs (batch, seq_len, 2 * hidden), as torch.nn.GRU.
+        A PackedSequence input gives a PackedSequence output (see the module docstring)."""
+        packed = input
+        input, lengths = self._unpack(input)
         self._check_input(input)
         if self.bidirectional:
-            out, (h,) = self._run_bidirectional(input, [states])
-            return out, h
-        sink = self._fused_step_log()
+            out, (h,) = self._run_bidirectional(input, [states], lengths)
+            return (out if lengths is None else pack_like(out, lengths, packed)), h
+        sink = None if lengths is not None else self._fused_step_log()
         if self.cell_step_mode and sink is None:
             return self._forward_cell_steps(input, states, layer_states=True)
-        return rnn_sequence(self.spec(), input, states, None, self.flat_parameters(), step_log=sink, layer_states=True,
-                            dropout=active_dropout(self, input.device))
+        out, h = rnn_sequence(self.spec(), input, states, None, self.flat_parameters(), step_log=sink, layer_states=True,
+                              dropout=active_dropout(self, input.device), lengths=lengths)
+        return (out if lengths is None else pack_like(out, lengths, packed)), h
 
     def _forward_cell_steps(self, input, init_states, layer_states=False):
         """The reference's own loop (gru.py:119-136); `layer_states` as for TTLSTM."""

@@ -11,7 +11,8 @@ the evaluation form of `similarity_matrix` (`enrollment_embeds` given) is not pr
 `proj_size=P` (appended to the reference signature; LSTM only, the GRU modules refuse it) builds the LSTM with a recurrent
 projection of the GE2E paper (LSTMP) on either side, `compression=None` (dense `LSTM`) or `'tt'` (`TTLSTM`); the embedding
 `linear` then reads the P-wide final state.  `embed_utterances` / `embed_speakers` (appended) give the utterance and speaker
-embeddings of enrollment and verification: sliding-window partials, embedded in one stack call and averaged (DESIGN.md §4.21).
+embeddings of enrollment and verification: sliding-window partials, embedded in one stack call and averaged (DESIGN.md §4.21),
+or with `using_partials=False` each whole utterance embedded by one variable-length stack call (DESIGN.md §4.22).
 """
 from __future__ import annotations
 
@@ -59,23 +60,31 @@ class SpeakerEncoder(nn.Module):
         torch.nn.utils.clip_grad_norm_(self.parameters(), self.clip, norm_type=2)
 
     def forward(self, utterances, hidden_init=None):
-        if not self.use_gru:
-            out, (last_hidden, _) = self.rnn(utterances)
-        else:
-            out, last_hidden = self.rnn(utterances)
+        return self._embed(self.rnn(utterances))
+
+    def _embed(self, rnn_result):
+        _, st = rnn_result
+        last_hidden = st if self.use_gru else st[0]
         return embed_normalize(self.linear(last_hidden))            # relu + L2 norm (speaker_encoder.py:86-89)
 
-    def embed_utterances(self, frames, lengths, partial_frames=160, overlap=0.5, min_coverage=0.75):
+    def embed_utterances(self, frames, lengths, partial_frames=160, overlap=0.5, min_coverage=0.75, using_partials=True):
         """Utterance d-vectors (N, E) of N utterances of any length, as GE2E and Real-Time-Voice-Cloning's `embed_utterance`
         define them: each utterance is cut into overlapping windows of `partial_frames` frames (`partial_windows`), every
         window is embedded by `forward`, and the window embeddings are averaged and L2-normalised.
+        using_partials=False: the reference's full mode, `forward` on each whole utterance alone (ReLU + L2 norm of
+        linear(h_n of the last layer)); the window arguments are then unused.
 
         frames: the utterances' frames packed in order, a CUDA float32 (sum(lengths), mel_n_channels) block (for a list of
         (n_i, mel) tensors: `torch.cat(utts)` with `[u.size(0) for u in utts]`); lengths: ints >= 1.  All windows of all
-        utterances go through one gather, one `forward` and one segment mean; the call is differentiable in the parameters."""
+        utterances go through one gather, one `forward` and one segment mean (full mode: one window per utterance of
+        max(lengths) frames, zero past the utterance, and one variable-length `forward`); the call is differentiable in
+        the parameters."""
         n = _counts(lengths, "lengths")
         if frames.dim() != 2 or frames.shape[0] != int(n.sum()):
             raise ValueError("frames must be (sum(lengths) = %d, mel_n_channels), got %s" % (int(n.sum()), tuple(frames.shape)))
+        if not using_partials:
+            padded = gather_partials(frames, np.cumsum(n) - n, n.astype(np.int32), int(n.max()))
+            return self._embed(self.rnn._forward_padded(padded, None, n))
         first, valid, n_windows = partial_windows(n, partial_frames, overlap, min_coverage)
         return segment_mean_normalize(self(gather_partials(frames, first, valid, partial_frames)), n_windows)
 
